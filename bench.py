@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the fused FPV step (flip task) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): env-steps/s, flip task, device-timed, max over ranks.  One "step" = one
@@ -17,6 +17,10 @@ algorithmic bytes of SURVEY.md section 8(d); `sustained` = an internal 300-step 
 samples (independent of --steps); `cpu_baseline` = the oracle port (the reference's torch modules' arithmetic + restated glue,
 pinned to the reference's own classes by tests/golden/glue_*.npz) timed on this host's cores on a bounded sample of the SAME
 workload; `policy_loop`, `config3_mix_actor`, `config4_rotate`, `config5_mix_dr` = the other BASELINE.json workloads.
+
+--dump-outputs DIR writes what the last of the K timed steps returned (obs, states, rew, reset, time_outs at a fixed seeded sample
+of envs, and the rollout statistics of the timed window) as DIR/*.npy.  Inputs depend only on the arguments (seeded env, Philox
+actions), so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -44,6 +48,7 @@ ALGO_BYTES_NO_DR = 1493      # SURVEY.md section 8(d): 16 + 637 + 416 + 424 (len
 ALGO_BYTES_DR = 1549
 TASK = "flip"
 SEED = 0x7AC0
+DUMP_MAX_ENVS = 65536        # --dump-outputs: 26 + 5 x 26 + 3 floats + an env id = 644 B per env, 42 MB at most
 
 
 def parse():
@@ -67,7 +72,15 @@ def parse():
     ap.add_argument("--no-actor", action="store_true", help="skip the BASELINE config 3 point (mix task + actor MLP in the rollout loop)")
     ap.add_argument("--actor-envs", type=int, default=262144)
     ap.add_argument("--actor-hidden", default="256,256,256", help="actor hidden sizes (not pinned by the reference: the YAML is missing; our stated default)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (rank 0's shard; a fixed seeded sample of at most "
+                         f"{DUMP_MAX_ENVS} envs) as DIR/<name>.npy, float32 / float64, for comparing two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -215,14 +228,16 @@ def run_reference(args, rank, world):
 
 # ------------------------------------------------------------------------------------------------ ours
 def time_steps(env, actions, steps, torch, dist, world):
-    """K consecutive steps bracketed by barrier + synchronize; CUDA events on the launching stream."""
+    """K consecutive steps bracketed by barrier + synchronize; CUDA events on the launching stream.  Returns (ms, rollout stats,
+    what the last step returned: (obs_dict, rew, reset, extras), views of the env's buffers that the next step overwrites)."""
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
+    last = None
     for t in range(steps):
-        env.step(actions[t % len(actions)])
+        last = env.step(actions[t % len(actions)])
     stats = env.stats()
     if world > 1:
         dist.all_reduce(stats)                       # the one collective of the path: 8 doubles per rollout
@@ -234,7 +249,29 @@ def time_steps(env, actions, steps, torch, dist, world):
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
         ms = float(tmax.item())
         dist.barrier()
-    return ms, stats
+    return ms, stats, last
+
+
+def dump_outputs(out_dir, last, stats, n, torch):
+    """--dump-outputs: the last timed step's return values at a fixed, seeded sample of env indices (all envs when there are at most
+    DUMP_MAX_ENVS), plus the rollout statistics of the timed window.  Called before the next step overwrites the buffers."""
+    import numpy as np
+    obs_dict, rew, reset, extras = last
+    if n > DUMP_MAX_ENVS:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(SEED))[:DUMP_MAX_ENVS].sort().values
+    else:
+        idx = torch.arange(n)
+    idx_dev = idx.to(rew.device)
+    arrays = {"env_index": idx.double(),
+              "obs": obs_dict["obs"][idx_dev].float(), "states": obs_dict["states"][idx_dev].float(),
+              "rew": rew[idx_dev].float(), "reset": reset[idx_dev].float(), "time_outs": extras["time_outs"][idx_dev].float(),
+              "rollout_stats": stats.double()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+    return {"dir": os.path.abspath(out_dir), "envs": int(idx.numel()), "files": sorted(k + ".npy" for k in arrays),
+            "note": "values returned by the last timed step at the envs listed in env_index.npy (rank 0's shard), "
+                    "and the rollout statistics of the timed window"}
 
 
 def _timed(torch, fn, iters, warm=3):
@@ -418,7 +455,7 @@ def shard_point(torch, dist, taco_b200, dev, rank, world, task, n, dr, strict_fp
     for t in range(warm):
         env.step(acts[t % 4])
     env.stats()
-    ms, _ = time_steps(env, acts, steps, torch, dist, world)
+    ms, _, _ = time_steps(env, acts, steps, torch, dist, world)
     env.close()
     algo = ALGO_BYTES_DR if dr else ALGO_BYTES_NO_DR
     ach = algo * n / (ms / steps * 1e-3) / 1e9
@@ -557,8 +594,9 @@ def main():
         dist.all_reduce(warm_stats)                  # NCCL communicator set-up happens here, outside the timed region
     launches0 = _capi.launch_count()
     t0 = sampler.mark()
-    ms, stats = time_steps(env, actions, args.steps, torch, dist, world)
+    ms, stats, last = time_steps(env, actions, args.steps, torch, dist, world)
     t1 = sampler.mark()
+    dumped = dump_outputs(args.dump_outputs, last, stats, n, torch) if (args.dump_outputs and rank == 0) else None
     launches = _capi.launch_count() - launches0      # counted by the library: one per kernel it launched in the timed region
     if world > 1:
         lt = torch.tensor([launches], dtype=torch.float64, device="cuda")
@@ -568,7 +606,7 @@ def main():
     value = total_env_steps / (ms * 1e-3)
     # ---- sustained window: 300 more steps of the same workload (episodes desynchronised by now), own clock samples
     s0 = sampler.mark()
-    ms_sus, _ = time_steps(env, actions, 300, torch, dist, world)
+    ms_sus, _, _ = time_steps(env, actions, 300, torch, dist, world)
     s1 = sampler.mark()
     # ---- end-to-end through the host-buffer C-ABI call
     e2e = None
@@ -648,7 +686,7 @@ def main():
         acts_s = [env_s.random_actions(t) for t in range(n_act)]
         for t in range(10):
             env_s.step(acts_s[t % n_act])
-        ms_s, _ = time_steps(env_s, acts_s, 200, torch, dist, 1)
+        ms_s, _, _ = time_steps(env_s, acts_s, 200, torch, dist, 1)
         small = {"workload": f"{args.task}, 4096 envs (BASELINE config 2, the reference's own scale), L2-resident; bound by instruction latency, not by bandwidth",
                  "value": 4096 * 200 / (ms_s * 1e-3), "unit": "env-steps/s", "us_per_step": ms_s / 200 * 1e3}
         env_s.close()
@@ -704,6 +742,8 @@ def main():
             "clocks": clocks,
             "rollout_stats": [float(x) for x in stats.cpu().tolist()],
         }
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         if e2e is not None:
             line["e2e"] = e2e
         if small is not None:

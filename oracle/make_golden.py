@@ -302,6 +302,8 @@ def _ppo_update_cases(ns, H, N, mb, actor_hidden, critic_hidden, lstm_hidden, fi
         out[f"{tag}_difficulty"] = torch.tensor(ppo.env.difficulty)
         for name, val in logged.items():
             out[f"{tag}_log__{name.split('/')[1].rstrip(':')}"] = torch.tensor(val)
+    if file_name == "ppo_update_native.npz":            # keeps the file under 1 MB: lip_ arrays equal to their plain_ twins are stored once
+        out = {k: v for k, v in out.items() if not (k.startswith("lip_") and torch.equal(v, out["plain_" + k[4:]]))}
     np.savez_compressed(os.path.join(OUT, file_name), **{k: np.asarray(t) for k, t in out.items()})
 
 

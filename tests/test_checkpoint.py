@@ -43,33 +43,38 @@ def test_state_dict_round_trip_and_reference_parameter_names(tmp_path):
     assert sa.keys() == sc.keys() and all(torch.equal(sa[k]["exp_avg_sq"], sc[k]["exp_avg_sq"]) for k in sa)
 
 
-def test_reference_state_dict_loads_when_the_reference_is_present(tmp_path):
-    """Build container only: a state dict saved by the reference's own PPO_ActorCritic loads into TorchActorCritic and gives the
-    same action mean and value."""
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("reference tree not present")
-    ns = ref_loader.load()
-    torch.manual_seed(0)
-    para = {"actor_critic_mlp_dict": {"actor_input_dim": 26, "actor_output_dim": 4, "critic_input_dim": 26, "critic_output_dim": 1,
-                                      "actor_hidden_sizes": [64, 64], "critic_hidden_sizes": [64], "activation": torch.nn.ReLU},
-            "use_actor_encoder": False, "use_critic_encoder": True, "share_encoder": False, "critic_encoder_type": "LSTM",
-            "critic_encoder_dict": {"encoder_type": "LSTM", "input_size": 26, "output_size": 32, "num_layers": 1, "bidirectional": False}}
-    try:
-        ref = ns.nets.PPO_ActorCritic(para)
-    except Exception as exc:                                   # constructor dict keys differ between reference revisions
-        pytest.skip(f"reference PPO_ActorCritic not constructible with the reconstructed dict: {exc!r}")
+def test_reference_state_dict_loads_and_gives_the_reference_outputs(golden_dir, tmp_path):
+    """State dicts in the reference's format load into TorchActorCritic and give the reference's own action mean and value.
+    tests/golden/ppo_update.npz holds PPO_ActorCritic.state_dict() of the reference (plain_init__<key>): it must load with exactly
+    its keys and shapes.  tests/golden/actor.npz and critic.npz hold weights, inputs and outputs of the reference's actor MLP /
+    act() and LSTM critic (case a); under the reference's parameter names they must reproduce those outputs."""
+    from taco_b200.ppo import TorchActorCritic, load_checkpoint
+    z = np.load(os.path.join(golden_dir, "ppo_update.npz"))
+    ref_sd = {k[len("plain_init__"):]: torch.from_numpy(z[k]) for k in z.files if k.startswith("plain_init__")}
     p = str(tmp_path / "ref_model.pt")
-    torch.save(ref.state_dict(), p)
-    from taco_b200.ppo import load_checkpoint
-    ours = _agent()
-    load_checkpoint(p, ours)
-    obs, st = torch.randn(16, 1, 26), torch.randn(16, 5, 26)
+    torch.save(ref_sd, p)
+    ours = TorchActorCritic(26, 4, [32, 24], 26, 16, [20])
+    assert load_checkpoint(p, ours) is None                    # strict load_state_dict: no missing or unexpected key
+    got = ours.state_dict()
+    assert got.keys() == ref_sd.keys() and all(torch.equal(got[k], ref_sd[k]) for k in ref_sd)
+    a, c = np.load(os.path.join(golden_dir, "actor.npz")), np.load(os.path.join(golden_dir, "critic.npz"))
+    sd = {"log_std": a["log_std"]}
+    for i in range(3):
+        sd[f"actor_mlp.layers.{2 * i}.weight"], sd[f"actor_mlp.layers.{2 * i}.bias"] = a[f"w{i}"], a[f"b{i}"]
+        sd[f"critic_mlp.layers.{2 * i}.weight"], sd[f"critic_mlp.layers.{2 * i}.bias"] = c[f"a_w{i}"], c[f"a_b{i}"]
+    for nm in ("weight_ih", "weight_hh", "bias_ih", "bias_hh"):
+        sd[f"critic_encoder.layers.{nm}_l0"] = c[f"a_{nm}_l0"]
+    p2 = str(tmp_path / "ref_model_2.pt")
+    torch.save({k: torch.from_numpy(np.asarray(v)) for k, v in sd.items()}, p2)
+    ours = TorchActorCritic(26, 4, [64, 128], 26, 48, [64, 32])
+    load_checkpoint(p2, ours)
     with torch.no_grad():
-        _, _, v_ref, m_ref, _ = ref.act(obs, st, deterministic=True)
-        m = ours(obs)
-        v = ours.critic_mlp(ours.critic_encoder(st))
-    assert torch.allclose(m, m_ref, atol=1e-6) and torch.allclose(v, v_ref, atol=1e-6)
+        m = ours(torch.from_numpy(a["obs"]))
+        v = ours.critic_mlp(ours.critic_encoder(torch.from_numpy(c["a_states"])))
+    for want in (a["mean"], a["act_mean"]):
+        assert torch.allclose(m, torch.from_numpy(want), atol=1e-6)
+    for want in (c["a_value"], c["a_act_value"]):
+        assert torch.allclose(v, torch.from_numpy(want), atol=1e-6)
 
 
 def test_export_actor_torchscript(tmp_path):

@@ -1,8 +1,8 @@
 #!/bin/bash
 # Copies the reference's PPO consumer (IsaacGymEnvs/algorithms/: ppo_asymmetry.py, nets_asymmetry.py, buffer_asymmetry.py)
-# UNMODIFIED into the git-ignored baseline/_ref/ so that it travels to the GPU box (gpurun ships baseline/_ref, git does not).
-# Used by tools/run_reference_ppo.py and tests/test_reference_consumer_gpu.py: the reference's own PPO.run drives FpvVecTask.
-# Build container only (needs /root/reference).
+# UNMODIFIED into the git-ignored baseline/_ref/, next to the project, so that it can be used on a machine without the reference tree.
+# Used by tools/run_reference_ppo.py: the reference's own PPO.run drives FpvVecTask.
+# Needs a copy of the reference (TACO_REFERENCE points to it).
 set -e
 REF=${TACO_REFERENCE:-/root/reference}
 ROOT=$(cd "$(dirname "$0")/.." && pwd)

@@ -93,7 +93,8 @@ print(json.dumps(out["parity_256"]), flush=True)
 # ---------------------------------------------------------------- 3. the reference-generated golden update
 z = np.load(os.path.join(ROOT, "tests", "golden", "ppo_update_native.npz"))
 for tag in ("plain", "lip"):
-    gg = {k[len(tag) + 1:]: torch.from_numpy(np.asarray(z[k])) for k in z.files if k.startswith(tag + "_")}
+    gg = {k[len("plain_"):]: torch.from_numpy(np.asarray(z[k])) for k in z.files if k.startswith("plain_")}   # shared arrays: plain_ only
+    gg.update({k[len(tag) + 1:]: torch.from_numpy(np.asarray(z[k])) for k in z.files if k.startswith(tag + "_")})
     init = {k[6:]: v for k, v in gg.items() if k.startswith("init__")}
     final = {k[7:]: v for k, v in gg.items() if k.startswith("final__")}
     buf = types.SimpleNamespace(**{k[5:]: v.cuda() for k, v in gg.items() if k.startswith("buf__")})
