@@ -22,35 +22,14 @@
 // warps 2..17 = epilogue: tile slot t = (warp-2)/8, column half of the part = ((warp-2)/4)&1, TMEM lane quadrant =
 // warp%4 (thread <-> TMEM lane <-> env row).
 #pragma once
-#include <cuda_bf16.h>
-#include <stdint.h>
+#include "mlp_common.cuh"
 #include "philox.cuh"
 
 namespace taco {
 namespace actor {
+using namespace taco::mlp;
 
-constexpr int kTileM = 128;                    // envs per tile = TMEM lanes
-constexpr int kKC = 64;                        // bf16 per K chunk: one 128-byte swizzle row
-constexpr int kMaxN = 256;                     // widest hidden layer
-constexpr int kPartN = 128;                    // rows of W per stage = columns of D per part
-constexpr int kSlots = 3;                      // weight ring: slots of one part (all K chunks)
-constexpr int kChunkBytes = kPartN * 128;      // 16 KB: 128 rows x 64 bf16
-constexpr int kSlotBytes = kChunkBytes * (kMaxN / kKC);   // 64 KB
-constexpr int kMaxHidden = 4;
-constexpr int kOutPad = 4;                     // num_acts = 4
-constexpr int kOutN = 16;                      // output layer as an MMA part: N padded to the instruction minimum
-constexpr int kEpiWarps = 16;
-constexpr int kTcThreads = (2 + kEpiWarps) * 32;   // 576
-constexpr int kTmemCols = 512;
-constexpr int kTmemSlot = 256;                 // columns per tile slot: A (128, packed bf16 pairs) + D (128, fp32)
-constexpr int kTmemD = 128;                    // offset of D inside a slot
 constexpr uint32_t STREAM_ACTOR = 6;           // Philox stream of the action noise
-
-struct TcLayer {
-    int n;               // output width of the layer (multiple of 64, <= 256)
-    int kchunks;         // ceil(K / 64)
-    uint32_t img_off;    // byte offset of the layer's first chunk image; chunk c is at img_off + c * n * 128
-};
 
 struct SampleParams {    // PPO_ActorCritic.act sampling (nets_asymmetry.py:336-346); enabled when action != nullptr
     float* action;       // (n, out) mean + std * eps
@@ -78,133 +57,10 @@ struct TcParams {
     SampleParams sp;
     unsigned long long* dbg;   // optional timeline of CTA 0 (TACO_ACTOR_TIMELINE=<file>): 3 regions of kDbgCap (clock << 8 | code) words
 };
-constexpr int kDbgCap = 4096;
-#define TACO_DBG(region, cnt, code)                                                                         \
-    do {                                                                                                    \
-        if (p.dbg && blockIdx.x == 0 && (cnt) < kDbgCap)                                                    \
-            p.dbg[(region) * kDbgCap + (cnt)++] = ((unsigned long long)clock64() << 8) | (unsigned)(code);  \
-    } while (0)
 
-constexpr int kSmemBias = kMaxHidden * kMaxN * 4;          // 4 KB
-constexpr int kTcSmemBytes = 1024 /*alignment slack*/ + kSlots * kSlotBytes + kSmemBias + 256;
 constexpr int kObsBulkMaxIn = 26;              // widest observation row the bulk-staged path takes (26 x len_obs = 1)
 constexpr int kObsStageBytes = kTileM * kObsBulkMaxIn * 4;        // one tile's observation block, fp32, as it lies in global memory
 constexpr int kActorSmemBytes = kTcSmemBytes + 2 * kObsStageBytes;
-
-// ---------------------------------------------------------------------------------------------- PTX wrappers
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"(bar), "r"(parity)
-            : "memory");
-    } while (!ok);
-}
-__device__ __forceinline__ uint32_t elect_one_sync() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred P1;\n\telect.sync _|P1, 0xFFFFFFFF;\n\tselp.b32 %0, 1, 0, P1;\n\t}" : "=r"(pred));
-    return pred;
-}
-__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// bulk async copy global -> shared (the TMA engine, 1-D form): completes `bytes` on the mbarrier
-__device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst_smem), "l"(src),
-                 "r"(bytes), "r"(bar)
-                 : "memory");
-}
-
-__device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-
-// shared-memory matrix descriptor, K-major, SWIZZLE_128B: 8-row x 128-byte atoms, consecutive atoms 1024 B apart
-// (cute::UMMA::SmemDescriptor: start>>4 [0,14), LBO>>4 [16,30), SBO>>4 [32,46), version=1 [46,48), layout=2 [61,64))
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
-    return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) |
-           ((uint64_t)2 << 61);
-}
-// instruction descriptor, kind::f16: D=f32 [4,6)=1, A=bf16 [7,10)=1, B=bf16 [10,13)=1, both K-major, N>>3 [17,23), M>>4 [24,29)
-__device__ __forceinline__ uint32_t umma_idesc_bf16(int m, int n) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// all previously issued tcgen05.mma of this thread arrive (once) on the mbarrier when they have completed
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// 32 lanes x 32 consecutive fp32 columns -> 32 registers per thread (thread t <-> lane base + t)
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]),
-          "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]),
-          "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld4(uint32_t taddr, uint32_t (&v)[4]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-// registers -> 32 lanes x 16 consecutive columns (thread t <-> lane base + t)
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t* v) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-        ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]),
-          "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-        : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-// D[tmem] (+)= A[tmem, packed bf16 pairs] * B[smem descriptor]^T   (the "TS" form: A operand from tensor memory)
-__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-
-__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
-    const __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);     // .x (low half) = lo
-    return *reinterpret_cast<const uint32_t*>(&v);
-}
-
-// byte offset of the 16-byte chunk c16 (0..7) of row r inside a [rows x 64 bf16] SWIZZLE_128B block
-__device__ __forceinline__ uint32_t sw128_off(int r, int c16) { return (uint32_t)(r * 128 + ((c16 ^ (r & 7)) << 4)); }
 
 // tanh output + optional sampling, shared by the tensor-core and the FP32 kernels (one thread = one env row)
 __device__ __forceinline__ void actor_tail(const float* pre, int out_dim, long long row, float* mean, const SampleParams& sp) {
@@ -244,16 +100,6 @@ __device__ __forceinline__ void actor_tail(const float* pre, int out_dim, long l
 }
 
 // ---------------------------------------------------------------------------------------------- the kernel
-// relu(D + bias) of 32 accumulator columns -> 16 packed bf16 pairs (column 2j in the low half)
-__device__ __forceinline__ void relu_pack32(const uint32_t (&v)[32], const float* bias, uint32_t* pk) {
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-        const float4 b = *reinterpret_cast<const float4*>(bias + q * 4);
-        pk[q * 2 + 0] = pack_bf16x2(fmaxf(__uint_as_float(v[q * 4 + 0]) + b.x, 0.0f), fmaxf(__uint_as_float(v[q * 4 + 1]) + b.y, 0.0f));
-        pk[q * 2 + 1] = pack_bf16x2(fmaxf(__uint_as_float(v[q * 4 + 2]) + b.z, 0.0f), fmaxf(__uint_as_float(v[q * 4 + 3]) + b.w, 0.0f));
-    }
-}
-
 // the observation features [32 g, 32 g + 32) of one row as 16 packed bf16 pairs (zero beyond in_dim / for invalid rows).  Rows of an
 // even width are 8-byte aligned ((N, in_dim) float32 contiguous): one 8-byte load per pair halves the L1 wavefronts of this
 // row-per-thread access pattern (every lane touches its own row, i.e. its own cache line).
@@ -287,7 +133,6 @@ __device__ __forceinline__ void read_staged_obs(const float* stage, int r, int i
     }
 }
 
-#ifndef TACO_TC_NO_ACTOR_KERNEL      // critic_tc.cuh reuses the wrappers above and the weight packer below, not this kernel
 __global__ void __launch_bounds__(kTcThreads, 1) actor_tc_kernel(const TcParams p) {
     extern __shared__ uint8_t smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
@@ -532,27 +377,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) actor_tc_kernel(const TcParams 
     if (warp == 1) {
         tc_fence_after();
         tmem_dealloc(tmem0, kTmemCols);
-    }
-}
-
-#endif  // TACO_TC_NO_ACTOR_KERNEL
-
-// fp32 (out, in) row-major weights -> bf16 K-chunk images in the SWIZZLE_128B K-major layout the kernel copies verbatim:
-// chunk c holds W[:, 64c .. 64c+63] as n rows of 128 bytes (rows >= n_real are zero); the 16-byte piece q of row r sits
-// at r*128 + ((q ^ (r&7)) << 4).
-static __global__ void pack_weights_kernel(const float* __restrict__ w, int n_real, int n, int k, uint8_t* __restrict__ img) {
-    const int kchunks = (k + kKC - 1) / kKC;
-    const int total = kchunks * n * 8;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
-        const int q = i & 7, r = (i >> 3) % n, c = (i >> 3) / n;
-        float f[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const int kk = c * kKC + q * 8 + j;
-            f[j] = (kk < k && r < n_real) ? w[(size_t)r * k + kk] : 0.0f;
-        }
-        const uint4 pk = make_uint4(pack_bf16x2(f[0], f[1]), pack_bf16x2(f[2], f[3]), pack_bf16x2(f[4], f[5]), pack_bf16x2(f[6], f[7]));
-        *reinterpret_cast<uint4*>(img + (size_t)c * n * 128 + sw128_off(r, q)) = pk;
     }
 }
 

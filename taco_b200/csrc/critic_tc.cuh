@@ -16,21 +16,21 @@
 //     free), read and rewritten by the thread that owns (env row, hidden unit); h_t is written back over the A operand as
 //     packed bf16 pairs next to the freshly staged x_{t+1};
 //   * the T = len_states steps reuse one weight image; then the MLP layers and the 16-wide output part follow as in the actor.
-// Gate non-linearities use MUFU.TANH on packed half pairs (tanh.approx.f16x2; sigmoid(x) = 0.5 + 0.5 tanh(x / 2)): 2.5 MUFU slots
-// per (env, unit, step) -- the LSTM phase is bound by the 16 MUFU lanes of the SM, not by the tensor core.
+// Gate non-linearities use MUFU.TANH (tanh.approx.f32; sigmoid(x) = 0.5 + 0.5 tanh(x / 2)): five per (env, unit, step) -- the
+// LSTM phase is bound by the 16 MUFU lanes of the SM, not by the tensor core.
 #pragma once
-#define TACO_TC_NO_ACTOR_KERNEL
 #include <cuda_fp16.h>
-#include "actor_tc.cuh"
+#include "mlp_common.cuh"
 
 namespace taco {
 namespace critic {
-using namespace taco::actor;
+using namespace taco::mlp;
 
 constexpr int kMaxSeq = 8;             // len_states of the reference runs is 5 (README.md:60-66)
 constexpr int kTcMaxLstmHidden = 64;   // the cell state lives in the 64 spare TMEM columns of the tile's A operand
 constexpr int kTcMaxIn = 30;           // features per frame (26) + two constant-1 bias columns, padded to 32 = 16 packed TMEM columns
 constexpr int kMaxMlpHidden = 3;       // s_bias rows: LSTM gates + up to 3 hidden layers
+static_assert(1 + kMaxMlpHidden <= kMaxHidden, "the LSTM step and the MLP's hidden layers share the kMaxHidden bias rows / TcImage layers");
 constexpr int kRing = kSlots - 1;        // ring slots of the MLP weights; the last 64 KB slot holds the LSTM image for the whole kernel
 constexpr int kAColH = 0;              // A operand columns (packed bf16 pairs): h in [0, 32), x_t in [32, 48), zero pad [48, 64)
 constexpr int kAColX = 32;
@@ -48,30 +48,10 @@ struct CriticTcParams {
     const float* bias;     // [kMaxHidden][kMaxN]: row 0 unused (the LSTM bias rides in the MMA), rows 1.. = MLP hidden biases
     const float* b_out;    // [kOutPad]
     TcLayer layer[2 + kMaxMlpHidden];   // [0] one LSTM step, [1 .. n_hidden] MLP hidden layers, [n_hidden + 1] output layer
-    unsigned long long* dbg;            // optional timeline of CTA 0 (TACO_CRITIC_TIMELINE=<file>), see TACO_DBG in actor_tc.cuh
+    unsigned long long* dbg;            // optional timeline of CTA 0 (TACO_CRITIC_TIMELINE=<file>), see TACO_DBG in mlp_common.cuh
 };
 
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t* v) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(v[0]), "r"(v[1]),
-                 "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
-                 : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr)
-        : "memory");
-}
-// non-blocking phase test of an mbarrier
-__device__ __forceinline__ bool mbar_test(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    return ok != 0;
-}
 constexpr int kCriticStagger = 1200;      // default of CriticTcParams::stagger (TACO_CRITIC_STAGGER in the environment overrides it: tuning)
-__device__ __forceinline__ float tanh_mufu(float x) { float y; asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 
 // TACO_CRITIC_GATES (tuning builds): 0 (default) = tanh.approx.f32; 1 = MUFU.TANH on packed half pairs (tanh.approx.f16x2: the same
 // 16.4 results per clock and SM as the f32 form, tools/probes/mufu_probe.cu, plus conversions -- no faster, twice the error);
@@ -106,9 +86,6 @@ __device__ __forceinline__ void lstm_group(const uint32_t (&v)[16], uint32_t (&c
         const float2 tc = tanh_pair(c0, c1);
         hp[u >> 1] = pack_bf16x2(fmaf(0.5f, to.x, 0.5f) * tc.x, fmaf(0.5f, to.y, 0.5f) * tc.y);
     }
-}
-__device__ __forceinline__ void tmem_st4(uint32_t taddr, const uint32_t (&v)[4]) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]) : "memory");
 }
 // one 64-column half of a gate part = 4 groups = 16 hidden units of this thread's env row; t_c = TMEM address of their cell
 // states; `early` = arrive on the tile's A/D barrier as soon as the last accumulator columns are in registers (the next part of

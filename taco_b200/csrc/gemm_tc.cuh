@@ -29,16 +29,10 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <stdint.h>
-
-#ifndef TACO_TC_NO_ACTOR_KERNEL
-#define TACO_TC_NO_ACTOR_KERNEL          // only the PTX wrappers of actor_tc.cuh are used here
-#endif
-#include "actor_tc.cuh"
+#include "tc_ptx.cuh"
 
 namespace taco {
 namespace gemm {
-
-using namespace taco::actor;
 
 constexpr int BM = 128, BK = 64;
 constexpr int kStages = 3;
@@ -82,43 +76,6 @@ struct GemmParams {
     const int* stop;                  // device flag (may be null): non-zero = the update stopped early (KL), the launch is a no-op
     LstmEpi lstm;
 };
-
-// MN-major SWIZZLE_128B operand: 64 (M or N) x 64 (K) blocks of 8 KB; inside a block k-row r is the 128-byte line r (8-row atoms,
-// 1024 bytes apart = stride byte offset), the next 64 M / N elements are the next block (leading byte offset).  cute's canonical
-// layout Swizzle<3,4,3> o ((8,n),(8,k)):((1,LBO),(8,SBO)) in 16-byte units.
-constexpr uint32_t kMnBlock = 64 * BK * 2;
-__device__ __forceinline__ uint64_t umma_desc_sw128_mn(uint32_t smem_addr) {
-    return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) | ((uint64_t)(kMnBlock >> 4) << 16) | ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) |
-           ((uint64_t)2 << 61);
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst_smem, const CUtensorMap* tm, int c0, int c1, uint32_t bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst_smem),
-                 "l"(tm), "r"(bar), "r"(c0), "r"(c1)
-                 : "memory");
-}
-// staging tile (shared memory, SWIZZLE_128B, 128 rows x 128 bytes) -> global tensor at (column c0, row c1), clipped at the tensor's edges
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* tm, uint32_t src_smem, int c0, int c1) {
-    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(tm), "r"(src_smem), "r"(c0), "r"(c1) : "memory");
-    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-}
-// all bulk stores of this thread have finished READING shared memory
-__device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-// programmatic dependent launch: a kernel launched with the stream-serialization attribute may start while its predecessor in the
-// stream is still running; nothing the predecessor wrote may be read (and nothing it reads overwritten) before pdl_wait()
-// returns = predecessor complete and flushed.  pdl_launch_dependents() lets the successor's CTAs be scheduled from here on.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-// generic-proxy writes to shared memory become visible to the async proxy (TMA)
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr)
-        : "memory");
-}
 
 // 8 bf16 = 4 packed pairs -> one 16-byte store
 __device__ __forceinline__ void st_u4(__nv_bfloat16* dst, const uint32_t* pk) {
@@ -382,7 +339,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                         for (int q = 0; q < 4; ++q)                       // own row, pieces 4 h2 .. 4 h2 + 3 (XOR-swizzled: conflict-free, and the TMA's SWIZZLE_128B)
                             *reinterpret_cast<uint4*>(sa + own + (((uint32_t)(4 * h2 + q) ^ key) << 4)) = make_uint4(pk[4 * q], pk[4 * q + 1], pk[4 * q + 2], pk[4 * q + 3]);
                     }
-                    fence_async_smem();
+                    fence_proxy_async_smem();
                     epi_barrier(half);
                     if (te == 0) tma_store_2d(&tmC, smem_u32(sa), c0, mt * BM);
                     sb ^= 1u;
@@ -402,7 +359,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     for (int q = 0; q < 8; ++q)
                         *reinterpret_cast<uint4*>(sa + own + (((uint32_t)q ^ key) << 4)) = make_uint4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
                     if (c0 + 64 < p.n_valid) tmem_ld32(t_row + c0 + 64, v);
-                    fence_async_smem();
+                    fence_proxy_async_smem();
                     epi_barrier(half);
                     if (te == 0) tma_store_2d(&tmC, smem_u32(sa), c0, sp * p.m + mt * BM);
                     sb ^= 1u;

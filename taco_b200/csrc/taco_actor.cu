@@ -17,32 +17,13 @@
 #include <string>
 #include <vector>
 
-#include "../../include/taco_b200.h"
+#include "host_common.h"
 #include "actor_tc.cuh"
 
 namespace taco {
-int fail(int code, const std::string& msg);      // taco_env.cu: sets the thread-local message behind taco_last_error
 namespace actor {
 
-static int afail(int code, const std::string& msg) { return taco::fail(code, msg); }   // one error slot for the whole library
-
-#define ACT_CUDA(expr)                                                                            \
-    do {                                                                                          \
-        cudaError_t _e = (expr);                                                                  \
-        if (_e != cudaSuccess)                                                                    \
-            return afail(TACO_E_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));        \
-    } while (0)
-
-struct DevGuard {
-    int prev = -1;
-    explicit DevGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
-    ~DevGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
-
 constexpr int kMaxLayers = 8;        // linear layers of the FP32 path
-constexpr int kFpEnvs = 32;          // envs per CTA of the FP32 kernel (one warp lane per env)
-constexpr int kFpThreads = 128;
-constexpr int kFpTile = 8;           // output neurons per warp pass of the FP32 kernel
 
 struct FpParams {
     const float* obs; float* mean;
@@ -177,23 +158,20 @@ __global__ void __launch_bounds__(kSnThreads) spectral_norm_kernel(float* w, int
 }  // namespace taco
 
 using namespace taco::actor;
+using taco::DevGuard;
+using taco::fail;
 
 struct TacoActor {
     int device = 0;
     std::vector<int> sizes;              // [in, h1, ..., hL, out]
     int n_layers = 0;
-    std::vector<size_t> w_off, b_off;    // float offsets into w_f32 / b_f32
-    float* w_f32 = nullptr;              // all layers, (out, in) row-major each
-    float* b_f32 = nullptr;
+    MlpF32 f32;                          // all layers, (out, in) row-major each
     double* sigma = nullptr;             // per layer, device
     bool loaded = false;
     // tensor-core path
     bool tc_ok = false;
     std::string tc_why;
-    uint8_t* wimg = nullptr;
-    float* bias_pad = nullptr;           // [kMaxHidden][kMaxN]
-    float* b_out = nullptr;              // [kOutPad]
-    TcLayer tc_layer[kMaxHidden + 1];    // hidden layers + the output layer (16-row padded image)
+    TcImage tc;                          // hidden layers + the output layer (16-row padded image)
     int num_sms = 148;
     int fp_smem = 0;
     // sampling constants [std0..3, logp_const, pad]: device copy read by the kernels, host copy to detect changes
@@ -215,24 +193,24 @@ static int actor_set_log_std(TacoActor* a, const float* log_std_host, cudaStream
     v[4] = (float)(-lsum - 0.5 * out * std::log(2.0 * M_PI));
     if (a->samp_set && memcmp(v, a->samp_host, sizeof(v)) == 0) return TACO_OK;
     cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    ACT_CUDA(cudaStreamIsCapturing(s, &cs));
+    TACO_CUDA(cudaStreamIsCapturing(s, &cs));
     if (cs != cudaStreamCaptureStatusNone)
-        return afail(TACO_E_INVALID, "taco_actor: log_std changed while the stream is capturing; call taco_actor_set_log_std before the capture");
+        return fail(TACO_E_INVALID, "taco_actor: log_std changed while the stream is capturing; call taco_actor_set_log_std before the capture");
     memcpy(a->samp_host, v, sizeof(v));
-    ACT_CUDA(cudaMemcpyAsync(a->samp_dev, a->samp_host, sizeof(v), cudaMemcpyHostToDevice, s));   // pageable source: staged before the call returns
+    TACO_CUDA(cudaMemcpyAsync(a->samp_dev, a->samp_host, sizeof(v), cudaMemcpyHostToDevice, s));   // pageable source: staged before the call returns
     a->samp_set = true;
     return TACO_OK;
 }
 
 static int actor_run(TacoActor* a, const float* obs_dev, float* mean_dev, int32_t n, int32_t use_tc, const SampleParams& sp, void* stream) {
-    if (!a || !obs_dev || !mean_dev) return afail(TACO_E_INVALID, "taco_actor: null argument");
-    if (!a->loaded) return afail(TACO_E_INVALID, "taco_actor: call taco_actor_load first");
-    if (n <= 0) return afail(TACO_E_INVALID, "taco_actor: n must be positive");
-    if (a->sizes.back() == 4 && ((uintptr_t)mean_dev & 15u)) return afail(TACO_E_INVALID, "taco_actor: mean must be 16-byte aligned");
+    if (!a || !obs_dev || !mean_dev) return fail(TACO_E_INVALID, "taco_actor: null argument");
+    if (!a->loaded) return fail(TACO_E_INVALID, "taco_actor: call taco_actor_load first");
+    if (n <= 0) return fail(TACO_E_INVALID, "taco_actor: n must be positive");
+    if (a->sizes.back() == 4 && ((uintptr_t)mean_dev & 15u)) return fail(TACO_E_INVALID, "taco_actor: mean must be 16-byte aligned");
     DevGuard guard(a->device);
     cudaStream_t s = (cudaStream_t)stream;
     if (use_tc) {
-        if (!a->tc_ok) return afail(TACO_E_INVALID, "taco_actor: tensor-core path unavailable for this shape: " + a->tc_why);
+        if (!a->tc_ok) return fail(TACO_E_INVALID, "taco_actor: tensor-core path unavailable for this shape: " + a->tc_why);
         TcParams p;
         memset(&p, 0, sizeof(p));
         p.obs = obs_dev; p.mean = mean_dev;
@@ -240,71 +218,52 @@ static int actor_run(TacoActor* a, const float* obs_dev, float* mean_dev, int32_
         p.n_hidden = a->n_layers - 1;
         p.obs_vec2 = ((p.in_dim & 1) == 0 && ((uintptr_t)obs_dev & 7u) == 0) ? 1 : 0;
         p.obs_bulk = ((p.in_dim & 1) == 0 && p.in_dim <= kObsBulkMaxIn && ((uintptr_t)obs_dev & 15u) == 0 && !getenv("TACO_ACTOR_NO_BULK_OBS")) ? 1 : 0;
-        p.wimg = a->wimg; p.bias = a->bias_pad; p.b_out = a->b_out;
-        for (int l = 0; l <= p.n_hidden; ++l) p.layer[l] = a->tc_layer[l];
+        p.wimg = a->tc.wimg; p.bias = a->tc.bias; p.b_out = a->tc.b_out;
+        for (int l = 0; l <= p.n_hidden; ++l) p.layer[l] = a->tc.layer[l];
         p.sp = sp;
-        p.tiles_per_cta = p.num_tiles <= a->num_sms ? 1 : 2;           // a CTA keeps two tiles in flight unless every tile can have its own SM
-        const int num_pairs = (p.num_tiles + p.tiles_per_cta - 1) / p.tiles_per_cta;
-        const int grid = num_pairs < a->num_sms ? num_pairs : a->num_sms;
-        // developer aid: TACO_ACTOR_TIMELINE=<file> records clock64 stamps of CTA 0's MMA issuer / epilogue (synchronous)
+        const int grid = tc_grid(p.num_tiles, a->num_sms, &p.tiles_per_cta);
         const char* tl = getenv("TACO_ACTOR_TIMELINE");
-        if (tl && *tl) {
-            ACT_CUDA(cudaMalloc(&p.dbg, 3 * kDbgCap * sizeof(unsigned long long)));
-            ACT_CUDA(cudaMemsetAsync(p.dbg, 0, 3 * kDbgCap * sizeof(unsigned long long), s));
-        }
+        if (int rc = timeline_begin(tl, &p.dbg, s)) return rc;
         actor_tc_kernel<<<grid, kTcThreads, kActorSmemBytes, s>>>(p); TACO_LAUNCHED();
-        if (p.dbg) {
-            std::vector<unsigned long long> h(3 * kDbgCap);
-            ACT_CUDA(cudaStreamSynchronize(s));
-            ACT_CUDA(cudaMemcpy(h.data(), p.dbg, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-            cudaFree(p.dbg);
-            if (FILE* f = fopen(tl, "wb")) { fwrite(h.data(), sizeof(unsigned long long), h.size(), f); fclose(f); }
-        }
+        if (int rc = timeline_end(tl, p.dbg, s)) return rc;
     } else {
         FpParams p;
         memset(&p, 0, sizeof(p));
         p.obs = obs_dev; p.mean = mean_dev; p.n_rows = n; p.n_layers = a->n_layers;
         int mx = 0;
         for (int l = 0; l <= a->n_layers; ++l) { p.sizes[l] = a->sizes[l]; mx = a->sizes[l] > mx ? a->sizes[l] : mx; }
-        for (int l = 0; l < a->n_layers; ++l) { p.w[l] = a->w_f32 + a->w_off[l]; p.b[l] = a->b_f32 + a->b_off[l]; }
+        for (int l = 0; l < a->n_layers; ++l) { p.w[l] = a->f32.w + a->f32.w_off[l]; p.b[l] = a->f32.b + a->f32.b_off[l]; }
         p.stride = mx + 1;
         p.sp = sp;
         actor_fp32_kernel<<<(n + kFpEnvs - 1) / kFpEnvs, kFpThreads, a->fp_smem, s>>>(p); TACO_LAUNCHED();
     }
-    ACT_CUDA(cudaGetLastError());
+    TACO_CUDA(cudaGetLastError());
     return TACO_OK;
 }
 
 extern "C" {
 
 int taco_actor_create(int device, const int32_t* sizes, int32_t n_sizes, TacoActor** out) {
-    if (!sizes || !out) return afail(TACO_E_INVALID, "taco_actor_create: null argument");
+    if (!sizes || !out) return fail(TACO_E_INVALID, "taco_actor_create: null argument");
     *out = nullptr;
-    if (n_sizes < 2 || n_sizes > kMaxLayers + 1) return afail(TACO_E_INVALID, "taco_actor_create: need 2..9 layer sizes [in, h1, ..., out]");
+    if (n_sizes < 2 || n_sizes > kMaxLayers + 1) return fail(TACO_E_INVALID, "taco_actor_create: need 2..9 layer sizes [in, h1, ..., out]");
     for (int i = 0; i < n_sizes; ++i)
-        if (sizes[i] < 1 || sizes[i] > 512) return afail(TACO_E_INVALID, "taco_actor_create: layer sizes must be in [1, 512]");
-    if (sizes[n_sizes - 1] > kOutPad) return afail(TACO_E_INVALID, "taco_actor_create: output width must be <= 4 (num_acts, fpv_asymmetry.py:102)");
+        if (sizes[i] < 1 || sizes[i] > 512) return fail(TACO_E_INVALID, "taco_actor_create: layer sizes must be in [1, 512]");
+    if (sizes[n_sizes - 1] > kOutPad) return fail(TACO_E_INVALID, "taco_actor_create: output width must be <= 4 (num_acts, fpv_asymmetry.py:102)");
     int ndev = 0;
-    ACT_CUDA(cudaGetDeviceCount(&ndev));
-    if (device < 0 || device >= ndev) return afail(TACO_E_INVALID, "taco_actor_create: no such CUDA device");
+    TACO_CUDA(cudaGetDeviceCount(&ndev));
+    if (device < 0 || device >= ndev) return fail(TACO_E_INVALID, "taco_actor_create: no such CUDA device");
     DevGuard guard(device);
     TacoActor* a = new (std::nothrow) TacoActor();
-    if (!a) return afail(TACO_E_NOMEM, "host allocation failed");
+    if (!a) return fail(TACO_E_NOMEM, "host allocation failed");
     a->device = device;
     a->sizes.assign(sizes, sizes + n_sizes);
     a->n_layers = n_sizes - 1;
-    size_t wo = 0, bo = 0;
     int mx = 0;
-    for (int l = 0; l < a->n_layers; ++l) {
-        a->w_off.push_back(wo); a->b_off.push_back(bo);
-        wo += (size_t)sizes[l] * sizes[l + 1];
-        wo = (wo + 3) & ~(size_t)3;
-        bo += (size_t)((sizes[l + 1] + 3) & ~3);
-    }
     for (int i = 0; i < n_sizes; ++i) mx = sizes[i] > mx ? sizes[i] : mx;
     a->fp_smem = 2 * kFpEnvs * (mx + 1) * (int)sizeof(float);
     cudaDeviceProp prop;
-    ACT_CUDA(cudaGetDeviceProperties(&prop, device));
+    TACO_CUDA(cudaGetDeviceProperties(&prop, device));
     a->num_sms = prop.multiProcessorCount;
     // ---- is the shape eligible for the tcgen05 path?
     const int n_hidden = a->n_layers - 1;
@@ -312,26 +271,13 @@ int taco_actor_create(int device, const int32_t* sizes, int32_t n_sizes, TacoAct
     if (prop.major != 10) { a->tc_ok = false; a->tc_why = "device is not sm_100"; }
     else if (n_hidden < 1 || n_hidden > kMaxHidden) { a->tc_ok = false; a->tc_why = "needs 1..4 hidden layers"; }
     else if (sizes[0] > kMaxN) { a->tc_ok = false; a->tc_why = "input width > 256"; }
-    else {
-        for (int l = 1; l <= n_hidden; ++l)
-            if (sizes[l] % 64 != 0 || sizes[l] > kMaxN) { a->tc_ok = false; a->tc_why = "hidden widths must be multiples of 64, <= 256"; }
-    }
-    cudaError_t ce = cudaMalloc(&a->w_f32, wo * sizeof(float));
-    if (ce == cudaSuccess) ce = cudaMalloc(&a->b_f32, bo * sizeof(float));
+    else if (!tc_hidden_widths_ok(sizes, n_hidden)) { a->tc_ok = false; a->tc_why = "hidden widths must be multiples of 64, <= 256"; }
+    cudaError_t ce = mlp_f32_alloc(a->f32, sizes, a->n_layers);
     if (ce == cudaSuccess) ce = cudaMalloc(&a->sigma, kMaxLayers * sizeof(double));
     if (ce == cudaSuccess) ce = cudaMemset(a->sigma, 0, kMaxLayers * sizeof(double));
     if (ce == cudaSuccess) ce = cudaMalloc(&a->samp_dev, 8 * sizeof(float));
     if (ce == cudaSuccess && a->tc_ok) {
-        size_t img = 0;
-        for (int l = 0; l <= n_hidden; ++l) {
-            const int k = sizes[l], nn = l < n_hidden ? sizes[l + 1] : kOutN;
-            const int kch = (k + kKC - 1) / kKC;
-            a->tc_layer[l].n = nn; a->tc_layer[l].kchunks = kch; a->tc_layer[l].img_off = (uint32_t)img;
-            img += (size_t)kch * nn * 128;
-        }
-        ce = cudaMalloc(&a->wimg, img);
-        if (ce == cudaSuccess) ce = cudaMalloc(&a->bias_pad, kMaxHidden * kMaxN * sizeof(float));
-        if (ce == cudaSuccess) ce = cudaMalloc(&a->b_out, kOutPad * sizeof(float));
+        ce = tc_image_alloc(a->tc, sizes, n_hidden, 0, 0);
         if (ce == cudaSuccess) ce = cudaFuncSetAttribute(actor_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kActorSmemBytes);
     }
     if (ce == cudaSuccess && a->fp_smem > 48 * 1024)
@@ -339,7 +285,7 @@ int taco_actor_create(int device, const int32_t* sizes, int32_t n_sizes, TacoAct
     if (ce != cudaSuccess) {
         const std::string msg = std::string("taco_actor_create: ") + cudaGetErrorString(ce);
         taco_actor_destroy(a);
-        return afail(ce == cudaErrorMemoryAllocation ? TACO_E_NOMEM : TACO_E_CUDA, msg);
+        return fail(ce == cudaErrorMemoryAllocation ? TACO_E_NOMEM : TACO_E_CUDA, msg);
     }
     *out = a;
     return TACO_OK;
@@ -348,63 +294,50 @@ int taco_actor_create(int device, const int32_t* sizes, int32_t n_sizes, TacoAct
 int taco_actor_destroy(TacoActor* a) {
     if (!a) return TACO_OK;
     DevGuard guard(a->device);
-    cudaFree(a->w_f32); cudaFree(a->b_f32); cudaFree(a->sigma); cudaFree(a->samp_dev);
-    cudaFree(a->wimg); cudaFree(a->bias_pad); cudaFree(a->b_out);
+    mlp_f32_free(a->f32); cudaFree(a->sigma); cudaFree(a->samp_dev);
+    tc_image_free(a->tc);
     delete a;
     return TACO_OK;
 }
 
 int taco_actor_load(TacoActor* a, const float* const* weights_host, const float* const* biases_host, float lipschitz_const, void* stream) {
-    if (!a || !weights_host || !biases_host) return afail(TACO_E_INVALID, "taco_actor_load: null argument");
+    if (!a || !weights_host || !biases_host) return fail(TACO_E_INVALID, "taco_actor_load: null argument");
     for (int l = 0; l < a->n_layers; ++l)
-        if (!weights_host[l] || !biases_host[l]) return afail(TACO_E_INVALID, "taco_actor_load: null layer pointer");
+        if (!weights_host[l] || !biases_host[l]) return fail(TACO_E_INVALID, "taco_actor_load: null layer pointer");
     DevGuard guard(a->device);
     cudaStream_t s = (cudaStream_t)stream;
-    for (int l = 0; l < a->n_layers; ++l) {
-        const int in = a->sizes[l], out = a->sizes[l + 1];
-        ACT_CUDA(cudaMemcpyAsync(a->w_f32 + a->w_off[l], weights_host[l], (size_t)in * out * sizeof(float), cudaMemcpyDefault, s));
-        ACT_CUDA(cudaMemcpyAsync(a->b_f32 + a->b_off[l], biases_host[l], (size_t)out * sizeof(float), cudaMemcpyDefault, s));
-    }
+    if (int rc = mlp_f32_upload(a->f32, weights_host, biases_host, a->sizes.data(), a->n_layers, s)) return rc;
     // spectral projection of every weight matrix (ppo_asymmetry.py:398-404); also records sigma when lipschitz_const <= 0
     for (int l = 0; l < a->n_layers && lipschitz_const >= 0.0f; ++l) {        // negative: weights are known to be projected, skip the measurement
         const int in = a->sizes[l], out = a->sizes[l + 1];
-        spectral_norm_kernel<<<1, kSnThreads, (size_t)(in + out) * sizeof(double), s>>>(a->w_f32 + a->w_off[l], out, in, lipschitz_const,
+        spectral_norm_kernel<<<1, kSnThreads, (size_t)(in + out) * sizeof(double), s>>>(a->f32.w + a->f32.w_off[l], out, in, lipschitz_const,
                                                                                          a->sigma + l, 20000, 1e-12); TACO_LAUNCHED();
     }
-    ACT_CUDA(cudaGetLastError());
+    TACO_CUDA(cudaGetLastError());
     if (a->tc_ok) {
-        const int n_hidden = a->n_layers - 1;
-        ACT_CUDA(cudaMemsetAsync(a->bias_pad, 0, kMaxHidden * kMaxN * sizeof(float), s));
-        for (int l = 0; l <= n_hidden; ++l) {
-            const int in = a->sizes[l], out = a->sizes[l + 1];
-            pack_weights_kernel<<<64, 256, 0, s>>>(a->w_f32 + a->w_off[l], out, a->tc_layer[l].n, in, a->wimg + a->tc_layer[l].img_off); TACO_LAUNCHED();
-            if (l < n_hidden)
-                ACT_CUDA(cudaMemcpyAsync(a->bias_pad + l * kMaxN, a->b_f32 + a->b_off[l], (size_t)out * sizeof(float), cudaMemcpyDeviceToDevice, s));
-        }
-        ACT_CUDA(cudaMemsetAsync(a->b_out, 0, kOutPad * sizeof(float), s));
-        ACT_CUDA(cudaMemcpyAsync(a->b_out, a->b_f32 + a->b_off[n_hidden], (size_t)a->sizes[n_hidden + 1] * sizeof(float), cudaMemcpyDeviceToDevice, s));
-        ACT_CUDA(cudaGetLastError());
+        TACO_CUDA(cudaMemsetAsync(a->tc.bias, 0, kMaxHidden * kMaxN * sizeof(float), s));
+        if (int rc = tc_image_pack(a->tc, a->f32, a->sizes.data(), a->n_layers - 1, s)) return rc;
     }
-    ACT_CUDA(cudaStreamSynchronize(s));     // the host weight buffers may be released by the caller on return
+    TACO_CUDA(cudaStreamSynchronize(s));     // the host weight buffers may be released by the caller on return
     a->loaded = true;
     return TACO_OK;
 }
 
 int taco_actor_sigmas(TacoActor* a, double* out_host) {
-    if (!a || !out_host) return afail(TACO_E_INVALID, "taco_actor_sigmas: null argument");
+    if (!a || !out_host) return fail(TACO_E_INVALID, "taco_actor_sigmas: null argument");
     DevGuard guard(a->device);
-    ACT_CUDA(cudaDeviceSynchronize());
-    ACT_CUDA(cudaMemcpy(out_host, a->sigma, (size_t)a->n_layers * sizeof(double), cudaMemcpyDeviceToHost));
+    TACO_CUDA(cudaDeviceSynchronize());
+    TACO_CUDA(cudaMemcpy(out_host, a->sigma, (size_t)a->n_layers * sizeof(double), cudaMemcpyDeviceToHost));
     return TACO_OK;
 }
 
 int taco_actor_weights(TacoActor* a, int32_t layer, float* w_host, float* b_host) {
-    if (!a || layer < 0 || layer >= a->n_layers) return afail(TACO_E_INVALID, "taco_actor_weights: bad argument");
+    if (!a || layer < 0 || layer >= a->n_layers) return fail(TACO_E_INVALID, "taco_actor_weights: bad argument");
     DevGuard guard(a->device);
-    ACT_CUDA(cudaDeviceSynchronize());
+    TACO_CUDA(cudaDeviceSynchronize());
     const int in = a->sizes[layer], out = a->sizes[layer + 1];
-    if (w_host) ACT_CUDA(cudaMemcpy(w_host, a->w_f32 + a->w_off[layer], (size_t)in * out * sizeof(float), cudaMemcpyDeviceToHost));
-    if (b_host) ACT_CUDA(cudaMemcpy(b_host, a->b_f32 + a->b_off[layer], (size_t)out * sizeof(float), cudaMemcpyDeviceToHost));
+    if (w_host) TACO_CUDA(cudaMemcpy(w_host, a->f32.w + a->f32.w_off[layer], (size_t)in * out * sizeof(float), cudaMemcpyDeviceToHost));
+    if (b_host) TACO_CUDA(cudaMemcpy(b_host, a->f32.b + a->f32.b_off[layer], (size_t)out * sizeof(float), cudaMemcpyDeviceToHost));
     return TACO_OK;
 }
 
@@ -413,14 +346,14 @@ int taco_actor_tc_available(TacoActor* a) { return (a && a->tc_ok) ? 1 : 0; }
 // PPO.spectral_normalize_actors for ONE parameter that already lives on the device (e.g. the storage of a torch nn.Linear weight
 // during PPO.update, ppo_asymmetry.py:248-249): in place, asynchronous, no SVD and no host round trip.
 int taco_spectral_project(int device, float* w_dev, int32_t rows, int32_t cols, float lipschitz_const, double* sigma_dev, void* stream) {
-    if (!w_dev || !sigma_dev) return afail(TACO_E_INVALID, "taco_spectral_project: null argument");
+    if (!w_dev || !sigma_dev) return fail(TACO_E_INVALID, "taco_spectral_project: null argument");
     if (rows < 1 || cols < 1 || (size_t)(rows + cols) * sizeof(double) > 200 * 1024)
-        return afail(TACO_E_INVALID, "taco_spectral_project: rows + cols must be in [2, 25600]");
+        return fail(TACO_E_INVALID, "taco_spectral_project: rows + cols must be in [2, 25600]");
     DevGuard guard(device);
     const size_t smem = (size_t)(rows + cols) * sizeof(double);
-    if (smem > 48 * 1024) ACT_CUDA(cudaFuncSetAttribute(spectral_norm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (smem > 48 * 1024) TACO_CUDA(cudaFuncSetAttribute(spectral_norm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     spectral_norm_kernel<<<1, kSnThreads, smem, (cudaStream_t)stream>>>(w_dev, rows, cols, lipschitz_const, sigma_dev, 20000, 1e-12); TACO_LAUNCHED();
-    ACT_CUDA(cudaGetLastError());
+    TACO_CUDA(cudaGetLastError());
     return TACO_OK;
 }
 
@@ -433,8 +366,8 @@ int taco_actor_forward(TacoActor* a, const float* obs_dev, float* mean_dev, int3
 int taco_actor_act_counter(TacoActor* a, const float* obs_dev, int32_t n, const float* log_std_host, int64_t env_offset, uint64_t seed,
                            uint32_t step_index, const uint32_t* step_base_dev, float* mean_dev, float* action_dev, float* clipped_dev,
                            float* logp_dev, int32_t use_tensor_cores, void* stream) {
-    if (!a || !action_dev) return afail(TACO_E_INVALID, "taco_actor_act: null argument");
-    if (!log_std_host && !a->samp_set) return afail(TACO_E_INVALID, "taco_actor_act: no log_std given and taco_actor_set_log_std was never called");
+    if (!a || !action_dev) return fail(TACO_E_INVALID, "taco_actor_act: null argument");
+    if (!log_std_host && !a->samp_set) return fail(TACO_E_INVALID, "taco_actor_act: no log_std given and taco_actor_set_log_std was never called");
     DevGuard guard(a->device);
     if (log_std_host) {
         const int rc = actor_set_log_std(a, log_std_host, (cudaStream_t)stream);
@@ -452,7 +385,7 @@ int taco_actor_act_counter(TacoActor* a, const float* obs_dev, int32_t n, const 
 }
 
 int taco_actor_set_log_std(TacoActor* a, const float* log_std_host, void* stream) {
-    if (!a || !log_std_host) return afail(TACO_E_INVALID, "taco_actor_set_log_std: null argument");
+    if (!a || !log_std_host) return fail(TACO_E_INVALID, "taco_actor_set_log_std: null argument");
     DevGuard guard(a->device);
     return actor_set_log_std(a, log_std_host, (cudaStream_t)stream);
 }

@@ -18,33 +18,14 @@
 #include <string>
 #include <vector>
 
-#include "../../include/taco_b200.h"
+#include "host_common.h"
 #include "critic_tc.cuh"
 
 namespace taco {
-int fail(int code, const std::string& msg);      // taco_env.cu
 namespace critic {
-
-static int cfail(int code, const std::string& msg) { return taco::fail(code, msg); }
-
-#define CRT_CUDA(expr)                                                                            \
-    do {                                                                                          \
-        cudaError_t _e = (expr);                                                                  \
-        if (_e != cudaSuccess)                                                                    \
-            return cfail(TACO_E_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));        \
-    } while (0)
-
-struct DevGuard {
-    int prev = -1;
-    explicit DevGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
-    ~DevGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
 
 constexpr int kMaxLstmLayers = 4;
 constexpr int kMaxMlpLayers = 8;     // linear layers of the FP32 path
-constexpr int kFpEnvs = 32;          // envs per CTA of the FP32 kernel (one warp lane per env)
-constexpr int kFpThreads = 128;
-constexpr int kFpTile = 8;           // output neurons per warp pass of the FP32 kernel's MLP part
 
 struct FpParams {
     const float* states; float* value;
@@ -197,6 +178,8 @@ __global__ void __launch_bounds__(kFpThreads) critic_fp32_kernel(const FpParams 
 }  // namespace taco
 
 using namespace taco::critic;
+using taco::DevGuard;
+using taco::fail;
 
 struct TacoCritic {
     int device = 0;
@@ -204,18 +187,13 @@ struct TacoCritic {
     std::vector<int> mlp_sizes;          // [hidden, h1, ..., 1]
     int n_mlp = 0;
     std::vector<size_t> lstm_off;        // per layer: float offsets of w_ih, w_hh, b_ih, b_hh (4 per layer)
-    std::vector<size_t> w_off, b_off;
     float* lstm_f32 = nullptr;
-    float* w_f32 = nullptr;
-    float* b_f32 = nullptr;
+    MlpF32 f32;
     bool loaded = false;
     int fp_smem = 0, fp_stride = 0, off_lstm = 0, off_mlp = 0, mlp_w = 0;
     bool tc_ok = false;
     std::string tc_why;
-    uint8_t* wimg = nullptr;
-    float* bias_pad = nullptr;           // [kMaxHidden][kMaxN]
-    float* b_out = nullptr;              // [kOutPad]
-    taco::actor::TcLayer tc_layer[2 + kMaxMlpHidden];
+    TcImage tc;                          // layer[0] / bias row 0: the LSTM step (its image in front of the MLP's), MLP from 1 on
     int num_sms = 148;
 };
 
@@ -225,22 +203,22 @@ int taco_critic_destroy(TacoCritic* c);
 
 int taco_critic_create(int device, int32_t in_dim, int32_t seq_len, int32_t lstm_hidden, int32_t lstm_layers, const int32_t* mlp_sizes,
                        int32_t n_mlp_sizes, TacoCritic** out) {
-    if (!mlp_sizes || !out) return cfail(TACO_E_INVALID, "taco_critic_create: null argument");
+    if (!mlp_sizes || !out) return fail(TACO_E_INVALID, "taco_critic_create: null argument");
     *out = nullptr;
-    if (in_dim < 1 || in_dim > 256 || seq_len < 1 || seq_len > 64) return cfail(TACO_E_INVALID, "taco_critic_create: in_dim must be in [1, 256], seq_len in [1, 64]");
+    if (in_dim < 1 || in_dim > 256 || seq_len < 1 || seq_len > 64) return fail(TACO_E_INVALID, "taco_critic_create: in_dim must be in [1, 256], seq_len in [1, 64]");
     if (lstm_hidden < 1 || lstm_hidden > 256 || lstm_layers < 1 || lstm_layers > kMaxLstmLayers)
-        return cfail(TACO_E_INVALID, "taco_critic_create: lstm_hidden must be in [1, 256], lstm_layers in [1, 4]");
-    if (n_mlp_sizes < 2 || n_mlp_sizes > kMaxMlpLayers + 1) return cfail(TACO_E_INVALID, "taco_critic_create: need 2..9 MLP sizes [lstm_hidden, h1, ..., 1]");
-    if (mlp_sizes[0] != lstm_hidden) return cfail(TACO_E_INVALID, "taco_critic_create: mlp_sizes[0] must equal lstm_hidden (the encoder output feeds the MLP)");
-    if (mlp_sizes[n_mlp_sizes - 1] != 1) return cfail(TACO_E_INVALID, "taco_critic_create: the critic output width is 1");
+        return fail(TACO_E_INVALID, "taco_critic_create: lstm_hidden must be in [1, 256], lstm_layers in [1, 4]");
+    if (n_mlp_sizes < 2 || n_mlp_sizes > kMaxMlpLayers + 1) return fail(TACO_E_INVALID, "taco_critic_create: need 2..9 MLP sizes [lstm_hidden, h1, ..., 1]");
+    if (mlp_sizes[0] != lstm_hidden) return fail(TACO_E_INVALID, "taco_critic_create: mlp_sizes[0] must equal lstm_hidden (the encoder output feeds the MLP)");
+    if (mlp_sizes[n_mlp_sizes - 1] != 1) return fail(TACO_E_INVALID, "taco_critic_create: the critic output width is 1");
     for (int i = 0; i < n_mlp_sizes; ++i)
-        if (mlp_sizes[i] < 1 || mlp_sizes[i] > 512) return cfail(TACO_E_INVALID, "taco_critic_create: layer sizes must be in [1, 512]");
+        if (mlp_sizes[i] < 1 || mlp_sizes[i] > 512) return fail(TACO_E_INVALID, "taco_critic_create: layer sizes must be in [1, 512]");
     int ndev = 0;
-    CRT_CUDA(cudaGetDeviceCount(&ndev));
-    if (device < 0 || device >= ndev) return cfail(TACO_E_INVALID, "taco_critic_create: no such CUDA device");
+    TACO_CUDA(cudaGetDeviceCount(&ndev));
+    if (device < 0 || device >= ndev) return fail(TACO_E_INVALID, "taco_critic_create: no such CUDA device");
     DevGuard guard(device);
     TacoCritic* c = new (std::nothrow) TacoCritic();
-    if (!c) return cfail(TACO_E_NOMEM, "host allocation failed");
+    if (!c) return fail(TACO_E_NOMEM, "host allocation failed");
     c->device = device; c->in_dim = in_dim; c->seq_len = seq_len; c->hidden = lstm_hidden; c->lstm_layers = lstm_layers;
     c->mlp_sizes.assign(mlp_sizes, mlp_sizes + n_mlp_sizes);
     c->n_mlp = n_mlp_sizes - 1;
@@ -251,13 +229,7 @@ int taco_critic_create(int device, int32_t in_dim, int32_t seq_len, int32_t lstm
         const size_t sz[4] = {(size_t)4 * H * in_l, (size_t)4 * H * H, (size_t)4 * H, (size_t)4 * H};
         for (int q = 0; q < 4; ++q) { c->lstm_off.push_back(lo); lo += (sz[q] + 3) & ~(size_t)3; }
     }
-    size_t wo = 0, bo = 0;
     int mx = 0;
-    for (int l = 0; l < c->n_mlp; ++l) {
-        c->w_off.push_back(wo); c->b_off.push_back(bo);
-        wo += ((size_t)mlp_sizes[l] * mlp_sizes[l + 1] + 3) & ~(size_t)3;
-        bo += (size_t)((mlp_sizes[l + 1] + 3) & ~3);
-    }
     for (int i = 0; i < n_mlp_sizes; ++i) mx = mlp_sizes[i] > mx ? mlp_sizes[i] : mx;
     c->off_lstm = seq_len * in_dim;
     c->off_mlp = c->off_lstm + lstm_layers * 3 * H;
@@ -268,7 +240,7 @@ int taco_critic_create(int device, int32_t in_dim, int32_t seq_len, int32_t lstm
     cudaError_t ce = cudaGetDeviceProperties(&prop, device);
     if (ce == cudaSuccess && (size_t)c->fp_smem > prop.sharedMemPerBlockOptin) {
         delete c;
-        return cfail(TACO_E_INVALID, "taco_critic_create: shape needs more shared memory per CTA than the device has");
+        return fail(TACO_E_INVALID, "taco_critic_create: shape needs more shared memory per CTA than the device has");
     }
     c->num_sms = prop.multiProcessorCount;
     // ---- is the shape eligible for the tcgen05 path?
@@ -280,27 +252,13 @@ int taco_critic_create(int device, int32_t in_dim, int32_t seq_len, int32_t lstm
     else if (in_dim > kTcMaxIn || (in_dim & 1)) { c->tc_ok = false; c->tc_why = "input width must be even, <= 30"; }
     else if (seq_len > kMaxSeq) { c->tc_ok = false; c->tc_why = "sequence length > 8"; }
     else if (n_hidden < 1 || n_hidden > kMaxMlpHidden) { c->tc_ok = false; c->tc_why = "needs 1..3 MLP hidden layers"; }
-    else {
-        for (int l = 1; l <= n_hidden; ++l)
-            if (mlp_sizes[l] % 64 != 0 || mlp_sizes[l] > taco::actor::kMaxN) { c->tc_ok = false; c->tc_why = "MLP hidden widths must be multiples of 64, <= 256"; }
-    }
+    else if (!tc_hidden_widths_ok(mlp_sizes, n_hidden)) { c->tc_ok = false; c->tc_why = "MLP hidden widths must be multiples of 64, <= 256"; }
     if (ce == cudaSuccess) ce = cudaMalloc(&c->lstm_f32, lo * sizeof(float));
-    if (ce == cudaSuccess) ce = cudaMalloc(&c->w_f32, wo * sizeof(float));
-    if (ce == cudaSuccess) ce = cudaMalloc(&c->b_f32, bo * sizeof(float));
+    if (ce == cudaSuccess) ce = mlp_f32_alloc(c->f32, mlp_sizes, c->n_mlp);
     if (ce == cudaSuccess && c->tc_ok) {
-        size_t img = 0;
-        // [0] the LSTM step: n = 4H gate rows, K = [h (64) | x (64)] = 2 chunks
-        c->tc_layer[0].n = 4 * H; c->tc_layer[0].kchunks = 2; c->tc_layer[0].img_off = 0;
-        img += (size_t)2 * 4 * H * 128;
-        for (int l = 0; l <= n_hidden; ++l) {          // MLP linear layer l: hidden layers, then the 16-row padded output layer
-            const int k = mlp_sizes[l], nn = l < n_hidden ? mlp_sizes[l + 1] : taco::actor::kOutN;
-            const int kch = (k + taco::actor::kKC - 1) / taco::actor::kKC;
-            c->tc_layer[1 + l].n = nn; c->tc_layer[1 + l].kchunks = kch; c->tc_layer[1 + l].img_off = (uint32_t)img;
-            img += (size_t)kch * nn * 128;
-        }
-        ce = cudaMalloc(&c->wimg, img);
-        if (ce == cudaSuccess) ce = cudaMalloc(&c->bias_pad, taco::actor::kMaxHidden * taco::actor::kMaxN * sizeof(float));
-        if (ce == cudaSuccess) ce = cudaMalloc(&c->b_out, taco::actor::kOutPad * sizeof(float));
+        // [0] the LSTM step: n = 4H gate rows, K = [h (64) | x (64)] = 2 chunks, in front of the MLP's images
+        c->tc.layer[0].n = 4 * H; c->tc.layer[0].kchunks = 2; c->tc.layer[0].img_off = 0;
+        ce = tc_image_alloc(c->tc, mlp_sizes, n_hidden, 1, (size_t)2 * 4 * H * 128);
         if (ce == cudaSuccess) ce = cudaFuncSetAttribute(critic_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCriticSmemBytes);
     }
     if (ce == cudaSuccess && c->fp_smem > 48 * 1024)
@@ -308,7 +266,7 @@ int taco_critic_create(int device, int32_t in_dim, int32_t seq_len, int32_t lstm
     if (ce != cudaSuccess) {
         const std::string msg = std::string("taco_critic_create: ") + cudaGetErrorString(ce);
         taco_critic_destroy(c);
-        return cfail(ce == cudaErrorMemoryAllocation ? TACO_E_NOMEM : TACO_E_CUDA, msg);
+        return fail(ce == cudaErrorMemoryAllocation ? TACO_E_NOMEM : TACO_E_CUDA, msg);
     }
     *out = c;
     return TACO_OK;
@@ -317,19 +275,19 @@ int taco_critic_create(int device, int32_t in_dim, int32_t seq_len, int32_t lstm
 int taco_critic_destroy(TacoCritic* c) {
     if (!c) return TACO_OK;
     DevGuard guard(c->device);
-    cudaFree(c->lstm_f32); cudaFree(c->w_f32); cudaFree(c->b_f32);
-    cudaFree(c->wimg); cudaFree(c->bias_pad); cudaFree(c->b_out);
+    cudaFree(c->lstm_f32); mlp_f32_free(c->f32);
+    tc_image_free(c->tc);
     delete c;
     return TACO_OK;
 }
 
 int taco_critic_load(TacoCritic* c, const float* const* lstm_host, const float* const* mlp_weights_host, const float* const* mlp_biases_host,
                      void* stream) {
-    if (!c || !lstm_host || !mlp_weights_host || !mlp_biases_host) return cfail(TACO_E_INVALID, "taco_critic_load: null argument");
+    if (!c || !lstm_host || !mlp_weights_host || !mlp_biases_host) return fail(TACO_E_INVALID, "taco_critic_load: null argument");
     for (int i = 0; i < 4 * c->lstm_layers; ++i)
-        if (!lstm_host[i]) return cfail(TACO_E_INVALID, "taco_critic_load: null LSTM parameter pointer");
+        if (!lstm_host[i]) return fail(TACO_E_INVALID, "taco_critic_load: null LSTM parameter pointer");
     for (int l = 0; l < c->n_mlp; ++l)
-        if (!mlp_weights_host[l] || !mlp_biases_host[l]) return cfail(TACO_E_INVALID, "taco_critic_load: null MLP layer pointer");
+        if (!mlp_weights_host[l] || !mlp_biases_host[l]) return fail(TACO_E_INVALID, "taco_critic_load: null MLP layer pointer");
     DevGuard guard(c->device);
     cudaStream_t s = (cudaStream_t)stream;
     const int H = c->hidden;
@@ -337,30 +295,16 @@ int taco_critic_load(TacoCritic* c, const float* const* lstm_host, const float* 
         const int in_l = l == 0 ? c->in_dim : H;
         const size_t sz[4] = {(size_t)4 * H * in_l, (size_t)4 * H * H, (size_t)4 * H, (size_t)4 * H};
         for (int q = 0; q < 4; ++q)
-            CRT_CUDA(cudaMemcpyAsync(c->lstm_f32 + c->lstm_off[4 * l + q], lstm_host[4 * l + q], sz[q] * sizeof(float), cudaMemcpyDefault, s));
+            TACO_CUDA(cudaMemcpyAsync(c->lstm_f32 + c->lstm_off[4 * l + q], lstm_host[4 * l + q], sz[q] * sizeof(float), cudaMemcpyDefault, s));
     }
-    for (int l = 0; l < c->n_mlp; ++l) {
-        const int in = c->mlp_sizes[l], out = c->mlp_sizes[l + 1];
-        CRT_CUDA(cudaMemcpyAsync(c->w_f32 + c->w_off[l], mlp_weights_host[l], (size_t)in * out * sizeof(float), cudaMemcpyDefault, s));
-        CRT_CUDA(cudaMemcpyAsync(c->b_f32 + c->b_off[l], mlp_biases_host[l], (size_t)out * sizeof(float), cudaMemcpyDefault, s));
-    }
+    if (int rc = mlp_f32_upload(c->f32, mlp_weights_host, mlp_biases_host, c->mlp_sizes.data(), c->n_mlp, s)) return rc;
     if (c->tc_ok) {
-        const int n_hidden = c->n_mlp - 1;
-        CRT_CUDA(cudaMemsetAsync(c->bias_pad, 0, taco::actor::kMaxHidden * taco::actor::kMaxN * sizeof(float), s));
+        TACO_CUDA(cudaMemsetAsync(c->tc.bias, 0, kMaxHidden * kMaxN * sizeof(float), s));
         pack_lstm_kernel<<<64, 256, 0, s>>>(c->lstm_f32 + c->lstm_off[0], c->lstm_f32 + c->lstm_off[1], c->lstm_f32 + c->lstm_off[2],
-                                            c->lstm_f32 + c->lstm_off[3], H, c->in_dim, 4 * H, c->wimg); TACO_LAUNCHED();
-        for (int l = 0; l <= n_hidden; ++l) {
-            const int in = c->mlp_sizes[l], out = c->mlp_sizes[l + 1];
-            taco::actor::pack_weights_kernel<<<64, 256, 0, s>>>(c->w_f32 + c->w_off[l], out, c->tc_layer[1 + l].n, in, c->wimg + c->tc_layer[1 + l].img_off); TACO_LAUNCHED();
-            if (l < n_hidden)
-                CRT_CUDA(cudaMemcpyAsync(c->bias_pad + (size_t)(1 + l) * taco::actor::kMaxN, c->b_f32 + c->b_off[l], (size_t)out * sizeof(float),
-                                         cudaMemcpyDeviceToDevice, s));
-        }
-        CRT_CUDA(cudaMemsetAsync(c->b_out, 0, taco::actor::kOutPad * sizeof(float), s));
-        CRT_CUDA(cudaMemcpyAsync(c->b_out, c->b_f32 + c->b_off[n_hidden], sizeof(float), cudaMemcpyDeviceToDevice, s));
-        CRT_CUDA(cudaGetLastError());
+                                            c->lstm_f32 + c->lstm_off[3], H, c->in_dim, 4 * H, c->tc.wimg); TACO_LAUNCHED();
+        if (int rc = tc_image_pack(c->tc, c->f32, c->mlp_sizes.data(), c->n_mlp - 1, s)) return rc;
     }
-    CRT_CUDA(cudaStreamSynchronize(s));     // the host buffers may be released by the caller on return
+    TACO_CUDA(cudaStreamSynchronize(s));     // the host buffers may be released by the caller on return
     c->loaded = true;
     return TACO_OK;
 }
@@ -368,39 +312,27 @@ int taco_critic_load(TacoCritic* c, const float* const* lstm_host, const float* 
 int taco_critic_tc_available(TacoCritic* c) { return (c && c->tc_ok) ? 1 : 0; }
 
 int taco_critic_forward(TacoCritic* c, const float* states_dev, float* value_dev, int32_t n, int32_t use_tensor_cores, void* stream) {
-    if (!c || !states_dev || !value_dev) return cfail(TACO_E_INVALID, "taco_critic_forward: null argument");
-    if (!c->loaded) return cfail(TACO_E_INVALID, "taco_critic_forward: call taco_critic_load first");
-    if (n <= 0) return cfail(TACO_E_INVALID, "taco_critic_forward: n must be positive");
+    if (!c || !states_dev || !value_dev) return fail(TACO_E_INVALID, "taco_critic_forward: null argument");
+    if (!c->loaded) return fail(TACO_E_INVALID, "taco_critic_forward: call taco_critic_load first");
+    if (n <= 0) return fail(TACO_E_INVALID, "taco_critic_forward: n must be positive");
     DevGuard guard(c->device);
     cudaStream_t s = (cudaStream_t)stream;
     if (use_tensor_cores) {
-        if (!c->tc_ok) return cfail(TACO_E_INVALID, "taco_critic_forward: tensor-core path unavailable for this shape: " + c->tc_why);
+        if (!c->tc_ok) return fail(TACO_E_INVALID, "taco_critic_forward: tensor-core path unavailable for this shape: " + c->tc_why);
         CriticTcParams p;
         memset(&p, 0, sizeof(p));
         p.states = states_dev; p.value = value_dev;
-        p.in_dim = c->in_dim; p.seq_len = c->seq_len; p.n_rows = n; p.num_tiles = (n + taco::actor::kTileM - 1) / taco::actor::kTileM;
+        p.in_dim = c->in_dim; p.seq_len = c->seq_len; p.n_rows = n; p.num_tiles = (n + kTileM - 1) / kTileM;
         p.lstm_hidden = c->hidden; p.n_hidden = c->n_mlp - 1;
-        p.wimg = c->wimg; p.bias = c->bias_pad; p.b_out = c->b_out;
-        for (int l = 0; l <= p.n_hidden + 1; ++l) p.layer[l] = c->tc_layer[l];
-        p.tiles_per_cta = p.num_tiles <= c->num_sms ? 1 : 2;
-        static const int stagger = [] { const char* e = getenv("TACO_CRITIC_STAGGER"); return e ? atoi(e) : taco::critic::kCriticStagger; }();
+        p.wimg = c->tc.wimg; p.bias = c->tc.bias; p.b_out = c->tc.b_out;
+        for (int l = 0; l <= p.n_hidden + 1; ++l) p.layer[l] = c->tc.layer[l];
+        static const int stagger = [] { const char* e = getenv("TACO_CRITIC_STAGGER"); return e ? atoi(e) : kCriticStagger; }();
         p.stagger = stagger;
-        const int num_pairs = (p.num_tiles + p.tiles_per_cta - 1) / p.tiles_per_cta;
-        const int grid = num_pairs < c->num_sms ? num_pairs : c->num_sms;
-        // developer aid: TACO_CRITIC_TIMELINE=<file> records clock64 stamps of CTA 0's MMA issuer / epilogue (synchronous)
+        const int grid = tc_grid(p.num_tiles, c->num_sms, &p.tiles_per_cta);
         const char* tl = getenv("TACO_CRITIC_TIMELINE");
-        if (tl && *tl) {
-            CRT_CUDA(cudaMalloc(&p.dbg, 3 * taco::actor::kDbgCap * sizeof(unsigned long long)));
-            CRT_CUDA(cudaMemsetAsync(p.dbg, 0, 3 * taco::actor::kDbgCap * sizeof(unsigned long long), s));
-        }
-        critic_tc_kernel<<<grid, taco::actor::kTcThreads, kCriticSmemBytes, s>>>(p); TACO_LAUNCHED();
-        if (p.dbg) {
-            std::vector<unsigned long long> h(3 * taco::actor::kDbgCap);
-            CRT_CUDA(cudaStreamSynchronize(s));
-            CRT_CUDA(cudaMemcpy(h.data(), p.dbg, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-            cudaFree(p.dbg);
-            if (FILE* f = fopen(tl, "wb")) { fwrite(h.data(), sizeof(unsigned long long), h.size(), f); fclose(f); }
-        }
+        if (int rc = timeline_begin(tl, &p.dbg, s)) return rc;
+        critic_tc_kernel<<<grid, kTcThreads, kCriticSmemBytes, s>>>(p); TACO_LAUNCHED();
+        if (int rc = timeline_end(tl, p.dbg, s)) return rc;
     } else {
         FpParams p;
         memset(&p, 0, sizeof(p));
@@ -411,11 +343,11 @@ int taco_critic_forward(TacoCritic* c, const float* states_dev, float* value_dev
             p.b_ih[l] = c->lstm_f32 + c->lstm_off[4 * l + 2]; p.b_hh[l] = c->lstm_f32 + c->lstm_off[4 * l + 3];
         }
         for (int l = 0; l <= c->n_mlp; ++l) p.mlp_sizes[l] = c->mlp_sizes[l];
-        for (int l = 0; l < c->n_mlp; ++l) { p.w[l] = c->w_f32 + c->w_off[l]; p.b[l] = c->b_f32 + c->b_off[l]; }
+        for (int l = 0; l < c->n_mlp; ++l) { p.w[l] = c->f32.w + c->f32.w_off[l]; p.b[l] = c->f32.b + c->f32.b_off[l]; }
         p.stride = c->fp_stride; p.off_lstm = c->off_lstm; p.off_mlp = c->off_mlp; p.mlp_w = c->mlp_w;
         critic_fp32_kernel<<<(n + kFpEnvs - 1) / kFpEnvs, kFpThreads, c->fp_smem, s>>>(p); TACO_LAUNCHED();
     }
-    CRT_CUDA(cudaGetLastError());
+    TACO_CUDA(cudaGetLastError());
     return TACO_OK;
 }
 

@@ -13,7 +13,7 @@
 #include <string>
 #include <vector>
 
-#include "../../include/taco_b200.h"
+#include "host_common.h"
 #include "philox.cuh"
 #include "fpv_math.cuh"
 #include "step_params.h"
@@ -23,18 +23,6 @@ namespace taco {
 std::atomic<unsigned long long> g_launches{0};
 static thread_local std::string g_err;
 int fail(int code, const std::string& msg) { g_err = msg; return code; }
-#define TACO_CUDA(expr)                                                                          \
-    do {                                                                                         \
-        cudaError_t _e = (expr);                                                                 \
-        if (_e != cudaSuccess)                                                                   \
-            return fail(TACO_E_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));        \
-    } while (0)
-
-struct DeviceGuard {
-    int prev = -1;
-    explicit DeviceGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
-    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
 
 }  // namespace taco
 
@@ -282,7 +270,7 @@ const char* taco_last_error(void) { return g_err.c_str(); }
 
 int taco_selftest_divc(int device, float dt, uint64_t* n_mismatch) {
     if (!n_mismatch) return fail(TACO_E_INVALID, "taco_selftest_divc: null argument");
-    DeviceGuard guard(device);
+    DevGuard guard(device);
     unsigned long long* d = nullptr;
     TACO_CUDA(cudaMalloc(&d, 2 * sizeof(unsigned long long) + 64 * sizeof(uint32_t)));
     TACO_CUDA(cudaMemset(d, 0, 2 * sizeof(unsigned long long) + 64 * sizeof(uint32_t)));
@@ -302,7 +290,7 @@ int taco_selftest_divc(int device, float dt, uint64_t* n_mismatch) {
 }
 int taco_selftest_atan2(int device, uint32_t n_angles, float* max_ulp, uint32_t* n_nonfinite) {
     if (!max_ulp || !n_nonfinite || n_angles == 0) return fail(TACO_E_INVALID, "taco_selftest_atan2: null / empty argument");
-    DeviceGuard guard(device);
+    DevGuard guard(device);
     uint32_t* d = nullptr;
     TACO_CUDA(cudaMalloc(&d, 2 * sizeof(uint32_t)));
     TACO_CUDA(cudaMemset(d, 0, 2 * sizeof(uint32_t)));
@@ -343,7 +331,7 @@ int taco_env_create(const TacoCfg* cfg, int device, TacoEnv** out) {
     int ndev = 0;
     TACO_CUDA(cudaGetDeviceCount(&ndev));
     if (device < 0 || device >= ndev) return fail(TACO_E_INVALID, "no such CUDA device");
-    DeviceGuard guard(device);
+    DevGuard guard(device);
 
     TacoEnv* e = new (std::nothrow) TacoEnv();
     if (!e) return fail(TACO_E_NOMEM, "host allocation failed");
@@ -423,7 +411,7 @@ int taco_env_create(const TacoCfg* cfg, int device, TacoEnv** out) {
 
 int taco_env_destroy(TacoEnv* env) {
     if (!env) return TACO_OK;
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     if (env->pipe_ready) {
         cudaStreamDestroy(env->s_h2d); cudaStreamDestroy(env->s_d2h);
         for (int k = 0; k < TacoEnv::kKernelStreams; ++k) cudaStreamDestroy(env->s_k[k]);
@@ -493,7 +481,7 @@ __global__ void step_counter_kernel(uint32_t* c, uint32_t value, int add) { *c =
 int taco_env_step(TacoEnv* env, const float* actions_dev, void* stream) {
     if (!env || !actions_dev) return fail(TACO_E_INVALID, "taco_env_step: null argument");
     if (((uintptr_t)actions_dev & 15u) != 0) return fail(TACO_E_INVALID, "actions must be 16-byte aligned (contiguous (N,4) float32)");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     StepParams& p = env->p;
     const int rc = bind_history(env);
     if (rc != TACO_OK) return rc;
@@ -540,7 +528,7 @@ static int pipe_init(TacoEnv* env) {
 int taco_env_step_host_compact(TacoEnv* env, const float* actions_host, float* rew_host, uint8_t* flags_host, void* stream) {
     if (!env || !actions_host || !flags_host) return fail(TACO_E_INVALID, "taco_env_step_host_compact: null argument");
     if (((uintptr_t)actions_host & 15u) != 0) return fail(TACO_E_INVALID, "taco_env_step_host_compact: actions must be 16-byte aligned");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     void* d_act = mapped_ptr(actions_host);
     void* d_rew = mapped_ptr(rew_host);
@@ -565,7 +553,7 @@ int taco_env_step_host_compact(TacoEnv* env, const float* actions_host, float* r
 int taco_env_step_host(TacoEnv* env, const float* actions_host, float* rew_host, int64_t* reset_host, uint8_t* time_outs_host,
                        void* stream) {
     if (!env || !actions_host) return fail(TACO_E_INVALID, "taco_env_step_host: null argument");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     int rc = pipe_init(env);
     if (rc != TACO_OK) return rc;
@@ -654,7 +642,7 @@ int taco_env_step_host(TacoEnv* env, const float* actions_host, float* rew_host,
 
 int taco_env_graph_begin(TacoEnv* env, void* stream) {
     if (!env) return fail(TACO_E_INVALID, "taco_env_graph_begin: null argument");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     if (!env->step_counter) TACO_CUDA(cudaMalloc(&env->step_counter, sizeof(uint32_t)));
     step_counter_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(env->step_counter, env->step_index, 0); TACO_LAUNCHED();
     TACO_CUDA(cudaGetLastError());
@@ -666,7 +654,7 @@ int taco_env_graph_begin(TacoEnv* env, void* stream) {
 
 int taco_env_graph_advance(TacoEnv* env, uint32_t steps, void* stream) {
     if (!env || !env->graph_mode) return fail(TACO_E_INVALID, "taco_env_graph_advance: call taco_env_graph_begin first");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     step_counter_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(env->step_counter, steps, 1); TACO_LAUNCHED();
     TACO_CUDA(cudaGetLastError());
     return TACO_OK;
@@ -675,7 +663,7 @@ int taco_env_graph_advance(TacoEnv* env, uint32_t steps, void* stream) {
 int taco_env_graph_end(TacoEnv* env, void* stream) {
     if (!env) return fail(TACO_E_INVALID, "taco_env_graph_end: null argument");
     if (!env->graph_mode) return TACO_OK;
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     uint32_t v = 0;
     TACO_CUDA(cudaMemcpyAsync(&v, env->step_counter, sizeof(v), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
     TACO_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
@@ -700,7 +688,7 @@ int taco_env_attach_rollout(TacoEnv* env, float* obs_ring, float* states_ring, i
         return fail(TACO_E_INVALID, "taco_env_attach_rollout: rew / done / time-out rows must be given together (or all NULL)");
     if (((uintptr_t)obs_ring | (uintptr_t)states_ring) & 7u) return fail(TACO_E_INVALID, "taco_env_attach_rollout: rings must be 8-byte aligned");
     if (env->ring_slots) return fail(TACO_E_INVALID, "taco_env_attach_rollout: a ring is already attached");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     // the newest observation / state history moves into slot 0
     TACO_CUDA(cudaMemcpyAsync(obs_ring, env->obs_ab[env->cur], (size_t)env->n * env->cfg.len_obs * kObs * sizeof(float), cudaMemcpyDeviceToDevice, s));
@@ -714,7 +702,7 @@ int taco_env_attach_rollout(TacoEnv* env, float* obs_ring, float* states_ring, i
 int taco_env_rewind_rollout(TacoEnv* env, void* stream) {
     if (!env) return fail(TACO_E_INVALID, "taco_env_rewind_rollout: null argument");
     if (!env->ring_slots) return fail(TACO_E_INVALID, "taco_env_rewind_rollout: no ring attached");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     if (env->ring_cur > 0) {
         const size_t so = (size_t)env->n * env->cfg.len_obs * kObs, ss = (size_t)env->n * env->cfg.len_states * kObs;
@@ -728,7 +716,7 @@ int taco_env_rewind_rollout(TacoEnv* env, void* stream) {
 int taco_env_detach_rollout(TacoEnv* env, void* stream) {
     if (!env) return fail(TACO_E_INVALID, "taco_env_detach_rollout: null argument");
     if (!env->ring_slots) return TACO_OK;
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t so = (size_t)env->n * env->cfg.len_obs * kObs, ss = (size_t)env->n * env->cfg.len_states * kObs;
     TACO_CUDA(cudaMemcpyAsync(env->obs_ab[env->cur], env->ring_obs + so * env->ring_cur, so * sizeof(float), cudaMemcpyDeviceToDevice, s));
@@ -742,7 +730,7 @@ int taco_env_rollout_cursor(TacoEnv* env) { return (env && env->ring_slots) ? en
 
 int taco_env_reset_all(TacoEnv* env, void* stream) {
     if (!env) return fail(TACO_E_INVALID, "taco_env_reset_all: null argument");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t np = (size_t)env->n_pad;
     for (int k = 0; k < 2; ++k) {
@@ -767,7 +755,7 @@ int taco_env_set_difficulty(TacoEnv* env, float difficulty) {
     if (!env) return fail(TACO_E_INVALID, "taco_env_set_difficulty: null argument");
     env->cfg.difficulty = difficulty;
     refresh_derived(env);
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     TACO_CUDA(upload_derived(env));       // captured launches (graph mode) read the device copy
     return TACO_OK;
 }
@@ -787,7 +775,7 @@ int taco_env_set_seed(TacoEnv* env, uint64_t seed) {
 
 int taco_env_stats(TacoEnv* env, double* out_dev, double* out_host, void* stream) {
     if (!env) return fail(TACO_E_INVALID, "taco_env_stats: null argument");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     double* dst = out_dev ? out_dev : env->stats_out;
     reduce_stats_kernel<<<1, 32, 0, s>>>(env->p.stats, dst); TACO_LAUNCHED();
@@ -801,7 +789,7 @@ int taco_env_stats(TacoEnv* env, double* out_dev, double* out_host, void* stream
 
 int taco_env_fill_random_actions(TacoEnv* env, float* actions_dev, uint32_t step_index, void* stream) {
     if (!env || !actions_dev) return fail(TACO_E_INVALID, "taco_env_fill_random_actions: null argument");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     fill_actions_kernel<<<(env->n + 255) / 256, 256, 0, (cudaStream_t)stream>>>((float4*)actions_dev, env->n, env->p.env_offset, step_index,
                                                                                env->p.seed_lo, env->p.seed_hi); TACO_LAUNCHED();
     TACO_CUDA(cudaGetLastError());
@@ -810,7 +798,7 @@ int taco_env_fill_random_actions(TacoEnv* env, float* actions_dev, uint32_t step
 
 int taco_env_export_state(TacoEnv* env, float* out_host) {
     if (!env || !out_host) return fail(TACO_E_INVALID, "taco_env_export_state: null argument");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     const size_t bytes = (size_t)env->n * TACO_STATE_WORDS * sizeof(float);
     if (!env->export_stage) TACO_CUDA(cudaMalloc(&env->export_stage, bytes));
     TACO_CUDA(cudaDeviceSynchronize());
@@ -822,7 +810,7 @@ int taco_env_export_state(TacoEnv* env, float* out_host) {
 
 int taco_env_import_state(TacoEnv* env, const float* in_host) {
     if (!env || !in_host) return fail(TACO_E_INVALID, "taco_env_import_state: null argument");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     const size_t bytes = (size_t)env->n * TACO_STATE_WORDS * sizeof(float);
     if (!env->export_stage) TACO_CUDA(cudaMalloc(&env->export_stage, bytes));
     TACO_CUDA(cudaDeviceSynchronize());
@@ -854,7 +842,7 @@ int taco_env_checkpoint_save(TacoEnv* env, void* out_host, uint64_t bytes) {
     if (!env || !out_host) return fail(TACO_E_INVALID, "taco_env_checkpoint_save: null argument");
     if (bytes != sizeof(CkptHeader) + env->arena_bytes) return fail(TACO_E_INVALID, "taco_env_checkpoint_save: wrong buffer size (taco_env_checkpoint_size)");
     if (env->ring_slots || env->graph_mode) return fail(TACO_E_INVALID, "taco_env_checkpoint_save: detach the rollout ring / leave graph mode first");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     CkptHeader h;
     memset(&h, 0, sizeof(h));
     memcpy(h.magic, "TACOENV1", 8);
@@ -877,7 +865,7 @@ int taco_env_checkpoint_load(TacoEnv* env, const void* in_host, uint64_t bytes) 
     TacoCfg a = h.cfg, b = env->cfg;
     a.difficulty = b.difficulty = 0.f; a.seed = b.seed = 0;
     if (memcmp(&a, &b, sizeof(TacoCfg)) != 0) return fail(TACO_E_INVALID, "taco_env_checkpoint_load: the checkpoint was written by an env with another configuration");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     TACO_CUDA(cudaDeviceSynchronize());
     TACO_CUDA(cudaMemcpy(env->arena, (const char*)in_host + sizeof(h), env->arena_bytes, cudaMemcpyHostToDevice));
     env->step_index = h.step_index; env->cur = h.cur;
@@ -891,7 +879,7 @@ int taco_env_checkpoint_load(TacoEnv* env, const void* in_host, uint64_t bytes) 
 int taco_env_debug_delay(TacoEnv* env, float* out_host) {
     if (!env || !out_host) return fail(TACO_E_INVALID, "taco_env_debug_delay: null argument");
     if (!env->dbg_delay) return fail(TACO_E_INVALID, "env was not created with TACO_F_DEBUG_DELAY");
-    DeviceGuard guard(env->device);
+    DevGuard guard(env->device);
     TACO_CUDA(cudaDeviceSynchronize());
     // device layout [cfi][n_pad] float4 -> host (n, cfi, 4)
     const int cfi = env->cfg.control_freq_inv;

@@ -17,10 +17,9 @@
 
 #include <cuda_runtime.h>
 
-#include "../../include/taco_b200.h"
+#include "host_common.h"
 
 namespace taco {
-int fail(int code, const std::string& msg);      // taco_env.cu
 namespace gae {
 
 constexpr int kThreads = 128;
@@ -79,16 +78,11 @@ __global__ void gae_normalize_kernel(float* __restrict__ adv, long long count, c
         adv[k] = (adv[k] - mean32) / den;
 }
 
-struct DevGuard {
-    int prev = -1;
-    explicit DevGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
-    ~DevGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
-
 }  // namespace gae
 }  // namespace taco
 
 using namespace taco::gae;
+using taco::DevGuard;
 
 extern "C" {
 

@@ -27,27 +27,14 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 
-#include "../../include/taco_b200.h"
+#include "host_common.h"
 #include "gemm_tc.cuh"
 
 namespace taco {
-int fail(int code, const std::string& msg);      // taco_env.cu
 namespace ppo {
 
 using namespace taco::gemm;
 typedef __nv_bfloat16 bf16;
-
-#define PPO_CUDA(expr)                                                                               \
-    do {                                                                                             \
-        cudaError_t _e = (expr);                                                                     \
-        if (_e != cudaSuccess) return ::taco::fail(TACO_E_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e)); \
-    } while (0)
-
-struct DevGuard {
-    int prev = -1;
-    explicit DevGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
-    ~DevGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
 
 constexpr int kMaxHiddenL = 4;
 constexpr int kH = 64;              // LSTM hidden width the LSTM epilogue is written for
@@ -511,6 +498,8 @@ __global__ void __launch_bounds__(256) pack_lstm_kernel(const float* w_ih, const
 }  // namespace taco
 
 using namespace taco::ppo;
+using taco::DevGuard;
+using taco::fail;
 
 // ---------------------------------------------------------------------------------------------- the trainer object
 struct MlpNet {
@@ -557,7 +546,6 @@ struct TacoPPO {
     std::vector<void*> allocs;
 };
 
-static int ppo_fail(int code, const std::string& m) { return taco::fail(code, m); }
 
 template <typename T>
 static cudaError_t dev_alloc(TacoPPO* t, T** p, size_t count) {
@@ -591,7 +579,7 @@ static int launch_gemm(TacoPPO* t, const CUtensorMap& a, const CUtensorMap& b, G
     const int total = ((p.m + BM - 1) / BM) * p.splits;
     const int grid = total < t->num_sms ? total : t->num_sms;
     p.tma_store = c != nullptr;
-    return launch_pdl(gemm_tc_kernel, dim3(grid), dim3(kGemmThreads), kGemmSmem, s, a, b, c ? *c : a, p) == cudaSuccess ? TACO_OK : ppo_fail(TACO_E_CUDA, "gemm_tc_kernel launch failed");
+    return launch_pdl(gemm_tc_kernel, dim3(grid), dim3(kGemmThreads), kGemmSmem, s, a, b, c ? *c : a, p) == cudaSuccess ? TACO_OK : fail(TACO_E_CUDA, "gemm_tc_kernel launch failed");
 }
 
 static int splits_for(int m, long long k, int num_sms) {
@@ -630,7 +618,7 @@ static int setup_net(TacoPPO* t, MlpNet& n, long long& off, bool actor) {
         ok = ok && make_map(&n.m_dz_mn[lz], n.dz_bm[lz], B, n.ld_dz[lz], n.ld_dz[lz], BK);   // A operand of the dW GEMM (MN-major)
         n.partial_tma[l] = out % BM == 0;
         if (n.partial_tma[l]) ok = ok && make_map_f32(&n.m_partial[l], n.partial[l], (long long)n.splits[l] * out, n.ld_p[l], n.ld_p[l]);
-        if (!ok) return ppo_fail(TACO_E_CUDA, "cuTensorMapEncodeTiled failed");
+        if (!ok) return fail(TACO_E_CUDA, "cuTensorMapEncodeTiled failed");
     }
     (void)actor;
     return TACO_OK;
@@ -639,35 +627,35 @@ static int setup_net(TacoPPO* t, MlpNet& n, long long& off, bool actor) {
 extern "C" {
 
 int taco_ppo_create(int device, const TacoPPOCfg* cfg, TacoPPO** out) {
-    if (!cfg || !out) return ppo_fail(TACO_E_INVALID, "taco_ppo_create: null argument");
+    if (!cfg || !out) return fail(TACO_E_INVALID, "taco_ppo_create: null argument");
     *out = nullptr;
-    if (cfg->batch < 128 || cfg->batch % 128) return ppo_fail(TACO_E_INVALID, "taco_ppo_create: the minibatch size must be a positive multiple of 128");
-    if (cfg->lstm_hidden != kH) return ppo_fail(TACO_E_INVALID, "taco_ppo_create: lstm_hidden must be 64");
-    if (cfg->act_dim < 1 || cfg->act_dim > 4) return ppo_fail(TACO_E_INVALID, "taco_ppo_create: act_dim must be in [1, 4]");
+    if (cfg->batch < 128 || cfg->batch % 128) return fail(TACO_E_INVALID, "taco_ppo_create: the minibatch size must be a positive multiple of 128");
+    if (cfg->lstm_hidden != kH) return fail(TACO_E_INVALID, "taco_ppo_create: lstm_hidden must be 64");
+    if (cfg->act_dim < 1 || cfg->act_dim > 4) return fail(TACO_E_INVALID, "taco_ppo_create: act_dim must be in [1, 4]");
     if (cfg->seq_len < 1 || cfg->seq_len > kSeqMax || cfg->state_dim < 1 || kH + cfg->state_dim + 2 > 128 || cfg->obs_dim < 1 || cfg->obs_dim > 256)
-        return ppo_fail(TACO_E_INVALID, "taco_ppo_create: seq_len <= 8, state_dim <= 62, obs_dim <= 256");
+        return fail(TACO_E_INVALID, "taco_ppo_create: seq_len <= 8, state_dim <= 62, obs_dim <= 256");
     if (cfg->n_actor_hidden < 1 || cfg->n_actor_hidden > kMaxHiddenL || cfg->n_critic_hidden < 1 || cfg->n_critic_hidden > kMaxHiddenL)
-        return ppo_fail(TACO_E_INVALID, "taco_ppo_create: 1..4 hidden layers per MLP");
+        return fail(TACO_E_INVALID, "taco_ppo_create: 1..4 hidden layers per MLP");
     for (int l = 0; l < cfg->n_actor_hidden; ++l)
-        if (cfg->actor_hidden[l] < 16 || cfg->actor_hidden[l] > 256 || cfg->actor_hidden[l] % 16) return ppo_fail(TACO_E_INVALID, "taco_ppo_create: hidden widths must be multiples of 16 in [16, 256]");
+        if (cfg->actor_hidden[l] < 16 || cfg->actor_hidden[l] > 256 || cfg->actor_hidden[l] % 16) return fail(TACO_E_INVALID, "taco_ppo_create: hidden widths must be multiples of 16 in [16, 256]");
     for (int l = 0; l < cfg->n_critic_hidden; ++l)
-        if (cfg->critic_hidden[l] < 16 || cfg->critic_hidden[l] > 256 || cfg->critic_hidden[l] % 16) return ppo_fail(TACO_E_INVALID, "taco_ppo_create: hidden widths must be multiples of 16 in [16, 256]");
+        if (cfg->critic_hidden[l] < 16 || cfg->critic_hidden[l] > 256 || cfg->critic_hidden[l] % 16) return fail(TACO_E_INVALID, "taco_ppo_create: hidden widths must be multiples of 16 in [16, 256]");
     int ndev = 0;
-    PPO_CUDA(cudaGetDeviceCount(&ndev));
-    if (device < 0 || device >= ndev) return ppo_fail(TACO_E_INVALID, "taco_ppo_create: no such CUDA device");
+    TACO_CUDA(cudaGetDeviceCount(&ndev));
+    if (device < 0 || device >= ndev) return fail(TACO_E_INVALID, "taco_ppo_create: no such CUDA device");
     DevGuard guard(device);
     cudaDeviceProp prop;
-    PPO_CUDA(cudaGetDeviceProperties(&prop, device));
-    if (prop.major != 10) return ppo_fail(TACO_E_INVALID, "taco_ppo_create: the native update needs an sm_100 device (tcgen05); there is no fallback");
-    if (!encode_fn()) return ppo_fail(TACO_E_CUDA, "taco_ppo_create: cuTensorMapEncodeTiled is not available from the driver");
+    TACO_CUDA(cudaGetDeviceProperties(&prop, device));
+    if (prop.major != 10) return fail(TACO_E_INVALID, "taco_ppo_create: the native update needs an sm_100 device (tcgen05); there is no fallback");
+    if (!encode_fn()) return fail(TACO_E_CUDA, "taco_ppo_create: cuTensorMapEncodeTiled is not available from the driver");
     TacoPPO* t = new (std::nothrow) TacoPPO();
-    if (!t) return ppo_fail(TACO_E_NOMEM, "host allocation failed");
+    if (!t) return fail(TACO_E_NOMEM, "host allocation failed");
     t->device = device; t->cfg = *cfg; t->num_sms = prop.multiProcessorCount;
     t->B = cfg->batch; t->A = cfg->act_dim; t->seq = cfg->seq_len; t->sd = cfg->state_dim;
     t->ld_u = pad8(kH + cfg->state_dim + 2);
     const int B = t->B;
     int rc = TACO_OK;
-    auto bail = [&](int code, const char* msg) { taco_ppo_destroy(t); return ppo_fail(code, msg); };
+    auto bail = [&](int code, const char* msg) { taco_ppo_destroy(t); return fail(code, msg); };
     // ---- flat parameter layout: log_std | actor MLP (W, b per layer) | LSTM W_ih, W_hh, b_ih, b_hh | critic MLP
     long long off = 0;
     t->off_log_std = off; off += t->A;
@@ -753,7 +741,7 @@ int taco_ppo_destroy(TacoPPO* t) {
 }
 
 int taco_ppo_num_params(TacoPPO* t, int64_t* n) {
-    if (!t || !n) return ppo_fail(TACO_E_INVALID, "taco_ppo_num_params: null argument");
+    if (!t || !n) return fail(TACO_E_INVALID, "taco_ppo_num_params: null argument");
     *n = t->n_params;
     return TACO_OK;
 }
@@ -761,13 +749,13 @@ int taco_ppo_num_params(TacoPPO* t, int64_t* n) {
 // offsets of the parameter tensors inside the flat vector, in this order: log_std; actor (W, b) x layers; LSTM weight_ih_l0,
 // weight_hh_l0, bias_ih_l0, bias_hh_l0; critic (W, b) x layers.  `count` = capacity of `offsets`; returns the number written.
 int taco_ppo_param_offsets(TacoPPO* t, int64_t* offsets, int32_t count, int32_t* n_out) {
-    if (!t || !offsets || !n_out) return ppo_fail(TACO_E_INVALID, "taco_ppo_param_offsets: null argument");
+    if (!t || !offsets || !n_out) return fail(TACO_E_INVALID, "taco_ppo_param_offsets: null argument");
     std::vector<int64_t> v;
     v.push_back(t->off_log_std);
     for (int l = 0; l < t->actor.L; ++l) { v.push_back(t->actor.w_off[l]); v.push_back(t->actor.b_off[l]); }
     v.push_back(t->off_wih); v.push_back(t->off_whh); v.push_back(t->off_bih); v.push_back(t->off_bhh);
     for (int l = 0; l < t->critic.L; ++l) { v.push_back(t->critic.w_off[l]); v.push_back(t->critic.b_off[l]); }
-    if ((int)v.size() > count) return ppo_fail(TACO_E_INVALID, "taco_ppo_param_offsets: buffer too small");
+    if ((int)v.size() > count) return fail(TACO_E_INVALID, "taco_ppo_param_offsets: buffer too small");
     for (size_t i = 0; i < v.size(); ++i) offsets[i] = v[i];
     *n_out = (int32_t)v.size();
     return TACO_OK;
@@ -776,7 +764,7 @@ int taco_ppo_param_offsets(TacoPPO* t, int64_t* offsets, int32_t count, int32_t*
 // device addresses of the flat fp32 vectors (each n_params floats): parameters, gradient of the last backward, Adam m, Adam v;
 // and of the int32 optimiser step counter.  Any pointer may be NULL.
 int taco_ppo_buffers(TacoPPO* t, float** params, float** grad, float** adam_m, float** adam_v, int32_t** step) {
-    if (!t) return ppo_fail(TACO_E_INVALID, "taco_ppo_buffers: null argument");
+    if (!t) return fail(TACO_E_INVALID, "taco_ppo_buffers: null argument");
     if (params) *params = t->prm;
     if (grad) *grad = t->grad;
     if (adam_m) *adam_m = t->adam_m;
@@ -788,7 +776,7 @@ int taco_ppo_buffers(TacoPPO* t, float** params, float** grad, float** adam_m, f
 // the caller's stream waits for the actor's projection / re-pack still running on the side stream
 static int join_actor(TacoPPO* t, cudaStream_t s) {
     if (t->actor_pending) {
-        PPO_CUDA(cudaStreamWaitEvent(s, t->ev_actor, 0));
+        TACO_CUDA(cudaStreamWaitEvent(s, t->ev_actor, 0));
         t->actor_pending = false;
     }
     return TACO_OK;
@@ -813,12 +801,12 @@ static int repack(TacoPPO* t, cudaStream_t s, bool honour_stop, int which = 0) {
         launch_pdl(pack_lstm_kernel, dim3(64), dim3(256), 0, s, (const float*)(t->prm + t->off_wih), (const float*)(t->prm + t->off_whh), (const float*)(t->prm + t->off_bih),
                    (const float*)(t->prm + t->off_bhh), t->sd, t->ld_u, t->wcat, t->whh_t, (const int*)(honour_stop ? t->stop : nullptr));
     }
-    return cudaGetLastError() == cudaSuccess ? TACO_OK : ppo_fail(TACO_E_CUDA, "pack kernels failed");
+    return cudaGetLastError() == cudaSuccess ? TACO_OK : fail(TACO_E_CUDA, "pack kernels failed");
 }
 
 // call after writing the parameter vector (taco_ppo_buffers) from outside: refreshes the bf16 operand copies
 int taco_ppo_params_changed(TacoPPO* t, void* stream) {
-    if (!t) return ppo_fail(TACO_E_INVALID, "taco_ppo_params_changed: null argument");
+    if (!t) return fail(TACO_E_INVALID, "taco_ppo_params_changed: null argument");
     DevGuard guard(t->device);
     const int rcj = join_actor(t, (cudaStream_t)stream);
     if (rcj != TACO_OK) return rcj;
@@ -827,12 +815,12 @@ int taco_ppo_params_changed(TacoPPO* t, void* stream) {
 
 // start of one PPO.update: clears the early-stop flag and the log
 int taco_ppo_begin_update(TacoPPO* t, void* stream) {
-    if (!t) return ppo_fail(TACO_E_INVALID, "taco_ppo_begin_update: null argument");
+    if (!t) return fail(TACO_E_INVALID, "taco_ppo_begin_update: null argument");
     DevGuard guard(t->device);
     cudaStream_t s = (cudaStream_t)stream;
-    PPO_CUDA(cudaMemsetAsync(t->stop, 0, sizeof(int), s));
-    PPO_CUDA(cudaMemsetAsync(t->n_logged, 0, sizeof(int), s));
-    PPO_CUDA(cudaMemsetAsync(t->acc, 0, kNumStat * sizeof(double), s));
+    TACO_CUDA(cudaMemsetAsync(t->stop, 0, sizeof(int), s));
+    TACO_CUDA(cudaMemsetAsync(t->n_logged, 0, sizeof(int), s));
+    TACO_CUDA(cudaMemsetAsync(t->acc, 0, kNumStat * sizeof(double), s));
     return TACO_OK;
 }
 
@@ -897,7 +885,7 @@ static int mlp_backward(TacoPPO* t, MlpNet& n, float* dx_out, cudaStream_t s) {
 // phase 1: gather + forward + loss.  The rollout tensors are flat views [N_total][...] on the device; idx_dev = B int64 row indices.
 int taco_ppo_forward_loss(TacoPPO* t, const TacoPPOHyper* hyper, const float* obs, const float* states, const float* act, const float* old_logp,
                           const float* adv, const float* ret, const int64_t* idx_dev, void* stream) {
-    if (!t || !hyper || !obs || !states || !act || !old_logp || !adv || !ret || !idx_dev) return ppo_fail(TACO_E_INVALID, "taco_ppo_forward_loss: null argument");
+    if (!t || !hyper || !obs || !states || !act || !old_logp || !adv || !ret || !idx_dev) return fail(TACO_E_INVALID, "taco_ppo_forward_loss: null argument");
     DevGuard guard(t->device);
     cudaStream_t s = (cudaStream_t)stream;
     const int B = t->B;
@@ -941,21 +929,21 @@ int taco_ppo_forward_loss(TacoPPO* t, const TacoPPOHyper* hyper, const float* ob
     L.dv_bm = t->critic.dz_bm[t->critic.L];
     L.acc = t->acc; L.stop = t->stop;
     launch_pdl(loss_kernel, dim3((B + 255) / 256), dim3(256), 0, s, L);
-    PPO_CUDA(cudaGetLastError());
+    TACO_CUDA(cudaGetLastError());
     return TACO_OK;
 }
 
 // device address of the 8 float64 loss accumulators [sum surrogate, sum value, sum kl, -, d log_std x 4]: a data-parallel job
 // all-reduces (SUM) them between taco_ppo_forward_loss and taco_ppo_decide and passes world > 1 in the hyper-parameters
 int taco_ppo_loss_sums(TacoPPO* t, double** acc_dev) {
-    if (!t || !acc_dev) return ppo_fail(TACO_E_INVALID, "taco_ppo_loss_sums: null argument");
+    if (!t || !acc_dev) return fail(TACO_E_INVALID, "taco_ppo_loss_sums: null argument");
     *acc_dev = t->acc;
     return TACO_OK;
 }
 
 // phase 2: log row + KL early-stop decision (device side)
 int taco_ppo_decide(TacoPPO* t, const TacoPPOHyper* hyper, void* stream) {
-    if (!t || !hyper) return ppo_fail(TACO_E_INVALID, "taco_ppo_decide: null argument");
+    if (!t || !hyper) return fail(TACO_E_INVALID, "taco_ppo_decide: null argument");
     DevGuard guard(t->device);
     DecideParams d;
     memset(&d, 0, sizeof(d));
@@ -963,13 +951,13 @@ int taco_ppo_decide(TacoPPO* t, const TacoPPOHyper* hyper, void* stream) {
     d.log_std = t->prm + t->off_log_std; d.act_dim = t->A; d.B = t->B; d.h = to_hyper(hyper);
     d.grad_log_std = t->grad + t->off_log_std;
     launch_pdl(decide_kernel, dim3(1), dim3(32), 0, (cudaStream_t)stream, d);
-    PPO_CUDA(cudaGetLastError());
+    TACO_CUDA(cudaGetLastError());
     return TACO_OK;
 }
 
 // phase 3: backward -> flat gradient (local; a data-parallel job all-reduces (SUM) it before taco_ppo_apply)
 int taco_ppo_backward(TacoPPO* t, void* stream) {
-    if (!t) return ppo_fail(TACO_E_INVALID, "taco_ppo_backward: null argument");
+    if (!t) return fail(TACO_E_INVALID, "taco_ppo_backward: null argument");
     DevGuard guard(t->device);
     cudaStream_t s = (cudaStream_t)stream;
     const int B = t->B;
@@ -1050,13 +1038,13 @@ int taco_ppo_backward(TacoPPO* t, void* stream) {
     }
     gp.grad = t->grad; gp.acc = t->acc; gp.stop = t->stop;
     launch_pdl(grad_assemble_kernel, dim3((unsigned)((elems + 255) / 256)), dim3(256), 0, s, gp);
-    PPO_CUDA(cudaGetLastError());
+    TACO_CUDA(cudaGetLastError());
     return TACO_OK;
 }
 
 // phase 4: clip_grad_norm_ + Adam + spectral projection + re-pack of the bf16 operand copies
 int taco_ppo_apply(TacoPPO* t, const TacoPPOHyper* hyper, void* stream) {
-    if (!t || !hyper) return ppo_fail(TACO_E_INVALID, "taco_ppo_apply: null argument");
+    if (!t || !hyper) return fail(TACO_E_INVALID, "taco_ppo_apply: null argument");
     DevGuard guard(t->device);
     cudaStream_t s = (cudaStream_t)stream;
     const Hyper h = to_hyper(hyper);
@@ -1075,17 +1063,17 @@ int taco_ppo_apply(TacoPPO* t, const TacoPPOHyper* hyper, void* stream) {
         t->spec_cold = false;
         // actor: projection, then the bf16 copies of the projected matrices, on the side stream (4 CTAs of latency-bound power
         // iteration); the caller's stream goes on with the critic's copies and the next minibatch until it needs the actor
-        PPO_CUDA(cudaEventRecord(t->ev_adam, s));
-        PPO_CUDA(cudaStreamWaitEvent(t->side, t->ev_adam, 0));
+        TACO_CUDA(cudaEventRecord(t->ev_adam, s));
+        TACO_CUDA(cudaStreamWaitEvent(t->side, t->ev_adam, 0));
         spectral_kernel<<<sp.n_seg, 512, 0, t->side>>>(sp); TACO_LAUNCHED();
-        PPO_CUDA(cudaGetLastError());
+        TACO_CUDA(cudaGetLastError());
         int rc = repack(t, t->side, true, 1);
         if (rc != TACO_OK) return rc;
-        PPO_CUDA(cudaEventRecord(t->ev_actor, t->side));
+        TACO_CUDA(cudaEventRecord(t->ev_actor, t->side));
         t->actor_pending = true;
         return repack(t, s, true, 2);
     }
-    PPO_CUDA(cudaGetLastError());
+    TACO_CUDA(cudaGetLastError());
     return repack(t, s, true);
 }
 
@@ -1093,7 +1081,7 @@ int taco_ppo_apply(TacoPPO* t, const TacoPPOHyper* hyper, void* stream) {
 // total loss, approx KL, gradient norm, stopped-here flag, clip coefficient), the number of optimiser steps taken overall and
 // whether the KL early stop fired.  log_host may be NULL.
 int taco_ppo_end_update(TacoPPO* t, float* log_host, int32_t max_rows, int32_t* n_rows, int32_t* optim_steps, int32_t* early_stop, void* stream) {
-    if (!t) return ppo_fail(TACO_E_INVALID, "taco_ppo_end_update: null argument");
+    if (!t) return fail(TACO_E_INVALID, "taco_ppo_end_update: null argument");
     DevGuard guard(t->device);
     cudaStream_t s = (cudaStream_t)stream;
     {
@@ -1101,13 +1089,13 @@ int taco_ppo_end_update(TacoPPO* t, float* log_host, int32_t max_rows, int32_t* 
         if (rcj != TACO_OK) return rcj;
     }
     int h[3] = {0, 0, 0};
-    PPO_CUDA(cudaMemcpyAsync(&h[0], t->n_logged, sizeof(int), cudaMemcpyDeviceToHost, s));
-    PPO_CUDA(cudaMemcpyAsync(&h[1], t->step, sizeof(int), cudaMemcpyDeviceToHost, s));
-    PPO_CUDA(cudaMemcpyAsync(&h[2], t->stop, sizeof(int), cudaMemcpyDeviceToHost, s));
-    PPO_CUDA(cudaStreamSynchronize(s));
+    TACO_CUDA(cudaMemcpyAsync(&h[0], t->n_logged, sizeof(int), cudaMemcpyDeviceToHost, s));
+    TACO_CUDA(cudaMemcpyAsync(&h[1], t->step, sizeof(int), cudaMemcpyDeviceToHost, s));
+    TACO_CUDA(cudaMemcpyAsync(&h[2], t->stop, sizeof(int), cudaMemcpyDeviceToHost, s));
+    TACO_CUDA(cudaStreamSynchronize(s));
     int rows = h[0] < t->max_log ? h[0] : t->max_log;
     if (rows > max_rows) rows = max_rows;
-    if (log_host && rows > 0) PPO_CUDA(cudaMemcpy(log_host, t->log, (size_t)rows * kLogCols * sizeof(float), cudaMemcpyDeviceToHost));
+    if (log_host && rows > 0) TACO_CUDA(cudaMemcpy(log_host, t->log, (size_t)rows * kLogCols * sizeof(float), cudaMemcpyDeviceToHost));
     if (n_rows) *n_rows = rows;
     if (optim_steps) *optim_steps = h[1];
     if (early_stop) *early_stop = h[2];
@@ -1116,16 +1104,16 @@ int taco_ppo_end_update(TacoPPO* t, float* log_host, int32_t max_rows, int32_t* 
 
 // sigma of every actor weight matrix as measured by the last projection (n_actor_layers doubles, host)
 int taco_ppo_sigmas(TacoPPO* t, double* out_host) {
-    if (!t || !out_host) return ppo_fail(TACO_E_INVALID, "taco_ppo_sigmas: null argument");
+    if (!t || !out_host) return fail(TACO_E_INVALID, "taco_ppo_sigmas: null argument");
     DevGuard guard(t->device);
-    PPO_CUDA(cudaDeviceSynchronize());
-    PPO_CUDA(cudaMemcpy(out_host, t->spec_sigma, (size_t)t->actor.L * sizeof(double), cudaMemcpyDeviceToHost));
+    TACO_CUDA(cudaDeviceSynchronize());
+    TACO_CUDA(cudaMemcpy(out_host, t->spec_sigma, (size_t)t->actor.L * sizeof(double), cudaMemcpyDeviceToHost));
     return TACO_OK;
 }
 
 // test hook: device addresses of the forward results of the last taco_ppo_forward_loss: action mean (batch, act_dim) and value (batch)
 int taco_ppo_debug_outputs(TacoPPO* t, float** mean_dev, float** value_dev) {
-    if (!t) return ppo_fail(TACO_E_INVALID, "taco_ppo_debug_outputs: null argument");
+    if (!t) return fail(TACO_E_INVALID, "taco_ppo_debug_outputs: null argument");
     if (mean_dev) *mean_dev = t->mean;
     if (value_dev) *value_dev = t->value;
     return TACO_OK;
@@ -1134,34 +1122,34 @@ int taco_ppo_debug_outputs(TacoPPO* t, float** mean_dev, float** value_dev) {
 // test hook: D[M][N] (fp32, ld = N) = A[M][K] B[N][K]^T for bf16 row-major device matrices (ld = K, K multiple of 8) through
 // gemm_tc_kernel with `splits` split-K partials summed on the host side of the call
 static int gemm_selftest_impl(int device, const void* a_bf16, const void* b_bf16, float* d_f32, int32_t m, int32_t n, int32_t k, int32_t splits, bool mn, void* stream) {
-    if (!a_bf16 || !b_bf16 || !d_f32 || m < 1 || n < 1 || n > 256 || k < 8 || (k & 7)) return ppo_fail(TACO_E_INVALID, "taco_gemm_selftest: bad argument");
+    if (!a_bf16 || !b_bf16 || !d_f32 || m < 1 || n < 1 || n > 256 || k < 8 || (k & 7)) return fail(TACO_E_INVALID, "taco_gemm_selftest: bad argument");
     DevGuard guard(device);
     cudaStream_t s = (cudaStream_t)stream;
-    if (!encode_fn()) return ppo_fail(TACO_E_CUDA, "cuTensorMapEncodeTiled unavailable");
+    if (!encode_fn()) return fail(TACO_E_CUDA, "cuTensorMapEncodeTiled unavailable");
     CUtensorMap ma, mb;
     const bool ok = mn ? make_map(&ma, (const bf16*)a_bf16, k, m, m, BK) && make_map(&mb, (const bf16*)b_bf16, k, n, n, BK)
                        : make_map(&ma, (const bf16*)a_bf16, m, k, k, BM) && make_map(&mb, (const bf16*)b_bf16, n, k, k, pad16(n));
-    if (!ok) return ppo_fail(TACO_E_CUDA, "tensor map");
-    PPO_CUDA(cudaFuncSetAttribute(gemm_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kGemmSmem));
+    if (!ok) return fail(TACO_E_CUDA, "tensor map");
+    TACO_CUDA(cudaFuncSetAttribute(gemm_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kGemmSmem));
     const int kb_total = (k + BK - 1) / BK;
     int sp = splits < 1 ? 1 : (splits > kb_total ? kb_total : splits);
     const int per = (kb_total + sp - 1) / sp;
     sp = (kb_total + per - 1) / per;
     float* part = nullptr;
-    PPO_CUDA(cudaMalloc(&part, (size_t)sp * m * n * sizeof(float)));
+    TACO_CUDA(cudaMalloc(&part, (size_t)sp * m * n * sizeof(float)));
     // (compute-sanitizer's initcheck does not observe writes made by cp.async.bulk.tensor stores: without this the partials the
     // TMA-store epilogue writes read as uninitialised in the assembly kernel below)
-    PPO_CUDA(cudaMemsetAsync(part, 0, (size_t)sp * m * n * sizeof(float), s));
+    TACO_CUDA(cudaMemsetAsync(part, 0, (size_t)sp * m * n * sizeof(float), s));
     GemmParams p;
     memset(&p, 0, sizeof(p));
     p.m = m; p.n = n; p.k = k; p.n_tile = pad16(n); p.splits = sp; p.kb_per_split = per; p.epi = EPI_F32; p.n_valid = n; p.mn_major = mn ? 1 : 0;
     p.out_f32 = part; p.ldc = n; p.split_stride = (long long)m * n;
     cudaDeviceProp prop;
-    PPO_CUDA(cudaGetDeviceProperties(&prop, device));
+    TACO_CUDA(cudaGetDeviceProperties(&prop, device));
     const int total = ((m + BM - 1) / BM) * sp;
     CUtensorMap mc = ma;
     p.tma_store = (m % BM == 0 && n % 4 == 0) ? 1 : 0;      // exercise the TMA-store epilogue where its shape rule holds
-    if (p.tma_store && !make_map_f32(&mc, part, (long long)sp * m, n, n)) return ppo_fail(TACO_E_CUDA, "tensor map");
+    if (p.tma_store && !make_map_f32(&mc, part, (long long)sp * m, n, n)) return fail(TACO_E_CUDA, "tensor map");
     gemm_tc_kernel<<<total < prop.multiProcessorCount ? total : prop.multiProcessorCount, kGemmThreads, kGemmSmem, s>>>(ma, mb, mc, p); TACO_LAUNCHED();
     GradParams gp;
     memset(&gp, 0, sizeof(gp));
@@ -1171,7 +1159,7 @@ static int gemm_selftest_impl(int device, const void* a_bf16, const void* b_bf16
     grad_assemble_kernel<<<(unsigned)(((long long)m * n + 255) / 256), 256, 0, s>>>(gp); TACO_LAUNCHED();
     const cudaError_t e = cudaStreamSynchronize(s);
     cudaFree(part);
-    if (e != cudaSuccess) return ppo_fail(TACO_E_CUDA, std::string("taco_gemm_selftest: ") + cudaGetErrorString(e));
+    if (e != cudaSuccess) return fail(TACO_E_CUDA, std::string("taco_gemm_selftest: ") + cudaGetErrorString(e));
     return TACO_OK;
 }
 
@@ -1181,7 +1169,7 @@ int taco_gemm_selftest(int device, const void* a_bf16, const void* b_bf16, float
 }
 // the same product from TRANSPOSED operands: at[k][m], bt[k][n] (m, n multiples of 8)
 int taco_gemm_selftest_mn(int device, const void* at_bf16, const void* bt_bf16, float* d_f32, int32_t m, int32_t n, int32_t k, int32_t splits, void* stream) {
-    if ((m & 7) || (n & 7)) return ppo_fail(TACO_E_INVALID, "taco_gemm_selftest_mn: m and n must be multiples of 8");
+    if ((m & 7) || (n & 7)) return fail(TACO_E_INVALID, "taco_gemm_selftest_mn: m and n must be multiples of 8");
     return gemm_selftest_impl(device, at_bf16, bt_bf16, d_f32, m, n, k, splits, true, stream);
 }
 
