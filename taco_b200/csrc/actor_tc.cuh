@@ -15,7 +15,8 @@
 // on one tile the epilogue warps of the other drain its accumulator.  The 4-wide output layer rides the same chain as
 // one more (N = 16, zero-padded) MMA part; tanh and the optional Gaussian sampling are CUDA-core work in its epilogue.
 //
-// TMEM map (512 columns): tile slot t owns columns [256 t, 256 t + 256): A = first 128 (K <= 256 as bf16 pairs),
+// This pipeline is shared with the critic kernel (mlp_common.cuh); this header adds the observation staging, the output part and the
+// tail.  TMEM map (512 columns): tile slot t owns columns [256 t, 256 t + 256): A = first 128 (K <= 256 as bf16 pairs),
 // D = last 128 (one part of N).
 // Warp roles (576 threads): warp 0 = weight producer, warp 1 = TMEM allocator + MMA issuer (both warp-uniform loops
 // with one elected lane issuing, so that every operand stays in uniform registers),
@@ -135,62 +136,27 @@ __device__ __forceinline__ void read_staged_obs(const float* stage, int r, int i
 
 __global__ void __launch_bounds__(kTcThreads, 1) actor_tc_kernel(const TcParams p) {
     extern __shared__ uint8_t smem_raw[];
-    const uint32_t raw = smem_u32(smem_raw);
-    const uint32_t base = (raw + 1023u) & ~1023u;                   // SWIZZLE_128B atoms need 1024-byte alignment
-    uint8_t* sm = smem_raw + (base - raw);
-    const uint32_t s_ring = base;                                    // kSlots x 64 KB weight ring
-    float* s_bias = reinterpret_cast<float*>(sm + kSlots * kSlotBytes);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(s_bias + kMaxHidden * kMaxN);
-    const uint32_t bar_full = smem_u32(bars);                        // [kSlots] producer -> MMA
-    const uint32_t bar_empty = bar_full + 8 * kSlots;                // [kSlots] MMA -> producer
-    const uint32_t bar_a = bar_empty + 8 * kSlots;                   // [2] epilogue(t) -> MMA: D(t) drained (and, for a new layer, A(t) written)
-    const uint32_t bar_d = bar_a + 16;                               // [2] MMA -> epilogue(t): the part of D(t) is complete
-    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bars + 2 * kSlots + 4);
-    const uint32_t bar_obs = bar_d + 16 + 8;                         // [2] a tile's observation block has landed in the staging buffer
-    float* s_obs = reinterpret_cast<float*>(sm + kTcSmemBytes - 1024);   // [2 tiles][128 rows x in_dim] (only with p.obs_bulk)
+    const TcSmem sm(smem_raw);
+    const uint32_t bar_obs = sm.bar_own;                             // [2] a tile's observation block has landed in the staging buffer
+    float* s_obs = reinterpret_cast<float*>(sm.base + kTcSmemBytes - 1024);   // [2 tiles][128 rows x in_dim] (only with p.obs_bulk)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int tps = p.tiles_per_cta;                                 // 2, or 1 when there are fewer tiles than SMs (small batches: one tile per CTA halves the latency)
     const int num_pairs = (p.num_tiles + tps - 1) / tps;
     const int n_layers = p.n_hidden + 1;                             // hidden layers + the output layer as a 16-wide part
 
-    for (int i = threadIdx.x; i < kMaxHidden * kMaxN; i += kTcThreads) s_bias[i] = p.bias[i];
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < kSlots; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, 1); }
-        for (int t = 0; t < 2; ++t) { mbar_init(bar_a + 8 * t, (kEpiWarps / 2) * 32); mbar_init(bar_d + 8 * t, 1); mbar_init(bar_obs + 8 * t, 1); }
-        fence_barrier_init();
-    }
-    if (warp == 1) tmem_alloc(smem_u32(s_tmem), kTmemCols);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem0 = *s_tmem;
+    const uint32_t tmem0 = sm.setup(warp, p.bias, [&] { for (int t = 0; t < 2; ++t) mbar_init(bar_obs + 8 * t, 1); });
 
     if (warp == 0) {
-        // ===================== weight producer: per pair, per layer, per 128-row part: one slot (all its K chunks)
+        // ===================== weight producer: per pair, per layer, per 128-row part one slot
         uint32_t slot = 0, phase = 0;
-        for (int pair = blockIdx.x; pair < num_pairs; pair += gridDim.x) {
-            for (int l = 0; l < n_layers; ++l) {
-                const int n = p.layer[l].n, kch = p.layer[l].kchunks;
-                const uint8_t* img = p.wimg + p.layer[l].img_off;
-                for (int h0 = 0; h0 < n; h0 += kPartN) {
-                    const uint32_t bytes = (uint32_t)min(kPartN, n - h0) * 128u;
-                    mbar_wait(bar_empty + 8 * slot, phase ^ 1u);
-                    if (elect_one_sync()) {
-                        mbar_arrive_expect_tx(bar_full + 8 * slot, bytes * (uint32_t)kch);
-                        for (int c = 0; c < kch; ++c)
-                            bulk_g2s(s_ring + slot * kSlotBytes + c * kChunkBytes, img + ((size_t)c * n + h0) * 128u, bytes, bar_full + 8 * slot);
-                    }
-                    __syncwarp();
-                    if (++slot == kSlots) { slot = 0; phase ^= 1u; }
-                }
-            }
-        }
+        for (int pair = blockIdx.x; pair < num_pairs; pair += gridDim.x)
+            for (int l = 0; l < n_layers; ++l) produce_layer(sm, p.wimg, p.layer[l], kSlots, slot, phase);
     } else if (warp == 1) {
         // ===================== MMA issuer: tiles A (slot 0) and B (slot 1) of the pair alternate part by part and share every weight slot
         uint32_t slot = 0, phase = 0, a_phase = 0;
         int dbg_n = lane == 0 ? 0 : kDbgCap;
-        const uint64_t bdesc0 = umma_desc_sw128(s_ring);
+        const uint64_t bdesc0 = umma_desc_sw128(sm.ring);
         for (int pair = blockIdx.x; pair < num_pairs; pair += gridDim.x) {
             const int nt = min(tps, p.num_tiles - tps * pair);
             for (int l = 0; l < n_layers; ++l) {
@@ -201,26 +167,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) actor_tc_kernel(const TcParams 
 #pragma unroll
                     for (int t = 0; t < 2; ++t) {
                         if (t < nt) {
-                            mbar_wait(bar_a + 8 * t, (a_phase >> t) & 1u); a_phase ^= (1u << t);   // D(t) free; A(t) of this layer in TMEM
-                            if (t == 0) mbar_wait(bar_full + 8 * slot, phase);
+                            mbar_wait(sm.bar_a + 8 * t, (a_phase >> t) & 1u); a_phase ^= (1u << t);   // D(t) free; A(t) of this layer in TMEM
+                            if (t == 0) mbar_wait(sm.bar_full + 8 * slot, phase);
                             tc_fence_after();
                             TACO_DBG(0, dbg_n, 0x20 | t);
-                            if (elect_one_sync()) {
-                                const uint32_t a_addr = tmem0 + (uint32_t)(t * kTmemSlot);
-                                const uint32_t d_addr = a_addr + (uint32_t)kTmemD;
-                                for (int c = 0; c < kch; ++c) {
-                                    const uint64_t b_c = bdesc + (uint64_t)(c * (kChunkBytes >> 4));
-                                    const uint32_t a_c = a_addr + (uint32_t)(c * (kKC / 2));
-                                    // 16 bf16 along K = 8 packed TMEM columns of A = 32 bytes inside the B swizzle atom
-                                    umma_bf16_ts(d_addr, a_c, b_c, idesc, (uint32_t)(c != 0));
-                                    umma_bf16_ts(d_addr, a_c + 8u, b_c + 2u, idesc, 1u);
-                                    umma_bf16_ts(d_addr, a_c + 16u, b_c + 4u, idesc, 1u);
-                                    umma_bf16_ts(d_addr, a_c + 24u, b_c + 6u, idesc, 1u);
-                                }
-                                if (t == nt - 1) umma_commit(bar_empty + 8 * slot);   // slot free once the last user's MMAs have read it
-                                umma_commit(bar_d + 8 * t);
-                            }
-                            __syncwarp();
+                            issue_part(tmem0 + (uint32_t)(t * kTmemSlot), bdesc, idesc, kch, false, t == nt - 1, sm.bar_empty + 8 * slot,
+                                       sm.bar_d + 8 * t);
                             TACO_DBG(0, dbg_n, 0x30 | t);
                         }
                     }
@@ -229,18 +181,15 @@ __global__ void __launch_bounds__(kTcThreads, 1) actor_tc_kernel(const TcParams 
             }
         }
     } else {
-        // ===================== epilogue warps: thread <-> TMEM lane <-> env row of tile slot t; the two 64-column halves of a
-        // part are handled by the warps `ch` = 0 / 1 of the same lane quadrant
-        const int e = warp - 2;
-        const int t = e >> 3, ch = (e >> 2) & 1, quad = warp & 3;    // a warp may only touch TMEM lanes 32*(warp%4)..+31
-        const int r = (quad << 5) | lane;
-        const uint32_t t_a = tmem0 + ((uint32_t)(quad << 5) << 16) + (uint32_t)(t * kTmemSlot);
-        const uint32_t t_d = t_a + (uint32_t)kTmemD + (uint32_t)(ch * 64);
+        // ===================== epilogue warps
+        const EpiThread ep(warp, lane, tmem0, tps, p.num_tiles);
+        const int e = ep.e, t = ep.t, ch = ep.ch, r = ep.r;
+        const uint32_t t_a = ep.t_a, t_d = ep.t_d;
         uint32_t d_phase = 0;
         const int kc0 = p.layer[0].kchunks;
-        int dbg_n = (ch == 0 && quad == 0 && lane == 0) ? 0 : kDbgCap;
-        int tile = t < tps ? tps * (int)blockIdx.x + t : p.num_tiles;      // tile slot 1 idles with one tile per CTA
-        const int tile_step = tps * (int)gridDim.x;
+        int dbg_n = (ch == 0 && ep.quad == 0 && lane == 0) ? 0 : kDbgCap;
+        int tile = ep.tile;
+        const int tile_step = ep.tile_step;
         // Bulk-staged observations (p.obs_bulk): a FULL tile's rows are one contiguous block of global memory (128 x in_dim floats), so
         // one elected thread of the tile has the bulk-copy engine fetch the block of the tile AFTER the one being staged; the
         // 128 x 26 row-per-thread scalar loads (one cache line per lane and instruction) leave the LSU.  Partial last tiles use loads.
@@ -282,7 +231,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) actor_tc_kernel(const TcParams 
             }
             tmem_st_wait();
             tc_fence_before();
-            mbar_arrive(bar_a + 8 * t);
+            mbar_arrive(sm.bar_a + 8 * t);
             TACO_DBG(1 + t, dbg_n, 0x01);
         }
         for (; tile < p.num_tiles; tile += tile_step) {
@@ -292,47 +241,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) actor_tc_kernel(const TcParams 
             const long long row_next = row + (long long)tile_step * kTileM;
             const float* x_next = p.obs + row_next * p.in_dim;
             if (has_next && row_next < p.n_rows) prefetch_l2(x_next + ch * 32);   // this thread's first group of the next tile
-            for (int l = 0; l < p.n_hidden; ++l) {
-                // hidden layer: relu(D + bias) as bf16 pairs, held in registers until every MMA of the layer has read A(t), then
-                // written over A(t) as the next layer's operand
-                const int n = p.layer[l].n;
-                const float* bl = s_bias + l * kMaxN;
-                const bool two_parts = n > kPartN;
-                uint32_t pk0[32];
-                const bool mine0 = ch * 64 < min(n, kPartN);                 // this warp has columns in part 0
-                const bool mine1 = two_parts && (kPartN + ch * 64 < n);      // ... in part 1
-                mbar_wait(bar_d + 8 * t, d_phase); d_phase ^= 1u;
-                tc_fence_after();
-                TACO_DBG(1 + t, dbg_n, 0x02);
-                if (mine0) {
-                    uint32_t v[32];
-                    tmem_ld32(t_d, v); tmem_ld_wait();
-                    relu_pack32(v, bl + ch * 64, pk0);
-                    tmem_ld32(t_d + 32u, v); tmem_ld_wait();
-                    if (two_parts) { tc_fence_before(); mbar_arrive(bar_a + 8 * t); TACO_DBG(1 + t, dbg_n, 0x03); }   // D drained: part 1 may start
-                    relu_pack32(v, bl + ch * 64 + 32, pk0 + 16);
-                } else if (two_parts) { tc_fence_before(); mbar_arrive(bar_a + 8 * t); }
-                if (two_parts) {
-                    mbar_wait(bar_d + 8 * t, d_phase); d_phase ^= 1u;
-                    tc_fence_after();
-                    TACO_DBG(1 + t, dbg_n, 0x04);
-                }
-                // every MMA of layer l on this tile is complete: overwrite A(t) (feature k -> packed column k/2)
-                if (mine0) { tmem_st16(t_a + (uint32_t)(ch * 32), pk0); tmem_st16(t_a + (uint32_t)(ch * 32 + 16), pk0 + 16); }
-                if (mine1) {
-                    uint32_t v[32], pk1[16];
-                    tmem_ld32(t_d, v); tmem_ld_wait();
-                    relu_pack32(v, bl + kPartN + ch * 64, pk1);
-                    tmem_st16(t_a + (uint32_t)(64 + ch * 32), pk1);
-                    tmem_ld32(t_d + 32u, v); tmem_ld_wait();
-                    relu_pack32(v, bl + kPartN + ch * 64 + 32, pk1);
-                    tmem_st16(t_a + (uint32_t)(64 + ch * 32 + 16), pk1);
-                }
-                tmem_st_wait();
-                tc_fence_before();
-                mbar_arrive(bar_a + 8 * t);
-                TACO_DBG(1 + t, dbg_n, 0x05);
-            }
+            for (int l = 0; l < p.n_hidden; ++l)
+                hidden_layer<true>(ep, sm.bias, l, p.layer[l].n, sm.bar_a, sm.bar_d, d_phase, p.dbg, dbg_n);
             // ---- output layer (columns 0..3 of its 16-wide part).  The next tile's first observation group is fetched while the
             // output MMAs run; once D is in registers the next A(t) is written and the issuer released, and only then the tanh /
             // sampling tail of this tile runs (overlapping the next tile's first MMAs).
@@ -347,7 +257,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) actor_tc_kernel(const TcParams 
                 }
                 if (bulk_tile(tile + 2 * tile_step)) fetch_obs(tile + 2 * tile_step);
             } else if (has_next) load_obs_group(x_next, ch, p.in_dim, row_next < p.n_rows, pkn, p.obs_vec2 != 0);
-            mbar_wait(bar_d + 8 * t, d_phase); d_phase ^= 1u;
+            mbar_wait(sm.bar_d + 8 * t, d_phase); d_phase ^= 1u;
             tc_fence_after();
             TACO_DBG(1 + t, dbg_n, 0x06);
             uint32_t v[4];
@@ -360,7 +270,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) actor_tc_kernel(const TcParams 
                 }
                 tmem_st_wait();
                 tc_fence_before();
-                mbar_arrive(bar_a + 8 * t);
+                mbar_arrive(sm.bar_a + 8 * t);
                 TACO_DBG(1 + t, dbg_n, 0x01);
             }
             if (ch == 0 && valid) {
@@ -372,12 +282,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) actor_tc_kernel(const TcParams 
             TACO_DBG(1 + t, dbg_n, 0x07);
         }
     }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem0, kTmemCols);
-    }
+    sm.teardown(warp, tmem0);
 }
 
 }  // namespace actor

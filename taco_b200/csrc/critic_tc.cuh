@@ -5,17 +5,17 @@
 //   LSTMEncoder.forward   nets_asymmetry.py:128-136   nn.LSTM(26, H, 1, batch_first=True) over (N, len_states, 26), output h_T
 //   MLP.forward           nets_asymmetry.py:23-39     [Linear -> ReLU] x L -> Linear(-> 1), Identity output (:318)
 //
-// Same machinery as the actor kernel (actor_tc.cuh: two 128-env tiles in flight per CTA, the A operand in TENSOR MEMORY,
-// weights streamed through a shared-memory ring by the bulk-copy engine and shared by both tiles, MMA parts of the two
-// tiles interleaved so that one tile's accumulator is drained while the tensor core works on the other).  What is new is
-// the schedule and the LSTM epilogue:
+// Runs the tcgen05 MLP pipeline of mlp_common.cuh, as the actor kernel does: two 128-env tiles in flight per CTA, the A operand in
+// TENSOR MEMORY, weights streamed through a shared-memory ring by the bulk-copy engine and shared by both tiles, MMA parts of the
+// two tiles interleaved so that one tile's accumulator is drained while the tensor core works on the other.  The critic's own
+// parts are the schedule and the LSTM epilogue:
 //   * one LSTM time step is ONE layer of the chain: gates[128 x 4H] = [h_{t-1} | x_t] (K = 64 + 64, zero padded) * Wcat^T,
 //     Wcat = [W_hh | W_ih] with its rows permuted so that every 16 accumulator columns hold the four gates (i, f, g, o; 4
 //     columns each) of the same 4 hidden units -- an epilogue thread reads 16 columns and owns those 4 units outright;
 //   * the cell state c lives in tensor memory too (fp32, in the 64 columns of the tile's A region the K = 128 LSTM operand leaves
 //     free), read and rewritten by the thread that owns (env row, hidden unit); h_t is written back over the A operand as
 //     packed bf16 pairs next to the freshly staged x_{t+1};
-//   * the T = len_states steps reuse one weight image; then the MLP layers and the 16-wide output part follow as in the actor.
+//   * the T = len_states steps reuse one weight image; then come the MLP layers and the 16-wide output part.
 // Gate non-linearities use MUFU.TANH (tanh.approx.f32; sigmoid(x) = 0.5 + 0.5 tanh(x / 2)): five per (env, unit, step) -- the
 // LSTM phase is bound by the 16 MUFU lanes of the SM, not by the tensor core.
 #pragma once
@@ -29,7 +29,7 @@ using namespace taco::mlp;
 constexpr int kMaxSeq = 8;             // len_states of the reference runs is 5 (README.md:60-66)
 constexpr int kTcMaxLstmHidden = 64;   // the cell state lives in the 64 spare TMEM columns of the tile's A operand
 constexpr int kTcMaxIn = 30;           // features per frame (26) + two constant-1 bias columns, padded to 32 = 16 packed TMEM columns
-constexpr int kMaxMlpHidden = 3;       // s_bias rows: LSTM gates + up to 3 hidden layers
+constexpr int kMaxMlpHidden = 3;       // bias rows: LSTM gates + up to 3 hidden layers
 static_assert(1 + kMaxMlpHidden <= kMaxHidden, "the LSTM step and the MLP's hidden layers share the kMaxHidden bias rows / TcImage layers");
 constexpr int kRing = kSlots - 1;        // ring slots of the MLP weights; the last 64 KB slot holds the LSTM image for the whole kernel
 constexpr int kAColH = 0;              // A operand columns (packed bf16 pairs): h in [0, 32), x_t in [32, 48), zero pad [48, 64)
@@ -180,19 +180,9 @@ __device__ __forceinline__ void stage_new_tile(uint32_t t_a, int ch, const uint3
 
 __global__ void __launch_bounds__(kTcThreads, 1) critic_tc_kernel(const CriticTcParams p) {
     extern __shared__ uint8_t smem_raw[];
-    const uint32_t raw = smem_u32(smem_raw);
-    const uint32_t base = (raw + 1023u) & ~1023u;
-    uint8_t* sm = smem_raw + (base - raw);
-    const uint32_t s_ring = base;
-    float* s_bias = reinterpret_cast<float*>(sm + kSlots * kSlotBytes);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(s_bias + kMaxHidden * kMaxN);
-    const uint32_t bar_full = smem_u32(bars);
-    const uint32_t bar_empty = bar_full + 8 * kSlots;
-    const uint32_t bar_a = bar_empty + 8 * kSlots;
-    const uint32_t bar_d = bar_a + 16;
-    const uint32_t bar_lstm = bar_d + 16 + 8;                       // the resident LSTM weight image has landed (the word after bar_d holds the TMEM address)
-    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bars + 2 * kSlots + 4);
-    uint32_t* s_x = reinterpret_cast<uint32_t*>(sm + kTcSmemBytes - 1024);       // [2 tiles][128 rows][kXStride] staged state frames (bf16 pairs)
+    const TcSmem sm(smem_raw);
+    const uint32_t bar_lstm = sm.bar_own;                             // the resident LSTM weight image has landed
+    uint32_t* s_x = reinterpret_cast<uint32_t*>(sm.base + kTcSmemBytes - 1024);     // [2 tiles][128 rows][kXStride] staged state frames (bf16 pairs)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int tps = p.tiles_per_cta;                                 // 2, or 1 when there are fewer tiles than SMs (small batches: one tile per CTA halves the latency)
@@ -202,18 +192,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) critic_tc_kernel(const CriticTc
 
     // constant part of the staged frames: pair in_dim / 2 = (1, 1) (the bias columns), zero elsewhere
     for (int i = threadIdx.x; i < 2 * kTileM * kXStride; i += kTcThreads) s_x[i] = (i % kXStride == (p.in_dim >> 1)) ? 0x3F803F80u : 0u;
-    for (int i = threadIdx.x; i < kMaxHidden * kMaxN; i += kTcThreads) s_bias[i] = p.bias[i];
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < kSlots; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, 1); }
-        for (int t = 0; t < 2; ++t) { mbar_init(bar_a + 8 * t, (kEpiWarps / 2) * 32); mbar_init(bar_d + 8 * t, 1); }
-        mbar_init(bar_lstm, 1);
-        fence_barrier_init();
-    }
-    if (warp == 1) tmem_alloc(smem_u32(s_tmem), kTmemCols);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem0 = *s_tmem;
+    const uint32_t tmem0 = sm.setup(warp, p.bias, [&] { mbar_init(bar_lstm, 1); });
 
     if (warp == 0) {
         // ===================== weight producer.  The LSTM image (<= 64 KB: [W_hh | W_ih] for 4H <= 256 gate rows) is the same for
@@ -227,34 +206,19 @@ __global__ void __launch_bounds__(kTcThreads, 1) critic_tc_kernel(const CriticTc
                 mbar_arrive_expect_tx(bar_lstm, (uint32_t)n * 128u * 2u);
                 for (int h0 = 0, part = 0; h0 < n; h0 += kPartN, ++part)
                     for (int c = 0; c < 2; ++c)
-                        bulk_g2s(s_ring + kRing * kSlotBytes + (part * 2 + c) * kChunkBytes, img + ((size_t)c * n + h0) * 128u,
+                        bulk_g2s(sm.ring + kRing * kSlotBytes + (part * 2 + c) * kChunkBytes, img + ((size_t)c * n + h0) * 128u,
                                  (uint32_t)min(kPartN, n - h0) * 128u, bar_lstm);
             }
             __syncwarp();
         }
         uint32_t slot = 0, phase = 0;
-        for (int pair = blockIdx.x; pair < num_pairs; pair += gridDim.x) {
-            for (int l = 1; l <= p.n_hidden + 1; ++l) {
-                const int n = p.layer[l].n, kch = p.layer[l].kchunks;
-                const uint8_t* img = p.wimg + p.layer[l].img_off;
-                for (int h0 = 0; h0 < n; h0 += kPartN) {
-                    const uint32_t bytes = (uint32_t)min(kPartN, n - h0) * 128u;
-                    mbar_wait(bar_empty + 8 * slot, phase ^ 1u);
-                    if (elect_one_sync()) {
-                        mbar_arrive_expect_tx(bar_full + 8 * slot, bytes * (uint32_t)kch);
-                        for (int c = 0; c < kch; ++c)
-                            bulk_g2s(s_ring + slot * kSlotBytes + c * kChunkBytes, img + ((size_t)c * n + h0) * 128u, bytes, bar_full + 8 * slot);
-                    }
-                    __syncwarp();
-                    if (++slot == kRing) { slot = 0; phase ^= 1u; }
-                }
-            }
-        }
+        for (int pair = blockIdx.x; pair < num_pairs; pair += gridDim.x)
+            for (int l = 1; l <= p.n_hidden + 1; ++l) produce_layer(sm, p.wimg, p.layer[l], kRing, slot, phase);
     } else if (warp == 1) {
-        // ===================== MMA issuer (see actor_tc.cuh): the two tiles alternate part by part and share every weight slot
+        // ===================== MMA issuer: the two tiles alternate part by part and share every weight slot
         uint32_t slot = 0, phase = 0, a_phase = 0;
         int dbg_n = lane == 0 ? 0 : kDbgCap;
-        const uint64_t bdesc0 = umma_desc_sw128(s_ring);
+        const uint64_t bdesc0 = umma_desc_sw128(sm.ring);
         mbar_wait(bar_lstm, 0u);                                       // the resident LSTM image
         for (int pair = blockIdx.x; pair < num_pairs; pair += gridDim.x) {
             const int nt = min(tps, p.num_tiles - tps * pair);
@@ -273,29 +237,14 @@ __global__ void __launch_bounds__(kTcThreads, 1) critic_tc_kernel(const CriticTc
                         const int dn = t == 0 ? done0 : done1;
                         if (dn >= total_parts) continue;
                         if (t == 1 && dn == 0 && (done0 == 0 || clock64() - t0_start < (long long)p.stagger)) continue;
-                        if (!mbar_test(bar_a + 8 * t, (a_phase >> t) & 1u)) continue;
+                        if (!mbar_test(sm.bar_a + 8 * t, (a_phase >> t) & 1u)) continue;
                         a_phase ^= (1u << t);
                         const int h0 = (dn % parts) * kPartN;
                         const uint32_t idesc = umma_idesc_bf16(kTileM, min(kPartN, n - h0));
                         const uint64_t bdesc = bdesc0 + (uint64_t)((kRing * kSlotBytes + (h0 / kPartN) * 2 * kChunkBytes) >> 4);
                         tc_fence_after();
                         TACO_DBG(0, dbg_n, 0x20 | t);
-                        if (elect_one_sync()) {
-                            const uint32_t a_addr = tmem0 + (uint32_t)(t * kTmemSlot);
-                            const uint32_t d_addr = a_addr + (uint32_t)kTmemD;
-                            for (int c = 0; c < p.layer[0].kchunks; ++c) {
-                                const uint64_t b_c = bdesc + (uint64_t)(c * (kChunkBytes >> 4));
-                                const uint32_t a_c = a_addr + (uint32_t)(c * (kKC / 2));
-                                umma_bf16_ts(d_addr, a_c, b_c, idesc, (uint32_t)(c != 0));
-                                umma_bf16_ts(d_addr, a_c + 8u, b_c + 2u, idesc, 1u);
-                                if (c == 0) {                          // the x_t chunk of an LSTM step holds only 32 K values (26 + 2 bias + pad)
-                                    umma_bf16_ts(d_addr, a_c + 16u, b_c + 4u, idesc, 1u);
-                                    umma_bf16_ts(d_addr, a_c + 24u, b_c + 6u, idesc, 1u);
-                                }
-                            }
-                            umma_commit(bar_d + 8 * t);
-                        }
-                        __syncwarp();
+                        issue_part(tmem0 + (uint32_t)(t * kTmemSlot), bdesc, idesc, p.layer[0].kchunks, true, false, 0u, sm.bar_d + 8 * t);
                         TACO_DBG(0, dbg_n, 0x30 | t);
                         if (t == 0) { if (done0 == 0) t0_start = clock64(); ++done0; } else ++done1;
                     }
@@ -314,27 +263,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) critic_tc_kernel(const CriticTc
 #pragma unroll
                     for (int t = 0; t < 2; ++t) {
                         if (t < nt) {
-                            mbar_wait(bar_a + 8 * t, (a_phase >> t) & 1u); a_phase ^= (1u << t);
-                            if (t == 0 && ring) mbar_wait(bar_full + 8 * slot, phase);
+                            mbar_wait(sm.bar_a + 8 * t, (a_phase >> t) & 1u); a_phase ^= (1u << t);
+                            if (t == 0 && ring) mbar_wait(sm.bar_full + 8 * slot, phase);
                             tc_fence_after();
                             TACO_DBG(0, dbg_n, 0x20 | t);
-                            if (elect_one_sync()) {
-                                const uint32_t a_addr = tmem0 + (uint32_t)(t * kTmemSlot);
-                                const uint32_t d_addr = a_addr + (uint32_t)kTmemD;
-                                for (int c = 0; c < kch; ++c) {
-                                    const uint64_t b_c = bdesc + (uint64_t)(c * (kChunkBytes >> 4));
-                                    const uint32_t a_c = a_addr + (uint32_t)(c * (kKC / 2));
-                                    umma_bf16_ts(d_addr, a_c, b_c, idesc, (uint32_t)(c != 0));
-                                    umma_bf16_ts(d_addr, a_c + 8u, b_c + 2u, idesc, 1u);
-                                    if (ring || c == 0) {                  // the x_t chunk of an LSTM step holds only 32 K values (26 + 2 bias + pad)
-                                        umma_bf16_ts(d_addr, a_c + 16u, b_c + 4u, idesc, 1u);
-                                        umma_bf16_ts(d_addr, a_c + 24u, b_c + 6u, idesc, 1u);
-                                    }
-                                }
-                                if (t == nt - 1 && ring) umma_commit(bar_empty + 8 * slot);
-                                umma_commit(bar_d + 8 * t);
-                            }
-                            __syncwarp();
+                            issue_part(tmem0 + (uint32_t)(t * kTmemSlot), bdesc, idesc, kch, !ring, t == nt - 1 && ring, sm.bar_empty + 8 * slot,
+                                       sm.bar_d + 8 * t);
                             TACO_DBG(0, dbg_n, 0x30 | t);
                         }
                     }
@@ -343,18 +277,16 @@ __global__ void __launch_bounds__(kTcThreads, 1) critic_tc_kernel(const CriticTc
             }
         }
     } else {
-        // ===================== epilogue warps: thread <-> TMEM lane <-> env row of tile slot t; `ch` = 64-column half of a part
-        const int e = warp - 2;
-        const int t = e >> 3, ch = (e >> 2) & 1, quad = warp & 3;
-        const int r = (quad << 5) | lane;
-        const uint32_t t_a = tmem0 + ((uint32_t)(quad << 5) << 16) + (uint32_t)(t * kTmemSlot);
-        const uint32_t t_d = t_a + (uint32_t)kTmemD + (uint32_t)(ch * 64);
+        // ===================== epilogue warps
+        const EpiThread ep(warp, lane, tmem0, tps, p.num_tiles);
+        const int t = ep.t, ch = ep.ch, r = ep.r;
+        const uint32_t t_a = ep.t_a, t_d = ep.t_d;
         uint32_t d_phase = 0;
-        int dbg_n = (ch == 0 && quad == 0 && lane == 0) ? 0 : kDbgCap;
+        int dbg_n = (ch == 0 && ep.quad == 0 && lane == 0) ? 0 : kDbgCap;
         const size_t row_floats = (size_t)T * p.in_dim;
-        int tile = t < tps ? tps * (int)blockIdx.x + t : p.num_tiles;      // tile slot 1 idles with one tile per CTA
-        const int tile_step = tps * (int)gridDim.x;
-        const int tt = ((e & 7) << 5) | lane;                       // index among the 256 epilogue threads of this tile
+        int tile = ep.tile;
+        const int tile_step = ep.tile_step;
+        const int tt = ((ep.e & 7) << 5) | lane;                       // index among the 256 epilogue threads of this tile
         const float inv_in = 1.0f / (float)(p.in_dim >> 1);           // 1 / feature pairs per frame
         uint32_t* s_xt = s_x + t * (kTileM * kXStride);
         if (tile < p.num_tiles) {
@@ -367,7 +299,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) critic_tc_kernel(const CriticTc
             stage_new_tile(t_a, ch, x0);
             tmem_st_wait();
             tc_fence_before();
-            mbar_arrive(bar_a + 8 * t);
+            mbar_arrive(sm.bar_a + 8 * t);
         }
         // the LSTM layer: n = 4H accumulator columns in parts of 128; this thread owns 16 hidden units of every part it has columns in
         const int n_g = p.layer[0].n;
@@ -390,16 +322,16 @@ __global__ void __launch_bounds__(kTcThreads, 1) critic_tc_kernel(const CriticTc
                 // x_{t+1}: with one gate part the loads fly while the step's MMAs run; with two they are issued between the parts
                 // (their latency then overlaps part 1's MMAs instead of delaying the drain of part 0)
                 if (have_x && !g_two) frame_load(p.states, (long long)tile * kTileM, ts + 1, T, p.in_dim, row_floats, p.n_rows, tt, inv_in, raw);
-                mbar_wait(bar_d + 8 * t, d_phase); d_phase ^= 1u;
+                mbar_wait(sm.bar_d + 8 * t, d_phase); d_phase ^= 1u;
                 tc_fence_after();
                 TACO_DBG(1 + t, dbg_n, 0x02);
-                if (g_mine0) lstm_half(t_d, t_a + (uint32_t)(kAColC + ch * 16), hp, g_two, bar_a + 8 * t);      // D drained: part 1 may start
-                else if (g_two) { tc_fence_before(); mbar_arrive(bar_a + 8 * t); }
+                if (g_mine0) lstm_half(t_d, t_a + (uint32_t)(kAColC + ch * 16), hp, g_two, sm.bar_a + 8 * t);      // D drained: part 1 may start
+                else if (g_two) { tc_fence_before(); mbar_arrive(sm.bar_a + 8 * t); }
                 TACO_DBG(1 + t, dbg_n, 0x0A);
                 if (have_x && g_two) frame_load(p.states, (long long)tile * kTileM, ts + 1, T, p.in_dim, row_floats, p.n_rows, tt, inv_in, raw);
                 TACO_DBG(1 + t, dbg_n, 0x09);
                 if (g_two) {
-                    mbar_wait(bar_d + 8 * t, d_phase); d_phase ^= 1u;
+                    mbar_wait(sm.bar_d + 8 * t, d_phase); d_phase ^= 1u;
                     tc_fence_after();
                     TACO_DBG(1 + t, dbg_n, 0x04);
                 }
@@ -419,49 +351,16 @@ __global__ void __launch_bounds__(kTcThreads, 1) critic_tc_kernel(const CriticTc
                 }
                 tmem_st_wait();
                 tc_fence_before();
-                mbar_arrive(bar_a + 8 * t);
+                mbar_arrive(sm.bar_a + 8 * t);
                 TACO_DBG(1 + t, dbg_n, 0x05);
             }
-            // ---- MLP hidden layers (as in the actor kernel)
-            for (int l = 1; l <= p.n_hidden; ++l) {
-                const int n = p.layer[l].n;
-                const float* bl = s_bias + l * kMaxN;
-                const bool two_parts = n > kPartN;
-                uint32_t pk0[32];
-                const bool mine0 = ch * 64 < min(n, kPartN);
-                const bool mine1 = two_parts && (kPartN + ch * 64 < n);
-                mbar_wait(bar_d + 8 * t, d_phase); d_phase ^= 1u;
-                tc_fence_after();
-                if (mine0) {
-                    uint32_t v[32];
-                    tmem_ld32(t_d, v); tmem_ld_wait();
-                    relu_pack32(v, bl + ch * 64, pk0);
-                    tmem_ld32(t_d + 32u, v); tmem_ld_wait();
-                    if (two_parts) { tc_fence_before(); mbar_arrive(bar_a + 8 * t); }
-                    relu_pack32(v, bl + ch * 64 + 32, pk0 + 16);
-                } else if (two_parts) { tc_fence_before(); mbar_arrive(bar_a + 8 * t); }
-                if (two_parts) {
-                    mbar_wait(bar_d + 8 * t, d_phase); d_phase ^= 1u;
-                    tc_fence_after();
-                }
-                if (mine0) { tmem_st16(t_a + (uint32_t)(ch * 32), pk0); tmem_st16(t_a + (uint32_t)(ch * 32 + 16), pk0 + 16); }
-                if (mine1) {
-                    uint32_t v[32], pk1[16];
-                    tmem_ld32(t_d, v); tmem_ld_wait();
-                    relu_pack32(v, bl + kPartN + ch * 64, pk1);
-                    tmem_st16(t_a + (uint32_t)(64 + ch * 32), pk1);
-                    tmem_ld32(t_d + 32u, v); tmem_ld_wait();
-                    relu_pack32(v, bl + kPartN + ch * 64 + 32, pk1);
-                    tmem_st16(t_a + (uint32_t)(64 + ch * 32 + 16), pk1);
-                }
-                tmem_st_wait();
-                tc_fence_before();
-                mbar_arrive(bar_a + 8 * t);
-            }
+            // ---- MLP hidden layers
+            for (int l = 1; l <= p.n_hidden; ++l)
+                hidden_layer<false>(ep, sm.bias, l, p.layer[l].n, sm.bar_a, sm.bar_d, d_phase, nullptr, dbg_n);
             // ---- output part (column 0 of 16): the next tile's A operand is staged before the value leaves
             uint32_t raw[kXRaw];
             if (has_next) frame_load(p.states, (long long)(tile + tile_step) * kTileM, 0, T, p.in_dim, row_floats, p.n_rows, tt, inv_in, raw);
-            mbar_wait(bar_d + 8 * t, d_phase); d_phase ^= 1u;
+            mbar_wait(sm.bar_d + 8 * t, d_phase); d_phase ^= 1u;
             tc_fence_after();
             uint32_t v[4];
             if (ch == 0) { tmem_ld4(t_d, v); tmem_ld_wait(); }
@@ -473,17 +372,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) critic_tc_kernel(const CriticTc
                 stage_new_tile(t_a, ch, x0);
                 tmem_st_wait();
                 tc_fence_before();
-                mbar_arrive(bar_a + 8 * t);
+                mbar_arrive(sm.bar_a + 8 * t);
             }
             if (ch == 0 && valid) p.value[row] = __uint_as_float(v[0]) + __ldg(p.b_out);
         }
     }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem0, kTmemCols);
-    }
+    sm.teardown(warp, tmem0);
 }
 
 // LSTM weights (torch layout: w_ih (4H, In), w_hh (4H, H), gate row blocks i, f, g, o) -> two bf16 K-chunk images of n = 4H

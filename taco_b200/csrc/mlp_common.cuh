@@ -1,5 +1,6 @@
 // What the actor and the critic (taco_actor.cu / actor_tc.cuh, taco_critic.cu / critic_tc.cuh) share: the tile, weight-ring
-// and TMEM geometry of their tcgen05 kernels, the MLP weight-image format and its packer, and the host code that sets these up.
+// and TMEM geometry of their tcgen05 kernels and the pipeline both kernels run, the MLP weight-image format and its packer, and
+// the host code that sets these up.
 #pragma once
 #include <cstdio>
 #include <cstdlib>
@@ -38,16 +39,143 @@ struct TcLayer {
 };
 
 // optional timeline of CTA 0 (TACO_ACTOR_TIMELINE / TACO_CRITIC_TIMELINE=<file>, see timeline_begin): 3 regions of kDbgCap
-// (clock << 8 | code) words in p.dbg
+// (clock << 8 | code) words in dbg; TACO_DBG writes to the kernel's p.dbg
 constexpr int kDbgCap = 4096;
-#define TACO_DBG(region, cnt, code)                                                                         \
+#define TACO_DBG_AT(dbg, region, cnt, code)                                                                 \
     do {                                                                                                    \
-        if (p.dbg && blockIdx.x == 0 && (cnt) < kDbgCap)                                                    \
-            p.dbg[(region) * kDbgCap + (cnt)++] = ((unsigned long long)clock64() << 8) | (unsigned)(code);  \
+        if ((dbg) && blockIdx.x == 0 && (cnt) < kDbgCap)                                                    \
+            (dbg)[(region) * kDbgCap + (cnt)++] = ((unsigned long long)clock64() << 8) | (unsigned)(code);  \
     } while (0)
+#define TACO_DBG(region, cnt, code) TACO_DBG_AT(p.dbg, region, cnt, code)
 
 constexpr int kSmemBias = kMaxHidden * kMaxN * 4;          // 4 KB
 constexpr int kTcSmemBytes = 1024 /*alignment slack*/ + kSlots * kSlotBytes + kSmemBias + 256;
+
+// ---------------------------------------------------------------------------------------------- the tcgen05 MLP pipeline
+// One persistent CTA per SM keeps two 128-env tiles in flight.  Warp 0 streams the weights through a ring of 64 KB slots in shared
+// memory, one 128-row part of a layer per slot; warp 1 issues the MMAs of every part for both tiles and releases the slot after the
+// last tile's; the 16 epilogue warps drain D(t) and write the next layer's A(t) in tensor memory.  Producer and issuer are
+// warp-uniform loops with one elected lane issuing, so that every descriptor stays in uniform registers (issuing from inside
+// `if (lane == 0)` halved the MMA issue rate).  The kernels keep the slot and phase counters in their own loops.
+
+// Shared memory from its 1024-byte aligned base (SWIZZLE_128B atoms need that alignment): the weight ring, the bias block, the
+// barriers, the TMEM address word, then the kernel's own barriers from bar_own on.  The kernel's own buffers start at
+// base + kTcSmemBytes - 1024.
+struct TcSmem {
+    uint8_t* base;
+    uint32_t ring;        // kSlots x 64 KB weight ring
+    float* bias;          // [kMaxHidden][kMaxN]
+    uint32_t bar_full;    // [kSlots] producer -> MMA
+    uint32_t bar_empty;   // [kSlots] MMA -> producer
+    uint32_t bar_a;       // [2] epilogue(t) -> MMA: D(t) drained (and, for a new layer, A(t) written)
+    uint32_t bar_d;       // [2] MMA -> epilogue(t): the part of D(t) is complete
+    uint32_t* tmem;       // written by tcgen05.alloc
+    uint32_t bar_own;
+
+    __device__ __forceinline__ explicit TcSmem(uint8_t* smem_raw) {
+        const uint32_t raw = smem_u32(smem_raw);
+        const uint32_t aligned = (raw + 1023u) & ~1023u;
+        base = smem_raw + (aligned - raw);
+        ring = aligned;
+        bias = reinterpret_cast<float*>(base + kSlots * kSlotBytes);
+        uint64_t* bars = reinterpret_cast<uint64_t*>(bias + kMaxHidden * kMaxN);
+        bar_full = smem_u32(bars);
+        bar_empty = bar_full + 8 * kSlots;
+        bar_a = bar_empty + 8 * kSlots;
+        bar_d = bar_a + 16;
+        tmem = reinterpret_cast<uint32_t*>(bars + 2 * kSlots + 4);
+        bar_own = bar_d + 16 + 8;
+    }
+
+    // copies the biases, initialises the barriers (own_init() adds the kernel's own, on the same thread before the init fence) and
+    // allocates all of tensor memory; returns its base address
+    template <class OwnInit>
+    __device__ __forceinline__ uint32_t setup(int warp, const float* bias_src, OwnInit own_init) const {
+        for (int i = threadIdx.x; i < kMaxHidden * kMaxN; i += kTcThreads) bias[i] = bias_src[i];
+        if (threadIdx.x == 0) {
+            for (int s = 0; s < kSlots; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, 1); }
+            for (int t = 0; t < 2; ++t) { mbar_init(bar_a + 8 * t, (kEpiWarps / 2) * 32); mbar_init(bar_d + 8 * t, 1); }
+            own_init();
+            fence_barrier_init();
+        }
+        if (warp == 1) tmem_alloc(smem_u32(tmem), kTmemCols);
+        tc_fence_before();
+        __syncthreads();
+        tc_fence_after();
+        return *tmem;
+    }
+
+    __device__ __forceinline__ void teardown(int warp, uint32_t tmem0) const {
+        tc_fence_before();
+        __syncthreads();
+        if (warp == 1) {
+            tc_fence_after();
+            tmem_dealloc(tmem0, kTmemCols);
+        }
+    }
+};
+
+// producer: every 128-row part of layer L, all its K chunks, into the next slot of a ring of ring_slots slots once the MMAs have
+// released that slot
+__device__ __forceinline__ void produce_layer(const TcSmem& s, const uint8_t* wimg, const TcLayer& L, int ring_slots, uint32_t& slot,
+                                              uint32_t& phase) {
+    const int n = L.n, kch = L.kchunks;
+    const uint8_t* img = wimg + L.img_off;
+    for (int h0 = 0; h0 < n; h0 += kPartN) {
+        const uint32_t bytes = (uint32_t)min(kPartN, n - h0) * 128u;
+        mbar_wait(s.bar_empty + 8 * slot, phase ^ 1u);
+        if (elect_one_sync()) {
+            mbar_arrive_expect_tx(s.bar_full + 8 * slot, bytes * (uint32_t)kch);
+            for (int c = 0; c < kch; ++c)
+                bulk_g2s(s.ring + slot * kSlotBytes + c * kChunkBytes, img + ((size_t)c * n + h0) * 128u, bytes, s.bar_full + 8 * slot);
+        }
+        __syncwarp();
+        if (++slot == ring_slots) { slot = 0; phase ^= 1u; }
+    }
+}
+
+// issuer: the MMAs of one part for one tile, D = A * B^T over kch K chunks of 64 (A at a_addr, D next to it), then a commit to
+// bar_free if `release` (the ring slot may be refilled once the last tile's MMAs have read it) and to bar_done.  lstm: an LSTM step,
+// whose second chunk (x_t: 26 features, 2 bias columns, padding) holds only 32 K values.
+__device__ __forceinline__ void issue_part(uint32_t a_addr, uint64_t bdesc, uint32_t idesc, int kch, bool lstm, bool release,
+                                           uint32_t bar_free, uint32_t bar_done) {
+    if (elect_one_sync()) {
+        const uint32_t d_addr = a_addr + (uint32_t)kTmemD;
+        for (int c = 0; c < kch; ++c) {
+            const uint64_t b_c = bdesc + (uint64_t)(c * (kChunkBytes >> 4));
+            const uint32_t a_c = a_addr + (uint32_t)(c * (kKC / 2));
+            // 16 bf16 along K = 8 packed TMEM columns of A = 32 bytes inside the B swizzle atom
+            umma_bf16_ts(d_addr, a_c, b_c, idesc, (uint32_t)(c != 0));
+            umma_bf16_ts(d_addr, a_c + 8u, b_c + 2u, idesc, 1u);
+            if (!lstm || c == 0) {
+                umma_bf16_ts(d_addr, a_c + 16u, b_c + 4u, idesc, 1u);
+                umma_bf16_ts(d_addr, a_c + 24u, b_c + 6u, idesc, 1u);
+            }
+        }
+        if (release) umma_commit(bar_free);
+        umma_commit(bar_done);
+    }
+    __syncwarp();
+}
+
+// An epilogue thread (warps 2..17): tile slot t, 64-column half ch of a part, TMEM lane quadrant quad (a warp may only touch TMEM
+// lanes 32 (warp % 4) .. + 31); thread <-> TMEM lane <-> env row r of the tile.  t_a / t_d: the thread's lane of A(t) and of its half
+// of D(t).  `tile` is the slot's first tile (num_tiles: slot 1 idles with one tile per CTA), tile_step the stride to its next.
+struct EpiThread {
+    int e, t, ch, quad, r;
+    uint32_t t_a, t_d;
+    int tile, tile_step;
+
+    __device__ __forceinline__ EpiThread(int warp, int lane, uint32_t tmem0, int tps, int num_tiles) {
+        e = warp - 2;
+        t = e >> 3; ch = (e >> 2) & 1; quad = warp & 3;
+        r = (quad << 5) | lane;
+        t_a = tmem0 + ((uint32_t)(quad << 5) << 16) + (uint32_t)(t * kTmemSlot);
+        t_d = t_a + (uint32_t)kTmemD + (uint32_t)(ch * 64);
+        tile = t < tps ? tps * (int)blockIdx.x + t : num_tiles;
+        tile_step = tps * (int)gridDim.x;
+    }
+};
 
 // relu(D + bias) of 32 accumulator columns -> 16 packed bf16 pairs (column 2j in the low half)
 __device__ __forceinline__ void relu_pack32(const uint32_t (&v)[32], const float* bias, uint32_t* pk) {
@@ -57,6 +185,52 @@ __device__ __forceinline__ void relu_pack32(const uint32_t (&v)[32], const float
         pk[q * 2 + 0] = pack_bf16x2(fmaxf(__uint_as_float(v[q * 4 + 0]) + b.x, 0.0f), fmaxf(__uint_as_float(v[q * 4 + 1]) + b.y, 0.0f));
         pk[q * 2 + 1] = pack_bf16x2(fmaxf(__uint_as_float(v[q * 4 + 2]) + b.z, 0.0f), fmaxf(__uint_as_float(v[q * 4 + 3]) + b.w, 0.0f));
     }
+}
+
+// Epilogue of hidden layer l (width n, bias row l of the bias block) on tile slot ep.t: relu(D + bias) as bf16 pairs, held in
+// registers until every MMA of the layer has read A(t), then written over A(t) as the next layer's operand (feature k -> packed
+// column k / 2).  With two parts, D is released as soon as part 0 is in registers, so part 1's MMAs overlap the rest of the drain.
+// bar_a / bar_d: the [2] barrier arrays of TcSmem.  kMark: timeline markers 0x02..0x05 in region 1 + t of dbg.
+template <bool kMark>
+__device__ __forceinline__ void hidden_layer(const EpiThread& ep, const float* bias, int l, int n, uint32_t bar_a, uint32_t bar_d, uint32_t& d_phase,
+                                             unsigned long long* dbg, int& dbg_n) {
+    const int ch = ep.ch, t = ep.t;
+    const uint32_t t_a = ep.t_a, t_d = ep.t_d;
+    const float* bl = bias + l * kMaxN;
+    const bool two_parts = n > kPartN;
+    uint32_t pk0[32];
+    const bool mine0 = ch * 64 < min(n, kPartN);                 // this warp has columns in part 0
+    const bool mine1 = two_parts && (kPartN + ch * 64 < n);      // ... in part 1
+    mbar_wait(bar_d + 8 * t, d_phase); d_phase ^= 1u;
+    tc_fence_after();
+    if (kMark) TACO_DBG_AT(dbg, 1 + t, dbg_n, 0x02);
+    if (mine0) {
+        uint32_t v[32];
+        tmem_ld32(t_d, v); tmem_ld_wait();
+        relu_pack32(v, bl + ch * 64, pk0);
+        tmem_ld32(t_d + 32u, v); tmem_ld_wait();
+        if (two_parts) { tc_fence_before(); mbar_arrive(bar_a + 8 * t); if (kMark) TACO_DBG_AT(dbg, 1 + t, dbg_n, 0x03); }
+        relu_pack32(v, bl + ch * 64 + 32, pk0 + 16);
+    } else if (two_parts) { tc_fence_before(); mbar_arrive(bar_a + 8 * t); }
+    if (two_parts) {
+        mbar_wait(bar_d + 8 * t, d_phase); d_phase ^= 1u;
+        tc_fence_after();
+        if (kMark) TACO_DBG_AT(dbg, 1 + t, dbg_n, 0x04);
+    }
+    if (mine0) { tmem_st16(t_a + (uint32_t)(ch * 32), pk0); tmem_st16(t_a + (uint32_t)(ch * 32 + 16), pk0 + 16); }
+    if (mine1) {
+        uint32_t v[32], pk1[16];
+        tmem_ld32(t_d, v); tmem_ld_wait();
+        relu_pack32(v, bl + kPartN + ch * 64, pk1);
+        tmem_st16(t_a + (uint32_t)(64 + ch * 32), pk1);
+        tmem_ld32(t_d + 32u, v); tmem_ld_wait();
+        relu_pack32(v, bl + kPartN + ch * 64 + 32, pk1);
+        tmem_st16(t_a + (uint32_t)(64 + ch * 32 + 16), pk1);
+    }
+    tmem_st_wait();
+    tc_fence_before();
+    mbar_arrive(bar_a + 8 * t);
+    if (kMark) TACO_DBG_AT(dbg, 1 + t, dbg_n, 0x05);
 }
 
 // fp32 (out, in) row-major weights -> bf16 K-chunk images in the SWIZZLE_128B K-major layout the kernel copies verbatim:
