@@ -33,6 +33,7 @@ def main():
     ap.add_argument("--actor-hidden", default="256,256,256")
     ap.add_argument("--critic-hidden", default="256,256")
     ap.add_argument("--lstm-hidden", type=int, default=64)
+    ap.add_argument("--lstm-layers", type=int, default=1, help="stacked LSTM layers of the critic encoder (num_layers of the reference's critic_encoder_dict)")
     ap.add_argument("--lipschitz", type=float, default=4.0, help="README training command: --lipschitz_para=4; 0 disables")
     ap.add_argument("--tensor-cores", default="auto", choices=["auto", "on", "off"])
     ap.add_argument("--update", default="native", choices=["native", "torch"])
@@ -59,7 +60,7 @@ def main():
                                env_offset=off, num_envs_global=n_glob, seed=args.seed)
     a_hid = [int(x) for x in args.actor_hidden.split(",")]
     c_hid = [int(x) for x in args.critic_hidden.split(",")]
-    agent = TorchActorCritic(26 * env.len_obs, 4, a_hid, 26, args.lstm_hidden, c_hid).to(dev)
+    agent = TorchActorCritic(26 * env.len_obs, 4, a_hid, 26, args.lstm_hidden, c_hid, lstm_layers=args.lstm_layers).to(dev)
     cfg = PPOConfig(epochs=args.epochs, train_iters=args.train_iters, lr=args.lr, use_lipschitz=args.lipschitz > 0,
                     lipschitz_para=args.lipschitz, lip_epoch_index=[args.epochs // 5, args.epochs],
                     diff_epoch_index=[args.epochs // 5, args.epochs], lr_epoch_index=int(0.7 * args.epochs))
@@ -69,10 +70,11 @@ def main():
         native = NativePPO(agent, n * args.horizon // args.mini_batch_num, device=dev)
         native._create(env.len_states)
     actor = taco_b200.ActorMLP(26 * env.len_obs, a_hid, 4, device=dev)
-    critic = taco_b200.CriticLSTM(26, env.len_states, args.lstm_hidden, c_hid, device=dev)
+    critic = taco_b200.CriticLSTM(26, env.len_states, args.lstm_hidden, c_hid, lstm_layers=args.lstm_layers, device=dev)
     buf = taco_b200.RolloutBuffer(n, 26, env.len_obs, 26, env.len_states, 4, args.horizon, args.mini_batch_num, 0.99, 0.95, dev)
     # the tensor-core kernels are also the fast path at small env counts (latency of one tile chain: ~12 us actor, ~36 us critic)
-    tc = args.tensor_cores != "off" and actor.tensor_cores_available and critic.tensor_cores_available
+    # a stacked critic has no tcgen05 kernel: its rollouts keep the actor's and run the critic on the FP32 kernel (with a warning)
+    tc = args.tensor_cores != "off" and actor.tensor_cores_available and (critic.tensor_cores_available or args.lstm_layers > 1)
     env.reset()
     graphed = None
     for epoch in range(args.epochs):

@@ -253,7 +253,8 @@ int taco_actor_act_counter(TacoActor* actor, const float* obs_dev, int32_t n, co
 
 /* -- native PPO update: PPO.update of the reference (IsaacGymEnvs/algorithms/ppo_asymmetry.py:137-258) for the network
  * configuration it trains with (README.md:60-66; nets_asymmetry.py:270-377): MLP actor (tanh mean, state-independent log_std,
- * std = exp(log_std)^2), critic = MLP(LSTMEncoder(states)).  Forward / backward are tcgen05 GEMMs fed by TMA tensor maps (bf16
+ * std = exp(log_std)^2), critic = MLP(LSTMEncoder(states)) with 1-4 stacked unidirectional LSTM layers of 64 units (taco_ppo_create_layers;
+ * the layers run one after another, each over all time steps, and back-propagate top layer first).  Forward / backward are tcgen05 GEMMs fed by TMA tensor maps (bf16
  * operands, fp32 accumulation), master weights / Adam moments / losses in fp32; the KL early stop (:223-226) is decided on the
  * device, so an update is a stream of launches without a host sync.  Per minibatch: taco_ppo_forward_loss -> [data parallel:
  * all-reduce SUM the 8 doubles of taco_ppo_loss_sums] -> taco_ppo_decide -> taco_ppo_backward -> [data parallel: all-reduce SUM
@@ -265,7 +266,7 @@ typedef struct TacoPPOCfg {
     int32_t obs_dim;             /* flattened actor input: num_obs * len_obs */
     int32_t act_dim;             /* <= 4 */
     int32_t state_dim, seq_len;  /* critic input (N, seq_len, state_dim): num_states, len_states */
-    int32_t lstm_hidden;         /* 64 */
+    int32_t lstm_hidden;         /* 64; the number of stacked LSTM layers is an argument of taco_ppo_create_layers */
     int32_t n_actor_hidden, actor_hidden[4];     /* hidden widths: multiples of 16 in [16, 256] */
     int32_t n_critic_hidden, critic_hidden[4];
 } TacoPPOCfg;
@@ -276,10 +277,14 @@ typedef struct TacoPPOHyper {
     int32_t world;               /* data-parallel ranks whose sums were all-reduced (1 = single process) */
 } TacoPPOHyper;
 int taco_ppo_create(int device, const TacoPPOCfg* cfg, TacoPPO** out);
+/* the same with a stacked LSTM encoder of lstm_layers in [1, 4] unidirectional layers (nn.LSTM(state_dim, 64, lstm_layers));
+ * taco_ppo_create is lstm_layers = 1 */
+int taco_ppo_create_layers(int device, const TacoPPOCfg* cfg, int32_t lstm_layers, TacoPPO** out);
 int taco_ppo_destroy(TacoPPO* ppo);
 int taco_ppo_num_params(TacoPPO* ppo, int64_t* n);
-/* offsets of the parameter tensors in the flat fp32 vector, in this order: log_std; actor (weight, bias) per layer; LSTM
- * weight_ih_l0, weight_hh_l0, bias_ih_l0, bias_hh_l0; critic MLP (weight, bias) per layer -- every tensor in torch's layout */
+/* offsets of the parameter tensors in the flat fp32 vector, in this order: log_std; actor (weight, bias) per layer; per LSTM
+ * layer k, bottom first: weight_ih_lk, weight_hh_lk, bias_ih_lk, bias_hh_lk; critic MLP (weight, bias) per layer -- every tensor
+ * in torch's layout */
 int taco_ppo_param_offsets(TacoPPO* ppo, int64_t* offsets, int32_t count, int32_t* n_out);
 /* device addresses of the flat vectors (n_params floats each) and of the int32 optimiser-step counter; any may be NULL */
 int taco_ppo_buffers(TacoPPO* ppo, float** params, float** grad, float** adam_m, float** adam_v, int32_t** step);

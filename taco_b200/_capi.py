@@ -105,6 +105,7 @@ def lib():
         "taco_critic_tc_available": (C.c_int, [vp]),
         "taco_critic_forward": (C.c_int, [vp, vp, vp, i32, i32, vp]),
         "taco_ppo_create": (C.c_int, [C.c_int, vp, C.POINTER(vp)]),
+        "taco_ppo_create_layers": (C.c_int, [C.c_int, vp, i32, C.POINTER(vp)]),
         "taco_ppo_destroy": (C.c_int, [vp]),
         "taco_ppo_num_params": (C.c_int, [vp, C.POINTER(C.c_int64)]),
         "taco_ppo_param_offsets": (C.c_int, [vp, C.POINTER(C.c_int64), i32, C.POINTER(i32)]),

@@ -53,6 +53,8 @@ struct LstmEpi {
                                       // (saved for the backward pass; a chunk's 128 bytes are what one epilogue round produces per row)
     __nv_bfloat16* h_bm;              // destination of h: row stride ld_h_bm elements (the next step's operand [h | x | 1 1])
     long long ld_h_bm;
+    __nv_bfloat16* h2_bm;             // second destination of h (null: none): the x columns of the next LSTM layer's operand
+    long long ld_h2_bm;
 };
 
 struct GemmParams {
@@ -277,6 +279,13 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                             for (int q = 0; q < 2; ++q) {
                                 const int row = row2 + 64 * q;
                                 if (full || m0 + row < p.m) *reinterpret_cast<uint4*>(L.h_bm + (m0 + row) * L.ld_h_bm + j0 + 8 * pc2) = oh[q];
+                            }
+                        }
+                        if (L.h2_bm) {
+#pragma unroll
+                            for (int q = 0; q < 2; ++q) {
+                                const int row = row2 + 64 * q;
+                                if (full || m0 + row < p.m) *reinterpret_cast<uint4*>(L.h2_bm + (m0 + row) * L.ld_h2_bm + j0 + 8 * pc2) = oh[q];
                             }
                         }
                         sb ^= 1u;

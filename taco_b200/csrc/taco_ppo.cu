@@ -37,6 +37,7 @@ using namespace taco::gemm;
 typedef __nv_bfloat16 bf16;
 
 constexpr int kMaxHiddenL = 4;
+constexpr int kMaxLstmL = 4;        // stacked LSTM layers of the critic encoder
 constexpr int kH = 64;              // LSTM hidden width the LSTM epilogue is written for
 constexpr int kG = 4 * kH;          // gate rows
 constexpr int kSeqMax = 8;
@@ -239,7 +240,9 @@ __global__ void decide_kernel(const DecideParams p) {
 
 // LSTM backward, point-wise part of one time step (the gate math of nn.LSTM): one thread per (sample, unit), lanes along the units
 struct LstmBwdParams {
-    const float* dh; float* dc;                     // [B][64]: dL/dh_t (total), dL/dc_t carried from step t+1 (in) -> dL/dc_{t-1} (out)
+    const float* dh; float* dc;                     // [B][ld_dh], [B][64]: dL/dh_t from this layer's step t+1 or the critic MLP (null: 0),
+    int ld_dh;                                      // dL/dc_t carried from step t+1 (in) -> dL/dc_{t-1} (out)
+    const float* dh_add; int ld_dh_add;             // [B][ld_dh_add]: dL/dh_t through the LSTM layer above (null: top layer), added to dh
     const bf16* gates; const float* c_prev; const float* c_cur;     // [B][256] activated gates of step t (chunked layout), c_{t-1} (null: 0), c_t
     bf16* dg_bm;                                    // [B][256] gate pre-activation gradients of step t
     int B; int first;                               // first = this is the last time step (dc_in = 0)
@@ -256,7 +259,8 @@ __global__ void __launch_bounds__(256) lstm_bwd_kernel(const LstmBwdParams p) {
     const float gi = __bfloat162float(g[0]), gf = __bfloat162float(g[16]), gg = __bfloat162float(g[32]), go = __bfloat162float(g[48]);
     const float c = p.c_cur[i * kH + j], cp = p.c_prev ? p.c_prev[i * kH + j] : 0.0f;
     const float tc = tanhf(c);
-    const float dh = p.dh[i * kH + j];
+    float dh = p.dh ? p.dh[i * p.ld_dh + j] : 0.0f;
+    if (p.dh_add) dh += p.dh_add[i * p.ld_dh_add + j];
     const float dc = (p.first ? 0.0f : p.dc[i * kH + j]) + dh * go * (1.0f - tc * tc);
     p.dc[i * kH + j] = dc * gf;
     bf16* d = p.dg_bm + i * kG + j;
@@ -299,7 +303,7 @@ __global__ void __launch_bounds__(256) colsum_kernel(const ColSumParams p) {
 
 // gradient assembly: flat_grad[dst + r * cols + c] = sum over splits of partial[s][r][col0 + c]; accumulates the global norm^2
 struct GradSeg { const float* partial; int splits; long long split_stride; int ld, col0, rows, cols; long long dst; };
-struct GradParams { GradSeg seg[32]; int n_seg; float* grad; double* acc; const int* stop; };
+struct GradParams { GradSeg seg[4 * (kMaxHiddenL + 1) + 4 * kMaxLstmL]; int n_seg; float* grad; double* acc; const int* stop; };
 __global__ void __launch_bounds__(256) grad_assemble_kernel(const GradParams p) {
     pdl_launch_dependents();
     pdl_wait();
@@ -468,13 +472,14 @@ __global__ void __launch_bounds__(256) pack_kernel(const PackParams p) {
         }
     }
 }
-// LSTM: Wcat [256][96] = [W_hh | W_ih | b_hi b_lo | 0] and W_hh^T [64][256]
+// one LSTM layer: Wcat [256][ld_u] = [W_hh | W_ih | b_hi b_lo | 0] and its transpose Wcat^T [t_rows][256]: rows 0..63 W_hh^T, then
+// (t_rows = 128, layers above the first) W_ih^T
 __global__ void __launch_bounds__(256) pack_lstm_kernel(const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, int in_dim, int ld_u,
-                                                        bf16* wcat, bf16* whh_t, const int* stop) {
+                                                        bf16* wcat, bf16* wcat_t, int t_rows, const int* stop) {
     pdl_launch_dependents();
     pdl_wait();
     if (stop && *stop) return;
-    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < kG * ld_u + kH * kG; e += gridDim.x * blockDim.x) {
+    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < kG * ld_u + t_rows * kG; e += gridDim.x * blockDim.x) {
         if (e < kG * ld_u) {
             const int r = e / ld_u, c = e % ld_u;
             float v = 0.0f;
@@ -488,8 +493,8 @@ __global__ void __launch_bounds__(256) pack_lstm_kernel(const float* w_ih, const
             wcat[e] = __float2bfloat16_rn(v);
         } else {
             const int f = e - kG * ld_u;
-            const int j = f / kG, r = f % kG;                             // W_hh^T[j][r] = W_hh[r][j]
-            whh_t[f] = __float2bfloat16_rn(w_hh[r * kH + j]);
+            const int j = f / kG, r = f % kG;                             // W_hh^T[j][r] = W_hh[r][j], W_ih^T[j - 64][r] = W_ih[r][j - 64]
+            wcat_t[f] = __float2bfloat16_rn(j < kH ? w_hh[r * kH + j] : w_ih[r * in_dim + (j - kH)]);
         }
     }
 }
@@ -519,19 +524,32 @@ struct MlpNet {
     CUtensorMap m_partial[kMaxHiddenL + 1]; bool partial_tma[kMaxHiddenL + 1];   // split-K partials as [splits * out][ld_p] fp32 (TMA-stored when out % 128 == 0)
 };
 
+// one layer k of the stacked LSTM encoder; its operand of step t is U_k[t] = [h^k_{t-1} | x^k_t | 1 1 | 0] with x^0_t = states[:, t] and
+// x^k_t = h^{k-1}_t (written by layer k-1's epilogue), so one GEMM U_k[t] Wcat_k^T gives the gate pre-activations with the bias
+struct LstmLayer {
+    int in = 0, ld_u = 0, t_rows = 0;               // input width (state_dim, or 64 above layer 0), U / Wcat row pitch, rows of Wcat^T
+    long long off_wih = 0, off_whh = 0, off_bih = 0, off_bhh = 0;
+    bf16 *wcat = nullptr, *wcat_t = nullptr;        // [256][ld_u], [t_rows][256] (W_hh^T, then W_ih^T for k >= 1)
+    bf16 *u_bm = nullptr, *gates = nullptr, *dg_bm = nullptr;       // [seq*B][ld_u], [seq*B][256] x 2 (all time steps)
+    float *c_state = nullptr, *partial = nullptr;   // [seq*B][64]; dWcat split-K partials [splits][256][ld_u]
+    float* dhx = nullptr;                           // k >= 1: [seq][B][128] = d[h_{t-1} | x_t] of step t (slot 0: the x half only)
+    int splits = 1;
+    CUtensorMap m_u_bm, m_u_mn, m_wcat, m_wcat_t, m_wih_t, m_dg_bm, m_dg_mn, m_partial;
+    CUtensorMap m_dhx[kSeqMax], m_dx0;              // k >= 1: output maps of the d[h | x] GEMM per step, and of the dx-only GEMM of step 0
+};
+
 struct TacoPPO {
     int device = 0, num_sms = 148;
     TacoPPOCfg cfg;
-    int B = 0, A = 0, seq = 0, sd = 0, ld_u = 0;
+    int B = 0, A = 0, seq = 0, sd = 0, n_lstm = 1;
     long long n_params = 0;
-    long long off_log_std = 0, off_wih = 0, off_whh = 0, off_bih = 0, off_bhh = 0;
+    long long off_log_std = 0;
     float *prm = nullptr, *grad = nullptr, *adam_m = nullptr, *adam_v = nullptr;
     MlpNet actor, critic;
-    // LSTM
-    bf16 *wcat = nullptr, *whh_t = nullptr, *u_bm = nullptr, *gates = nullptr, *dg_bm = nullptr;     // dg_bm: [seq*B][256], all time steps
-    float *c_state = nullptr, *dh = nullptr, *dc = nullptr, *lstm_partial = nullptr, *colsum_partial = nullptr;
-    int lstm_splits = 1;
-    CUtensorMap m_u_bm, m_u_mn, m_wcat, m_whh_t, m_dg_bm, m_dg_mn, m_lstm_partial, m_dh;
+    // LSTM: the layers, dL/dh of layer 0's recurrence (and of the top layer's last step, from the critic MLP), dL/dc of the layer in flight
+    LstmLayer lstm[kMaxLstmL];
+    float *dh = nullptr, *dc = nullptr, *colsum_partial = nullptr;
+    CUtensorMap m_dh;
     // heads / side arrays
     float *mean = nullptr, *value = nullptr, *g_act = nullptr, *g_logp = nullptr, *g_adv = nullptr, *g_ret = nullptr;
     // bookkeeping
@@ -627,8 +645,13 @@ static int setup_net(TacoPPO* t, MlpNet& n, long long& off, bool actor) {
 extern "C" {
 
 int taco_ppo_create(int device, const TacoPPOCfg* cfg, TacoPPO** out) {
+    return taco_ppo_create_layers(device, cfg, 1, out);
+}
+
+int taco_ppo_create_layers(int device, const TacoPPOCfg* cfg, int32_t lstm_layers, TacoPPO** out) {
     if (!cfg || !out) return fail(TACO_E_INVALID, "taco_ppo_create: null argument");
     *out = nullptr;
+    if (lstm_layers < 1 || lstm_layers > kMaxLstmL) return fail(TACO_E_INVALID, "taco_ppo_create_layers: lstm_layers must be in [1, 4]");
     if (cfg->batch < 128 || cfg->batch % 128) return fail(TACO_E_INVALID, "taco_ppo_create: the minibatch size must be a positive multiple of 128");
     if (cfg->lstm_hidden != kH) return fail(TACO_E_INVALID, "taco_ppo_create: lstm_hidden must be 64");
     if (cfg->act_dim < 1 || cfg->act_dim > 4) return fail(TACO_E_INVALID, "taco_ppo_create: act_dim must be in [1, 4]");
@@ -651,12 +674,11 @@ int taco_ppo_create(int device, const TacoPPOCfg* cfg, TacoPPO** out) {
     TacoPPO* t = new (std::nothrow) TacoPPO();
     if (!t) return fail(TACO_E_NOMEM, "host allocation failed");
     t->device = device; t->cfg = *cfg; t->num_sms = prop.multiProcessorCount;
-    t->B = cfg->batch; t->A = cfg->act_dim; t->seq = cfg->seq_len; t->sd = cfg->state_dim;
-    t->ld_u = pad8(kH + cfg->state_dim + 2);
+    t->B = cfg->batch; t->A = cfg->act_dim; t->seq = cfg->seq_len; t->sd = cfg->state_dim; t->n_lstm = lstm_layers;
     const int B = t->B;
     int rc = TACO_OK;
     auto bail = [&](int code, const char* msg) { taco_ppo_destroy(t); return fail(code, msg); };
-    // ---- flat parameter layout: log_std | actor MLP (W, b per layer) | LSTM W_ih, W_hh, b_ih, b_hh | critic MLP
+    // ---- flat parameter layout: log_std | actor MLP (W, b per layer) | LSTM W_ih, W_hh, b_ih, b_hh per layer (bottom first) | critic MLP
     long long off = 0;
     t->off_log_std = off; off += t->A;
     t->actor.L = cfg->n_actor_hidden + 1;
@@ -664,10 +686,16 @@ int taco_ppo_create(int device, const TacoPPOCfg* cfg, TacoPPO** out) {
     for (int l = 0; l < cfg->n_actor_hidden; ++l) t->actor.s[l + 1] = cfg->actor_hidden[l];
     t->actor.s[t->actor.L] = t->A;
     if ((rc = setup_net(t, t->actor, off, true)) != TACO_OK) return bail(rc, "taco_ppo_create: actor buffers");
-    t->off_wih = off; off += (long long)kG * t->sd;
-    t->off_whh = off; off += (long long)kG * kH;
-    t->off_bih = off; off += kG;
-    t->off_bhh = off; off += kG;
+    for (int k = 0; k < t->n_lstm; ++k) {
+        LstmLayer& Ly = t->lstm[k];
+        Ly.in = k == 0 ? t->sd : kH;
+        Ly.ld_u = pad8(kH + Ly.in + 2);
+        Ly.t_rows = k == 0 ? kH : 2 * kH;
+        Ly.off_wih = off; off += (long long)kG * Ly.in;
+        Ly.off_whh = off; off += (long long)kG * kH;
+        Ly.off_bih = off; off += kG;
+        Ly.off_bhh = off; off += kG;
+    }
     t->critic.L = cfg->n_critic_hidden + 1;
     t->critic.s[0] = kH;
     for (int l = 0; l < cfg->n_critic_hidden; ++l) t->critic.s[l + 1] = cfg->critic_hidden[l];
@@ -680,17 +708,28 @@ int taco_ppo_create(int device, const TacoPPOCfg* cfg, TacoPPO** out) {
     if (ce == cudaSuccess) ce = dev_alloc(t, &t->adam_v, (size_t)off);
     // ---- LSTM buffers
     const long long SB = (long long)t->seq * B;
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->wcat, (size_t)kG * t->ld_u);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->whh_t, (size_t)kH * kG);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->u_bm, (size_t)SB * t->ld_u);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->gates, (size_t)SB * kG);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->dg_bm, (size_t)SB * kG);
+    for (int k = 0; k < t->n_lstm; ++k) {
+        LstmLayer& Ly = t->lstm[k];
+        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.wcat, (size_t)kG * Ly.ld_u);
+        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.wcat_t, (size_t)Ly.t_rows * kG);
+        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.u_bm, (size_t)SB * Ly.ld_u);
+        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.gates, (size_t)SB * kG);
+        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.dg_bm, (size_t)SB * kG);
+        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.c_state, (size_t)SB * kH);
+        Ly.splits = splits_for(kG, SB, t->num_sms);
+        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.partial, (size_t)Ly.splits * kG * Ly.ld_u);
+        if (k > 0 && ce == cudaSuccess) ce = dev_alloc(t, &Ly.dhx, (size_t)SB * 2 * kH);
+        if (k > 0 && ce == cudaSuccess) {
+            // the constant-1 columns of U_k (layer 0's come with the gather); the h columns of slot 0 (h_0 = 0) stay as allocated
+            const uint32_t ones = 0x3F803F80u;                            // two bf16 1.0
+            std::vector<uint32_t> col((size_t)SB, ones);
+            ce = cudaMemcpy2D(Ly.u_bm + kH + Ly.in, (size_t)Ly.ld_u * sizeof(bf16), col.data(), sizeof(uint32_t), sizeof(uint32_t), (size_t)SB,
+                              cudaMemcpyHostToDevice);
+        }
+    }
     if (ce == cudaSuccess) ce = dev_alloc(t, &t->colsum_partial, (size_t)2 * (kMaxHiddenL + 1) * ((B + kColRows - 1) / kColRows) * kColLd);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->c_state, (size_t)SB * kH);
     if (ce == cudaSuccess) ce = dev_alloc(t, &t->dh, (size_t)B * kH);
     if (ce == cudaSuccess) ce = dev_alloc(t, &t->dc, (size_t)B * kH);
-    t->lstm_splits = splits_for(kG, SB, t->num_sms);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->lstm_partial, (size_t)t->lstm_splits * kG * t->ld_u);
     if (ce == cudaSuccess) ce = dev_alloc(t, &t->mean, (size_t)B * t->A);
     if (ce == cudaSuccess) ce = dev_alloc(t, &t->value, (size_t)B);
     if (ce == cudaSuccess) ce = dev_alloc(t, &t->g_act, (size_t)B * t->A);
@@ -711,13 +750,22 @@ int taco_ppo_create(int device, const TacoPPOCfg* cfg, TacoPPO** out) {
         }
     }
     if (ce != cudaSuccess) return bail(ce == cudaErrorMemoryAllocation ? TACO_E_NOMEM : TACO_E_CUDA, "taco_ppo_create: device allocation failed");
-    bool ok = make_map(&t->m_u_bm, t->u_bm, SB, t->ld_u, t->ld_u, BM);
-    ok = ok && make_map(&t->m_u_mn, t->u_bm, SB, t->ld_u, t->ld_u, BK);
-    ok = ok && make_map(&t->m_wcat, t->wcat, kG, t->ld_u, t->ld_u, kG);
-    ok = ok && make_map(&t->m_whh_t, t->whh_t, kH, kG, kG, kH);
-    ok = ok && make_map(&t->m_dg_bm, t->dg_bm, SB, kG, kG, BM);
-    ok = ok && make_map(&t->m_dg_mn, t->dg_bm, SB, kG, kG, BK);
-    ok = ok && make_map_f32(&t->m_lstm_partial, t->lstm_partial, (long long)t->lstm_splits * kG, t->ld_u, t->ld_u);
+    bool ok = true;
+    for (int k = 0; k < t->n_lstm; ++k) {
+        LstmLayer& Ly = t->lstm[k];
+        ok = ok && make_map(&Ly.m_u_bm, Ly.u_bm, SB, Ly.ld_u, Ly.ld_u, BM);
+        ok = ok && make_map(&Ly.m_u_mn, Ly.u_bm, SB, Ly.ld_u, Ly.ld_u, BK);
+        ok = ok && make_map(&Ly.m_wcat, Ly.wcat, kG, Ly.ld_u, Ly.ld_u, kG);
+        ok = ok && make_map(&Ly.m_wcat_t, Ly.wcat_t, Ly.t_rows, kG, kG, Ly.t_rows);      // B operand of d[h | x] (k >= 1) or dh (k = 0)
+        ok = ok && make_map(&Ly.m_dg_bm, Ly.dg_bm, SB, kG, kG, BM);
+        ok = ok && make_map(&Ly.m_dg_mn, Ly.dg_bm, SB, kG, kG, BK);
+        ok = ok && make_map_f32(&Ly.m_partial, Ly.partial, (long long)Ly.splits * kG, Ly.ld_u, Ly.ld_u);
+        if (k > 0) {
+            ok = ok && make_map(&Ly.m_wih_t, Ly.wcat_t + (size_t)kH * kG, kH, kG, kG, kH);   // W_ih^T alone: the dx-only GEMM of step 0
+            for (int s = 0; s < t->seq; ++s) ok = ok && make_map_f32(&Ly.m_dhx[s], Ly.dhx + (size_t)s * B * 2 * kH, B, 2 * kH, 2 * kH);
+            ok = ok && make_map_f32(&Ly.m_dx0, Ly.dhx + kH, B, kH, 2 * kH);                  // the x half of slot 0
+        }
+    }
     ok = ok && make_map_f32(&t->m_dh, t->dh, B, kH, kH);
     if (!ok) return bail(TACO_E_CUDA, "taco_ppo_create: cuTensorMapEncodeTiled failed");
     if (cudaFuncSetAttribute(gemm_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kGemmSmem) != cudaSuccess)
@@ -746,14 +794,18 @@ int taco_ppo_num_params(TacoPPO* t, int64_t* n) {
     return TACO_OK;
 }
 
-// offsets of the parameter tensors inside the flat vector, in this order: log_std; actor (W, b) x layers; LSTM weight_ih_l0,
-// weight_hh_l0, bias_ih_l0, bias_hh_l0; critic (W, b) x layers.  `count` = capacity of `offsets`; returns the number written.
+// offsets of the parameter tensors inside the flat vector, in this order: log_std; actor (W, b) x layers; LSTM weight_ih_lk,
+// weight_hh_lk, bias_ih_lk, bias_hh_lk for k = 0 .. lstm_layers - 1; critic (W, b) x layers.  `count` = capacity of `offsets`;
+// returns the number written.
 int taco_ppo_param_offsets(TacoPPO* t, int64_t* offsets, int32_t count, int32_t* n_out) {
     if (!t || !offsets || !n_out) return fail(TACO_E_INVALID, "taco_ppo_param_offsets: null argument");
     std::vector<int64_t> v;
     v.push_back(t->off_log_std);
     for (int l = 0; l < t->actor.L; ++l) { v.push_back(t->actor.w_off[l]); v.push_back(t->actor.b_off[l]); }
-    v.push_back(t->off_wih); v.push_back(t->off_whh); v.push_back(t->off_bih); v.push_back(t->off_bhh);
+    for (int k = 0; k < t->n_lstm; ++k) {
+        const LstmLayer& Ly = t->lstm[k];
+        v.push_back(Ly.off_wih); v.push_back(Ly.off_whh); v.push_back(Ly.off_bih); v.push_back(Ly.off_bhh);
+    }
     for (int l = 0; l < t->critic.L; ++l) { v.push_back(t->critic.w_off[l]); v.push_back(t->critic.b_off[l]); }
     if ((int)v.size() > count) return fail(TACO_E_INVALID, "taco_ppo_param_offsets: buffer too small");
     for (size_t i = 0; i < v.size(); ++i) offsets[i] = v[i];
@@ -798,8 +850,12 @@ static int repack(TacoPPO* t, cudaStream_t s, bool honour_stop, int which = 0) {
     pp.stop = honour_stop ? t->stop : nullptr;
     launch_pdl(pack_kernel, dim3(32, pp.n_seg), dim3(256), 0, s, pp);
     if (which != 1) {
-        launch_pdl(pack_lstm_kernel, dim3(64), dim3(256), 0, s, (const float*)(t->prm + t->off_wih), (const float*)(t->prm + t->off_whh), (const float*)(t->prm + t->off_bih),
-                   (const float*)(t->prm + t->off_bhh), t->sd, t->ld_u, t->wcat, t->whh_t, (const int*)(honour_stop ? t->stop : nullptr));
+        for (int k = 0; k < t->n_lstm; ++k) {
+            const LstmLayer& Ly = t->lstm[k];
+            launch_pdl(pack_lstm_kernel, dim3(64), dim3(256), 0, s, (const float*)(t->prm + Ly.off_wih), (const float*)(t->prm + Ly.off_whh),
+                       (const float*)(t->prm + Ly.off_bih), (const float*)(t->prm + Ly.off_bhh), Ly.in, Ly.ld_u, Ly.wcat, Ly.wcat_t, Ly.t_rows,
+                       (const int*)(honour_stop ? t->stop : nullptr));
+        }
     }
     return cudaGetLastError() == cudaSuccess ? TACO_OK : fail(TACO_E_CUDA, "pack kernels failed");
 }
@@ -894,26 +950,35 @@ int taco_ppo_forward_loss(TacoPPO* t, const TacoPPOHyper* hyper, const float* ob
     g.obs = obs; g.obs_dim = t->cfg.obs_dim; g.states = states; g.seq = t->seq; g.state_dim = t->sd;
     g.act = act; g.logp = old_logp; g.adv = adv; g.ret = ret; g.idx = (const long long*)idx_dev; g.B = B; g.act_dim = t->A;
     g.x0_bm = t->actor.x_bm[0]; g.ld_x0 = t->actor.ld_x[0];
-    g.u_bm = t->u_bm; g.ld_u = t->ld_u;
+    g.u_bm = t->lstm[0].u_bm; g.ld_u = t->lstm[0].ld_u;
     g.g_act = t->g_act; g.g_logp = t->g_logp; g.g_adv = t->g_adv; g.g_ret = t->g_ret; g.stop = t->stop;
     launch_pdl(gather_kernel, dim3((B + 31) / 32), dim3(256), 0, s, g);
     int rc = TACO_OK;
-    // critic first: seq LSTM steps, each one GEMM [h_{t-1} | x_t | 1 1] Wcat^T with the gate math in the epilogue, then its MLP.  The
+    // critic first: seq LSTM steps per layer, bottom layer first, each one GEMM [h_{t-1} | x_t | 1 1] Wcat^T with the gate math in the
+    // epilogue, then its MLP.  A layer below the top also writes h_t into the x columns of the next layer's operand of step t.  The
     // previous optimiser step's projection + re-pack of the ACTOR may still be running on the side stream under these launches.
-    for (int k = 0; k < t->seq; ++k) {
-        GemmParams p;
-        memset(&p, 0, sizeof(p));
-        p.m = B; p.n = kG; p.k = t->ld_u; p.n_tile = kG; p.splits = 1; p.a_row0 = k * B; p.epi = EPI_LSTM; p.n_valid = kG;
-        p.lstm.c_prev = k > 0 ? t->c_state + (size_t)(k - 1) * B * kH : nullptr;
-        p.lstm.c_out = t->c_state + (size_t)k * B * kH;
-        p.lstm.gates_out = t->gates + (size_t)k * B * kG;
-        if (k + 1 < t->seq) {
-            p.lstm.h_bm = t->u_bm + (size_t)(k + 1) * B * t->ld_u; p.lstm.ld_h_bm = t->ld_u;
-        } else {
-            p.lstm.h_bm = t->critic.x_bm[0]; p.lstm.ld_h_bm = t->critic.ld_x[0];
+    for (int l = 0; l < t->n_lstm; ++l) {
+        const LstmLayer& Ly = t->lstm[l];
+        const LstmLayer* up = l + 1 < t->n_lstm ? &t->lstm[l + 1] : nullptr;
+        for (int k = 0; k < t->seq; ++k) {
+            GemmParams p;
+            memset(&p, 0, sizeof(p));
+            p.m = B; p.n = kG; p.k = Ly.ld_u; p.n_tile = kG; p.splits = 1; p.a_row0 = k * B; p.epi = EPI_LSTM; p.n_valid = kG;
+            p.lstm.c_prev = k > 0 ? Ly.c_state + (size_t)(k - 1) * B * kH : nullptr;
+            p.lstm.c_out = Ly.c_state + (size_t)k * B * kH;
+            p.lstm.gates_out = Ly.gates + (size_t)k * B * kG;
+            bf16* h_up = up ? up->u_bm + (size_t)k * B * up->ld_u + kH : nullptr;      // x columns of U_{l+1}[k]
+            if (k + 1 < t->seq) {
+                p.lstm.h_bm = Ly.u_bm + (size_t)(k + 1) * B * Ly.ld_u; p.lstm.ld_h_bm = Ly.ld_u;
+                if (up) { p.lstm.h2_bm = h_up; p.lstm.ld_h2_bm = up->ld_u; }
+            } else if (up) {
+                p.lstm.h_bm = h_up; p.lstm.ld_h_bm = up->ld_u;
+            } else {
+                p.lstm.h_bm = t->critic.x_bm[0]; p.lstm.ld_h_bm = t->critic.ld_x[0];
+            }
+            rc = launch_gemm(t, Ly.m_u_bm, Ly.m_wcat, p, s);
+            if (rc != TACO_OK) return rc;
         }
-        rc = launch_gemm(t, t->m_u_bm, t->m_wcat, p, s);
-        if (rc != TACO_OK) return rc;
     }
     rc = mlp_forward(t, t->critic, false, s);
     if (rc != TACO_OK) return rc;
@@ -966,30 +1031,55 @@ int taco_ppo_backward(TacoPPO* t, void* stream) {
     rc = mlp_backward(t, t->critic, t->dh, s);
     if (rc != TACO_OK) return rc;
     const long long SB = (long long)t->seq * B;
-    for (int k = t->seq - 1; k >= 0; --k) {
-        LstmBwdParams b;
-        memset(&b, 0, sizeof(b));
-        b.dh = t->dh; b.dc = t->dc; b.gates = t->gates + (size_t)k * B * kG;
-        b.c_prev = k > 0 ? t->c_state + (size_t)(k - 1) * B * kH : nullptr; b.c_cur = t->c_state + (size_t)k * B * kH;
-        b.dg_bm = t->dg_bm + (size_t)k * B * kG; b.B = B; b.first = (k == t->seq - 1); b.stop = t->stop;
-        launch_pdl(lstm_bwd_kernel, dim3((B + 3) / 4), dim3(256), 0, s, b);
-        if (k > 0) {   // dh_{t-1} = dgates_t W_hh: M = batch, N = 64, K = 256
+    // LSTM backward through time, top layer first.  Layer 0 back-propagates dh_{t-1} = dgates_t W_hh (N = 64) into t->dh; a layer
+    // l >= 1 computes d[h_{t-1} | x_t] = dgates_t [W_hh | W_ih] (N = 128) into its dhx slot t, whose x half the layer below adds to
+    // its dh at step t
+    for (int l = t->n_lstm - 1; l >= 0; --l) {
+        LstmLayer& Ly = t->lstm[l];
+        const LstmLayer* up = l + 1 < t->n_lstm ? &t->lstm[l + 1] : nullptr;
+        const bool top = up == nullptr;
+        for (int k = t->seq - 1; k >= 0; --k) {
+            LstmBwdParams b;
+            memset(&b, 0, sizeof(b));
+            if (l == 0 || k == t->seq - 1) {        // the critic MLP's dh (top layer, last step) or layer 0's recurrence
+                b.dh = (k < t->seq - 1 || top) ? t->dh : nullptr; b.ld_dh = kH;
+            } else {
+                b.dh = Ly.dhx + (size_t)(k + 1) * B * 2 * kH; b.ld_dh = 2 * kH;
+            }
+            if (up) { b.dh_add = up->dhx + (size_t)k * B * 2 * kH + kH; b.ld_dh_add = 2 * kH; }
+            b.dc = t->dc; b.gates = Ly.gates + (size_t)k * B * kG;
+            b.c_prev = k > 0 ? Ly.c_state + (size_t)(k - 1) * B * kH : nullptr; b.c_cur = Ly.c_state + (size_t)k * B * kH;
+            b.dg_bm = Ly.dg_bm + (size_t)k * B * kG; b.B = B; b.first = (k == t->seq - 1); b.stop = t->stop;
+            launch_pdl(lstm_bwd_kernel, dim3((B + 3) / 4), dim3(256), 0, s, b);
             GemmParams p;
             memset(&p, 0, sizeof(p));
-            p.m = B; p.n = kH; p.k = kG; p.n_tile = kH; p.splits = 1; p.a_row0 = k * B; p.epi = EPI_F32; p.n_valid = kH; p.out_f32 = t->dh; p.ldc = kH;
-            rc = launch_gemm(t, t->m_dg_bm, t->m_whh_t, p, s, &t->m_dh);
+            p.m = B; p.k = kG; p.splits = 1; p.a_row0 = k * B; p.epi = EPI_F32;
+            if (l == 0) {
+                if (k == 0) continue;
+                // dh_{t-1} = dgates_t W_hh: M = batch, N = 64, K = 256
+                p.n = kH; p.n_tile = kH; p.n_valid = kH; p.out_f32 = t->dh; p.ldc = kH;
+                rc = launch_gemm(t, Ly.m_dg_bm, Ly.m_wcat_t, p, s, &t->m_dh);
+            } else if (k > 0) {
+                // d[h_{t-1} | x_t] = dgates_t [W_hh | W_ih]: M = batch, N = 128, K = 256
+                p.n = 2 * kH; p.n_tile = 2 * kH; p.n_valid = 2 * kH; p.out_f32 = Ly.dhx + (size_t)k * B * 2 * kH; p.ldc = 2 * kH;
+                rc = launch_gemm(t, Ly.m_dg_bm, Ly.m_wcat_t, p, s, &Ly.m_dhx[k]);
+            } else {
+                // step 0 has no h_{-1} to differentiate: dx_0 = dgates_0 W_ih alone (N = 64)
+                p.n = kH; p.n_tile = kH; p.n_valid = kH; p.out_f32 = Ly.dhx + kH; p.ldc = 2 * kH;
+                rc = launch_gemm(t, Ly.m_dg_bm, Ly.m_wih_t, p, s, &Ly.m_dx0);
+            }
             if (rc != TACO_OK) return rc;
         }
-    }
-    {   // dWcat = dgates^T [h | x | 1 1] over all time steps: M = 256, N = ld_u, K = seq * batch (both operands read transposed)
-        GemmParams p;
-        memset(&p, 0, sizeof(p));
-        p.m = kG; p.n = t->ld_u; p.k = (int)SB; p.n_tile = pad16(t->ld_u); p.splits = t->lstm_splits; p.epi = EPI_F32; p.n_valid = pad16(t->ld_u);
-        p.out_f32 = t->lstm_partial; p.ldc = t->ld_u; p.split_stride = (long long)kG * t->ld_u;
-        if (p.n_valid > t->ld_u) p.n_valid = t->ld_u;
-        p.mn_major = 1;
-        rc = launch_gemm(t, t->m_dg_mn, t->m_u_mn, p, s, &t->m_lstm_partial);
-        if (rc != TACO_OK) return rc;
+        {   // dWcat = dgates^T [h | x | 1 1] over all time steps: M = 256, N = ld_u, K = seq * batch (both operands read transposed)
+            GemmParams p;
+            memset(&p, 0, sizeof(p));
+            p.m = kG; p.n = Ly.ld_u; p.k = (int)SB; p.n_tile = pad16(Ly.ld_u); p.splits = Ly.splits; p.epi = EPI_F32; p.n_valid = pad16(Ly.ld_u);
+            p.out_f32 = Ly.partial; p.ldc = Ly.ld_u; p.split_stride = (long long)kG * Ly.ld_u;
+            if (p.n_valid > Ly.ld_u) p.n_valid = Ly.ld_u;
+            p.mn_major = 1;
+            rc = launch_gemm(t, Ly.m_dg_mn, Ly.m_u_mn, p, s, &Ly.m_partial);
+            if (rc != TACO_OK) return rc;
+        }
     }
     // bias gradients = column sums of the batch-major dZ: partial rows here, summed by the assembly kernel below
     ColSumParams cs;
@@ -1025,16 +1115,17 @@ int taco_ppo_backward(TacoPPO* t, void* stream) {
             add(t->colsum_partial + (long long)(k * t->actor.L + l) * col_chunks * kColLd, col_chunks, kColLd, kColLd, 0, 1, n.s[l + 1], n.b_off[l]);
         }
     }
-    {
+    for (int l = 0; l < t->n_lstm; ++l) {
+        const LstmLayer& Ly = t->lstm[l];
         const int kb_total = (int)((SB + BK - 1) / BK);
-        int sp = t->lstm_splits > kb_total ? kb_total : t->lstm_splits;
+        int sp = Ly.splits > kb_total ? kb_total : Ly.splits;
         const int per = (kb_total + sp - 1) / sp;
         sp = (kb_total + per - 1) / per;
-        const long long stride = (long long)kG * t->ld_u;
-        add(t->lstm_partial, sp, stride, t->ld_u, 0, kG, kH, t->off_whh);
-        add(t->lstm_partial, sp, stride, t->ld_u, kH, kG, t->sd, t->off_wih);
-        add(t->lstm_partial, sp, stride, t->ld_u, kH + t->sd, kG, 1, t->off_bih);
-        add(t->lstm_partial, sp, stride, t->ld_u, kH + t->sd, kG, 1, t->off_bhh);
+        const long long stride = (long long)kG * Ly.ld_u;
+        add(Ly.partial, sp, stride, Ly.ld_u, 0, kG, kH, Ly.off_whh);
+        add(Ly.partial, sp, stride, Ly.ld_u, kH, kG, Ly.in, Ly.off_wih);
+        add(Ly.partial, sp, stride, Ly.ld_u, kH + Ly.in, kG, 1, Ly.off_bih);
+        add(Ly.partial, sp, stride, Ly.ld_u, kH + Ly.in, kG, 1, Ly.off_bhh);
     }
     gp.grad = t->grad; gp.acc = t->acc; gp.stop = t->stop;
     launch_pdl(grad_assemble_kernel, dim3((unsigned)((elems + 255) / 256)), dim3(256), 0, s, gp);

@@ -263,7 +263,7 @@ def sync_rollout_nets_native(native, actor=None, critic=None):
                    lipschitz_const=-1.0, log_std=v["log_std"])
     if critic is not None:
         n = native._cfg.n_critic_hidden + 1
-        critic.load([tuple(v[f"critic_encoder.layers.{k}_l0"] for k in ("weight_ih", "weight_hh", "bias_ih", "bias_hh"))],
+        critic.load([tuple(v[f"critic_encoder.layers.{k}_l{l}"] for k in ("weight_ih", "weight_hh", "bias_ih", "bias_hh")) for l in range(native.lstm_layers)],
                     [v[f"critic_mlp.layers.{2 * l}.weight"] for l in range(n)], [v[f"critic_mlp.layers.{2 * l}.bias"] for l in range(n)])
 
 

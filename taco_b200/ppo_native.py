@@ -2,7 +2,7 @@
 
 ``NativePPO`` owns the training state of one ``TorchActorCritic``-shaped agent on the device -- flat fp32 parameters, gradient,
 Adam moments -- and runs the reference's update (IsaacGymEnvs/algorithms/ppo_asymmetry.py:137-258) as a stream of kernel launches:
-gather -> tcgen05 GEMM forward (actor MLP; critic = 5 LSTM steps + MLP) -> loss / KL -> device-side early-stop decision ->
+gather -> tcgen05 GEMM forward (actor MLP; critic = 5 LSTM steps per stacked LSTM layer + MLP) -> loss / KL -> device-side early-stop decision ->
 GEMM backward (split-K weight gradients, LSTM backward through time) -> gradient norm + clip + Adam -> spectral projection of the
 actor weights -> bf16 re-pack.  Nothing synchronises with the host until ``end``: the KL early stop of :223-226 is a device flag.
 
@@ -35,8 +35,9 @@ class NativePPO:
         self.device = f"cuda:{self.device_id}"
         a_lin, c_lin = _linears(agent.actor_mlp), _linears(agent.critic_mlp)
         lstm = agent.critic_encoder.layers
-        if lstm.num_layers != 1 or lstm.bidirectional:
-            raise ValueError("NativePPO: one unidirectional LSTM layer")
+        if not 1 <= lstm.num_layers <= 4 or lstm.bidirectional:
+            raise ValueError("NativePPO: 1 to 4 unidirectional LSTM layers")
+        self.lstm_layers = int(lstm.num_layers)
         self.batch = int(batch)
         self.obs_dim, self.act_dim = a_lin[0].in_features, a_lin[-1].out_features
         self.state_dim, self.lstm_hidden = lstm.input_size, lstm.hidden_size
@@ -56,7 +57,7 @@ class NativePPO:
         self._lib = _capi.lib()
         self._h = None
         self._names = (["log_std"] + [f"actor_mlp.layers.{2 * l}.{k}" for l in range(len(a_lin)) for k in ("weight", "bias")] +
-                       [f"critic_encoder.layers.{k}_l0" for k in ("weight_ih", "weight_hh", "bias_ih", "bias_hh")] +
+                       [f"critic_encoder.layers.{k}_l{l}" for l in range(self.lstm_layers) for k in ("weight_ih", "weight_hh", "bias_ih", "bias_hh")] +
                        [f"critic_mlp.layers.{2 * l}.{k}" for l in range(len(c_lin)) for k in ("weight", "bias")])
         self._pending_agent = agent
 
@@ -64,7 +65,7 @@ class NativePPO:
     def _create(self, seq_len):
         self._cfg.seq_len = int(seq_len)
         h = C.c_void_p()
-        _capi.check(self._lib.taco_ppo_create(self.device_id, C.byref(self._cfg), C.byref(h)), "taco_ppo_create")
+        _capi.check(self._lib.taco_ppo_create_layers(self.device_id, C.byref(self._cfg), self.lstm_layers, C.byref(h)), "taco_ppo_create_layers")
         self._h = h
         n = C.c_int64()
         _capi.check(self._lib.taco_ppo_num_params(h, C.byref(n)), "taco_ppo_num_params")
