@@ -59,28 +59,25 @@ static EncodeTiledFn encode_fn() {
     }();
     return fn;
 }
-// row-major bf16 matrix [rows][cols], row pitch ld elements; box = 64 columns (one 128-byte swizzle row) x box_rows rows
-static bool make_map(CUtensorMap* tm, const bf16* ptr, long long rows, long long cols, long long ld, int box_rows) {
+// row-major matrix [rows][cols] of elem_bytes-sized elements, row pitch ld elements, 128-byte swizzle; box = box_cols x box_rows
+static bool encode_map(CUtensorMap* tm, CUtensorMapDataType type, size_t elem_bytes, const void* ptr, long long rows, long long cols, long long ld,
+                       int box_cols, int box_rows) {
     EncodeTiledFn f = encode_fn();
     if (!f) return false;
     const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    const cuuint64_t strides[1] = {(cuuint64_t)ld * sizeof(bf16)};
-    const cuuint32_t box[2] = {(cuuint32_t)BK, (cuuint32_t)box_rows};
+    const cuuint64_t strides[1] = {(cuuint64_t)ld * elem_bytes};
+    const cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
     const cuuint32_t estr[2] = {1, 1};
-    return f(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<bf16*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    return f(tm, type, 2, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+             CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-
-// fp32 [rows][cols] output of the split-K GEMMs, stored tile by tile (32 columns x 128 rows) by the TMA store engine
+// bf16 operand: box = 64 columns (one 128-byte swizzle row) x box_rows rows
+static bool make_map(CUtensorMap* tm, const bf16* ptr, long long rows, long long cols, long long ld, int box_rows) {
+    return encode_map(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, sizeof(bf16), ptr, rows, cols, ld, BK, box_rows);
+}
+// fp32 output of the split-K GEMMs, stored tile by tile (32 columns x 128 rows) by the TMA store engine
 static bool make_map_f32(CUtensorMap* tm, const float* ptr, long long rows, long long cols, long long ld) {
-    EncodeTiledFn f = encode_fn();
-    if (!f) return false;
-    const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    const cuuint64_t strides[1] = {(cuuint64_t)ld * sizeof(float)};
-    const cuuint32_t box[2] = {32u, (cuuint32_t)BM};
-    const cuuint32_t estr[2] = {1, 1};
-    return f(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    return encode_map(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, sizeof(float), ptr, rows, cols, ld, 32, BM);
 }
 
 // ---------------------------------------------------------------------------------------------- small kernels
@@ -507,21 +504,35 @@ using taco::DevGuard;
 using taco::fail;
 
 // ---------------------------------------------------------------------------------------------- the trainer object
-struct MlpNet {
-    int L = 0;                        // linear layers
-    int s[kMaxHiddenL + 2] = {0};     // sizes [in, h1, ..., out]
-    long long w_off[kMaxHiddenL + 1], b_off[kMaxHiddenL + 1];      // offsets into the flat parameter vector
-    bf16* wb[kMaxHiddenL + 1]; int ld_w[kMaxHiddenL + 1];          // [out_pad16][pad8(in)]
-    bf16* wt[kMaxHiddenL + 1]; int ld_t[kMaxHiddenL + 1];          // [in][pad8(out) (>= 16)]
-    bf16* x_bm[kMaxHiddenL + 1]; int ld_x[kMaxHiddenL + 1];        // activations X_0 .. X_{L-1}: [B][pad8(s_l)]
-    uint32_t* relu_mask[kMaxHiddenL + 1];                          // l >= 1: [ceil(s_l / 32)][B] words, bit j = pre-activation (sample, 32 c + j) > 0
-    bf16* dz_bm[kMaxHiddenL + 2];                                  // dZ_1 .. dZ_L (index l): [B][ld]
-    int ld_dz[kMaxHiddenL + 2];
-    float* partial[kMaxHiddenL + 1]; int splits[kMaxHiddenL + 1]; int ld_p[kMaxHiddenL + 1];
+// split-K plan of a GEMM of depth k: `splits` work items of kb_per_split k-blocks each, none of them empty
+struct SplitK { int splits = 1, kb_per_split = 1; };
+static SplitK split_k(int requested, long long k) {
+    const int kb_total = (int)((k + BK - 1) / BK);
+    SplitK r;
+    r.splits = requested < 1 ? 1 : (requested > kb_total ? kb_total : requested);
+    r.kb_per_split = (kb_total + r.splits - 1) / r.splits;
+    r.splits = (kb_total + r.kb_per_split - 1) / r.kb_per_split;      // merge the splits that would be left empty
+    return r;
+}
+
+// one linear layer Y = X W^T + b of an MLP (M = batch)
+struct MlpLayer {
+    int in = 0, out = 0;
+    long long w_off = 0, b_off = 0;                 // offsets into the flat parameter vector
+    bf16* wb = nullptr; int ld_w = 0;               // [out_pad16][pad8(in)]
+    bf16* wt = nullptr; int ld_t = 0;               // [in][pad8(out) (>= 16)]
+    bf16* x_bm = nullptr; int ld_x = 0;             // input activation X: [B][pad8(in)]
+    uint32_t* mask = nullptr;                       // layers >= 1: ReLU mask of X, [ceil(in / 32)][B] words, bit j = pre-activation (sample, 32 c + j) > 0
+    bf16* dz_bm = nullptr; int ld_dz = 0;           // dZ, the gradient of this layer's output pre-activation: [B][pad16(out)]
+    float* partial = nullptr; int ld_p = 0;         // dW split-K partials: [split.splits][out][ld_p]
+    SplitK split;
     // K-major maps (forward / dX GEMMs) and MN-major maps of the same batch-major tensors (dW = dZ^T X reads both transposed)
-    CUtensorMap m_x_bm[kMaxHiddenL + 1], m_x_mn[kMaxHiddenL + 1], m_w[kMaxHiddenL + 1], m_wt[kMaxHiddenL + 1];
-    CUtensorMap m_dz_bm[kMaxHiddenL + 2], m_dz_mn[kMaxHiddenL + 2];
-    CUtensorMap m_partial[kMaxHiddenL + 1]; bool partial_tma[kMaxHiddenL + 1];   // split-K partials as [splits * out][ld_p] fp32 (TMA-stored when out % 128 == 0)
+    CUtensorMap m_x_bm, m_x_mn, m_w, m_wt, m_dz_bm, m_dz_mn;
+    CUtensorMap m_partial;                          // only when out % 128 == 0: the partials are then TMA-stored
+};
+struct MlpNet {
+    int L = 0;                                      // linear layers
+    MlpLayer layer[kMaxHiddenL + 1];
 };
 
 // one layer k of the stacked LSTM encoder; its operand of step t is U_k[t] = [h^k_{t-1} | x^k_t | 1 1 | 0] with x^0_t = states[:, t] and
@@ -531,9 +542,9 @@ struct LstmLayer {
     long long off_wih = 0, off_whh = 0, off_bih = 0, off_bhh = 0;
     bf16 *wcat = nullptr, *wcat_t = nullptr;        // [256][ld_u], [t_rows][256] (W_hh^T, then W_ih^T for k >= 1)
     bf16 *u_bm = nullptr, *gates = nullptr, *dg_bm = nullptr;       // [seq*B][ld_u], [seq*B][256] x 2 (all time steps)
-    float *c_state = nullptr, *partial = nullptr;   // [seq*B][64]; dWcat split-K partials [splits][256][ld_u]
+    float *c_state = nullptr, *partial = nullptr;   // [seq*B][64]; dWcat split-K partials [split.splits][256][ld_u]
     float* dhx = nullptr;                           // k >= 1: [seq][B][128] = d[h_{t-1} | x_t] of step t (slot 0: the x half only)
-    int splits = 1;
+    SplitK split;
     CUtensorMap m_u_bm, m_u_mn, m_wcat, m_wcat_t, m_wih_t, m_dg_bm, m_dg_mn, m_partial;
     CUtensorMap m_dhx[kSeqMax], m_dx0;              // k >= 1: output maps of the d[h | x] GEMM per step, and of the dx-only GEMM of step 0
 };
@@ -564,13 +575,18 @@ struct TacoPPO {
     std::vector<void*> allocs;
 };
 
-
-template <typename T>
-static cudaError_t dev_alloc(TacoPPO* t, T** p, size_t count) {
-    cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
-    if (e == cudaSuccess) { e = cudaMemset(*p, 0, count * sizeof(T)); t->allocs.push_back((void*)*p); }
-    return e;
-}
+// zero-filled device allocations owned by t (the h_0 columns and the LSTM rings' zero padding rely on the zero fill).  The first
+// failure stays in `err` and turns every later call into a no-op, so a run of allocations is checked once, at its end.
+struct DevAlloc {
+    TacoPPO* t;
+    cudaError_t err = cudaSuccess;
+    template <typename T>
+    void operator()(T** p, size_t count) {
+        if (err != cudaSuccess) return;
+        err = cudaMalloc((void**)p, count * sizeof(T));
+        if (err == cudaSuccess) { err = cudaMemset(*p, 0, count * sizeof(T)); t->allocs.push_back((void*)*p); }
+    }
+};
 
 // launch with programmatic stream serialization: the kernel may be scheduled while its predecessor in the stream drains; every
 // kernel launched this way starts with pdl_wait() (gemm_tc.cuh)
@@ -586,18 +602,27 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
-// c: tensor map of the output when the epilogue stores through TMA (p.tma_store is set from it)
-static int launch_gemm(TacoPPO* t, const CUtensorMap& a, const CUtensorMap& b, GemmParams p, cudaStream_t s, const CUtensorMap* c = nullptr) {
-    const int kb_total = (p.k + BK - 1) / BK;
-    if (p.splits < 1) p.splits = 1;
-    if (p.splits > kb_total) p.splits = kb_total;
-    p.kb_per_split = (kb_total + p.splits - 1) / p.splits;
-    p.splits = (kb_total + p.kb_per_split - 1) / p.kb_per_split;       // no empty split
+// c: tensor map of the output when the epilogue stores through TMA (p.tma_store is set from it); sk: split-K plan (null: one split)
+static int launch_gemm(TacoPPO* t, const CUtensorMap& a, const CUtensorMap& b, GemmParams p, cudaStream_t s, const CUtensorMap* c = nullptr,
+                       const SplitK* sk = nullptr) {
+    const SplitK plan = sk ? *sk : split_k(1, p.k);
+    p.splits = plan.splits; p.kb_per_split = plan.kb_per_split;
     p.stop = t->stop;
     const int total = ((p.m + BM - 1) / BM) * p.splits;
     const int grid = total < t->num_sms ? total : t->num_sms;
     p.tma_store = c != nullptr;
     return launch_pdl(gemm_tc_kernel, dim3(grid), dim3(kGemmThreads), kGemmSmem, s, a, b, c ? *c : a, p) == cudaSuccess ? TACO_OK : fail(TACO_E_CUDA, "gemm_tc_kernel launch failed");
+}
+
+// weight gradient dW = dY^T X over K = batch rows, both operands batch-major and read transposed (MN-major): M = out, N = in.  Writes
+// the fp32 split-K partials [sk.splits][m][ldc], padding columns included, through the TMA store engine when m is a multiple of 128
+// (m_partial is only encoded then)
+static int launch_wgrad(TacoPPO* t, const CUtensorMap& dy_mn, const CUtensorMap& x_mn, int m, int n, long long k, float* partial, int ldc,
+                        const SplitK& sk, const CUtensorMap& m_partial, cudaStream_t s) {
+    GemmParams p{};
+    p.m = m; p.n = n; p.k = (int)k; p.n_tile = pad16(n); p.mn_major = 1;
+    p.epi = EPI_F32; p.n_valid = ldc; p.out_f32 = partial; p.ldc = ldc; p.split_stride = (long long)m * ldc;
+    return launch_gemm(t, dy_mn, x_mn, p, s, m % BM == 0 ? &m_partial : nullptr, &sk);
 }
 
 static int splits_for(int m, long long k, int num_sms) {
@@ -608,37 +633,39 @@ static int splits_for(int m, long long k, int num_sms) {
     return s < 1 ? 1 : s;
 }
 
-static int setup_net(TacoPPO* t, MlpNet& n, long long& off, bool actor) {
+// layer sizes (in -> hidden[0 .. n_hidden) -> out), parameter offsets, buffers and tensor maps of one MLP
+static int setup_net(TacoPPO* t, MlpNet& n, int in, const int32_t* hidden, int n_hidden, int out, long long& off) {
     const int B = t->B;
+    n.L = n_hidden + 1;
+    DevAlloc alloc{t};
     for (int l = 0; l < n.L; ++l) {
-        const int in = n.s[l], out = n.s[l + 1];
-        n.w_off[l] = off; off += (long long)in * out;
-        n.b_off[l] = off; off += out;
-        n.ld_w[l] = pad8(in);
-        n.ld_t[l] = pad8(out) < 16 ? 16 : pad8(out);
-        if (dev_alloc(t, &n.wb[l], (size_t)pad16(out) * n.ld_w[l]) != cudaSuccess) return TACO_E_NOMEM;
-        if (dev_alloc(t, &n.wt[l], (size_t)pad8(in) * n.ld_t[l]) != cudaSuccess) return TACO_E_NOMEM;
-        n.ld_x[l] = pad8(in);
-        if (dev_alloc(t, &n.x_bm[l], (size_t)B * n.ld_x[l]) != cudaSuccess) return TACO_E_NOMEM;
-        n.relu_mask[l] = nullptr;
-        if (l > 0 && dev_alloc(t, &n.relu_mask[l], (size_t)((in + 31) / 32) * B) != cudaSuccess) return TACO_E_NOMEM;
-        const int lz = l + 1;
-        n.ld_dz[lz] = pad16(out);
-        if (dev_alloc(t, &n.dz_bm[lz], (size_t)B * n.ld_dz[lz]) != cudaSuccess) return TACO_E_NOMEM;
-        n.splits[l] = splits_for(out, B, t->num_sms);
-        n.ld_p[l] = pad16(in);
-        if (dev_alloc(t, &n.partial[l], (size_t)n.splits[l] * out * n.ld_p[l]) != cudaSuccess) return TACO_E_NOMEM;
-        bool ok = make_map(&n.m_x_bm[l], n.x_bm[l], B, in, n.ld_x[l], BM);
-        ok = ok && make_map(&n.m_x_mn[l], n.x_bm[l], B, n.ld_x[l], n.ld_x[l], BK);           // B operand of the dW GEMM (MN-major: 64 x 64 boxes)
-        ok = ok && make_map(&n.m_w[l], n.wb[l], out, in, n.ld_w[l], pad16(out));             // B operand of the forward GEMM
-        ok = ok && make_map(&n.m_wt[l], n.wt[l], in, pad8(out) < 16 ? 16 : out, n.ld_t[l], pad16(in));   // B operand of the dX GEMM
-        ok = ok && make_map(&n.m_dz_bm[lz], n.dz_bm[lz], B, n.ld_dz[lz], n.ld_dz[lz], BM);   // A operand of the dX GEMM
-        ok = ok && make_map(&n.m_dz_mn[lz], n.dz_bm[lz], B, n.ld_dz[lz], n.ld_dz[lz], BK);   // A operand of the dW GEMM (MN-major)
-        n.partial_tma[l] = out % BM == 0;
-        if (n.partial_tma[l]) ok = ok && make_map_f32(&n.m_partial[l], n.partial[l], (long long)n.splits[l] * out, n.ld_p[l], n.ld_p[l]);
+        MlpLayer& Ly = n.layer[l];
+        Ly.in = l == 0 ? in : hidden[l - 1];
+        Ly.out = l + 1 < n.L ? hidden[l] : out;
+        Ly.w_off = off; off += (long long)Ly.in * Ly.out;
+        Ly.b_off = off; off += Ly.out;
+        Ly.ld_w = pad8(Ly.in);
+        Ly.ld_t = pad8(Ly.out) < 16 ? 16 : pad8(Ly.out);
+        alloc(&Ly.wb, (size_t)pad16(Ly.out) * Ly.ld_w);
+        alloc(&Ly.wt, (size_t)pad8(Ly.in) * Ly.ld_t);
+        Ly.ld_x = pad8(Ly.in);
+        alloc(&Ly.x_bm, (size_t)B * Ly.ld_x);
+        if (l > 0) alloc(&Ly.mask, (size_t)((Ly.in + 31) / 32) * B);
+        Ly.ld_dz = pad16(Ly.out);
+        alloc(&Ly.dz_bm, (size_t)B * Ly.ld_dz);
+        Ly.split = split_k(splits_for(Ly.out, B, t->num_sms), B);
+        Ly.ld_p = pad16(Ly.in);
+        alloc(&Ly.partial, (size_t)Ly.split.splits * Ly.out * Ly.ld_p);
+        if (alloc.err != cudaSuccess) return TACO_E_NOMEM;
+        bool ok = make_map(&Ly.m_x_bm, Ly.x_bm, B, Ly.in, Ly.ld_x, BM);
+        ok = ok && make_map(&Ly.m_x_mn, Ly.x_bm, B, Ly.ld_x, Ly.ld_x, BK);                    // B operand of the dW GEMM (MN-major: 64 x 64 boxes)
+        ok = ok && make_map(&Ly.m_w, Ly.wb, Ly.out, Ly.in, Ly.ld_w, pad16(Ly.out));           // B operand of the forward GEMM
+        ok = ok && make_map(&Ly.m_wt, Ly.wt, Ly.in, pad8(Ly.out) < 16 ? 16 : Ly.out, Ly.ld_t, pad16(Ly.in));   // B operand of the dX GEMM
+        ok = ok && make_map(&Ly.m_dz_bm, Ly.dz_bm, B, Ly.ld_dz, Ly.ld_dz, BM);                // A operand of the dX GEMM
+        ok = ok && make_map(&Ly.m_dz_mn, Ly.dz_bm, B, Ly.ld_dz, Ly.ld_dz, BK);                // A operand of the dW GEMM (MN-major)
+        if (Ly.out % BM == 0) ok = ok && make_map_f32(&Ly.m_partial, Ly.partial, (long long)Ly.split.splits * Ly.out, Ly.ld_p, Ly.ld_p);
         if (!ok) return fail(TACO_E_CUDA, "cuTensorMapEncodeTiled failed");
     }
-    (void)actor;
     return TACO_OK;
 }
 
@@ -681,11 +708,8 @@ int taco_ppo_create_layers(int device, const TacoPPOCfg* cfg, int32_t lstm_layer
     // ---- flat parameter layout: log_std | actor MLP (W, b per layer) | LSTM W_ih, W_hh, b_ih, b_hh per layer (bottom first) | critic MLP
     long long off = 0;
     t->off_log_std = off; off += t->A;
-    t->actor.L = cfg->n_actor_hidden + 1;
-    t->actor.s[0] = cfg->obs_dim;
-    for (int l = 0; l < cfg->n_actor_hidden; ++l) t->actor.s[l + 1] = cfg->actor_hidden[l];
-    t->actor.s[t->actor.L] = t->A;
-    if ((rc = setup_net(t, t->actor, off, true)) != TACO_OK) return bail(rc, "taco_ppo_create: actor buffers");
+    if ((rc = setup_net(t, t->actor, cfg->obs_dim, cfg->actor_hidden, cfg->n_actor_hidden, t->A, off)) != TACO_OK)
+        return bail(rc, "taco_ppo_create: actor buffers");
     for (int k = 0; k < t->n_lstm; ++k) {
         LstmLayer& Ly = t->lstm[k];
         Ly.in = k == 0 ? t->sd : kH;
@@ -696,60 +720,60 @@ int taco_ppo_create_layers(int device, const TacoPPOCfg* cfg, int32_t lstm_layer
         Ly.off_bih = off; off += kG;
         Ly.off_bhh = off; off += kG;
     }
-    t->critic.L = cfg->n_critic_hidden + 1;
-    t->critic.s[0] = kH;
-    for (int l = 0; l < cfg->n_critic_hidden; ++l) t->critic.s[l + 1] = cfg->critic_hidden[l];
-    t->critic.s[t->critic.L] = 1;
-    if ((rc = setup_net(t, t->critic, off, false)) != TACO_OK) return bail(rc, "taco_ppo_create: critic buffers");
+    if ((rc = setup_net(t, t->critic, kH, cfg->critic_hidden, cfg->n_critic_hidden, 1, off)) != TACO_OK)
+        return bail(rc, "taco_ppo_create: critic buffers");
     t->n_params = off;
-    cudaError_t ce = dev_alloc(t, &t->prm, (size_t)off);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->grad, (size_t)off);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->adam_m, (size_t)off);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->adam_v, (size_t)off);
+    DevAlloc alloc{t};
+    alloc(&t->prm, (size_t)off);
+    alloc(&t->grad, (size_t)off);
+    alloc(&t->adam_m, (size_t)off);
+    alloc(&t->adam_v, (size_t)off);
     // ---- LSTM buffers
     const long long SB = (long long)t->seq * B;
     for (int k = 0; k < t->n_lstm; ++k) {
         LstmLayer& Ly = t->lstm[k];
-        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.wcat, (size_t)kG * Ly.ld_u);
-        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.wcat_t, (size_t)Ly.t_rows * kG);
-        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.u_bm, (size_t)SB * Ly.ld_u);
-        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.gates, (size_t)SB * kG);
-        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.dg_bm, (size_t)SB * kG);
-        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.c_state, (size_t)SB * kH);
-        Ly.splits = splits_for(kG, SB, t->num_sms);
-        if (ce == cudaSuccess) ce = dev_alloc(t, &Ly.partial, (size_t)Ly.splits * kG * Ly.ld_u);
-        if (k > 0 && ce == cudaSuccess) ce = dev_alloc(t, &Ly.dhx, (size_t)SB * 2 * kH);
-        if (k > 0 && ce == cudaSuccess) {
+        alloc(&Ly.wcat, (size_t)kG * Ly.ld_u);
+        alloc(&Ly.wcat_t, (size_t)Ly.t_rows * kG);
+        alloc(&Ly.u_bm, (size_t)SB * Ly.ld_u);
+        alloc(&Ly.gates, (size_t)SB * kG);
+        alloc(&Ly.dg_bm, (size_t)SB * kG);
+        alloc(&Ly.c_state, (size_t)SB * kH);
+        Ly.split = split_k(splits_for(kG, SB, t->num_sms), SB);
+        alloc(&Ly.partial, (size_t)Ly.split.splits * kG * Ly.ld_u);
+        if (k > 0) alloc(&Ly.dhx, (size_t)SB * 2 * kH);
+        if (k > 0 && alloc.err == cudaSuccess) {
             // the constant-1 columns of U_k (layer 0's come with the gather); the h columns of slot 0 (h_0 = 0) stay as allocated
             const uint32_t ones = 0x3F803F80u;                            // two bf16 1.0
             std::vector<uint32_t> col((size_t)SB, ones);
-            ce = cudaMemcpy2D(Ly.u_bm + kH + Ly.in, (size_t)Ly.ld_u * sizeof(bf16), col.data(), sizeof(uint32_t), sizeof(uint32_t), (size_t)SB,
-                              cudaMemcpyHostToDevice);
+            alloc.err = cudaMemcpy2D(Ly.u_bm + kH + Ly.in, (size_t)Ly.ld_u * sizeof(bf16), col.data(), sizeof(uint32_t), sizeof(uint32_t), (size_t)SB,
+                                     cudaMemcpyHostToDevice);
         }
     }
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->colsum_partial, (size_t)2 * (kMaxHiddenL + 1) * ((B + kColRows - 1) / kColRows) * kColLd);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->dh, (size_t)B * kH);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->dc, (size_t)B * kH);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->mean, (size_t)B * t->A);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->value, (size_t)B);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->g_act, (size_t)B * t->A);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->g_logp, (size_t)B);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->g_adv, (size_t)B);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->g_ret, (size_t)B);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->acc, (size_t)kNumStat);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->log, (size_t)t->max_log * kLogCols);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->n_logged, 1);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->stop, 1);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->step, 1);
-    if (ce == cudaSuccess) ce = dev_alloc(t, &t->spec_sigma, (size_t)(kMaxHiddenL + 1));
-    for (int l = 0; l < t->actor.L && ce == cudaSuccess; ++l) {
-        ce = dev_alloc(t, &t->spec_v[l], (size_t)t->actor.s[l]);
-        if (ce == cudaSuccess) {
-            std::vector<float> ones((size_t)t->actor.s[l], 1.0f / std::sqrt((float)t->actor.s[l]));
-            ce = cudaMemcpy(t->spec_v[l], ones.data(), ones.size() * sizeof(float), cudaMemcpyHostToDevice);
+    alloc(&t->colsum_partial, (size_t)2 * (kMaxHiddenL + 1) * ((B + kColRows - 1) / kColRows) * kColLd);
+    alloc(&t->dh, (size_t)B * kH);
+    alloc(&t->dc, (size_t)B * kH);
+    alloc(&t->mean, (size_t)B * t->A);
+    alloc(&t->value, (size_t)B);
+    alloc(&t->g_act, (size_t)B * t->A);
+    alloc(&t->g_logp, (size_t)B);
+    alloc(&t->g_adv, (size_t)B);
+    alloc(&t->g_ret, (size_t)B);
+    alloc(&t->acc, (size_t)kNumStat);
+    alloc(&t->log, (size_t)t->max_log * kLogCols);
+    alloc(&t->n_logged, 1);
+    alloc(&t->stop, 1);
+    alloc(&t->step, 1);
+    alloc(&t->spec_sigma, (size_t)(kMaxHiddenL + 1));
+    for (int l = 0; l < t->actor.L; ++l) {
+        const int in = t->actor.layer[l].in;
+        alloc(&t->spec_v[l], (size_t)in);
+        if (alloc.err == cudaSuccess) {
+            std::vector<float> ones((size_t)in, 1.0f / std::sqrt((float)in));
+            alloc.err = cudaMemcpy(t->spec_v[l], ones.data(), ones.size() * sizeof(float), cudaMemcpyHostToDevice);
         }
     }
-    if (ce != cudaSuccess) return bail(ce == cudaErrorMemoryAllocation ? TACO_E_NOMEM : TACO_E_CUDA, "taco_ppo_create: device allocation failed");
+    if (alloc.err != cudaSuccess)
+        return bail(alloc.err == cudaErrorMemoryAllocation ? TACO_E_NOMEM : TACO_E_CUDA, "taco_ppo_create: device allocation failed");
     bool ok = true;
     for (int k = 0; k < t->n_lstm; ++k) {
         LstmLayer& Ly = t->lstm[k];
@@ -759,7 +783,7 @@ int taco_ppo_create_layers(int device, const TacoPPOCfg* cfg, int32_t lstm_layer
         ok = ok && make_map(&Ly.m_wcat_t, Ly.wcat_t, Ly.t_rows, kG, kG, Ly.t_rows);      // B operand of d[h | x] (k >= 1) or dh (k = 0)
         ok = ok && make_map(&Ly.m_dg_bm, Ly.dg_bm, SB, kG, kG, BM);
         ok = ok && make_map(&Ly.m_dg_mn, Ly.dg_bm, SB, kG, kG, BK);
-        ok = ok && make_map_f32(&Ly.m_partial, Ly.partial, (long long)Ly.splits * kG, Ly.ld_u, Ly.ld_u);
+        ok = ok && make_map_f32(&Ly.m_partial, Ly.partial, (long long)Ly.split.splits * kG, Ly.ld_u, Ly.ld_u);
         if (k > 0) {
             ok = ok && make_map(&Ly.m_wih_t, Ly.wcat_t + (size_t)kH * kG, kH, kG, kG, kH);   // W_ih^T alone: the dx-only GEMM of step 0
             for (int s = 0; s < t->seq; ++s) ok = ok && make_map_f32(&Ly.m_dhx[s], Ly.dhx + (size_t)s * B * 2 * kH, B, 2 * kH, 2 * kH);
@@ -801,12 +825,12 @@ int taco_ppo_param_offsets(TacoPPO* t, int64_t* offsets, int32_t count, int32_t*
     if (!t || !offsets || !n_out) return fail(TACO_E_INVALID, "taco_ppo_param_offsets: null argument");
     std::vector<int64_t> v;
     v.push_back(t->off_log_std);
-    for (int l = 0; l < t->actor.L; ++l) { v.push_back(t->actor.w_off[l]); v.push_back(t->actor.b_off[l]); }
+    for (int l = 0; l < t->actor.L; ++l) { v.push_back(t->actor.layer[l].w_off); v.push_back(t->actor.layer[l].b_off); }
     for (int k = 0; k < t->n_lstm; ++k) {
         const LstmLayer& Ly = t->lstm[k];
         v.push_back(Ly.off_wih); v.push_back(Ly.off_whh); v.push_back(Ly.off_bih); v.push_back(Ly.off_bhh);
     }
-    for (int l = 0; l < t->critic.L; ++l) { v.push_back(t->critic.w_off[l]); v.push_back(t->critic.b_off[l]); }
+    for (int l = 0; l < t->critic.L; ++l) { v.push_back(t->critic.layer[l].w_off); v.push_back(t->critic.layer[l].b_off); }
     if ((int)v.size() > count) return fail(TACO_E_INVALID, "taco_ppo_param_offsets: buffer too small");
     for (size_t i = 0; i < v.size(); ++i) offsets[i] = v[i];
     *n_out = (int32_t)v.size();
@@ -834,22 +858,25 @@ static int join_actor(TacoPPO* t, cudaStream_t s) {
     return TACO_OK;
 }
 
-// which: 0 = everything, 1 = the actor's matrices only, 2 = critic MLP + LSTM only
-static int repack(TacoPPO* t, cudaStream_t s, bool honour_stop, int which = 0) {
+// the networks whose bf16 operand copies repack() refreshes; the critic's include its LSTM
+enum PackNets { kPackActor = 1, kPackCritic = 2, kPackBoth = kPackActor | kPackCritic };
+
+static int repack(TacoPPO* t, cudaStream_t s, bool honour_stop, PackNets nets) {
     PackParams pp;
     memset(&pp, 0, sizeof(pp));
-    for (int k = 0; k < 2; ++k) {
-        if ((which == 1 && k == 1) || (which == 2 && k == 0)) continue;
-        MlpNet& n = k == 0 ? t->actor : t->critic;
+    auto add = [&](const MlpNet& n) {
         for (int l = 0; l < n.L; ++l) {
+            const MlpLayer& Ly = n.layer[l];
             PackSeg& S = pp.seg[pp.n_seg++];
-            S.w = t->prm + n.w_off[l]; S.out = n.s[l + 1]; S.in = n.s[l];
-            S.wb = n.wb[l]; S.ld_w = n.ld_w[l]; S.wt = n.wt[l]; S.ld_t = n.ld_t[l]; S.rows_t = pad8(n.s[l]);
+            S.w = t->prm + Ly.w_off; S.out = Ly.out; S.in = Ly.in;
+            S.wb = Ly.wb; S.ld_w = Ly.ld_w; S.wt = Ly.wt; S.ld_t = Ly.ld_t; S.rows_t = pad8(Ly.in);
         }
-    }
+    };
+    if (nets & kPackActor) add(t->actor);
+    if (nets & kPackCritic) add(t->critic);
     pp.stop = honour_stop ? t->stop : nullptr;
     launch_pdl(pack_kernel, dim3(32, pp.n_seg), dim3(256), 0, s, pp);
-    if (which != 1) {
+    if (nets & kPackCritic) {
         for (int k = 0; k < t->n_lstm; ++k) {
             const LstmLayer& Ly = t->lstm[k];
             launch_pdl(pack_lstm_kernel, dim3(64), dim3(256), 0, s, (const float*)(t->prm + Ly.off_wih), (const float*)(t->prm + Ly.off_whh),
@@ -866,7 +893,7 @@ int taco_ppo_params_changed(TacoPPO* t, void* stream) {
     DevGuard guard(t->device);
     const int rcj = join_actor(t, (cudaStream_t)stream);
     if (rcj != TACO_OK) return rcj;
-    return repack(t, (cudaStream_t)stream, false);
+    return repack(t, (cudaStream_t)stream, false, kPackBoth);
 }
 
 // start of one PPO.update: clears the early-stop flag and the log
@@ -889,49 +916,43 @@ static Hyper to_hyper(const TacoPPOHyper* h) {
 
 static int mlp_forward(TacoPPO* t, MlpNet& n, bool actor, cudaStream_t s) {
     for (int l = 0; l < n.L; ++l) {
-        GemmParams p;
-        memset(&p, 0, sizeof(p));
-        p.m = t->B; p.n = n.s[l + 1]; p.k = n.s[l]; p.n_tile = pad16(n.s[l + 1]); p.splits = 1;
-        p.bias = t->prm + n.b_off[l];
-        if (l + 1 < n.L) {
-            p.epi = EPI_BIAS_RELU; p.n_valid = pad8(n.s[l + 1]);
-            p.mask_out = n.relu_mask[l + 1]; p.ld_mask = t->B;
+        const MlpLayer& Ly = n.layer[l];
+        const MlpLayer* next = l + 1 < n.L ? &n.layer[l + 1] : nullptr;
+        GemmParams p{};
+        p.m = t->B; p.n = Ly.out; p.k = Ly.in; p.n_tile = pad16(Ly.out);
+        p.bias = t->prm + Ly.b_off;
+        if (next) {
+            p.epi = EPI_BIAS_RELU; p.n_valid = pad8(Ly.out);
+            p.mask_out = next->mask; p.ld_mask = t->B;
         } else if (actor) {
             p.epi = EPI_TANH_F32; p.n_valid = t->A; p.out_f32 = t->mean; p.ldc = t->A;
         } else {
             p.epi = EPI_F32; p.n_valid = 1; p.out_f32 = t->value; p.ldc = 1;
         }
-        const int rc = launch_gemm(t, n.m_x_bm[l], n.m_w[l], p, s, l + 1 < n.L ? &n.m_x_bm[l + 1] : nullptr);   // X_{l+1} leaves through its own (operand) map
+        const int rc = launch_gemm(t, Ly.m_x_bm, Ly.m_w, p, s, next ? &next->m_x_bm : nullptr);   // the next layer's X leaves through its own (operand) map
         if (rc != TACO_OK) return rc;
     }
     return TACO_OK;
 }
 
-// backward of an MLP whose dZ_L (both layouts) is already written.  dx_out != null: also d loss / d input as fp32 [B][s0] (critic -> LSTM)
-static int mlp_backward(TacoPPO* t, MlpNet& n, float* dx_out, cudaStream_t s) {
+// backward of an MLP whose last layer's dZ (both layouts) is already written.  dx_out != null: also d loss / d input as fp32 [B][in]
+// (critic -> LSTM), stored through dx_map when that is not null
+static int mlp_backward(TacoPPO* t, MlpNet& n, float* dx_out, const CUtensorMap* dx_map, cudaStream_t s) {
     for (int l = n.L - 1; l >= 0; --l) {
-        const int lz = l + 1, in = n.s[l], out = n.s[l + 1];
-        {   // dW_l = dZ^T X_{l-1}: M = out, N = in, K = batch
-            GemmParams p;
-            memset(&p, 0, sizeof(p));
-            p.m = out; p.n = in; p.k = t->B; p.n_tile = pad16(in); p.splits = n.splits[l];
-            p.epi = EPI_F32; p.n_valid = pad16(in);
-            p.out_f32 = n.partial[l]; p.ldc = n.ld_p[l]; p.split_stride = (long long)out * n.ld_p[l];
-            p.mn_major = 1;
-            const int rc = launch_gemm(t, n.m_dz_mn[lz], n.m_x_mn[l], p, s, n.partial_tma[l] ? &n.m_partial[l] : nullptr);
-            if (rc != TACO_OK) return rc;
-        }
-        if (l > 0 || dx_out) {   // dX_{l-1} = dZ W_l: M = batch, N = in, K = out
-            GemmParams p;
-            memset(&p, 0, sizeof(p));
-            p.m = t->B; p.n = in; p.k = n.ld_dz[lz] < n.ld_t[l] ? n.ld_dz[lz] : n.ld_t[l]; p.n_tile = pad16(in); p.splits = 1;
+        const MlpLayer& Ly = n.layer[l];
+        // dW = dZ^T X: M = out, N = in, K = batch
+        int rc = launch_wgrad(t, Ly.m_dz_mn, Ly.m_x_mn, Ly.out, Ly.in, t->B, Ly.partial, Ly.ld_p, Ly.split, Ly.m_partial, s);
+        if (rc != TACO_OK) return rc;
+        if (l > 0 || dx_out) {   // dX = dZ W, through the ReLU mask of X into the dZ of layer l - 1: M = batch, N = in, K = out
+            GemmParams p{};
+            p.m = t->B; p.n = Ly.in; p.k = Ly.ld_dz < Ly.ld_t ? Ly.ld_dz : Ly.ld_t; p.n_tile = pad16(Ly.in);
             if (l > 0) {
-                p.epi = EPI_RELUBWD; p.n_valid = pad8(in);
-                p.mask_in = n.relu_mask[l]; p.ld_mask = t->B;
+                p.epi = EPI_RELUBWD; p.n_valid = pad8(Ly.in);
+                p.mask_in = Ly.mask; p.ld_mask = t->B;
             } else {
-                p.epi = EPI_F32; p.n_valid = in; p.out_f32 = dx_out; p.ldc = in;
+                p.epi = EPI_F32; p.n_valid = Ly.in; p.out_f32 = dx_out; p.ldc = Ly.in;
             }
-            const int rc = launch_gemm(t, n.m_dz_bm[lz], n.m_wt[l], p, s, l > 0 ? &n.m_dz_bm[l] : (dx_out == t->dh ? &t->m_dh : nullptr));
+            rc = launch_gemm(t, Ly.m_dz_bm, Ly.m_wt, p, s, l > 0 ? &n.layer[l - 1].m_dz_bm : dx_map);
             if (rc != TACO_OK) return rc;
         }
     }
@@ -949,7 +970,7 @@ int taco_ppo_forward_loss(TacoPPO* t, const TacoPPOHyper* hyper, const float* ob
     memset(&g, 0, sizeof(g));
     g.obs = obs; g.obs_dim = t->cfg.obs_dim; g.states = states; g.seq = t->seq; g.state_dim = t->sd;
     g.act = act; g.logp = old_logp; g.adv = adv; g.ret = ret; g.idx = (const long long*)idx_dev; g.B = B; g.act_dim = t->A;
-    g.x0_bm = t->actor.x_bm[0]; g.ld_x0 = t->actor.ld_x[0];
+    g.x0_bm = t->actor.layer[0].x_bm; g.ld_x0 = t->actor.layer[0].ld_x;
     g.u_bm = t->lstm[0].u_bm; g.ld_u = t->lstm[0].ld_u;
     g.g_act = t->g_act; g.g_logp = t->g_logp; g.g_adv = t->g_adv; g.g_ret = t->g_ret; g.stop = t->stop;
     launch_pdl(gather_kernel, dim3((B + 31) / 32), dim3(256), 0, s, g);
@@ -961,9 +982,8 @@ int taco_ppo_forward_loss(TacoPPO* t, const TacoPPOHyper* hyper, const float* ob
         const LstmLayer& Ly = t->lstm[l];
         const LstmLayer* up = l + 1 < t->n_lstm ? &t->lstm[l + 1] : nullptr;
         for (int k = 0; k < t->seq; ++k) {
-            GemmParams p;
-            memset(&p, 0, sizeof(p));
-            p.m = B; p.n = kG; p.k = Ly.ld_u; p.n_tile = kG; p.splits = 1; p.a_row0 = k * B; p.epi = EPI_LSTM; p.n_valid = kG;
+            GemmParams p{};
+            p.m = B; p.n = kG; p.k = Ly.ld_u; p.n_tile = kG; p.a_row0 = k * B; p.epi = EPI_LSTM; p.n_valid = kG;
             p.lstm.c_prev = k > 0 ? Ly.c_state + (size_t)(k - 1) * B * kH : nullptr;
             p.lstm.c_out = Ly.c_state + (size_t)k * B * kH;
             p.lstm.gates_out = Ly.gates + (size_t)k * B * kG;
@@ -974,7 +994,7 @@ int taco_ppo_forward_loss(TacoPPO* t, const TacoPPOHyper* hyper, const float* ob
             } else if (up) {
                 p.lstm.h_bm = h_up; p.lstm.ld_h_bm = up->ld_u;
             } else {
-                p.lstm.h_bm = t->critic.x_bm[0]; p.lstm.ld_h_bm = t->critic.ld_x[0];
+                p.lstm.h_bm = t->critic.layer[0].x_bm; p.lstm.ld_h_bm = t->critic.layer[0].ld_x;
             }
             rc = launch_gemm(t, Ly.m_u_bm, Ly.m_wcat, p, s);
             if (rc != TACO_OK) return rc;
@@ -990,8 +1010,8 @@ int taco_ppo_forward_loss(TacoPPO* t, const TacoPPOHyper* hyper, const float* ob
     memset(&L, 0, sizeof(L));
     L.mean = t->mean; L.value = t->value; L.act = t->g_act; L.old_logp = t->g_logp; L.adv = t->g_adv; L.ret = t->g_ret;
     L.log_std = t->prm + t->off_log_std; L.B = B; L.act_dim = t->A; L.h = to_hyper(hyper);
-    L.dz_bm = t->actor.dz_bm[t->actor.L];
-    L.dv_bm = t->critic.dz_bm[t->critic.L];
+    L.dz_bm = t->actor.layer[t->actor.L - 1].dz_bm;
+    L.dv_bm = t->critic.layer[t->critic.L - 1].dz_bm;
     L.acc = t->acc; L.stop = t->stop;
     launch_pdl(loss_kernel, dim3((B + 255) / 256), dim3(256), 0, s, L);
     TACO_CUDA(cudaGetLastError());
@@ -1026,9 +1046,9 @@ int taco_ppo_backward(TacoPPO* t, void* stream) {
     DevGuard guard(t->device);
     cudaStream_t s = (cudaStream_t)stream;
     const int B = t->B;
-    int rc = mlp_backward(t, t->actor, nullptr, s);
+    int rc = mlp_backward(t, t->actor, nullptr, nullptr, s);
     if (rc != TACO_OK) return rc;
-    rc = mlp_backward(t, t->critic, t->dh, s);
+    rc = mlp_backward(t, t->critic, t->dh, &t->m_dh, s);
     if (rc != TACO_OK) return rc;
     const long long SB = (long long)t->seq * B;
     // LSTM backward through time, top layer first.  Layer 0 back-propagates dh_{t-1} = dgates_t W_hh (N = 64) into t->dh; a layer
@@ -1051,9 +1071,8 @@ int taco_ppo_backward(TacoPPO* t, void* stream) {
             b.c_prev = k > 0 ? Ly.c_state + (size_t)(k - 1) * B * kH : nullptr; b.c_cur = Ly.c_state + (size_t)k * B * kH;
             b.dg_bm = Ly.dg_bm + (size_t)k * B * kG; b.B = B; b.first = (k == t->seq - 1); b.stop = t->stop;
             launch_pdl(lstm_bwd_kernel, dim3((B + 3) / 4), dim3(256), 0, s, b);
-            GemmParams p;
-            memset(&p, 0, sizeof(p));
-            p.m = B; p.k = kG; p.splits = 1; p.a_row0 = k * B; p.epi = EPI_F32;
+            GemmParams p{};
+            p.m = B; p.k = kG; p.a_row0 = k * B; p.epi = EPI_F32;
             if (l == 0) {
                 if (k == 0) continue;
                 // dh_{t-1} = dgates_t W_hh: M = batch, N = 64, K = 256
@@ -1070,63 +1089,43 @@ int taco_ppo_backward(TacoPPO* t, void* stream) {
             }
             if (rc != TACO_OK) return rc;
         }
-        {   // dWcat = dgates^T [h | x | 1 1] over all time steps: M = 256, N = ld_u, K = seq * batch (both operands read transposed)
-            GemmParams p;
-            memset(&p, 0, sizeof(p));
-            p.m = kG; p.n = Ly.ld_u; p.k = (int)SB; p.n_tile = pad16(Ly.ld_u); p.splits = Ly.splits; p.epi = EPI_F32; p.n_valid = pad16(Ly.ld_u);
-            p.out_f32 = Ly.partial; p.ldc = Ly.ld_u; p.split_stride = (long long)kG * Ly.ld_u;
-            if (p.n_valid > Ly.ld_u) p.n_valid = Ly.ld_u;
-            p.mn_major = 1;
-            rc = launch_gemm(t, Ly.m_dg_mn, Ly.m_u_mn, p, s, &Ly.m_partial);
-            if (rc != TACO_OK) return rc;
-        }
+        // dWcat = dgates^T [h | x | 1 1] over all time steps: M = 256, N = ld_u, K = seq * batch
+        rc = launch_wgrad(t, Ly.m_dg_mn, Ly.m_u_mn, kG, Ly.ld_u, SB, Ly.partial, Ly.ld_u, Ly.split, Ly.m_partial, s);
+        if (rc != TACO_OK) return rc;
     }
-    // bias gradients = column sums of the batch-major dZ: partial rows here, summed by the assembly kernel below
+    // the flat gradient: weight gradients from the split-K partials, and MLP bias gradients = column sums of the batch-major dZ (partial
+    // rows from colsum_kernel, summed by the assembly kernel)
     ColSumParams cs;
     memset(&cs, 0, sizeof(cs));
-    const int col_chunks = (B + kColRows - 1) / kColRows;
-    for (int k = 0; k < 2; ++k) {
-        MlpNet& n = k == 0 ? t->actor : t->critic;
-        for (int l = 0; l < n.L; ++l) {
-            ColSumSeg& S = cs.seg[cs.n_seg++];
-            S.src = n.dz_bm[l + 1]; S.ld = n.ld_dz[l + 1];
-        }
-    }
-    cs.B = B; cs.partial = t->colsum_partial; cs.stop = t->stop;
-    launch_pdl(colsum_kernel, dim3(col_chunks, cs.n_seg), dim3(256), 0, s, cs);
-    // weight gradients from the split-K partials
     GradParams gp;
     memset(&gp, 0, sizeof(gp));
+    const int col_chunks = (B + kColRows - 1) / kColRows;
     long long elems = 0;
     auto add = [&](const float* partial, int splits, long long stride, int ld, int col0, int rows, int cols, long long dst) {
         GradSeg& S = gp.seg[gp.n_seg++];
         S.partial = partial; S.splits = splits; S.split_stride = stride; S.ld = ld; S.col0 = col0; S.rows = rows; S.cols = cols; S.dst = dst;
         elems += (long long)rows * cols;
     };
-    for (int k = 0; k < 2; ++k) {
-        MlpNet& n = k == 0 ? t->actor : t->critic;
-        for (int l = 0; l < n.L; ++l) {
-            // the launch may have merged splits: recompute the number actually written
-            const int kb_total = (B + BK - 1) / BK;
-            int sp = n.splits[l] > kb_total ? kb_total : n.splits[l];
-            const int per = (kb_total + sp - 1) / sp;
-            sp = (kb_total + per - 1) / per;
-            add(n.partial[l], sp, (long long)n.s[l + 1] * n.ld_p[l], n.ld_p[l], 0, n.s[l + 1], n.s[l], n.w_off[l]);
-            add(t->colsum_partial + (long long)(k * t->actor.L + l) * col_chunks * kColLd, col_chunks, kColLd, kColLd, 0, 1, n.s[l + 1], n.b_off[l]);
+    for (const MlpNet* n : {&t->actor, &t->critic}) {
+        for (int l = 0; l < n->L; ++l) {
+            const MlpLayer& Ly = n->layer[l];
+            const int c = cs.n_seg++;
+            cs.seg[c].src = Ly.dz_bm; cs.seg[c].ld = Ly.ld_dz;
+            add(Ly.partial, Ly.split.splits, (long long)Ly.out * Ly.ld_p, Ly.ld_p, 0, Ly.out, Ly.in, Ly.w_off);
+            add(t->colsum_partial + (long long)c * col_chunks * kColLd, col_chunks, kColLd, kColLd, 0, 1, Ly.out, Ly.b_off);
         }
     }
     for (int l = 0; l < t->n_lstm; ++l) {
         const LstmLayer& Ly = t->lstm[l];
-        const int kb_total = (int)((SB + BK - 1) / BK);
-        int sp = Ly.splits > kb_total ? kb_total : Ly.splits;
-        const int per = (kb_total + sp - 1) / sp;
-        sp = (kb_total + per - 1) / per;
+        const int sp = Ly.split.splits;
         const long long stride = (long long)kG * Ly.ld_u;
         add(Ly.partial, sp, stride, Ly.ld_u, 0, kG, kH, Ly.off_whh);
         add(Ly.partial, sp, stride, Ly.ld_u, kH, kG, Ly.in, Ly.off_wih);
         add(Ly.partial, sp, stride, Ly.ld_u, kH + Ly.in, kG, 1, Ly.off_bih);
         add(Ly.partial, sp, stride, Ly.ld_u, kH + Ly.in, kG, 1, Ly.off_bhh);
     }
+    cs.B = B; cs.partial = t->colsum_partial; cs.stop = t->stop;
+    launch_pdl(colsum_kernel, dim3(col_chunks, cs.n_seg), dim3(256), 0, s, cs);
     gp.grad = t->grad; gp.acc = t->acc; gp.stop = t->stop;
     launch_pdl(grad_assemble_kernel, dim3((unsigned)((elems + 255) / 256)), dim3(256), 0, s, gp);
     TACO_CUDA(cudaGetLastError());
@@ -1148,7 +1147,8 @@ int taco_ppo_apply(TacoPPO* t, const TacoPPOHyper* hyper, void* stream) {
         memset(&sp, 0, sizeof(sp));
         for (int l = 0; l < t->actor.L; ++l) {
             SpecSeg& S = sp.seg[sp.n_seg++];
-            S.w = t->prm + t->actor.w_off[l]; S.rows = t->actor.s[l + 1]; S.cols = t->actor.s[l]; S.v = t->spec_v[l]; S.sigma = t->spec_sigma + l;
+            const MlpLayer& Ly = t->actor.layer[l];
+            S.w = t->prm + Ly.w_off; S.rows = Ly.out; S.cols = Ly.in; S.v = t->spec_v[l]; S.sigma = t->spec_sigma + l;
         }
         sp.lipschitz = h.lipschitz; sp.max_iter = t->spec_cold ? 4000 : 200; sp.stop = t->stop;
         t->spec_cold = false;
@@ -1158,14 +1158,14 @@ int taco_ppo_apply(TacoPPO* t, const TacoPPOHyper* hyper, void* stream) {
         TACO_CUDA(cudaStreamWaitEvent(t->side, t->ev_adam, 0));
         spectral_kernel<<<sp.n_seg, 512, 0, t->side>>>(sp); TACO_LAUNCHED();
         TACO_CUDA(cudaGetLastError());
-        int rc = repack(t, t->side, true, 1);
+        int rc = repack(t, t->side, true, kPackActor);
         if (rc != TACO_OK) return rc;
         TACO_CUDA(cudaEventRecord(t->ev_actor, t->side));
         t->actor_pending = true;
-        return repack(t, s, true, 2);
+        return repack(t, s, true, kPackCritic);
     }
     TACO_CUDA(cudaGetLastError());
-    return repack(t, s, true);
+    return repack(t, s, true, kPackBoth);
 }
 
 // end of an update: synchronises and returns the log rows (n_rows x 8 floats: policy-gradient loss, value loss, entropy loss,
@@ -1222,18 +1222,15 @@ static int gemm_selftest_impl(int device, const void* a_bf16, const void* b_bf16
                        : make_map(&ma, (const bf16*)a_bf16, m, k, k, BM) && make_map(&mb, (const bf16*)b_bf16, n, k, k, pad16(n));
     if (!ok) return fail(TACO_E_CUDA, "tensor map");
     TACO_CUDA(cudaFuncSetAttribute(gemm_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kGemmSmem));
-    const int kb_total = (k + BK - 1) / BK;
-    int sp = splits < 1 ? 1 : (splits > kb_total ? kb_total : splits);
-    const int per = (kb_total + sp - 1) / sp;
-    sp = (kb_total + per - 1) / per;
+    const SplitK sk = split_k(splits, k);
+    const int sp = sk.splits;
     float* part = nullptr;
     TACO_CUDA(cudaMalloc(&part, (size_t)sp * m * n * sizeof(float)));
     // (compute-sanitizer's initcheck does not observe writes made by cp.async.bulk.tensor stores: without this the partials the
     // TMA-store epilogue writes read as uninitialised in the assembly kernel below)
     TACO_CUDA(cudaMemsetAsync(part, 0, (size_t)sp * m * n * sizeof(float), s));
-    GemmParams p;
-    memset(&p, 0, sizeof(p));
-    p.m = m; p.n = n; p.k = k; p.n_tile = pad16(n); p.splits = sp; p.kb_per_split = per; p.epi = EPI_F32; p.n_valid = n; p.mn_major = mn ? 1 : 0;
+    GemmParams p{};
+    p.m = m; p.n = n; p.k = k; p.n_tile = pad16(n); p.splits = sp; p.kb_per_split = sk.kb_per_split; p.epi = EPI_F32; p.n_valid = n; p.mn_major = mn ? 1 : 0;
     p.out_f32 = part; p.ldc = n; p.split_stride = (long long)m * n;
     cudaDeviceProp prop;
     TACO_CUDA(cudaGetDeviceProperties(&prop, device));
