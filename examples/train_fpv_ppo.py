@@ -73,8 +73,7 @@ def main():
     critic = taco_b200.CriticLSTM(26, env.len_states, args.lstm_hidden, c_hid, lstm_layers=args.lstm_layers, device=dev)
     buf = taco_b200.RolloutBuffer(n, 26, env.len_obs, 26, env.len_states, 4, args.horizon, args.mini_batch_num, 0.99, 0.95, dev)
     # the tensor-core kernels are also the fast path at small env counts (latency of one tile chain: ~12 us actor, ~36 us critic)
-    # a stacked critic has no tcgen05 kernel: its rollouts keep the actor's and run the critic on the FP32 kernel (with a warning)
-    tc = args.tensor_cores != "off" and actor.tensor_cores_available and (critic.tensor_cores_available or args.lstm_layers > 1)
+    tc = args.tensor_cores != "off" and actor.tensor_cores_available and critic.tensor_cores_available
     env.reset()
     graphed = None
     for epoch in range(args.epochs):

@@ -226,8 +226,11 @@ int taco_actor_act(TacoActor* actor, const float* obs_dev, int32_t n, const floa
  * value = MLP(LSTMEncoder(states)), LSTMEncoder = nn.LSTM(in_dim, lstm_hidden, lstm_layers, batch_first=True) with zero initial
  * state, output = top layer's h after the last time step (nets_asymmetry.py:128-136); MLP = [Linear -> ReLU] x L -> Linear(-> 1)
  * (nets_asymmetry.py:23-39, :318).  Two kernels compute the same function: an FP32 CUDA-core path (any shape; parity) and a
- * tcgen05/TMEM bf16 path (one LSTM layer of width multiple of 16 up to 64, even in_dim <= 30, seq_len <= 8, 1..3 MLP hidden layers of
- * widths multiples of 64 up to 256). */
+ * tcgen05/TMEM bf16 path (1..4 LSTM layers of width multiple of 16 up to 64, even in_dim <= 30, seq_len <= 8, 1..3 MLP hidden layers
+ * of widths multiples of 64 up to 256).  A stacked LSTM hands its layers' outputs over through a workspace owned by the handle:
+ * one forward at a time per handle.  taco_critic_create allocates it for a fixed chunk of the batch (4 waves of 2-tile pairs of
+ * 128 rows, whatever n later calls pass): seq_len x 16 KB per tile, i.e. 97 MB at seq_len = 5 and 155 MB at seq_len = 8 on a
+ * 148-SM B200, one buffer for 2 layers and two for 3-4 layers, so that a captured graph never sees it move. */
 typedef struct TacoCritic TacoCritic;
 /* mlp_sizes = [lstm_hidden, h1, ..., hL, 1] (n_mlp_sizes entries) */
 int taco_critic_create(int device, int32_t in_dim, int32_t seq_len, int32_t lstm_hidden, int32_t lstm_layers,

@@ -7,7 +7,9 @@ Mirrors (IsaacGymEnvs/algorithms/nets_asymmetry.py), in the configuration the re
   * ``PPO_ActorCritic.act`` (critic branch)  :350-352  ``value = critic_mlp(critic_encoder(critic_input))``
 
 The math runs in libtaco_b200.so (FP32 CUDA-core kernel, or the tcgen05 bf16 kernel with ``tensor_cores=True``); torch only
-provides device memory and the stream.  No CPU fallback.
+provides device memory and the stream.  No CPU fallback.  The tcgen05 kernel takes 1 to 4 stacked LSTM layers (one launch per
+layer over chunks of the batch); ``tensor_cores_available`` says whether it takes this critic's shape.  A stacked critic's
+workspace belongs to the handle, so one handle runs one ``forward`` at a time.
 """
 import ctypes as C
 

@@ -286,7 +286,7 @@ static inline void mlp_f32_free(MlpF32& m) { cudaFree(m.w); cudaFree(m.b); }
 // The tensor-core kernels' copy of an MLP [in, h1, ..., hL, out]: the bf16 K-chunk images of its layers back to back in wimg (the
 // output layer as a kOutN-row part), the hidden biases as rows of a [kMaxHidden][kMaxN] block, the output bias padded to kOutPad.
 // MLP layer l is layer[first + l] and its bias row first + l; the slots before `first` (and the image bytes before the MLP's)
-// belong to the caller: the critic's LSTM step and its unused bias row 0.
+// belong to the caller: the critic's LSTM step and bias row 0 (the gate biases of a stacked critic's top layer, unused otherwise).
 struct TcImage {
     uint8_t* wimg = nullptr;
     float* bias = nullptr;               // [kMaxHidden][kMaxN]; cleared on the stream by the caller before tc_image_pack

@@ -8,7 +8,8 @@
 //   MLP.forward           nets_asymmetry.py:23-39     [Linear -> ReLU] x L -> Linear -> Identity (:318)
 //
 // Two kernels compute the same function: an FP32 CUDA-core path (any shape; the parity path) and the tcgen05 bf16 path in
-// critic_tc.cuh (one LSTM layer of width <= 64, MLP widths multiples of 64 up to 256).
+// critic_tc.cuh (1..4 LSTM layers of width <= 64, MLP widths multiples of 64 up to 256).  A stacked LSTM runs on the tcgen05
+// path as one launch per layer over a chunk of the batch (kChunkWaves), the layers handing h over through a workspace.
 #include "launch_count.h"
 #include <cmath>
 #include <cstdio>
@@ -26,6 +27,11 @@ namespace critic {
 
 constexpr int kMaxLstmLayers = 4;
 constexpr int kMaxMlpLayers = 8;     // linear layers of the FP32 path
+// Stacked LSTM on the tensor cores: the batch is walked in chunks of kChunkWaves full waves of tile pairs (2 x SMs tiles each), and
+// each chunk runs layer 0 -> top, so that much of a chunk's hand-off between the layers (128 B per row and step and buffer) is read
+// back from L2.  Measured on a B200 (DESIGN.md 6c): 4 waves beat 1 and 2 (fewer launches and wave tails outweigh the part of the
+// hand-off that no longer fits L2).  TACO_CRITIC_CHUNK_WAVES in the environment at create time overrides it (tuning).
+constexpr int kChunkWaves = 4;
 
 struct FpParams {
     const float* states; float* value;
@@ -195,7 +201,30 @@ struct TacoCritic {
     std::string tc_why;
     TcImage tc;                          // layer[0] / bias row 0: the LSTM step (its image in front of the MLP's), MLP from 1 on
     int num_sms = 148;
+    // stacked LSTM on the tensor cores (lstm_layers > 1).  The image of LSTM layer k is at k * lstm_img_bytes in tc.wimg.  Layer k's
+    // launch reads its gate biases from row 0 of its bias block: tc.bias for the top layer (whose rows 1.. hold the MLP's; the bottom
+    // layer's bias rides in its image), seq_bias[k - 1] for a middle layer.  Everything is allocated at create: a captured graph
+    // keeps these addresses across taco_critic_load.
+    size_t lstm_img_bytes = 0;
+    float* seq_bias = nullptr;           // [lstm_layers - 2][kMaxHidden][kMaxN]
+    uint4* seq_ws[2] = {nullptr, nullptr};   // hand-off buffers (two from three layers on: ping-pong), chunk_tiles x seq_len x 16 KB each
+    int chunk_tiles = 0;
 };
+
+static float* tc_bias_block(const TacoCritic* c, int k) {
+    return (k == 0 || k + 1 == c->lstm_layers) ? c->tc.bias : c->seq_bias + (size_t)(k - 1) * kMaxHidden * kMaxN;
+}
+
+template <bool kSeqIn, bool kSeqOut>
+static void set_tc_smem(cudaError_t& ce) {
+    if (ce == cudaSuccess)
+        ce = cudaFuncSetAttribute(critic_tc_kernel<kSeqIn, kSeqOut>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  kSeqIn ? kCriticSeqSmemBytes : kCriticSmemBytes);
+}
+template <bool kSeqIn, bool kSeqOut>
+static void launch_tc(const CriticTcParams& p, int grid, cudaStream_t s) {
+    critic_tc_kernel<kSeqIn, kSeqOut><<<grid, kTcThreads, kSeqIn ? kCriticSeqSmemBytes : kCriticSmemBytes, s>>>(p); TACO_LAUNCHED();
+}
 
 extern "C" {
 
@@ -247,7 +276,6 @@ int taco_critic_create(int device, int32_t in_dim, int32_t seq_len, int32_t lstm
     const int n_hidden = c->n_mlp - 1;
     c->tc_ok = true;
     if (prop.major != 10) { c->tc_ok = false; c->tc_why = "device is not sm_100"; }
-    else if (lstm_layers != 1) { c->tc_ok = false; c->tc_why = "needs a single LSTM layer"; }
     else if (H % 16 != 0 || H > kTcMaxLstmHidden) { c->tc_ok = false; c->tc_why = "LSTM width must be a multiple of 16, <= 64"; }
     else if (in_dim > kTcMaxIn || (in_dim & 1)) { c->tc_ok = false; c->tc_why = "input width must be even, <= 30"; }
     else if (seq_len > kMaxSeq) { c->tc_ok = false; c->tc_why = "sequence length > 8"; }
@@ -256,10 +284,24 @@ int taco_critic_create(int device, int32_t in_dim, int32_t seq_len, int32_t lstm
     if (ce == cudaSuccess) ce = cudaMalloc(&c->lstm_f32, lo * sizeof(float));
     if (ce == cudaSuccess) ce = mlp_f32_alloc(c->f32, mlp_sizes, c->n_mlp);
     if (ce == cudaSuccess && c->tc_ok) {
-        // [0] the LSTM step: n = 4H gate rows, K = [h (64) | x (64)] = 2 chunks, in front of the MLP's images
+        // [0] the LSTM step: n = 4H gate rows, K = [h (64) | x (64)] = 2 chunks; every layer's image in front of the MLP's
         c->tc.layer[0].n = 4 * H; c->tc.layer[0].kchunks = 2; c->tc.layer[0].img_off = 0;
-        ce = tc_image_alloc(c->tc, mlp_sizes, n_hidden, 1, (size_t)2 * 4 * H * 128);
-        if (ce == cudaSuccess) ce = cudaFuncSetAttribute(critic_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCriticSmemBytes);
+        c->lstm_img_bytes = (size_t)2 * 4 * H * 128;
+        ce = tc_image_alloc(c->tc, mlp_sizes, n_hidden, 1, lstm_layers * c->lstm_img_bytes);
+        if (lstm_layers == 1) {
+            set_tc_smem<false, false>(ce);
+        } else {
+            const char* e = getenv("TACO_CRITIC_CHUNK_WAVES");
+            const int waves = (e && atoi(e) > 0) ? atoi(e) : kChunkWaves;
+            c->chunk_tiles = waves * 2 * c->num_sms;
+            const size_t ws_bytes = (size_t)c->chunk_tiles * seq_len * kTileM * 128;
+            for (int b = 0; b < (lstm_layers > 2 ? 2 : 1); ++b)
+                if (ce == cudaSuccess) ce = cudaMalloc(&c->seq_ws[b], ws_bytes);
+            if (ce == cudaSuccess && lstm_layers > 2) ce = cudaMalloc(&c->seq_bias, (size_t)(lstm_layers - 2) * kMaxHidden * kMaxN * sizeof(float));
+            set_tc_smem<false, true>(ce);
+            set_tc_smem<true, true>(ce);
+            set_tc_smem<true, false>(ce);
+        }
     }
     if (ce == cudaSuccess && c->fp_smem > 48 * 1024)
         ce = cudaFuncSetAttribute(critic_fp32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, c->fp_smem);
@@ -277,6 +319,7 @@ int taco_critic_destroy(TacoCritic* c) {
     DevGuard guard(c->device);
     cudaFree(c->lstm_f32); mlp_f32_free(c->f32);
     tc_image_free(c->tc);
+    cudaFree(c->seq_bias); cudaFree(c->seq_ws[0]); cudaFree(c->seq_ws[1]);
     delete c;
     return TACO_OK;
 }
@@ -300,8 +343,14 @@ int taco_critic_load(TacoCritic* c, const float* const* lstm_host, const float* 
     if (int rc = mlp_f32_upload(c->f32, mlp_weights_host, mlp_biases_host, c->mlp_sizes.data(), c->n_mlp, s)) return rc;
     if (c->tc_ok) {
         TACO_CUDA(cudaMemsetAsync(c->tc.bias, 0, kMaxHidden * kMaxN * sizeof(float), s));
+        if (c->seq_bias) TACO_CUDA(cudaMemsetAsync(c->seq_bias, 0, (size_t)(c->lstm_layers - 2) * kMaxHidden * kMaxN * sizeof(float), s));
         pack_lstm_kernel<<<64, 256, 0, s>>>(c->lstm_f32 + c->lstm_off[0], c->lstm_f32 + c->lstm_off[1], c->lstm_f32 + c->lstm_off[2],
                                             c->lstm_f32 + c->lstm_off[3], H, c->in_dim, 4 * H, c->tc.wimg); TACO_LAUNCHED();
+        for (int l = 1; l < c->lstm_layers; ++l) {
+            pack_lstm_seq_kernel<<<64, 256, 0, s>>>(c->lstm_f32 + c->lstm_off[4 * l], c->lstm_f32 + c->lstm_off[4 * l + 1],
+                                                    c->lstm_f32 + c->lstm_off[4 * l + 2], c->lstm_f32 + c->lstm_off[4 * l + 3], H, 4 * H,
+                                                    c->tc.wimg + l * c->lstm_img_bytes, tc_bias_block(c, l)); TACO_LAUNCHED();
+        }
         if (int rc = tc_image_pack(c->tc, c->f32, c->mlp_sizes.data(), c->n_mlp - 1, s)) return rc;
     }
     TACO_CUDA(cudaStreamSynchronize(s));     // the host buffers may be released by the caller on return
@@ -328,11 +377,33 @@ int taco_critic_forward(TacoCritic* c, const float* states_dev, float* value_dev
         for (int l = 0; l <= p.n_hidden + 1; ++l) p.layer[l] = c->tc.layer[l];
         static const int stagger = [] { const char* e = getenv("TACO_CRITIC_STAGGER"); return e ? atoi(e) : kCriticStagger; }();
         p.stagger = stagger;
-        const int grid = tc_grid(p.num_tiles, c->num_sms, &p.tiles_per_cta);
-        const char* tl = getenv("TACO_CRITIC_TIMELINE");
-        if (int rc = timeline_begin(tl, &p.dbg, s)) return rc;
-        critic_tc_kernel<<<grid, kTcThreads, kCriticSmemBytes, s>>>(p); TACO_LAUNCHED();
-        if (int rc = timeline_end(tl, p.dbg, s)) return rc;
+        if (c->lstm_layers == 1) {
+            const int grid = tc_grid(p.num_tiles, c->num_sms, &p.tiles_per_cta);
+            const char* tl = getenv("TACO_CRITIC_TIMELINE");
+            if (int rc = timeline_begin(tl, &p.dbg, s)) return rc;
+            launch_tc<false, false>(p, grid, s);
+            if (int rc = timeline_end(tl, p.dbg, s)) return rc;
+        } else {
+            // chunk by chunk, layer 0 -> top on the stream (no timeline); the next layer reads the hand-off of a chunk while much
+            // of it is still in L2.  The workspace is the handle's: one forward at a time per handle.
+            const int L = c->lstm_layers, T = c->seq_len;
+            const long long chunk_rows = (long long)c->chunk_tiles * kTileM;
+            for (long long row0 = 0; row0 < n; row0 += chunk_rows) {
+                const int rows = (int)(n - row0 < chunk_rows ? n - row0 : chunk_rows);
+                p.states = states_dev + row0 * T * c->in_dim; p.value = value_dev + row0;
+                p.n_rows = rows; p.num_tiles = (rows + kTileM - 1) / kTileM;
+                const int grid = tc_grid(p.num_tiles, c->num_sms, &p.tiles_per_cta);
+                for (int k = 0; k < L; ++k) {
+                    p.layer[0].img_off = (uint32_t)(k * c->lstm_img_bytes);
+                    p.bias = tc_bias_block(c, k);
+                    p.seq_in = k > 0 ? c->seq_ws[(k - 1) & 1] : nullptr;
+                    p.seq_out = k + 1 < L ? c->seq_ws[k & 1] : nullptr;
+                    if (k == 0) launch_tc<false, true>(p, grid, s);
+                    else if (k + 1 < L) launch_tc<true, true>(p, grid, s);
+                    else launch_tc<true, false>(p, grid, s);
+                }
+            }
+        }
     } else {
         FpParams p;
         memset(&p, 0, sizeof(p));
