@@ -291,7 +291,8 @@ int taco_ppo_num_params(TacoPPO* ppo, int64_t* n);
 int taco_ppo_param_offsets(TacoPPO* ppo, int64_t* offsets, int32_t count, int32_t* n_out);
 /* device addresses of the flat vectors (n_params floats each) and of the int32 optimiser-step counter; any may be NULL */
 int taco_ppo_buffers(TacoPPO* ppo, float** params, float** grad, float** adam_m, float** adam_v, int32_t** step);
-/* after writing the parameter vector from outside: refresh the bf16 operand copies */
+/* after writing the parameter vector from outside: refresh the bf16 operand copies; the next spectral projection starts its
+ * power iteration over (cold start) instead of from the singular vectors of the old weights */
 int taco_ppo_params_changed(TacoPPO* ppo, void* stream);
 int taco_ppo_begin_update(TacoPPO* ppo, void* stream);
 /* rollout tensors as flat device views [N_total][...] (obs (N, obs_dim), states (N, seq_len, state_dim), act (N, act_dim),

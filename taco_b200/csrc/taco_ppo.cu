@@ -350,12 +350,13 @@ __global__ void __launch_bounds__(256) adam_kernel(float* prm, float* m, float* 
     const float coef = fminf((float)((double)h.max_grad / (norm + 1e-6)), 1.0f) / (float)h.world;     // the 1 / world averages the summed gradient
     const int t = *step + 1;
     const float b1 = 0.9f, b2 = 0.999f;
+    const float a1 = 0.1f, a2 = 0.001f;             // 1 - beta rounded from the exact value, as torch passes it (1.0f - b2 is 1.3e-5 off)
     const float bc1 = 1.0f - powf(b1, (float)t), bc2 = 1.0f - powf(b2, (float)t);
     const float step_size = h.lr / bc1, inv_sqrt_bc2 = rsqrtf(bc2);
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
         const float g = grad[e] * coef;
-        const float mm = b1 * m[e] + (1.0f - b1) * g;
-        const float vv = b2 * v[e] + (1.0f - b2) * g * g;
+        const float mm = b1 * m[e] + a1 * g;
+        const float vv = b2 * v[e] + a2 * g * g;
         m[e] = mm; v[e] = vv;
         prm[e] -= step_size * (mm / (sqrtf(vv) * inv_sqrt_bc2 + 1e-5f));
     }
@@ -374,8 +375,18 @@ __global__ void finish_step_kernel(int* step, double* acc, const int* stop) {
 
 // PPO.spectral_normalize_actors (:398-404): sigma = ||W||_2 by power iteration on W^T W, warm-started from the previous optimiser
 // step's right singular vector; W *= c / sigma when sigma > c.  One CTA per weight matrix, all matrices in one launch.
-struct SpecSeg { float* w; int rows, cols; float* v; double* sigma; };
-struct SpecParams { SpecSeg seg[kMaxHiddenL + 1]; int n_seg; float lipschitz; int max_iter; const int* stop; };
+//
+// A matrix whose `cold` flag is set (a new handle, or weights loaded from outside) starts from the constant vector with the cold
+// iteration cap and clears its flag; a launch the early-stop flag turns into a no-op leaves it set.  Power iteration only ever
+// underestimates sigma, and the estimate can rise slowly for many iterations (a small top gap, or a start vector with little
+// weight on the top singular vector), so a single small change is not convergence: the loop stops once sigma has risen by at
+// most kSpecTol over the last kSpecWindow iterations (fp32 rounding moves sigma by ~1e-7, far below what a window may gain).
+// sigma is estimated as sqrt(||W^T W v||) for ||v|| = 1: a lower bound like ||W v||, closer to sigma_1, and it needs only the
+// norm that normalises v.
+constexpr int kSpecWindow = 8, kSpecColdIter = 4000, kSpecWarmIter = 200;
+constexpr double kSpecTol = 1e-6;
+struct SpecSeg { float* w; int rows, cols; float* v; double* sigma; int* cold; };
+struct SpecParams { SpecSeg seg[kMaxHiddenL + 1]; int n_seg; float lipschitz; const int* stop; };
 __global__ void __launch_bounds__(512) spectral_kernel(const SpecParams p) {
     pdl_launch_dependents();
     pdl_wait();
@@ -383,24 +394,16 @@ __global__ void __launch_bounds__(512) spectral_kernel(const SpecParams p) {
     const SpecSeg& S = p.seg[blockIdx.x];
     __shared__ float v[256], u[256], part[2][256];
     __shared__ float red[16];
-    __shared__ float s_norm;
+    __shared__ double hist[kSpecWindow], s_norm, s_sigma;
+    __shared__ int s_done;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int rows = S.rows, cols = S.cols;
     const float* __restrict__ W = S.w;
-    for (int c = tid; c < cols; c += 512) v[c] = S.v[c];
+    const bool cold = *S.cold != 0;
+    const int max_iter = cold ? kSpecColdIter : kSpecWarmIter;
+    for (int c = tid; c < cols; c += 512) v[c] = cold ? 1.0f / sqrtf((float)cols) : S.v[c];
     __syncthreads();
-    // block-wide sum of squares of a shared vector of length n -> s_norm
-    auto sumsq = [&](const float* x, int n) {
-        float a = 0.f;
-        for (int k = tid; k < n; k += 512) a += x[k] * x[k];
-        for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-        if (lane == 0) red[warp] = a;
-        __syncthreads();
-        if (tid == 0) { float t = 0.f; for (int w = 0; w < 16; ++w) t += red[w]; s_norm = t; }
-        __syncthreads();
-    };
-    float sigma = 0.f, prev = -1.f;
-    for (int it = 0; it < p.max_iter; ++it) {
+    for (int it = 0; it < max_iter; ++it) {
         // u = W v: a warp per row (two rows in flight), lanes along the row: coalesced reads of W from L2
         for (int r0 = warp * 2; r0 < rows; r0 += 32) {
             float a0 = 0.f, a1 = 0.f;
@@ -414,9 +417,7 @@ __global__ void __launch_bounds__(512) spectral_kernel(const SpecParams p) {
             if (lane == 0) { u[r0] = a0; if (two) u[r0 + 1] = a1; }
         }
         __syncthreads();
-        sumsq(u, rows);                                              // sigma^2 estimate = ||W v||^2 for ||v|| = 1
-        sigma = sqrtf(s_norm);
-        // v = W^T u: thread <-> (column, half of the rows): lanes read consecutive columns of one row, 8 loads in flight
+        // W^T u: thread <-> (column, half of the rows): lanes read consecutive columns of one row, 8 loads in flight
         {
             const int c = tid & 255, half = tid >> 8;
             if (c < cols) {
@@ -432,19 +433,34 @@ __global__ void __launch_bounds__(512) spectral_kernel(const SpecParams p) {
             }
         }
         __syncthreads();
-        for (int c = tid; c < cols; c += 512) v[c] = part[0][c] + part[1][c];
+        // v = W^T u and ||v||^2; thread 0 takes sigma and the stop test
+        {
+            float a = 0.f;
+            for (int c = tid; c < cols; c += 512) { const float x = part[0][c] + part[1][c]; v[c] = x; a = fmaf(x, x, a); }
+            for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+            if (lane == 0) red[warp] = a;
+            __syncthreads();
+            if (tid == 0) {
+                double t = 0.0;
+                for (int w = 0; w < 16; ++w) t += (double)red[w];
+                const double sg = sqrt(sqrt(t));
+                const int slot = it % kSpecWindow;
+                s_done = it >= kSpecWindow && sg - hist[slot] <= kSpecTol * sg;
+                hist[slot] = sg;
+                s_norm = t; s_sigma = sg;
+            }
+            __syncthreads();
+        }
+        const float inv = s_norm > 0.0 ? (float)(1.0 / sqrt(s_norm)) : 0.f;
+        for (int c = tid; c < cols; c += 512) v[c] *= inv;                  // (each thread its own columns, as written above)
+        if (s_done) break;
         __syncthreads();
-        sumsq(v, cols);
-        const float inv = s_norm > 0.f ? rsqrtf(s_norm) : 0.f;
-        for (int c = tid; c < cols; c += 512) v[c] *= inv;
-        __syncthreads();
-        if (it >= 2 && fabsf(sigma - prev) <= 1e-6f * sigma) break;
-        prev = sigma;
     }
+    const float sig = (float)s_sigma;
     for (int c = tid; c < cols; c += 512) S.v[c] = v[c];
-    if (tid == 0) *S.sigma = (double)sigma;
-    if (p.lipschitz > 0.0f && sigma > p.lipschitz) {
-        const float sc = p.lipschitz / sigma;                           // param.data *= lipschitz_const / spectral_norm
+    if (tid == 0) { *S.sigma = (double)sig; *S.cold = 0; }
+    if (p.lipschitz > 0.0f && sig > p.lipschitz) {
+        const float sc = p.lipschitz / sig;                             // param.data *= lipschitz_const / spectral_norm
         for (long long e = tid; e < (long long)rows * cols; e += 512) S.w[e] *= sc;
     }
 }
@@ -566,8 +582,8 @@ struct TacoPPO {
     // bookkeeping
     double* acc = nullptr; float* log = nullptr; int *n_logged = nullptr, *stop = nullptr, *step = nullptr;
     int max_log = 4096;
-    float* spec_v[kMaxHiddenL + 1] = {nullptr}; double* spec_sigma = nullptr;
-    bool spec_cold = true;
+    // power iteration state per actor matrix: right singular vector, sigma, cold-start flag (set: the next projection starts over)
+    float* spec_v[kMaxHiddenL + 1] = {nullptr}; double* spec_sigma = nullptr; int* spec_cold = nullptr;
     // the spectral projection + re-pack of the ACTOR runs on a side stream under the next minibatch's gather and critic forward
     cudaStream_t side = nullptr;
     cudaEvent_t ev_adam = nullptr, ev_actor = nullptr;
@@ -764,14 +780,9 @@ int taco_ppo_create_layers(int device, const TacoPPOCfg* cfg, int32_t lstm_layer
     alloc(&t->stop, 1);
     alloc(&t->step, 1);
     alloc(&t->spec_sigma, (size_t)(kMaxHiddenL + 1));
-    for (int l = 0; l < t->actor.L; ++l) {
-        const int in = t->actor.layer[l].in;
-        alloc(&t->spec_v[l], (size_t)in);
-        if (alloc.err == cudaSuccess) {
-            std::vector<float> ones((size_t)in, 1.0f / std::sqrt((float)in));
-            alloc.err = cudaMemcpy(t->spec_v[l], ones.data(), ones.size() * sizeof(float), cudaMemcpyHostToDevice);
-        }
-    }
+    alloc(&t->spec_cold, (size_t)(kMaxHiddenL + 1));
+    if (alloc.err == cudaSuccess) alloc.err = cudaMemset(t->spec_cold, 1, (kMaxHiddenL + 1) * sizeof(int));
+    for (int l = 0; l < t->actor.L; ++l) alloc(&t->spec_v[l], (size_t)t->actor.layer[l].in);
     if (alloc.err != cudaSuccess)
         return bail(alloc.err == cudaErrorMemoryAllocation ? TACO_E_NOMEM : TACO_E_CUDA, "taco_ppo_create: device allocation failed");
     bool ok = true;
@@ -887,12 +898,14 @@ static int repack(TacoPPO* t, cudaStream_t s, bool honour_stop, PackNets nets) {
     return cudaGetLastError() == cudaSuccess ? TACO_OK : fail(TACO_E_CUDA, "pack kernels failed");
 }
 
-// call after writing the parameter vector (taco_ppo_buffers) from outside: refreshes the bf16 operand copies
+// call after writing the parameter vector (taco_ppo_buffers) from outside: refreshes the bf16 operand copies, and the next
+// projection starts its power iteration over (the stored singular vectors belong to the old weights)
 int taco_ppo_params_changed(TacoPPO* t, void* stream) {
     if (!t) return fail(TACO_E_INVALID, "taco_ppo_params_changed: null argument");
     DevGuard guard(t->device);
     const int rcj = join_actor(t, (cudaStream_t)stream);
     if (rcj != TACO_OK) return rcj;
+    TACO_CUDA(cudaMemsetAsync(t->spec_cold, 1, (kMaxHiddenL + 1) * sizeof(int), (cudaStream_t)stream));
     return repack(t, (cudaStream_t)stream, false, kPackBoth);
 }
 
@@ -1148,10 +1161,9 @@ int taco_ppo_apply(TacoPPO* t, const TacoPPOHyper* hyper, void* stream) {
         for (int l = 0; l < t->actor.L; ++l) {
             SpecSeg& S = sp.seg[sp.n_seg++];
             const MlpLayer& Ly = t->actor.layer[l];
-            S.w = t->prm + Ly.w_off; S.rows = Ly.out; S.cols = Ly.in; S.v = t->spec_v[l]; S.sigma = t->spec_sigma + l;
+            S.w = t->prm + Ly.w_off; S.rows = Ly.out; S.cols = Ly.in; S.v = t->spec_v[l]; S.sigma = t->spec_sigma + l; S.cold = t->spec_cold + l;
         }
-        sp.lipschitz = h.lipschitz; sp.max_iter = t->spec_cold ? 4000 : 200; sp.stop = t->stop;
-        t->spec_cold = false;
+        sp.lipschitz = h.lipschitz; sp.stop = t->stop;
         // actor: projection, then the bf16 copies of the projected matrices, on the side stream (4 CTAs of latency-bound power
         // iteration); the caller's stream goes on with the critic's copies and the next minibatch until it needs the actor
         TACO_CUDA(cudaEventRecord(t->ev_adam, s));
