@@ -86,18 +86,20 @@ typedef struct TacoCfg {
     uint64_t seed;              /* Philox key */
 } TacoCfg;
 
-/* Device pointers of the buffers VecTask exposes (vec_task_asymmetry.py:231-254).  obs and
- * states are double-buffered: the pointers change on every step; call taco_env_buffers
- * again after each taco_env_step (the two alternating addresses are obs_ab / states_ab). */
+/* Device pointers of the buffers VecTask exposes (vec_task_asymmetry.py:231-254).  obs is
+ * double-buffered (the two alternating addresses are obs_ab).  The state history lives in a strip
+ * (taco_env_states_strip): states points at the current window, whose env stride is the strip's row,
+ * not len_states * 26.  Both pointers change on every step; call taco_env_buffers again after each
+ * taco_env_step.  While a rollout ring is attached, obs and states point into its newest slot. */
 typedef struct TacoBuffers {
     float* obs;          /* (num_envs, len_obs, 26) f32, newest frame last */
-    float* states;       /* (num_envs, len_states, 26) f32 */
+    float* states;       /* (num_envs, len_states, 26) f32, env stride frames * 26 floats (contiguous in a ring slot) */
     float* rew;          /* (num_envs) f32 */
     int64_t* reset;      /* (num_envs) i64, read at the start of step (lazy reset), written at the end */
     uint8_t* time_outs;  /* (num_envs) bool */
     int32_t* progress;   /* (num_envs) i32 (reference: i64 progress_buf) */
     float* obs_ab[2];
-    float* states_ab[2];
+    float* states_ab[2]; /* [0] = base of the state history strip, [1] = NULL */
     int32_t num_envs, len_obs, len_states, num_obs;
 } TacoBuffers;
 
@@ -149,6 +151,11 @@ int taco_env_attach_rollout(TacoEnv* env, float* obs_ring, float* states_ring, i
 int taco_env_rewind_rollout(TacoEnv* env, void* stream);
 int taco_env_detach_rollout(TacoEnv* env, void* stream);
 int taco_env_rollout_cursor(TacoEnv* env);   /* newest slot index, or -1 when no ring is attached */
+/* The env-owned state history: `frames` = len_states + period - 1 frames of 26 f32 per env row (num_envs rows).  After a step
+ * that ran at step index t the window is the len_states frames from offset (t + 1) % period; a step writes only its newest frame,
+ * and the step that wraps the offset to 0 first moves the kept frames to the start of the row.  (Not written while a rollout
+ * ring is attached: detaching copies the ring's newest slot back into the window.) */
+int taco_env_states_strip(TacoEnv* env, float** base, int32_t* frames, int32_t* period);
 /* -- env.difficulty is written by the trainer every epoch (algorithms/ppo_asymmetry.py:173-175) */
 int taco_env_set_difficulty(TacoEnv* env, float difficulty);
 int taco_env_get_difficulty(TacoEnv* env, float* out);

@@ -76,6 +76,7 @@ def lib():
         "taco_env_rewind_rollout": (C.c_int, [vp, vp]),
         "taco_env_detach_rollout": (C.c_int, [vp, vp]),
         "taco_env_rollout_cursor": (C.c_int, [vp]),
+        "taco_env_states_strip": (C.c_int, [vp, C.POINTER(vp), C.POINTER(i32), C.POINTER(i32)]),
         "taco_env_set_difficulty": (C.c_int, [vp, f32]),
         "taco_env_set_seed": (C.c_int, [vp, u64]),
         "taco_env_stats": (C.c_int, [vp, vp, vp, vp]),

@@ -174,12 +174,50 @@ __device__ __forceinline__ void write_rows(const float* __restrict__ in, float* 
     } else write_rows_impl<LC, false>(in, out, frames, L_rt, blk_env0, tid, nv);
 }
 
+// The env-owned state history (no rollout ring attached): each env's row of the strip holds strip_frames = L + K - 1 frames, and
+// after the step that ran at step index t the env's window is the L frames from offset (t + 1) mod K.  A step writes only the newest
+// frame, at the end of the new window: 104 B per env instead of re-reading 4 frames and rewriting 5 (936 B).  The step that wraps the
+// offset to 0 first moves the L - 1 kept frames (K .. K + L - 2) to the start of the row (0 .. L - 2) -- the "rebase", once per K
+// steps.  K >= L, so the moved frames, their destination and the newest frame (L - 1) are disjoint: no ordering inside the CTA.
+__device__ __forceinline__ void write_strip(const StepParams& p, const float* frames, size_t blk_env0, int tid, int nv) {
+    const uint32_t t = p.step_index + (p.step_base ? __ldg(p.step_base) : 0u);
+    const int L = p.len_states, q = (int)((t + 1u) % (uint32_t)p.strip_period);
+    const int row2 = 13 * p.strip_frames;
+    float2* s2 = reinterpret_cast<float2*>(p.states_strip) + blk_env0 * row2;
+    if (q == 0 && L > 1) {
+        const int keep2 = 13 * (L - 1), src2 = 13 * p.strip_period, total = nv * keep2;
+        constexpr int U = 13;                                   // loads in flight per thread
+        for (int k0 = tid; k0 < total; k0 += kBlock * U) {
+            float2 v[U];
+            int dst[U];
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                const int k = k0 + u * kBlock;
+                const int e = k / keep2, j = k - e * keep2;
+                dst[u] = e * row2 + j;
+                v[u] = (k < total) ? s2[dst[u] + src2] : make_float2(0.f, 0.f);
+            }
+#pragma unroll
+            for (int u = 0; u < U; ++u)
+                if (k0 + u * kBlock < total) s2[dst[u]] = v[u];
+        }
+    }
+    const int new2 = 13 * (q + L - 1);
+#pragma unroll
+    for (int u = 0; u < 13; ++u) {                               // nv rows x 13 float2 of the newest frame
+        const int k = tid + u * kBlock;
+        const int e = k / 13, j = k - e * 13;
+        const float* fr = frames + e * kFramePad + 2 * j;
+        if (e < nv) s2[e * row2 + new2 + j] = make_float2(fr[0], fr[1]);
+    }
+}
+
 // TASK: task_mode (mix = per-env task from the global env id).  DR: per-env randomised model parameters live in the
 // D planes; when false the rotor polynomial / aero coefficients fold into instruction immediates.
 // SUB: physics sub-steps per simulate call (1 / 2 unrolled; 0 = runtime p.substeps).
 // DEVDIFF: graph-mode variant (difficulty scalars from device memory; costs two spilled registers, so eager launches do not use it).
-// CW: extra warps of the CTA (threads >= 128) that do nothing but the kept-history copy of the states buffer, from the first cycle of
-// the CTA -- the copy depends on nothing the step computes.  CW = 4 for launches of at most one CTA per SM (the 4096-env scale of
+// CW: extra warps of the CTA (threads >= 128) that do nothing but the kept-history copy into the slot of an attached rollout ring, from
+// the first cycle of the CTA -- the copy depends on nothing the step computes (the env-owned strip, write_strip, has no such copy).  CW = 4 for launches of at most one CTA per SM (the 4096-env scale of
 // the reference: one env's instruction stream is latency-bound there, and the copy's four load -> store round trips were a third of
 // the kernel's time when they ran after it: 14.4 -> 13.1 us); CW = 0 otherwise (the copy warps' registers cost resident compute
 // warps: one copy warp per CTA at 2 Mi envs measured 0.636 against 0.609 ms, profiles/ab_r02y.txt).
@@ -199,7 +237,7 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
     const bool is_copy = CW > 0 && tid >= kBlock;              // copy warps: no env of their own
     const bool valid = !is_copy && i < p.n;
     // split copy: else the compute warps copy after the step, as with CW = 0 (where nothing of this is kept live across the step)
-    const bool split_copy = CW > 0 && min(kBlock, p.n - blk * kBlock) == kBlock && p.len_states == 5;
+    const bool split_copy = CW > 0 && !p.states_strip && min(kBlock, p.n - blk * kBlock) == kBlock && p.len_states == 5;
     const uint32_t flags = p.flags;
     const bool obs_noise = (flags & TACO_F_OBSERVATION_NOISE) != 0;
     if (tid < kNumStats) s_stats[tid] = 0.0;
@@ -803,10 +841,12 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
     }
 
     // ---------------------------------------------------------------------- history shift + newest frame (:392,:413)
-    // out[e][f][:] = in[e][f+1][:] for f < L-1, newest frame last; ping-pong buffers, so no in-place hazard.
+    // states: the newest frame into the env-owned strip, or (rollout ring attached) out[e][f][:] = in[e][f+1][:] for f < L-1 and the
+    // newest frame last, slot k -> slot k + 1 of the ring.  obs: the same shift between ping-pong buffers.  No in-place hazard.
     const size_t blk_env0 = (size_t)blk * kBlock;
     const int nv = min(kBlock, p.n - blk * kBlock);             // valid rows of this CTA
-    if (CW > 0 && split_copy) write_newest_rows<5>(p.states_out, s_clean, blk_env0, tid);   // the copy warps moved the kept part
+    if (p.states_strip) write_strip(p, s_clean, blk_env0, tid, nv);
+    else if (CW > 0 && split_copy) write_newest_rows<5>(p.states_out, s_clean, blk_env0, tid);   // the copy warps moved the kept part
     else if (p.len_states == 5) write_rows<5, !DR>(p.states_in, p.states_out, s_clean, 5, blk_env0, tid, nv);
     else write_rows<0, false>(p.states_in, p.states_out, s_clean, p.len_states, blk_env0, tid, nv);
     const float* sf = obs_noise ? s_noisy : s_clean;
@@ -822,7 +862,7 @@ constexpr int kSmallGrid = 148;     // one CTA per SM
 template <int TASK, bool DR, bool DEVDIFF>
 static void launch_variant(const StepParams& p, int grid, cudaStream_t stream) {
     if (p.substeps == 2) {
-        if (TACO_COPY_WARPS_SMALL > 0 && grid <= kSmallGrid)
+        if (TACO_COPY_WARPS_SMALL > 0 && grid <= kSmallGrid && !p.states_strip)   // the ring path's kept-history copy
             fpv_step_kernel<TASK, DR, 2, DEVDIFF, TACO_COPY_WARPS_SMALL><<<grid, kBlock + 32 * TACO_COPY_WARPS_SMALL, 0, stream>>>(p);
         else if (!DEVDIFF && (p.host_tout || p.host_flags)) fpv_step_kernel<TASK, DR, 2, false, 0, true><<<grid, kBlock, 0, stream>>>(p);
         else fpv_step_kernel<TASK, DR, 2, DEVDIFF><<<grid, kBlock, 0, stream>>>(p);

@@ -47,8 +47,10 @@ struct StepParams {
     float* rew;
     const float* obs_in;
     float* obs_out;
-    const float* states_in;
+    const float* states_in;        // attached rollout ring: slot k (read) and slot k + 1 (written), contiguous (n, len_states, 26)
     float* states_out;
+    float* states_strip;           // else the env's own history strip (see write_strip in fpv_step_kernel.cuh), null while a ring is attached
+    int strip_frames, strip_period;   // frames per env row of the strip, and the period K of the window offset
     float* roll_rew;               // row of the attached rollout buffer for this step (or null): rew, done as f32, time-outs
     float* roll_done;
     uint8_t* roll_tout;

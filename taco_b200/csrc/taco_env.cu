@@ -34,8 +34,9 @@ struct TacoEnv {
     void* arena = nullptr;       // one cudaMalloc for everything
     size_t arena_bytes = 0;
     float* obs_ab[2] = {nullptr, nullptr};
-    float* states_ab[2] = {nullptr, nullptr};
-    int cur = 0;                 // index of the buffers holding the latest obs/states
+    float* strip = nullptr;      // state history: strip_frames frames per env, window at offset step_index % strip_period (write_strip)
+    int strip_frames = 0, strip_period = 0;
+    int cur = 0;                 // index of the obs buffer holding the latest observation history
     // caller-owned rollout ring (taco_env_attach_rollout): slot k of obs / states, row k of rew / done / time-outs
     float* ring_obs = nullptr;
     float* ring_states = nullptr;
@@ -378,8 +379,12 @@ int taco_env_create(const TacoCfg* cfg, int device, TacoEnv** out) {
     const size_t oProg = take(np * sizeof(int)), oMeta = take(np * sizeof(uint32_t));
     const size_t oQact = take((size_t)kQueueCap * np * sizeof(float4)), oQend = take((size_t)kQueueCap * np * sizeof(uint16_t));
     const size_t oReset = take(np * sizeof(long long)), oTout = take(np), oRew = take(np * sizeof(float));
-    const size_t obs_bytes = np * cfg->len_obs * kObs * sizeof(float), st_bytes = np * cfg->len_states * kObs * sizeof(float);
-    const size_t oObs0 = take(obs_bytes), oObs1 = take(obs_bytes), oSt0 = take(st_bytes), oSt1 = take(st_bytes);
+    // state history strip: L + K - 1 frames per env with K = max(16, L) (K >= L keeps the rebase of write_strip free of overlap;
+    // at L = 5 an env's row is 20 frames = 2080 B, a multiple of the 32-byte sector)
+    e->strip_period = cfg->len_states > 16 ? cfg->len_states : 16;
+    e->strip_frames = cfg->len_states + e->strip_period - 1;
+    const size_t obs_bytes = np * cfg->len_obs * kObs * sizeof(float), st_bytes = np * e->strip_frames * kObs * sizeof(float);
+    const size_t oObs0 = take(obs_bytes), oObs1 = take(obs_bytes), oSt = take(st_bytes);
     const size_t oStats = take((size_t)kStatSlots * kStatStride * sizeof(double)), oStatsOut = take(kNumStats * sizeof(double));
     const size_t oStage = take(np * sizeof(float4));
     const size_t oDbg = (cfg->flags & TACO_F_DEBUG_DELAY) ? take((size_t)cfg->control_freq_inv * np * sizeof(float4)) : 0;
@@ -395,7 +400,8 @@ int taco_env_create(const TacoCfg* cfg, int device, TacoEnv** out) {
     p.qact = (float4*)(base + oQact); p.qend = (uint16_t*)(base + oQend);
     p.reset_buf = (long long*)(base + oReset); p.time_outs = (uint8_t*)(base + oTout); p.rew = (float*)(base + oRew);
     e->obs_ab[0] = (float*)(base + oObs0); e->obs_ab[1] = (float*)(base + oObs1);
-    e->states_ab[0] = (float*)(base + oSt0); e->states_ab[1] = (float*)(base + oSt1);
+    e->strip = (float*)(base + oSt);
+    p.strip_frames = e->strip_frames; p.strip_period = e->strip_period;
     p.stats = (double*)(base + oStats); e->stats_out = (double*)(base + oStatsOut);
     e->actions_stage = (float4*)(base + oStage);
     e->dbg_delay = (cfg->flags & TACO_F_DEBUG_DELAY) ? (float4*)(base + oDbg) : nullptr;
@@ -426,6 +432,12 @@ int taco_env_destroy(TacoEnv* env) {
     return TACO_OK;
 }
 
+// first frame of the current window of the state history strip (rows of strip_frames frames: not a contiguous (n, L, 26) array)
+static float* strip_window(TacoEnv* env) {
+    return env->strip + (size_t)(env->step_index % (uint32_t)env->strip_period) * kObs;
+}
+static size_t strip_row_bytes(TacoEnv* env) { return (size_t)env->strip_frames * kObs * sizeof(float); }
+
 int taco_env_buffers(TacoEnv* env, TacoBuffers* out) {
     if (!env || !out) return fail(TACO_E_INVALID, "taco_env_buffers: null argument");
     if (env->ring_slots) {
@@ -433,13 +445,14 @@ int taco_env_buffers(TacoEnv* env, TacoBuffers* out) {
         out->states = env->ring_states + (size_t)env->n * env->cfg.len_states * kObs * env->ring_cur;
     } else {
         out->obs = env->obs_ab[env->cur];
-        out->states = env->states_ab[env->cur];
+        out->states = strip_window(env);
     }
     out->rew = env->p.rew;
     out->reset = (int64_t*)env->p.reset_buf;
     out->time_outs = env->p.time_outs;
     out->progress = env->p.progress;
-    for (int k = 0; k < 2; ++k) { out->obs_ab[k] = env->obs_ab[k]; out->states_ab[k] = env->states_ab[k]; }
+    for (int k = 0; k < 2; ++k) out->obs_ab[k] = env->obs_ab[k];
+    out->states_ab[0] = env->strip; out->states_ab[1] = nullptr;
     out->num_envs = env->n; out->len_obs = env->cfg.len_obs; out->len_states = env->cfg.len_states; out->num_obs = kObs;
     return TACO_OK;
 }
@@ -453,13 +466,14 @@ static int bind_history(TacoEnv* env) {
         const size_t so = (size_t)env->n * env->cfg.len_obs * kObs, ss = (size_t)env->n * env->cfg.len_states * kObs;
         p.obs_in = env->ring_obs + so * env->ring_cur; p.obs_out = env->ring_obs + so * (env->ring_cur + 1);
         p.states_in = env->ring_states + ss * env->ring_cur; p.states_out = env->ring_states + ss * (env->ring_cur + 1);
+        p.states_strip = nullptr;
         p.roll_rew = env->ring_rew ? env->ring_rew + (size_t)env->n * env->ring_cur : nullptr;
         p.roll_done = env->ring_rew ? env->ring_done + (size_t)env->n * env->ring_cur : nullptr;
         p.roll_tout = env->ring_rew ? env->ring_tout + (size_t)env->n * env->ring_cur : nullptr;
     } else {
         const int nxt = env->cur ^ 1;
         p.obs_in = env->obs_ab[env->cur]; p.obs_out = env->obs_ab[nxt];
-        p.states_in = env->states_ab[env->cur]; p.states_out = env->states_ab[nxt];
+        p.states_in = nullptr; p.states_out = nullptr; p.states_strip = env->strip;
         p.roll_rew = nullptr; p.roll_done = nullptr; p.roll_tout = nullptr;
     }
     return TACO_OK;
@@ -692,7 +706,8 @@ int taco_env_attach_rollout(TacoEnv* env, float* obs_ring, float* states_ring, i
     cudaStream_t s = (cudaStream_t)stream;
     // the newest observation / state history moves into slot 0
     TACO_CUDA(cudaMemcpyAsync(obs_ring, env->obs_ab[env->cur], (size_t)env->n * env->cfg.len_obs * kObs * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    TACO_CUDA(cudaMemcpyAsync(states_ring, env->states_ab[env->cur], (size_t)env->n * env->cfg.len_states * kObs * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    const size_t win = (size_t)env->cfg.len_states * kObs * sizeof(float);
+    TACO_CUDA(cudaMemcpy2DAsync(states_ring, win, strip_window(env), strip_row_bytes(env), win, env->n, cudaMemcpyDeviceToDevice, s));
     env->ring_obs = obs_ring; env->ring_states = states_ring;
     env->ring_rew = rew_rows; env->ring_done = done_rows; env->ring_tout = time_out_rows;
     env->ring_slots = slots; env->ring_cur = 0;
@@ -720,9 +735,16 @@ int taco_env_detach_rollout(TacoEnv* env, void* stream) {
     cudaStream_t s = (cudaStream_t)stream;
     const size_t so = (size_t)env->n * env->cfg.len_obs * kObs, ss = (size_t)env->n * env->cfg.len_states * kObs;
     TACO_CUDA(cudaMemcpyAsync(env->obs_ab[env->cur], env->ring_obs + so * env->ring_cur, so * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    TACO_CUDA(cudaMemcpyAsync(env->states_ab[env->cur], env->ring_states + ss * env->ring_cur, ss * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    const size_t win = (size_t)env->cfg.len_states * kObs * sizeof(float);
+    TACO_CUDA(cudaMemcpy2DAsync(strip_window(env), strip_row_bytes(env), env->ring_states + ss * env->ring_cur, win, win, env->n, cudaMemcpyDeviceToDevice, s));
     env->ring_obs = env->ring_states = env->ring_rew = env->ring_done = nullptr; env->ring_tout = nullptr;
     env->ring_slots = 0; env->ring_cur = 0;
+    return TACO_OK;
+}
+
+int taco_env_states_strip(TacoEnv* env, float** base, int32_t* frames, int32_t* period) {
+    if (!env || !base || !frames || !period) return fail(TACO_E_INVALID, "taco_env_states_strip: null argument");
+    *base = env->strip; *frames = env->strip_frames; *period = env->strip_period;
     return TACO_OK;
 }
 
@@ -733,10 +755,8 @@ int taco_env_reset_all(TacoEnv* env, void* stream) {
     DevGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t np = (size_t)env->n_pad;
-    for (int k = 0; k < 2; ++k) {
-        TACO_CUDA(cudaMemsetAsync(env->obs_ab[k], 0, np * env->cfg.len_obs * kObs * sizeof(float), s));
-        TACO_CUDA(cudaMemsetAsync(env->states_ab[k], 0, np * env->cfg.len_states * kObs * sizeof(float), s));
-    }
+    for (int k = 0; k < 2; ++k) TACO_CUDA(cudaMemsetAsync(env->obs_ab[k], 0, np * env->cfg.len_obs * kObs * sizeof(float), s));
+    TACO_CUDA(cudaMemsetAsync(env->strip, 0, np * strip_row_bytes(env), s));
     if (env->ring_slots) {                                           // restart the attached ring from a zeroed slot 0
         TACO_CUDA(cudaMemsetAsync(env->ring_obs, 0, (size_t)env->n * env->cfg.len_obs * kObs * sizeof(float), s));
         TACO_CUDA(cudaMemsetAsync(env->ring_states, 0, (size_t)env->n * env->cfg.len_states * kObs * sizeof(float), s));
@@ -822,7 +842,7 @@ int taco_env_import_state(TacoEnv* env, const float* in_host) {
 }
 
 // ---- env-state checkpoint: the whole device arena (SoA state planes, DR planes, pending-action ring, reward / reset / time-out
-// buffers, both observation / state history buffers, statistics partials) + a header.  The reference never checkpoints the env
+// buffers, both observation history buffers, the state history strip, statistics partials) + a header.  The reference never checkpoints the env
 // (SURVEY.md section 5); here a resumed run continues bit-identically.
 struct CkptHeader {
     char magic[8];              // "TACOENV1"

@@ -127,7 +127,10 @@ class FpvVecTask:
         _capi.check(self._lib.taco_env_buffers(self._h, C.byref(b)), "taco_env_buffers")
         N, dev = self.num_envs, self.device
         self._obs_ab = [_capi.wrap(b.obs_ab[k], (N, self.len_obs, self.num_obs), "<f4", dev, self) for k in range(2)]
-        self._states_ab = [_capi.wrap(b.states_ab[k], (N, self.len_states, self.num_states), "<f4", dev, self) for k in range(2)]
+        base, frames, period = C.c_void_p(), C.c_int32(), C.c_int32()
+        _capi.check(self._lib.taco_env_states_strip(self._h, C.byref(base), C.byref(frames), C.byref(period)), "taco_env_states_strip")
+        self._strip = _capi.wrap(base.value, (N, frames.value, self.num_states), "<f4", dev, self)
+        self._strip_period = period.value
         self._ab_ptr = [int(b.obs_ab[0]), int(b.obs_ab[1])]
         self.rew_buf = _capi.wrap(b.rew, (N,), "<f4", dev, self)
         self.reset_buf = _capi.wrap(b.reset, (N,), "<i8", dev, self)
@@ -143,9 +146,12 @@ class FpvVecTask:
 
     @property
     def states_buf(self):
+        """(num_envs, len_states, 26) state history.  Without a rollout ring attached: a strided view of the library's history strip
+        (taco_env_states_strip), the window of the current step; the next period - len_states steps leave it intact."""
         if self.rollout_buffer is not None:
             return self.rollout_buffer.states_ring[self._ring_cur]
-        return self._states_ab[self._cur]
+        p = self.step_count % self._strip_period
+        return self._strip[:, p:p + self.len_states]
 
     @property
     def progress_buf(self):
@@ -181,7 +187,7 @@ class FpvVecTask:
         re-initialisation happens lazily at the start of the next step (reset_buf starts all ones)."""
         # Fresh tensors, like the reference's out-of-place clamp: PPO.run keeps these two as ITS persistent observation storage
         # (``obs.copy_(next_obs)``, ppo_asymmetry.py:297-299,328-329) and stores them AFTER env.step (:326); a view of the
-        # library's ping-pong buffer would be overwritten by every second step.
+        # library's history buffers would be overwritten by later steps.
         self.obs_dict["obs"] = torch.clamp(self.obs_buf, -self.clip_obs, self.clip_obs).to(self.rl_device)
         self.obs_dict["states"] = torch.clamp(self.states_buf, -self.clip_states, self.clip_states).to(self.rl_device)
         return self.obs_dict
