@@ -39,13 +39,14 @@ def main():
     ap.add_argument("--update", default="native", choices=["native", "torch"])
     ap.add_argument("--no-graph", action="store_true", help="collect rollouts with the eager loop instead of one CUDA-graph replay per rollout")
     ap.add_argument("--seed", type=int, default=42)
+    ap.add_argument("--save", default=None, help="after training, write the agent's state dict (save_checkpoint(para_only=True)) to this path")
     args = ap.parse_args()
 
     import torch
     import torch.distributed as dist
     import taco_b200
     from taco_b200 import dist as tdist
-    from taco_b200.ppo import PPOConfig, TorchActorCritic, make_optimizer, ppo_update, sync_rollout_nets, sync_rollout_nets_native
+    from taco_b200.ppo import PPOConfig, TorchActorCritic, make_optimizer, ppo_update, save_checkpoint, sync_rollout_nets, sync_rollout_nets_native
     from taco_b200.ppo_native import NativePPO
 
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
@@ -114,6 +115,8 @@ def main():
     if native is not None:
         native.store_to(agent, opt)                 # the torch module / optimiser hold the trained state again (checkpoints, export)
         native.close()
+    if args.save and rank == 0:
+        save_checkpoint(args.save, agent, para_only=True)         # loads with examples/eval_fpv_policy.py --checkpoint
     env.close(); actor.close(); critic.close()
     if world > 1:
         dist.destroy_process_group()

@@ -185,6 +185,41 @@ int taco_env_checkpoint_load(TacoEnv* env, const void* in_host, uint64_t bytes);
 /* delayed action read at each control sub-step of the last step: (num_envs, control_freq_inv, 4) f32, host */
 int taco_env_debug_delay(TacoEnv* env, float* out_host);
 
+/* -- evaluation: per-episode outcome records (DESIGN.md section 6f).  With a log attached, every step (taco_env_step and the
+ * host-buffer steps) is followed by one more launch on the step's stream -- capturable in a CUDA graph -- that accumulates per env
+ * the quantities below and, for each env whose episode ended in that step (reset_buf != 0), appends one record.  Only whole
+ * episodes are recorded: at attach, an env with reset_buf != 0 starts fresh and every other env is mid-episode and is not recorded
+ * until after its next end.  taco_env_reset_all, taco_env_import_state and taco_env_checkpoint_load discard the episodes in
+ * progress and re-run that initialisation.  The record order is unspecified (records of one step are appended in warp order by
+ * atomics); records past the capacity are dropped but counted: dropped = *count - capacity.  Not allowed together with a rollout
+ * ring (TACO_E_INVALID either way round).  48 bytes, a multiple of 16. */
+typedef struct TacoEpisode {
+    int64_t env_id;          /* global env id (env_offset + local index) */
+    uint32_t end_step;       /* RL step index (0-based, the Philox step index) of the step that ended the episode */
+    int32_t length;          /* progress_buf at the end, the episode length taco_env_stats adds */
+    int16_t task;            /* TACO_TASK_POS / _ROTATE / _FLIP; a mix env: the task of its third of the global ids */
+    int16_t timed_out;       /* time_outs of the ending step */
+    float ret;               /* float32 sum of the rewards in step order: bit-identical to the return taco_env_stats adds */
+    float pos_err_mean;      /* |pos - target pos| in m: mean over the episode's steps (after each step) */
+    float pos_err_final;     /* ... and its value at the end */
+    float tilt_max;          /* largest angle between body z and world z, acos(clamp(1 - 2 (qx^2 + qy^2))), rad */
+    float speed_mean;        /* mean |linvel|, m/s */
+    float angvel_max;        /* largest |angvel| (world frame), rad/s */
+    float roll_travel;       /* flip envs: roll_continuous at the end minus after the first step (flips = roll_travel / 2 pi); else 0 */
+} TacoEpisode;
+/* allocates the log (capacity records, a counter, two accumulator planes) once, so a captured graph never sees it move; clears the
+ * counter and runs the attach initialisation on `stream` */
+int taco_env_attach_episode_log(TacoEnv* env, int64_t capacity, void* stream);
+int taco_env_detach_episode_log(TacoEnv* env);
+/* zero-copy access: records_dev = capacity TacoEpisode, count_dev = one uint64 (records appended since attach / the last clear) */
+int taco_env_episode_log_buffers(TacoEnv* env, TacoEpisode** records_dev, uint64_t** count_dev, int64_t* capacity);
+/* rewinds the counter on `stream`; the per-env accumulators are kept, so the episodes in progress continue */
+int taco_env_episode_log_clear(TacoEnv* env, void* stream);
+/* trajectory recorder: the TACO_STATE_WORDS-float taco_env_export_state row of each of the k local env ids in ids_dev (device
+ * int32) into out_dev (k, TACO_STATE_WORDS) f32 on the device; an id outside [0, num_envs) gives a row of NaN.  Asynchronous on
+ * `stream`, no host sync (capturable). */
+int taco_env_record_state(TacoEnv* env, const int32_t* ids_dev, int32_t k, float* out_dev, void* stream);
+
 /* -- actor MLP inference in the rollout loop: MLP.forward + the actor branch of PPO_ActorCritic.act
  * (IsaacGymEnvs/algorithms/nets_asymmetry.py:23-39, :326-346) and PPO.spectral_normalize_actors
  * (IsaacGymEnvs/algorithms/ppo_asymmetry.py:398-404).  Two kernels compute the same function: an FP32 CUDA-core

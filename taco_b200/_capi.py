@@ -8,6 +8,8 @@ The library must exist -- there is no CPU fallback; a missing or unloadable .so 
 import ctypes as C
 import os
 
+import numpy as np
+
 _LIB_PATH = os.environ.get("TACO_B200_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libtaco_b200.so")
 
 ABI_VERSION = 1
@@ -84,6 +86,11 @@ def lib():
         "taco_env_export_state": (C.c_int, [vp, vp]),
         "taco_env_import_state": (C.c_int, [vp, vp]),
         "taco_env_debug_delay": (C.c_int, [vp, vp]),
+        "taco_env_attach_episode_log": (C.c_int, [vp, C.c_int64, vp]),
+        "taco_env_detach_episode_log": (C.c_int, [vp]),
+        "taco_env_episode_log_buffers": (C.c_int, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(C.c_int64)]),
+        "taco_env_episode_log_clear": (C.c_int, [vp, vp]),
+        "taco_env_record_state": (C.c_int, [vp, vp, i32, vp, vp]),
         "taco_selftest_divc": (C.c_int, [C.c_int, f32, C.POINTER(u64)]),
         "taco_selftest_atan2": (C.c_int, [C.c_int, C.c_uint32, C.POINTER(f32), C.POINTER(C.c_uint32)]),
         "taco_actor_create": (C.c_int, [C.c_int, C.POINTER(i32), i32, C.POINTER(vp)]),
@@ -150,6 +157,13 @@ class TacoPPOCfg(C.Structure):
 class TacoPPOHyper(C.Structure):
     _fields_ = [("lr", C.c_float), ("clip", C.c_float), ("target_kl", C.c_float), ("max_grad", C.c_float), ("pi_coef", C.c_float),
                 ("vf_coef", C.c_float), ("ent_coef", C.c_float), ("lipschitz", C.c_float), ("use_lipschitz", C.c_int32), ("world", C.c_int32)]
+
+
+# TacoEpisode (include/taco_b200.h), 48 bytes per record
+EPISODE_DTYPE = np.dtype([("env_id", "<i8"), ("end_step", "<u4"), ("length", "<i4"), ("task", "<i2"), ("timed_out", "<i2"),
+                          ("ret", "<f4"), ("pos_err_mean", "<f4"), ("pos_err_final", "<f4"), ("tilt_max", "<f4"),
+                          ("speed_mean", "<f4"), ("angvel_max", "<f4"), ("roll_travel", "<f4")])
+assert EPISODE_DTYPE.itemsize == 48
 
 
 class _CudaView:

@@ -17,6 +17,7 @@
 #include "philox.cuh"
 #include "fpv_math.cuh"
 #include "step_params.h"
+#include "episode_log.cuh"
 
 namespace taco {
 
@@ -48,6 +49,12 @@ struct TacoEnv {
     double* stats_out = nullptr;       // 8 doubles, device
     float* export_stage = nullptr;     // n * TACO_STATE_WORDS floats, device
     float4* dbg_delay = nullptr;
+    // episode log (taco_env_attach_episode_log): one allocation = counter, two accumulator planes, records
+    void* log_mem = nullptr;
+    unsigned long long* log_count = nullptr;
+    float4* log_acc[2] = {nullptr, nullptr};
+    TacoEpisode* log_rec = nullptr;
+    unsigned long long log_cap = 0;
     uint32_t step_index = 0;
     // graph mode (taco_env_graph_begin .. _end): the step index of a launch = *step_counter (device) + its offset since
     // graph_begin, so a CUDA graph captured over a rollout replays with fresh Philox counters / queue time slots
@@ -132,11 +139,17 @@ __global__ void reduce_stats_kernel(double* partial, double* out) {
     out[j] = acc;
 }
 
-// SoA planes <-> TACO_STATE_WORDS floats per env (layout documented in DESIGN.md "state export")
-__global__ void export_state_kernel(StepParams p, float* out) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= p.n) return;
-    float* o = out + (size_t)i * TACO_STATE_WORDS;
+// SoA planes <-> TACO_STATE_WORDS floats per env (layout documented in DESIGN.md "state export").  Row j of `out` is env ids[j]
+// (ids = null: env j) for j < count; an id outside [0, n) gives a row of NaN (taco_env_record_state takes device ids unchecked)
+__global__ void export_state_kernel(StepParams p, const int32_t* ids, int count, float* out) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= count) return;
+    const int i = ids ? ids[j] : j;
+    float* o = out + (size_t)j * TACO_STATE_WORDS;
+    if (i < 0 || i >= p.n) {
+        for (int w = 0; w < TACO_STATE_WORDS; ++w) o[w] = __int_as_float(0x7fc00000);
+        return;
+    }
     const float4 s0 = p.S[0][i], s1 = p.S[1][i], s2 = p.S[2][i], s3 = p.S[3][i], s4 = p.S[4][i], s5 = p.S[5][i], s6 = p.S[6][i], s7 = p.S[7][i];
     o[0] = s0.x; o[1] = s0.y; o[2] = s0.z;                    // pos
     o[3] = s0.w; o[4] = s1.x; o[5] = s1.y; o[6] = s1.z;       // quat xyzw
@@ -425,6 +438,7 @@ int taco_env_destroy(TacoEnv* env) {
         cudaEventDestroy(env->ev_begin); cudaEventDestroy(env->ev_end);
     }
     if (env->export_stage) cudaFree(env->export_stage);
+    if (env->log_mem) cudaFree(env->log_mem);
     if (env->arena) cudaFree(env->arena);
     if (env->step_counter) cudaFree(env->step_counter);
     if (env->diff_dev) cudaFree(env->diff_dev);
@@ -492,6 +506,26 @@ static void bind_step_index(TacoEnv* env) {
 
 __global__ void step_counter_kernel(uint32_t* c, uint32_t value, int add) { *c = add ? *c + value : value; }
 
+// the episode log's update for the step just taken (after advance_history): a launch of its own, never part of the step kernel
+static int log_after_step(TacoEnv* env, cudaStream_t s) {
+    if (!env->log_mem) return TACO_OK;
+    const uint32_t t = env->step_index - 1u;
+    const uint32_t step = env->graph_mode ? t - env->graph_origin : t;
+    episode_log_update_kernel<<<(env->n + 255) / 256, 256, 0, s>>>(env->p, env->log_acc[0], env->log_acc[1], env->log_rec, env->log_count,
+                                                                  env->log_cap, step, env->graph_mode ? env->step_counter : nullptr);
+    TACO_LAUNCHED();
+    TACO_CUDA(cudaGetLastError());
+    return TACO_OK;
+}
+
+// the attach initialisation of an attached log (a no-op without one): the episodes in progress are discarded
+static int log_restart(TacoEnv* env, cudaStream_t s) {
+    if (!env->log_mem) return TACO_OK;
+    episode_log_init_kernel<<<(env->n_pad + 255) / 256, 256, 0, s>>>(env->p, env->log_acc[0], env->log_acc[1]); TACO_LAUNCHED();
+    TACO_CUDA(cudaGetLastError());
+    return TACO_OK;
+}
+
 int taco_env_step(TacoEnv* env, const float* actions_dev, void* stream) {
     if (!env || !actions_dev) return fail(TACO_E_INVALID, "taco_env_step: null argument");
     if (((uintptr_t)actions_dev & 15u) != 0) return fail(TACO_E_INVALID, "actions must be 16-byte aligned (contiguous (N,4) float32)");
@@ -505,7 +539,7 @@ int taco_env_step(TacoEnv* env, const float* actions_dev, void* stream) {
     else launch_fpv_step_fast(p, (cudaStream_t)stream);
     TACO_CUDA(cudaGetLastError());
     advance_history(env);
-    return TACO_OK;
+    return log_after_step(env, (cudaStream_t)stream);
 }
 
 // device-visible address of a pinned (cudaHostAlloc / cudaHostRegister) host buffer, or null for pageable memory
@@ -550,7 +584,7 @@ int taco_env_step_host_compact(TacoEnv* env, const float* actions_host, float* r
     if (!d_act || (rew_host && !d_rew) || !d_flags)
         return fail(TACO_E_INVALID, "taco_env_step_host_compact: the host buffers must be pinned (device-mapped); use taco_env_step_host for pageable memory");
     StepParams& p = env->p;
-    const int rc = bind_history(env);
+    int rc = bind_history(env);
     if (rc != TACO_OK) return rc;
     p.actions = (const float4*)d_act;
     p.host_rew = (float*)d_rew; p.host_flags = (uint8_t*)d_flags;
@@ -560,6 +594,8 @@ int taco_env_step_host_compact(TacoEnv* env, const float* actions_host, float* r
     p.host_rew = nullptr; p.host_flags = nullptr;
     TACO_CUDA(le);
     advance_history(env);
+    rc = log_after_step(env, s);
+    if (rc != TACO_OK) return rc;
     TACO_CUDA(cudaStreamSynchronize(s));
     return TACO_OK;
 }
@@ -592,6 +628,8 @@ int taco_env_step_host(TacoEnv* env, const float* actions_host, float* rew_host,
             p.host_rew = nullptr; p.host_reset = nullptr; p.host_tout = nullptr;
             TACO_CUDA(le);
             advance_history(env);
+            rc = log_after_step(env, s);
+            if (rc != TACO_OK) return rc;
             TACO_CUDA(cudaStreamSynchronize(s));
             return TACO_OK;
         }
@@ -650,6 +688,8 @@ int taco_env_step_host(TacoEnv* env, const float* actions_host, float* rew_host,
         TACO_CUDA(cudaEventRecord(env->ev_end, env->s_d2h));         // s_d2h has waited for every chunk kernel
         TACO_CUDA(cudaStreamWaitEvent(s, env->ev_end, 0));
     }
+    rc = log_after_step(env, s);                                     // s has waited for every chunk kernel
+    if (rc != TACO_OK) return rc;
     TACO_CUDA(cudaStreamSynchronize(s));
     return TACO_OK;
 }
@@ -702,6 +742,7 @@ int taco_env_attach_rollout(TacoEnv* env, float* obs_ring, float* states_ring, i
         return fail(TACO_E_INVALID, "taco_env_attach_rollout: rew / done / time-out rows must be given together (or all NULL)");
     if (((uintptr_t)obs_ring | (uintptr_t)states_ring) & 7u) return fail(TACO_E_INVALID, "taco_env_attach_rollout: rings must be 8-byte aligned");
     if (env->ring_slots) return fail(TACO_E_INVALID, "taco_env_attach_rollout: a ring is already attached");
+    if (env->log_mem) return fail(TACO_E_INVALID, "taco_env_attach_rollout: an episode log is attached (evaluation only; detach it first)");
     DevGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     // the newest observation / state history moves into slot 0
@@ -765,6 +806,8 @@ int taco_env_reset_all(TacoEnv* env, void* stream) {
     TACO_CUDA(cudaMemsetAsync(env->p.stats, 0, (size_t)kStatSlots * kStatStride * sizeof(double), s));
     init_state_kernel<<<(env->n_pad + 255) / 256, 256, 0, s>>>(env->p); TACO_LAUNCHED();
     TACO_CUDA(cudaGetLastError());
+    const int rc = log_restart(env, s);
+    if (rc != TACO_OK) return rc;
     env->step_index = 0;
     env->graph_mode = false;                                         // host-side counting again; taco_env_graph_begin re-arms
     env->p.diff_dev = nullptr;
@@ -822,7 +865,7 @@ int taco_env_export_state(TacoEnv* env, float* out_host) {
     const size_t bytes = (size_t)env->n * TACO_STATE_WORDS * sizeof(float);
     if (!env->export_stage) TACO_CUDA(cudaMalloc(&env->export_stage, bytes));
     TACO_CUDA(cudaDeviceSynchronize());
-    export_state_kernel<<<(env->n + 255) / 256, 256>>>(env->p, env->export_stage); TACO_LAUNCHED();
+    export_state_kernel<<<(env->n + 255) / 256, 256>>>(env->p, nullptr, env->n, env->export_stage); TACO_LAUNCHED();
     TACO_CUDA(cudaGetLastError());
     TACO_CUDA(cudaMemcpy(out_host, env->export_stage, bytes, cudaMemcpyDeviceToHost));
     return TACO_OK;
@@ -837,6 +880,8 @@ int taco_env_import_state(TacoEnv* env, const float* in_host) {
     TACO_CUDA(cudaMemcpy(env->export_stage, in_host, bytes, cudaMemcpyHostToDevice));
     import_state_kernel<<<(env->n + 255) / 256, 256>>>(env->p, env->export_stage); TACO_LAUNCHED();
     TACO_CUDA(cudaGetLastError());
+    const int rc = log_restart(env, 0);
+    if (rc != TACO_OK) return rc;
     TACO_CUDA(cudaDeviceSynchronize());
     return TACO_OK;
 }
@@ -893,6 +938,71 @@ int taco_env_checkpoint_load(TacoEnv* env, const void* in_host, uint64_t bytes) 
     refresh_derived(env);
     TACO_CUDA(upload_derived(env));
     taco_env_set_seed(env, h.cfg.seed);
+    if (env->log_mem) {
+        const int rc = log_restart(env, 0);
+        if (rc != TACO_OK) return rc;
+        TACO_CUDA(cudaDeviceSynchronize());
+    }
+    return TACO_OK;
+}
+
+int taco_env_attach_episode_log(TacoEnv* env, int64_t capacity, void* stream) {
+    if (!env) return fail(TACO_E_INVALID, "taco_env_attach_episode_log: null argument");
+    if (capacity < 1) return fail(TACO_E_INVALID, "taco_env_attach_episode_log: capacity must be >= 1");
+    if (env->log_mem) return fail(TACO_E_INVALID, "taco_env_attach_episode_log: a log is already attached");
+    if (env->ring_slots) return fail(TACO_E_INVALID, "taco_env_attach_episode_log: a rollout ring is attached (the log reads the env's own result buffers)");
+    DevGuard guard(env->device);
+    const size_t acc_bytes = (size_t)env->n_pad * sizeof(float4);
+    const size_t bytes = 256 + 2 * acc_bytes + (size_t)capacity * sizeof(TacoEpisode);
+    void* mem = nullptr;
+    const cudaError_t ce = cudaMalloc(&mem, bytes);
+    if (ce != cudaSuccess) { cudaGetLastError(); return fail(TACO_E_NOMEM, std::string("cudaMalloc of the episode log failed: ") + cudaGetErrorString(ce)); }
+    char* base = (char*)mem;
+    env->log_mem = mem;
+    env->log_count = (unsigned long long*)base;
+    env->log_acc[0] = (float4*)(base + 256);
+    env->log_acc[1] = (float4*)(base + 256 + acc_bytes);
+    env->log_rec = (TacoEpisode*)(base + 256 + 2 * acc_bytes);
+    env->log_cap = (unsigned long long)capacity;
+    cudaStream_t s = (cudaStream_t)stream;
+    TACO_CUDA(cudaMemsetAsync(env->log_count, 0, sizeof(unsigned long long), s));
+    return log_restart(env, s);
+}
+
+int taco_env_detach_episode_log(TacoEnv* env) {
+    if (!env) return fail(TACO_E_INVALID, "taco_env_detach_episode_log: null argument");
+    if (!env->log_mem) return TACO_OK;
+    DevGuard guard(env->device);
+    TACO_CUDA(cudaDeviceSynchronize());
+    cudaFree(env->log_mem);
+    env->log_mem = nullptr; env->log_count = nullptr; env->log_acc[0] = env->log_acc[1] = nullptr; env->log_rec = nullptr;
+    env->log_cap = 0;
+    return TACO_OK;
+}
+
+int taco_env_episode_log_buffers(TacoEnv* env, TacoEpisode** records_dev, uint64_t** count_dev, int64_t* capacity) {
+    if (!env || !records_dev || !count_dev) return fail(TACO_E_INVALID, "taco_env_episode_log_buffers: null argument");
+    if (!env->log_mem) return fail(TACO_E_INVALID, "taco_env_episode_log_buffers: no episode log attached");
+    *records_dev = env->log_rec;
+    *count_dev = (uint64_t*)env->log_count;
+    if (capacity) *capacity = (int64_t)env->log_cap;
+    return TACO_OK;
+}
+
+int taco_env_episode_log_clear(TacoEnv* env, void* stream) {
+    if (!env) return fail(TACO_E_INVALID, "taco_env_episode_log_clear: null argument");
+    if (!env->log_mem) return fail(TACO_E_INVALID, "taco_env_episode_log_clear: no episode log attached");
+    DevGuard guard(env->device);
+    TACO_CUDA(cudaMemsetAsync(env->log_count, 0, sizeof(unsigned long long), (cudaStream_t)stream));
+    return TACO_OK;
+}
+
+int taco_env_record_state(TacoEnv* env, const int32_t* ids_dev, int32_t k, float* out_dev, void* stream) {
+    if (!env || !ids_dev || !out_dev) return fail(TACO_E_INVALID, "taco_env_record_state: null argument");
+    if (k < 1) return fail(TACO_E_INVALID, "taco_env_record_state: k must be >= 1");
+    DevGuard guard(env->device);
+    export_state_kernel<<<(k + 255) / 256, 256, 0, (cudaStream_t)stream>>>(env->p, ids_dev, k, out_dev); TACO_LAUNCHED();
+    TACO_CUDA(cudaGetLastError());
     return TACO_OK;
 }
 

@@ -336,6 +336,21 @@ class FpvVecTask:
         _capi.check(self._lib.taco_env_export_state(self._h, out.ctypes.data_as(C.c_void_p)), "taco_env_export_state")
         return out
 
+    def record_state(self, ids, out=None):
+        """Trajectory recorder (``taco_env_record_state``): the ``export_state`` rows of the local env ids ``ids`` (int32 CUDA tensor,
+        (k,)) into ``out`` ((k, 64) float32 CUDA tensor) on the device, without a host sync (capturable in a CUDA graph)."""
+        if ids.dtype != torch.int32 or ids.device.type != "cuda" or not ids.is_contiguous():
+            raise ValueError("record_state: ids must be a contiguous int32 CUDA tensor")
+        k = ids.numel()
+        if out is None:
+            out = torch.empty(k, _capi.STATE_WORDS, dtype=torch.float32, device=self.device)
+        if out.dtype != torch.float32 or not out.is_contiguous() or out.numel() != k * _capi.STATE_WORDS:
+            raise ValueError("record_state: out must be a contiguous float32 (k, 64) tensor")
+        stream = torch.cuda.current_stream(self.device_id).cuda_stream
+        _capi.check(self._lib.taco_env_record_state(self._h, C.c_void_p(ids.data_ptr()), k, C.c_void_p(out.data_ptr()), C.c_void_p(stream)),
+                    "taco_env_record_state")
+        return out
+
     def import_state(self, arr):
         arr = np.ascontiguousarray(arr, dtype=np.float32)
         assert arr.shape == (self.num_envs, _capi.STATE_WORDS)
