@@ -16,6 +16,8 @@
 // This header is compiled twice: fpv_step_fast.cu (FMA contraction on) and
 // fpv_step_strict.cu (-fmad=false: every multiply/add rounds separately, like eager torch).
 #pragma once
+#include <climits>
+#include <type_traits>
 #include "fpv_math.cuh"
 #include "philox.cuh"
 #include "step_params.h"
@@ -497,7 +499,25 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
         const Q4 qc0 = conj(q);
         V3 vb = qrot(qc0, vel), wb = qrot(qc0, wld);
 
+        // The control iteration reads the head run at buffer position min(len-1, k) (:366-368), i.e. at slot
+        // clk + min(q_len - 1, k), which never decreases in k.  So the head run changes only at the iteration head_k computes, and
+        // the values the PID derives from the head run's action (angular_vel_control, :637-650) are formed when it is loaded.
+        auto head_k = [&]() { const int r = run_end - clk; return (q_left > 1 && q_len - 1 >= r) ? r : INT_MAX; };
+        float u0, hu0, sp[3];
+        auto derive = [&]() {
+            u0 = (dact.x + 1.0f) / 2.0f * 1000.0f;
+            hu0 = u0 / 2.0f;
+            sp[0] = dact.y * 20.0f; sp[1] = dact.z * 20.0f; sp[2] = dact.w * 20.0f;
+        };
+        derive();
+        int k_next = head_k();
+
         // ------------------------------------------------------------------ control_freq_inv x (mid_physics_step + simulate)
+        // Two instantiations of the loop, chosen once per launch: GEN tests the debug-delay, battery and rotor-noise switches in every
+        // iteration; the other is the configuration of the training defaults (battery on, no rotor noise, no debug output) with
+        // none of those tests.
+        auto control = [&](auto gen) {
+        constexpr bool GEN = decltype(gen)::value;
         for (int k = 0; k < p.cfi; ++k) {
             // refresh_state (:334-360): roll unwrap with the 1 rad threshold; body-frame velocities
             if (track_roll) {
@@ -509,21 +529,21 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
                 roll_old = roll;
             }
             if (k > 0) vb = qrot(conj(q), vel);               // wb is carried by the integrator between sub-steps
-            // delayed action (:366-368): buffer position min(len-1, k)
-            {
+            // delayed action (:366-368)
+            if (k >= k_next) {
                 const int slot_abs = clk + min(q_len - 1, k);
                 while (slot_abs >= run_end && q_left > 1) {
                     q_cur = (q_cur + 1) & 15u; q_left -= 1;
                     dact = p.qact[(size_t)q_cur * p.n_pad + i];
                     run_end = p.qend[(size_t)q_cur * p.n_pad + i];
                 }
-                if (p.dbg_delay) p.dbg_delay[(size_t)k * p.n_pad + i] = dact;
+                derive();
+                k_next = head_k();
             }
-            // angular_vel_control (:637-650) + rate PID (angvel_control.py:67-88)
-            const float u0 = (dact.x + 1.0f) / 2.0f * 1000.0f;
+            if constexpr (GEN) { if (p.dbg_delay) p.dbg_delay[(size_t)k * p.n_pad + i] = dact; }
+            // rate PID (angvel_control.py:67-88)
             float uu[3];
             {
-                const float sp[3] = {dact.y * 20.0f, dact.z * 20.0f, dact.w * 20.0f};
                 const float wbv[3] = {wb.x, wb.y, wb.z};
                 const float kp[3] = {27.5f, 50.0f, 200.0f};
 #pragma unroll
@@ -540,7 +560,7 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
             float thr[4];
             {
                 const float u1 = uu[0], u2 = uu[1];
-                const float u3 = fminf(fmaxf(uu[2], -u0 / 2.0f), u0 / 2.0f);
+                const float u3 = fminf(fmaxf(uu[2], -hu0), hu0);      // -u0 / 2 == -(u0 / 2)
                 thr[0] = u0 - u1 + u2 - u3;
                 thr[1] = u0 - u1 - u2 + u3;
                 thr[2] = u0 + u1 - u2 - u3;
@@ -555,11 +575,12 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
             {
                 float c[4];
 #pragma unroll
-                for (int r = 0; r < 4; ++r) { const float x = TACO_DIVC(om[r] * 2.0f * kPi, 4500.0f); c[r] = 400.0f * (x * x * x); }
+                // om * 2 * pi rounds once, as om * (2 pi): the doubling is exact for every float (tests/test_exact_folds.py)
+                for (int r = 0; r < 4; ++r) { const float x = TACO_DIVC(om[r] * kTwoPi, 4500.0f); c[r] = 400.0f * (x * x * x); }
                 pm = ((c[0] + c[1]) + c[2]) + c[3];
             }
             // battery sag (battery_dynamics.py:47-75)
-            if (battery_on) {
+            if (GEN ? battery_on : true) {
                 bt = bt + dt;
                 const float pc = TACO_DIVC(TACO_DIVC(pm, 0.75f), 9000.0f);
                 bec = bec + pc * dt;
@@ -581,7 +602,7 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
                     const float tgt = (((p01 + poly[2] * y) + poly[3] * (x * x)) + poly[4] * x * y) * 100.0f;
                     om[r] = om[r] + lag[r] * (tgt - om[r]);
                 }
-                if (flags & TACO_F_ROTOR_NOISE) {
+                if (GEN && (flags & TACO_F_ROTOR_NOISE)) {
                     const uint4 nb = philox4x32_10(g, t_rl, (uint32_t)k, STREAM_ROTOR_NOISE, k0, k1);
                     const float rng = (float)((1.0 + 10.0 / 700.0) - (1.0 - 10.0 / 700.0)), lo = (float)(1.0 - 10.0 / 700.0);
                     om[0] = om[0] * rr(rng, lo, u01(nb.x)); om[1] = om[1] * rr(rng, lo, u01(nb.y));
@@ -642,7 +663,10 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
                 }
             }
         }
-        wld = qrot(q, wb);                                            // world-frame root state at the end of the RL step
+        };
+        if (battery_on && !(flags & TACO_F_ROTOR_NOISE) && !p.dbg_delay) control(std::false_type{});
+        else control(std::true_type{});
+        wld = qrot(q, wb);                                           // world-frame root state at the end of the RL step
 
         // ------------------------------------------------------------------ post_physics_step (:374-388)
         progress += 1;
