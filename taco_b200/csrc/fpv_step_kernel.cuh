@@ -41,56 +41,60 @@
 namespace taco {
 namespace TACO_VARIANT {   // distinct symbols per translation unit: the two builds must not be merged by the linker
 
-// nominal model parameters (thrust_dynamics.py:46-47,156-167)
-__device__ constexpr float kPolyNom[5] = {0.0f, 12.9466f, 0.1872f, -5.1220f, 0.5906f};
-__device__ constexpr float kAeroNom[5] = {1.13e-05f, 0.05f, -0.386f, -0.53f, 0.009f};
 __device__ constexpr float kTurns[8] = {-3.f, -2.f, -1.f, 0.f, 0.f, 1.f, 2.f, 3.f};   // fpv_asymmetry.py:892-901
 
 __device__ __forceinline__ float4 ldg4(const float4* p) { return __ldg(p); }
+// refresh_state's roll unwrap (fpv_asymmetry.py:334-360): the continuous roll follows the roll angle, a step over 1 rad is a wrap
+__device__ __forceinline__ void unwrap_roll(const Q4& q, float& roll_old, float& roll_cont) {
+    const float roll = roll_of(q);
+    float dl = roll - roll_old;
+    if (dl > 1.0f) dl = dl - kTwoPi;
+    if (dl < -1.0f) dl = dl + kTwoPi;
+    roll_cont += dl;
+    roll_old = roll;
+}
 
-// One CTA writes its 128 rows of an (N, L, 26) history buffer: frames 1..L-1 of the previous buffer shifted down by one
-// (coalesced 64-bit copies: a row is 13*L float2, the shift is 13 float2) and the newest frame from shared memory.
-// LC = compile-time L (fast paths for the README shapes L=5 / L=1), 0 = runtime L.  nv = valid rows of this CTA (only the
-// last CTA of a shard whose env count is not a multiple of 128 has nv < 128): rows >= nv are never touched, so the
-// buffers may be exactly (num_envs, L, 26) -- e.g. a slot of a caller-owned rollout ring.
-template <int LC, bool FULL>
-__device__ __forceinline__ void write_rows_impl(const float* __restrict__ in, float* __restrict__ out, const float* frames,
-                                                int L_rt, size_t blk_env0, int tid, int nv) {
-    const int L = LC ? LC : L_rt;
-    const int row2 = 13 * L, keep2 = 13 * (L - 1);
-    const float2* in2 = reinterpret_cast<const float2*>(in) + blk_env0 * row2;
-    float2* out2 = reinterpret_cast<float2*>(out) + blk_env0 * row2;
-    if (keep2 > 0) {
-        const int total = (FULL ? kBlock : nv) * keep2;       // FULL: compile-time trip count (multiple of kBlock)
-        constexpr int U = 13;                                   // loads in flight per thread
-        for (int k0 = tid; k0 < total; k0 += kBlock * U) {
-            float2 v[U];
-            int dst[U];
+// The history writers.  A CTA writes its 128 rows of an (N, L, 26) history buffer: frames 1..L-1 of the previous buffer shifted
+// down by one (coalesced 64-bit copies: a row is 13*L float2, the shift is 13 float2) and the newest frame from shared memory.
+// nv = valid rows of this CTA (only the last CTA of a shard whose env count is not a multiple of 128 has nv < 128): rows >= nv
+// are never touched, so the buffers may be exactly (num_envs, L, 26) -- e.g. a slot of a caller-owned rollout ring.
+
+// kept part, flat walk over the CTA's keep2 * rows kept float2 (every request 256 contiguous bytes, 13 loads in flight per
+// thread): out2 row e, column j <- in2 row e, column 13 + j, for j < keep2 (> 0) and rows of row2 float2
+__device__ __forceinline__ void copy_kept_flat(const float2* __restrict__ in2, float2* __restrict__ out2, int row2, int keep2,
+                                               int rows, int tid) {
+    const int total = rows * keep2;
+    constexpr int U = 13;                                       // loads in flight per thread
+    for (int k0 = tid; k0 < total; k0 += kBlock * U) {
+        float2 v[U];
+        int dst[U];
 #pragma unroll
-            for (int u = 0; u < U; ++u) {
-                const int k = k0 + u * kBlock;
-                const int e = k / (keep2 > 0 ? keep2 : 1), j = k - e * keep2;
-                dst[u] = e * row2 + j;
-                v[u] = (k < total) ? __ldg(in2 + dst[u] + 13) : make_float2(0.f, 0.f);
-            }
-#pragma unroll
-            for (int u = 0; u < U; ++u)
-                if (k0 + u * kBlock < total) out2[dst[u]] = v[u];
+        for (int u = 0; u < U; ++u) {
+            const int k = k0 + u * kBlock;
+            const int e = k / keep2, j = k - e * keep2;
+            dst[u] = e * row2 + j;
+            v[u] = (k < total) ? __ldg(in2 + dst[u] + 13) : make_float2(0.f, 0.f);
         }
-    }
 #pragma unroll
-    for (int u = 0; u < 13; ++u) {                               // 128 rows x 13 float2 of the newest frame
+        for (int u = 0; u < U; ++u)
+            if (k0 + u * kBlock < total) out2[dst[u]] = v[u];
+    }
+}
+// newest frame, generic walk: 13 float2 of each of the rows (all 128 if FULL, else nv) at column new2 of rows of row2 float2
+template <bool FULL>
+__device__ __forceinline__ void write_newest_flat(float2* out2, const float* frames, int row2, int new2, int tid, int nv) {
+#pragma unroll
+    for (int u = 0; u < 13; ++u) {
         const int k = tid + u * kBlock;
         const int e = k / 13, j = k - e * 13;
         const float* fr = frames + e * kFramePad + 2 * j;
-        if (FULL || e < nv) out2[e * row2 + keep2 + j] = make_float2(fr[0], fr[1]);
+        if (FULL || e < nv) out2[e * row2 + new2 + j] = make_float2(fr[0], fr[1]);
     }
 }
-// The same copy for a full CTA and a compile-time L, with no index arithmetic in the instruction stream: warp w owns the 32
-// consecutive rows [32 w, 32 w + 32) and its lanes run ALONG a row, so every load / store is `base + immediate` (the row and
-// column offsets are compile-time constants of the unrolled loops).  Kept part: lanes 0..31 and 32..keep2-1 of each row;
-// newest frame: two rows per store instruction (13 float2 each, lanes 26..31 idle).  Same bytes touched as the generic walk,
-// a third of its instructions (8 per element there: division by keep2, address, bounds predicate).
+// Forms for a full CTA and a compile-time L, with no index arithmetic in the instruction stream: warp w owns the 32 consecutive
+// rows [32 w, 32 w + 32) and its lanes run ALONG a row, so every load / store is `base + immediate` (the row and column offsets are
+// compile-time constants of the unrolled loops).  Same bytes touched as the flat walk, a third of its instructions (8 per element
+// there: division by keep2, address, bounds predicate).
 // kept part of rows [row0, row0 + NR) of the CTA by ONE warp (lanes along the row)
 template <int LC, int NR>
 __device__ __forceinline__ void copy_kept_rows(const float* __restrict__ in, float* __restrict__ out, size_t blk_env0, int row0, int lane) {
@@ -131,49 +135,36 @@ __device__ __forceinline__ void write_newest_rows(float* __restrict__ out, const
         for (int e = 0; e < 32; e += 2) d[e * row2] = make_float2(fr[e * kFramePad], fr[e * kFramePad + 1]);
     }
 }
-// A full CTA with a compile-time L.  Newest frame: write_newest_rows.  Kept part, two forms, chosen per kernel variant by
-// measurement (tools/step_ab.py, profiles/ab_r02ab.txt / ab_r02ac.txt):
+// the flat walks for rows of L frames (FULL: nv == 128)
+template <int LC, bool FULL>
+__device__ __forceinline__ void write_rows_flat(const float* __restrict__ in, float* __restrict__ out, const float* frames,
+                                                int L_rt, size_t blk_env0, int tid, int nv) {
+    const int L = LC ? LC : L_rt;
+    const int row2 = 13 * L, keep2 = 13 * (L - 1);
+    const float2* in2 = reinterpret_cast<const float2*>(in) + blk_env0 * row2;
+    float2* out2 = reinterpret_cast<float2*>(out) + blk_env0 * row2;
+    if (keep2 > 0) copy_kept_flat(in2, out2, row2, keep2, FULL ? kBlock : nv, tid);
+    write_newest_flat<FULL>(out2, frames, row2, keep2, tid, nv);
+}
+// LC = compile-time L (the README shapes L = 5 / L = 1), 0 = runtime L.  A full CTA with a compile-time L writes the newest frame
+// with write_newest_rows and the kept part in one of two forms, chosen per kernel variant by measurement (tools/step_ab.py,
+// profiles/ab_r02ab.txt / ab_r02ac.txt):
 //   FLAT = false  lanes along the rows (copy_kept_rows): a third of the instructions, but the second column chunk of a 52-element row
 //                 fills 20 of 32 lanes -- best for the DR variants (96 registers, 5 CTAs per SM: mix + DR 0.719 against 0.731 ms)
-//   FLAT = true   the flat walk over the CTA's kept elements (every request 256 contiguous bytes, 13 loads in flight per thread):
-//                 best for the variants at 80 registers / 6 CTAs per SM (flip: 0.560 against 0.584 ms over the first synchronised
-//                 steps, 0.602 against 0.607 in steady state)
-template <int LC, bool FLAT>
-__device__ __forceinline__ void write_rows_full(const float* __restrict__ in, float* __restrict__ out, const float* frames,
-                                                size_t blk_env0, int tid) {
-    if constexpr (FLAT) {
-        constexpr int row2 = 13 * LC, keep2 = 13 * (LC - 1);
-        const float2* in2 = reinterpret_cast<const float2*>(in) + blk_env0 * row2;
-        float2* out2 = reinterpret_cast<float2*>(out) + blk_env0 * row2;
-        if constexpr (keep2 > 0) {
-            constexpr int total = kBlock * keep2, U = 13;
-            for (int k0 = tid; k0 < total; k0 += kBlock * U) {
-                float2 v[U];
-                int dst[U];
-#pragma unroll
-                for (int u = 0; u < U; ++u) {
-                    const int k = k0 + u * kBlock;
-                    const int e = k / keep2, j = k - e * keep2;
-                    dst[u] = e * row2 + j;
-                    v[u] = (k < total) ? __ldg(in2 + dst[u] + 13) : make_float2(0.f, 0.f);
-                }
-#pragma unroll
-                for (int u = 0; u < U; ++u)
-                    if (k0 + u * kBlock < total) out2[dst[u]] = v[u];
-            }
-        }
-    } else {
-        copy_kept_rows<LC, 32>(in, out, blk_env0, 32 * (tid >> 5), tid & 31);
-    }
-    write_newest_rows<LC>(out, frames, blk_env0, tid);
-}
+//   FLAT = true   the flat walk (copy_kept_flat): best for the variants at 80 registers / 6 CTAs per SM (flip: 0.560 against
+//                 0.584 ms over the first synchronised steps, 0.602 against 0.607 in steady state)
 template <int LC, bool FLAT>
 __device__ __forceinline__ void write_rows(const float* __restrict__ in, float* __restrict__ out, const float* frames,
                                            int L_rt, size_t blk_env0, int tid, int nv) {
     if (nv == kBlock) {                                                                        // every CTA but (at most) the last
-        if constexpr (LC > 0) write_rows_full<LC, FLAT>(in, out, frames, blk_env0, tid);
-        else write_rows_impl<LC, true>(in, out, frames, L_rt, blk_env0, tid, nv);
-    } else write_rows_impl<LC, false>(in, out, frames, L_rt, blk_env0, tid, nv);
+        if constexpr (LC > 0) {
+            if constexpr (!FLAT) copy_kept_rows<LC, 32>(in, out, blk_env0, 32 * (tid >> 5), tid & 31);
+            else if constexpr (LC > 1)
+                copy_kept_flat(reinterpret_cast<const float2*>(in) + blk_env0 * (13 * LC), reinterpret_cast<float2*>(out) + blk_env0 * (13 * LC),
+                               13 * LC, 13 * (LC - 1), kBlock, tid);
+            write_newest_rows<LC>(out, frames, blk_env0, tid);
+        } else write_rows_flat<LC, true>(in, out, frames, L_rt, blk_env0, tid, nv);
+    } else write_rows_flat<LC, false>(in, out, frames, L_rt, blk_env0, tid, nv);
 }
 
 // The env-owned state history (no rollout ring attached): each env's row of the strip holds strip_frames = L + K - 1 frames, and
@@ -181,6 +172,8 @@ __device__ __forceinline__ void write_rows(const float* __restrict__ in, float* 
 // frame, at the end of the new window: 104 B per env instead of re-reading 4 frames and rewriting 5 (936 B).  The step that wraps the
 // offset to 0 first moves the L - 1 kept frames (K .. K + L - 2) to the start of the row (0 .. L - 2) -- the "rebase", once per K
 // steps.  K >= L, so the moved frames, their destination and the newest frame (L - 1) are disjoint: no ordering inside the CTA.
+// The rebase is the flat walk of copy_kept_flat with another source column, but it reads and writes one buffer: it keeps a loop of
+// its own with plain loads rather than copy_kept_flat's __ldg from a second, read-only buffer.
 __device__ __forceinline__ void write_strip(const StepParams& p, const float* frames, size_t blk_env0, int tid, int nv) {
     const uint32_t t = p.step_index + (p.step_base ? __ldg(p.step_base) : 0u);
     const int L = p.len_states, q = (int)((t + 1u) % (uint32_t)p.strip_period);
@@ -204,14 +197,7 @@ __device__ __forceinline__ void write_strip(const StepParams& p, const float* fr
                 if (k0 + u * kBlock < total) s2[dst[u]] = v[u];
         }
     }
-    const int new2 = 13 * (q + L - 1);
-#pragma unroll
-    for (int u = 0; u < 13; ++u) {                               // nv rows x 13 float2 of the newest frame
-        const int k = tid + u * kBlock;
-        const int e = k / 13, j = k - e * 13;
-        const float* fr = frames + e * kFramePad + 2 * j;
-        if (e < nv) s2[e * row2 + new2 + j] = make_float2(fr[0], fr[1]);
-    }
+    write_newest_flat<false>(s2, frames, row2, 13 * (q + L - 1), tid, nv);
 }
 
 // TASK: task_mode (mix = per-env task from the global env id).  DR: per-env randomised model parameters live in the
@@ -306,9 +292,9 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
         // every env of the launch -> coalesced planes however desynchronised the episodes are); an env's live runs are
         // the last q_n slots, so the head is implied
         const uint32_t tslot = t_rl & 15u;
-        uint32_t q_n = (qm >> QM_N_SHIFT) & 31u;
-        int q_len = (int)((qm >> QM_LEN_SHIFT) & 2047u);
-        uint32_t q_ovf = (qm >> QM_OVF_SHIFT) & 1u;
+        uint32_t q_n = qm_runs(qm);
+        int q_len = (int)qm_len(qm);
+        uint32_t q_ovf = qm_ovf(qm);
 
         // ------------------------------------------------------------------ reset draws, generated by the WARP for its resetting envs
         // In steady state ~1 % of the envs reset per step, i.e. ~29 % of the warps hold one or two resetting lanes, and such a warp
@@ -519,15 +505,8 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
         auto control = [&](auto gen) {
         constexpr bool GEN = decltype(gen)::value;
         for (int k = 0; k < p.cfi; ++k) {
-            // refresh_state (:334-360): roll unwrap with the 1 rad threshold; body-frame velocities
-            if (track_roll) {
-                const float roll = roll_of(q);
-                float dl = roll - roll_old;
-                if (dl > 1.0f) dl = dl - kTwoPi;
-                if (dl < -1.0f) dl = dl + kTwoPi;
-                roll_cont += dl;
-                roll_old = roll;
-            }
+            // refresh_state (:334-360): roll unwrap, body-frame velocities
+            if (track_roll) unwrap_roll(q, roll_old, roll_cont);
             if (k > 0) vb = qrot(conj(q), vel);               // wb is carried by the integrator between sub-steps
             // delayed action (:366-368)
             if (k >= k_next) {
@@ -680,14 +659,7 @@ __global__ void __launch_bounds__(kBlock + 32 * CW, CW ? 1 : (DR ? TACO_MIN_BLOC
             q_len = max(q_len - 10, 0);
         }
         // refresh_state
-        if (track_roll) {
-            const float roll = roll_of(q);
-            float dl = roll - roll_old;
-            if (dl > 1.0f) dl = dl - kTwoPi;
-            if (dl < -1.0f) dl = dl + kTwoPi;
-            roll_cont += dl;
-            roll_old = roll;
-        }
+        if (track_roll) unwrap_roll(q, roll_old, roll_cont);
         const Q4 qc = conj(q);
         vb = qrot(qc, vel);
         wb = qrot(qc, wld);

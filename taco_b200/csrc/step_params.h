@@ -14,8 +14,19 @@ constexpr int kStatSlots = 64;    // spread of the per-block stats atomics
 constexpr int kStatStride = 16;   // doubles per slot (128 B)
 constexpr int kNumStats = 8;
 
+// nominal model parameters (thrust_dynamics.py:46-47,156-167): rotor speed polynomial, aero k_f, k_tau, d_x, d_y, k_th
+__device__ constexpr float kPolyNom[5] = {0.0f, 12.9466f, 0.1872f, -5.1220f, 0.5906f};
+__device__ constexpr float kAeroNom[5] = {1.13e-05f, 0.05f, -0.386f, -0.53f, 0.009f};
+
 // qmeta bit layout: live runs (5 b), actions_remained_length (11 b), overflow flag
 constexpr uint32_t QM_N_SHIFT = 4, QM_LEN_SHIFT = 9, QM_OVF_SHIFT = 20;
+__host__ __device__ __forceinline__ uint32_t qm_runs(uint32_t qm) { return (qm >> QM_N_SHIFT) & 31u; }
+__host__ __device__ __forceinline__ uint32_t qm_len(uint32_t qm) { return (qm >> QM_LEN_SHIFT) & 2047u; }
+__host__ __device__ __forceinline__ uint32_t qm_ovf(uint32_t qm) { return (qm >> QM_OVF_SHIFT) & 1u; }
+// each field cut to its width (the step kernel packs values already in range: it clamps the length instead)
+__host__ __device__ __forceinline__ uint32_t qm_pack(uint32_t runs, uint32_t len, uint32_t ovf) {
+    return ((runs & 31u) << QM_N_SHIFT) | ((len & 2047u) << QM_LEN_SHIFT) | ((ovf & 1u) << QM_OVF_SHIFT);
+}
 
 struct StepParams {
     int n, n_pad;

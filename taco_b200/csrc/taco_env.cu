@@ -111,14 +111,14 @@ __global__ void init_state_kernel(StepParams p) {
     p.S[6][i] = make_float4(0.f, 0.f, 0.f, 0.f);
     p.S[7][i] = make_float4(0.f, 0.f, 0.f, 0.f);
     p.progress[i] = 0;
-    p.qmeta[i] = ((uint32_t)p.delay_time << QM_LEN_SHIFT);
+    p.qmeta[i] = qm_pack(0, (uint32_t)p.delay_time, 0);
     p.reset_buf[i] = 1;
     p.time_outs[i] = 0;
     p.rew[i] = 0.f;
     if (p.has_dr) {
-        p.D[0][i] = make_float4(0.0f, 12.9466f, 0.1872f, -5.1220f);
-        p.D[1][i] = make_float4(0.5906f, 1.13e-05f, 0.05f, -0.386f);
-        p.D[2][i] = make_float4(-0.53f, 0.009f, 0.f, 0.f);
+        p.D[0][i] = make_float4(kPolyNom[0], kPolyNom[1], kPolyNom[2], kPolyNom[3]);
+        p.D[1][i] = make_float4(kPolyNom[4], kAeroNom[0], kAeroNom[1], kAeroNom[2]);
+        p.D[2][i] = make_float4(kAeroNom[3], kAeroNom[4], 0.f, 0.f);
         p.D[3][i] = make_float4(p.lag_gain_fixed, p.lag_gain_fixed, p.lag_gain_fixed, p.lag_gain_fixed);
     }
 }
@@ -165,9 +165,9 @@ __global__ void export_state_kernel(StepParams p, const int32_t* ids, int count,
     o[33] = s7.w;                                             // running episode return
     const uint32_t qm = p.qmeta[i];
     o[34] = (float)p.progress[i];
-    o[35] = (float)((qm >> QM_LEN_SHIFT) & 2047u);            // actions_remained_length
-    o[36] = (float)((qm >> QM_N_SHIFT) & 31u);                // live runs in the action queue
-    o[37] = (float)((qm >> QM_OVF_SHIFT) & 1u);               // delay overflow flag
+    o[35] = (float)qm_len(qm);                                // actions_remained_length
+    o[36] = (float)qm_runs(qm);                               // live runs in the action queue
+    o[37] = (float)qm_ovf(qm);                                // delay overflow flag
     o[38] = (float)p.reset_buf[i];
     o[39] = 0.f;                                              // (was: queue head; the head is implied by the step clock)
     if (p.has_dr) {
@@ -176,8 +176,7 @@ __global__ void export_state_kernel(StepParams p, const int32_t* ids, int count,
         o[45] = d1.y; o[46] = d1.z; o[47] = d1.w; o[48] = d2.x; o[49] = d2.y;             // aero k_f,k_tau,d_x,d_y,k_th
         o[50] = d3.x; o[51] = d3.y; o[52] = d3.z; o[53] = d3.w;                           // lag gains
     } else {
-        o[40] = 0.0f; o[41] = 12.9466f; o[42] = 0.1872f; o[43] = -5.1220f; o[44] = 0.5906f;
-        o[45] = 1.13e-05f; o[46] = 0.05f; o[47] = -0.386f; o[48] = -0.53f; o[49] = 0.009f;
+        for (int j = 0; j < 5; ++j) { o[40 + j] = kPolyNom[j]; o[45 + j] = kAeroNom[j]; }
         o[50] = o[51] = o[52] = o[53] = p.lag_gain_fixed;
     }
     for (int j = 54; j < TACO_STATE_WORDS; ++j) o[j] = 0.f;
@@ -206,8 +205,7 @@ __global__ void import_state_kernel(StepParams p, const float* in) {
         }
     p.progress[i] = (int)o[34];
     p.reset_buf[i] = (long long)o[38];
-    p.qmeta[i] = (((uint32_t)o[36] & 31u) << QM_N_SHIFT) |
-                 (((uint32_t)o[35] & 2047u) << QM_LEN_SHIFT) | (((uint32_t)o[37] & 1u) << QM_OVF_SHIFT);
+    p.qmeta[i] = qm_pack((uint32_t)o[36], (uint32_t)o[35], (uint32_t)o[37]);
     if (p.has_dr) {
         p.D[0][i] = make_float4(o[40], o[41], o[42], o[43]);
         p.D[1][i] = make_float4(o[44], o[45], o[46], o[47]);
@@ -526,20 +524,39 @@ static int log_restart(TacoEnv* env, cudaStream_t s) {
     return TACO_OK;
 }
 
+// the step kernel of the env's build (-fmad=false or FMA contraction) with the bound StepParams
+static void launch_step(TacoEnv* env, cudaStream_t s) {
+    if (env->cfg.flags & TACO_F_STRICT_FP) launch_fpv_step_strict(env->p, s);
+    else launch_fpv_step_fast(env->p, s);
+}
+
+// The step as one launch over the whole shard.  actions and the host_* result buffers (null, or device-visible addresses of the
+// caller's pinned host memory) are bound for this launch only: the host pointers are cleared whatever the launch returns, and a
+// failed launch leaves the history and the step index where they were.  sync: return after the step has finished.
+static int step_single(TacoEnv* env, const void* actions, float* host_rew, long long* host_reset, uint8_t* host_tout, uint8_t* host_flags,
+                       cudaStream_t s, bool sync) {
+    StepParams& p = env->p;
+    int rc = bind_history(env);
+    if (rc != TACO_OK) return rc;
+    p.actions = (const float4*)actions;
+    p.host_rew = host_rew; p.host_reset = host_reset; p.host_tout = host_tout; p.host_flags = host_flags;
+    bind_step_index(env);
+    launch_step(env, s);
+    const cudaError_t launch = cudaGetLastError();
+    p.host_rew = nullptr; p.host_reset = nullptr; p.host_tout = nullptr; p.host_flags = nullptr;
+    TACO_CUDA(launch);
+    advance_history(env);
+    rc = log_after_step(env, s);
+    if (rc != TACO_OK) return rc;
+    if (sync) TACO_CUDA(cudaStreamSynchronize(s));
+    return TACO_OK;
+}
+
 int taco_env_step(TacoEnv* env, const float* actions_dev, void* stream) {
     if (!env || !actions_dev) return fail(TACO_E_INVALID, "taco_env_step: null argument");
     if (((uintptr_t)actions_dev & 15u) != 0) return fail(TACO_E_INVALID, "actions must be 16-byte aligned (contiguous (N,4) float32)");
     DevGuard guard(env->device);
-    StepParams& p = env->p;
-    const int rc = bind_history(env);
-    if (rc != TACO_OK) return rc;
-    p.actions = (const float4*)actions_dev;
-    bind_step_index(env);
-    if (env->cfg.flags & TACO_F_STRICT_FP) launch_fpv_step_strict(p, (cudaStream_t)stream);
-    else launch_fpv_step_fast(p, (cudaStream_t)stream);
-    TACO_CUDA(cudaGetLastError());
-    advance_history(env);
-    return log_after_step(env, (cudaStream_t)stream);
+    return step_single(env, actions_dev, nullptr, nullptr, nullptr, nullptr, (cudaStream_t)stream, false);
 }
 
 // device-visible address of a pinned (cudaHostAlloc / cudaHostRegister) host buffer, or null for pageable memory
@@ -583,21 +600,7 @@ int taco_env_step_host_compact(TacoEnv* env, const float* actions_host, float* r
     void* d_flags = mapped_ptr(flags_host);
     if (!d_act || (rew_host && !d_rew) || !d_flags)
         return fail(TACO_E_INVALID, "taco_env_step_host_compact: the host buffers must be pinned (device-mapped); use taco_env_step_host for pageable memory");
-    StepParams& p = env->p;
-    int rc = bind_history(env);
-    if (rc != TACO_OK) return rc;
-    p.actions = (const float4*)d_act;
-    p.host_rew = (float*)d_rew; p.host_flags = (uint8_t*)d_flags;
-    bind_step_index(env);
-    if (env->cfg.flags & TACO_F_STRICT_FP) launch_fpv_step_strict(p, s); else launch_fpv_step_fast(p, s);
-    const cudaError_t le = cudaGetLastError();
-    p.host_rew = nullptr; p.host_flags = nullptr;
-    TACO_CUDA(le);
-    advance_history(env);
-    rc = log_after_step(env, s);
-    if (rc != TACO_OK) return rc;
-    TACO_CUDA(cudaStreamSynchronize(s));
-    return TACO_OK;
+    return step_single(env, d_act, (float*)d_rew, nullptr, nullptr, (uint8_t*)d_flags, s, true);
 }
 
 int taco_env_step_host(TacoEnv* env, const float* actions_host, float* rew_host, int64_t* reset_host, uint8_t* time_outs_host,
@@ -617,22 +620,8 @@ int taco_env_step_host(TacoEnv* env, const float* actions_host, float* rew_host,
     if (host_mode == 0 && ((uintptr_t)actions_host & 15u) == 0) {
         void* d_act = mapped_ptr(actions_host);
         void* d_rew = mapped_ptr(rew_host); void* d_reset = mapped_ptr(reset_host); void* d_tout = mapped_ptr(time_outs_host);
-        if (d_act && (!rew_host || d_rew) && (!reset_host || d_reset) && (!time_outs_host || d_tout)) {
-            rc = bind_history(env);
-            if (rc != TACO_OK) return rc;
-            p.actions = (const float4*)d_act;
-            p.host_rew = (float*)d_rew; p.host_reset = (long long*)d_reset; p.host_tout = (uint8_t*)d_tout;
-            bind_step_index(env);
-            if (env->cfg.flags & TACO_F_STRICT_FP) launch_fpv_step_strict(p, s); else launch_fpv_step_fast(p, s);
-            const cudaError_t le = cudaGetLastError();
-            p.host_rew = nullptr; p.host_reset = nullptr; p.host_tout = nullptr;
-            TACO_CUDA(le);
-            advance_history(env);
-            rc = log_after_step(env, s);
-            if (rc != TACO_OK) return rc;
-            TACO_CUDA(cudaStreamSynchronize(s));
-            return TACO_OK;
-        }
+        if (d_act && (!rew_host || d_rew) && (!reset_host || d_reset) && (!time_outs_host || d_tout))
+            return step_single(env, d_act, (float*)d_rew, (long long*)d_reset, (uint8_t*)d_tout, nullptr, s, true);
     }
     const int total_blocks = env->n_pad / kBlock;
     // 4 equal chunks of at least 512 CTAs (64 Ki envs): measured best of 4 / 8 / 12 / 16 equal chunks and of a graded
@@ -654,7 +643,6 @@ int taco_env_step_host(TacoEnv* env, const float* actions_host, float* rew_host,
     if (rc != TACO_OK) return rc;
     p.actions = (const float4*)env->actions_stage;
     bind_step_index(env);
-    const bool strict = (env->cfg.flags & TACO_F_STRICT_FP) != 0;
     const bool want_out = rew_host || reset_host || time_outs_host;
     TACO_CUDA(cudaEventRecord(env->ev_begin, s));                    // work already queued on the caller's stream comes first
     TACO_CUDA(cudaStreamWaitEvent(env->s_h2d, env->ev_begin, 0));
@@ -670,7 +658,7 @@ int taco_env_step_host(TacoEnv* env, const float* actions_host, float* rew_host,
         TACO_CUDA(cudaEventRecord(env->ev_h2d[c], env->s_h2d));
         TACO_CUDA(cudaStreamWaitEvent(sk, env->ev_h2d[c], 0));
         p.block0 = b0; p.nblocks = b1 - b0;
-        if (strict) launch_fpv_step_strict(p, sk); else launch_fpv_step_fast(p, sk);
+        launch_step(env, sk);
         TACO_CUDA(cudaGetLastError());
         TACO_CUDA(cudaEventRecord(env->ev_k[c], sk));
         if (want_out) {
