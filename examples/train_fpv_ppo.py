@@ -11,6 +11,8 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 examples/train_fpv_ppo.py --num-envs 65536
 
 Prints one JSON line per epoch on rank 0 (mean reward per env-step, episode return / length, losses, env-steps/s of the whole loop).
+--episode-summary adds, per task, the rollout's finished episodes, survival (time-outs / episodes), mean and std of the return and
+the mean length (taco_b200.RolloutEpisodes: one scan of the rollout ring per rollout, all-reduced over ranks).
 """
 import argparse
 import json
@@ -39,6 +41,7 @@ def main():
     ap.add_argument("--update", default="native", choices=["native", "torch"])
     ap.add_argument("--no-graph", action="store_true", help="collect rollouts with the eager loop instead of one CUDA-graph replay per rollout")
     ap.add_argument("--seed", type=int, default=42)
+    ap.add_argument("--episode-summary", action="store_true", help="log per-task episode counts, survival, return mean / std and mean length")
     ap.add_argument("--save", default=None, help="after training, write the agent's state dict (save_checkpoint(para_only=True)) to this path")
     args = ap.parse_args()
 
@@ -76,6 +79,8 @@ def main():
     # the tensor-core kernels are also the fast path at small env counts (latency of one tile chain: ~12 us actor, ~36 us critic)
     tc = args.tensor_cores != "off" and actor.tensor_cores_available and critic.tensor_cores_available
     env.reset()
+    # only the summaries are logged; they count every finished episode, records dropped past the capacity included
+    episodes = taco_b200.RolloutEpisodes(env, n) if args.episode_summary else None
     graphed = None
     for epoch in range(args.epochs):
         ts = time.perf_counter()
@@ -86,9 +91,9 @@ def main():
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         if args.no_graph:
-            stats = taco_b200.collect_rollout(env, actor, buf, critic, seed=args.seed, tensor_cores=tc)
+            stats = taco_b200.collect_rollout(env, actor, buf, critic, seed=args.seed, tensor_cores=tc, episodes=episodes)
         elif graphed is None:                       # the first rollout runs eagerly inside the constructor, then the loop is one graph
-            graphed = taco_b200.GraphedRollout(env, actor, buf, critic, seed=args.seed, tensor_cores=tc)
+            graphed = taco_b200.GraphedRollout(env, actor, buf, critic, seed=args.seed, tensor_cores=tc, episodes=episodes)
             stats = graphed.first_stats
         else:
             stats = graphed.run()
@@ -104,14 +109,20 @@ def main():
         t2 = time.perf_counter()
         if rank == 0:
             s = tdist.summarise(stats)
-            print(json.dumps({"epoch": epoch, "mean_reward": s["mean_reward"], "episode_return": s["mean_episode_return"],
-                              "episode_length": s["mean_episode_length"], "difficulty": out["difficulty"], "lipschitz": out["lipschitz_para"],
-                              "pg_loss": out["policy_gradient_loss"], "value_loss": out["value_loss"], "kl": out["approx_kl"],
-                              "optim_steps": out["optim_steps"], "sync_s": t0 - ts, "rollout_s": t1 - t0, "update_s": t2 - t1,
-                              "rollout_env_steps_per_s": world * n_s / (t1 - t0), "loop_env_steps_per_s": world * n_s / (t2 - ts),
-                              "tensor_cores": bool(tc), "update": args.update, "early_stop": out["early_stop"], "world": world}), flush=True)
+            line = {"epoch": epoch, "mean_reward": s["mean_reward"], "episode_return": s["mean_episode_return"],
+                    "episode_length": s["mean_episode_length"], "difficulty": out["difficulty"], "lipschitz": out["lipschitz_para"],
+                    "pg_loss": out["policy_gradient_loss"], "value_loss": out["value_loss"], "kl": out["approx_kl"],
+                    "optim_steps": out["optim_steps"], "sync_s": t0 - ts, "rollout_s": t1 - t0, "update_s": t2 - t1,
+                    "rollout_env_steps_per_s": world * n_s / (t1 - t0), "loop_env_steps_per_s": world * n_s / (t2 - ts),
+                    "tensor_cores": bool(tc), "update": args.update, "early_stop": out["early_stop"], "world": world}
+            if episodes is not None:
+                line["episodes_by_task"] = {task: {k: e[k] for k in ("episodes", "survival", "ret_mean", "ret_std", "length_mean")}
+                                            for task, e in episodes.summary().items()}
+            print(json.dumps(line), flush=True)
     if graphed is not None:
         graphed.close()
+    if episodes is not None:
+        episodes.close()
     if native is not None:
         native.store_to(agent, opt)                 # the torch module / optimiser hold the trained state again (checkpoints, export)
         native.close()

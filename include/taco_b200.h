@@ -220,6 +220,42 @@ int taco_env_episode_log_clear(TacoEnv* env, void* stream);
  * `stream`, no host sync (capturable). */
 int taco_env_record_state(TacoEnv* env, const int32_t* ids_dev, int32_t k, float* out_dev, void* stream);
 
+/* -- training-time episode records and per-task summaries from the rollout ring (DESIGN.md section 6f).  No launch is added to the
+ * step: one scan per rollout (taco_env_scan_rollout_episodes, capturable) walks the ring's rew / done / time-out rows written since
+ * the last scan or rewind, in step order, one thread per env.  Per env it carries the running return (float32, rew added in step
+ * order: bit-identical to TacoEpisode.ret and to the return taco_env_stats adds), the running length and a live flag from one
+ * scan to the next, and appends one record per episode that ended in the scanned rows.  Only whole episodes are recorded: at
+ * attach, an env with reset_buf != 0 starts fresh and every other env is not recorded until after its next end; taco_env_reset_all,
+ * taco_env_import_state, taco_env_attach_rollout (steps taken without a ring are unseen) and a taco_env_rewind_rollout over rows
+ * not yet scanned re-run that rule.  The record order is unspecified (one atomic per block); records past the capacity are
+ * dropped but counted: dropped = *count - capacity.  The first six fields of TacoEpisode, same order and layout; 24 bytes. */
+typedef struct TacoRolloutEpisode {
+    int64_t env_id;          /* global env id (env_offset + local index) */
+    uint32_t end_step;       /* RL step index (the Philox step index) of the step that ended the episode */
+    int32_t length;          /* steps of the episode: the progress_buf value taco_env_stats adds */
+    int16_t task;            /* TACO_TASK_POS / _ROTATE / _FLIP; a mix env: the task of its third of the global ids */
+    int16_t timed_out;       /* time_outs of the ending step */
+    float ret;               /* float32 sum of the rewards in step order */
+} TacoRolloutEpisode;
+/* summary of one scan, float64: for task t in POS, ROTATE, FLIP, words 5 t .. 5 t + 4 = [episodes, time-outs, sum of lengths,
+ * sum of returns, sum of squared returns] over every episode that ended in the scanned rows (dropped records included).  Each env's
+ * episodes are summed in step order and the envs in a fixed tree order, so the same rows give a bit-identical summary whatever
+ * the launch timing; the vector is SUM-reducible across ranks. */
+#define TACO_EPISODE_SUMMARY_WORDS 15
+/* allocates records, counter and the per-env planes once (a captured graph never sees them move); clears the counter and runs the
+ * start rule on `stream`.  Rows already in an attached ring are treated as scanned. */
+int taco_env_attach_rollout_episodes(TacoEnv* env, int64_t capacity, void* stream);
+int taco_env_detach_rollout_episodes(TacoEnv* env);
+/* zero-copy access: records_dev = capacity records, count_dev = one uint64 (records appended since attach / the last clear) */
+int taco_env_rollout_episodes_buffers(TacoEnv* env, TacoRolloutEpisode** records_dev, uint64_t** count_dev, int64_t* capacity);
+/* rewinds the counter on `stream`; the per-env planes are kept, so the episodes in progress continue */
+int taco_env_rollout_episodes_clear(TacoEnv* env, void* stream);
+/* scans the ring rows written since the last scan or rewind and writes the TACO_EPISODE_SUMMARY_WORDS doubles of their episodes to
+ * summary_dev (device).  Asynchronous on `stream`, capturable; in graph mode the end steps are read from the device step counter,
+ * so capture the scan before the rollout's taco_env_graph_advance, like the steps it scans.  TACO_E_INVALID without attached
+ * rollout episodes or without an attached ring with result rows. */
+int taco_env_scan_rollout_episodes(TacoEnv* env, double* summary_dev, void* stream);
+
 /* -- actor MLP inference in the rollout loop: MLP.forward + the actor branch of PPO_ActorCritic.act
  * (IsaacGymEnvs/algorithms/nets_asymmetry.py:23-39, :326-346) and PPO.spectral_normalize_actors
  * (IsaacGymEnvs/algorithms/ppo_asymmetry.py:398-404).  Two kernels compute the same function: an FP32 CUDA-core

@@ -15,6 +15,7 @@ _LIB_PATH = os.environ.get("TACO_B200_LIB") or os.path.join(os.path.dirname(os.p
 ABI_VERSION = 1
 TASK = {"pos": 0, "rotate": 1, "flip": 2, "mix": 3}
 NUM_OBS, NUM_ACTS, NUM_STATS, STATE_WORDS = 26, 4, 8, 64
+EPISODE_SUMMARY_WORDS = 15        # TACO_EPISODE_SUMMARY_WORDS: 3 tasks x [episodes, time-outs, sum length, sum ret, sum ret^2]
 
 FLAGS = {  # cfg key -> bit (include/taco_b200.h TACO_F_*)
     "random_copter_pos": 1 << 0, "random_copter_quat": 1 << 1, "random_copter_vel": 1 << 2,
@@ -91,6 +92,11 @@ def lib():
         "taco_env_episode_log_buffers": (C.c_int, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(C.c_int64)]),
         "taco_env_episode_log_clear": (C.c_int, [vp, vp]),
         "taco_env_record_state": (C.c_int, [vp, vp, i32, vp, vp]),
+        "taco_env_attach_rollout_episodes": (C.c_int, [vp, C.c_int64, vp]),
+        "taco_env_detach_rollout_episodes": (C.c_int, [vp]),
+        "taco_env_rollout_episodes_buffers": (C.c_int, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(C.c_int64)]),
+        "taco_env_rollout_episodes_clear": (C.c_int, [vp, vp]),
+        "taco_env_scan_rollout_episodes": (C.c_int, [vp, vp, vp]),
         "taco_selftest_divc": (C.c_int, [C.c_int, f32, C.POINTER(u64)]),
         "taco_selftest_atan2": (C.c_int, [C.c_int, C.c_uint32, C.POINTER(f32), C.POINTER(C.c_uint32)]),
         "taco_actor_create": (C.c_int, [C.c_int, C.POINTER(i32), i32, C.POINTER(vp)]),
@@ -164,6 +170,10 @@ EPISODE_DTYPE = np.dtype([("env_id", "<i8"), ("end_step", "<u4"), ("length", "<i
                           ("ret", "<f4"), ("pos_err_mean", "<f4"), ("pos_err_final", "<f4"), ("tilt_max", "<f4"),
                           ("speed_mean", "<f4"), ("angvel_max", "<f4"), ("roll_travel", "<f4")])
 assert EPISODE_DTYPE.itemsize == 48
+
+# TacoRolloutEpisode: the first six fields of TacoEpisode, 24 bytes per record
+ROLLOUT_EPISODE_DTYPE = np.dtype(EPISODE_DTYPE.descr[:6])
+assert ROLLOUT_EPISODE_DTYPE.itemsize == 24
 
 
 class _CudaView:

@@ -18,6 +18,7 @@
 #include "fpv_math.cuh"
 #include "step_params.h"
 #include "episode_log.cuh"
+#include "rollout_episodes.cuh"
 
 namespace taco {
 
@@ -55,6 +56,18 @@ struct TacoEnv {
     float4* log_acc[2] = {nullptr, nullptr};
     TacoEpisode* log_rec = nullptr;
     unsigned long long log_cap = 0;
+    // rollout episodes (taco_env_attach_rollout_episodes): one allocation = counters, per-env ret / len / live planes, block
+    // partials, records; rep_scanned = the first ring row the next scan reads
+    void* rep_mem = nullptr;
+    unsigned long long* rep_count = nullptr;
+    unsigned int* rep_blocks_done = nullptr;
+    float* rep_ret = nullptr;
+    int* rep_len = nullptr;
+    uint8_t* rep_live = nullptr;
+    double* rep_partial = nullptr;
+    TacoRolloutEpisode* rep_rec = nullptr;
+    unsigned long long rep_cap = 0;
+    int rep_scanned = 0;
     uint32_t step_index = 0;
     // graph mode (taco_env_graph_begin .. _end): the step index of a launch = *step_counter (device) + its offset since
     // graph_begin, so a CUDA graph captured over a rollout replays with fresh Philox counters / queue time slots
@@ -437,6 +450,7 @@ int taco_env_destroy(TacoEnv* env) {
     }
     if (env->export_stage) cudaFree(env->export_stage);
     if (env->log_mem) cudaFree(env->log_mem);
+    if (env->rep_mem) cudaFree(env->rep_mem);
     if (env->arena) cudaFree(env->arena);
     if (env->step_counter) cudaFree(env->step_counter);
     if (env->diff_dev) cudaFree(env->diff_dev);
@@ -521,6 +535,17 @@ static int log_restart(TacoEnv* env, cudaStream_t s) {
     if (!env->log_mem) return TACO_OK;
     episode_log_init_kernel<<<(env->n_pad + 255) / 256, 256, 0, s>>>(env->p, env->log_acc[0], env->log_acc[1]); TACO_LAUNCHED();
     TACO_CUDA(cudaGetLastError());
+    return TACO_OK;
+}
+
+// the start rule of attached rollout episodes (a no-op without them): the episodes in progress are discarded, and the ring rows
+// written so far count as scanned
+static int rep_restart(TacoEnv* env, cudaStream_t s) {
+    if (!env->rep_mem) return TACO_OK;
+    rollout_episodes_init_kernel<<<(env->n + 255) / 256, 256, 0, s>>>(env->p.reset_buf, env->n, env->rep_ret, env->rep_len, env->rep_live);
+    TACO_LAUNCHED();
+    TACO_CUDA(cudaGetLastError());
+    env->rep_scanned = env->ring_slots ? env->ring_cur : 0;
     return TACO_OK;
 }
 
@@ -740,7 +765,7 @@ int taco_env_attach_rollout(TacoEnv* env, float* obs_ring, float* states_ring, i
     env->ring_obs = obs_ring; env->ring_states = states_ring;
     env->ring_rew = rew_rows; env->ring_done = done_rows; env->ring_tout = time_out_rows;
     env->ring_slots = slots; env->ring_cur = 0;
-    return TACO_OK;
+    return rep_restart(env, s);
 }
 
 int taco_env_rewind_rollout(TacoEnv* env, void* stream) {
@@ -748,6 +773,11 @@ int taco_env_rewind_rollout(TacoEnv* env, void* stream) {
     if (!env->ring_slots) return fail(TACO_E_INVALID, "taco_env_rewind_rollout: no ring attached");
     DevGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
+    if (env->rep_scanned < env->ring_cur) {                          // unscanned rows: their episodes would be lost half-seen
+        const int rc = rep_restart(env, s);
+        if (rc != TACO_OK) return rc;
+    }
+    env->rep_scanned = 0;
     if (env->ring_cur > 0) {
         const size_t so = (size_t)env->n * env->cfg.len_obs * kObs, ss = (size_t)env->n * env->cfg.len_states * kObs;
         TACO_CUDA(cudaMemcpyAsync(env->ring_obs, env->ring_obs + so * env->ring_cur, so * sizeof(float), cudaMemcpyDeviceToDevice, s));
@@ -768,6 +798,7 @@ int taco_env_detach_rollout(TacoEnv* env, void* stream) {
     TACO_CUDA(cudaMemcpy2DAsync(strip_window(env), strip_row_bytes(env), env->ring_states + ss * env->ring_cur, win, win, env->n, cudaMemcpyDeviceToDevice, s));
     env->ring_obs = env->ring_states = env->ring_rew = env->ring_done = nullptr; env->ring_tout = nullptr;
     env->ring_slots = 0; env->ring_cur = 0;
+    env->rep_scanned = 0;
     return TACO_OK;
 }
 
@@ -794,7 +825,9 @@ int taco_env_reset_all(TacoEnv* env, void* stream) {
     TACO_CUDA(cudaMemsetAsync(env->p.stats, 0, (size_t)kStatSlots * kStatStride * sizeof(double), s));
     init_state_kernel<<<(env->n_pad + 255) / 256, 256, 0, s>>>(env->p); TACO_LAUNCHED();
     TACO_CUDA(cudaGetLastError());
-    const int rc = log_restart(env, s);
+    int rc = log_restart(env, s);
+    if (rc != TACO_OK) return rc;
+    rc = rep_restart(env, s);
     if (rc != TACO_OK) return rc;
     env->step_index = 0;
     env->graph_mode = false;                                         // host-side counting again; taco_env_graph_begin re-arms
@@ -868,7 +901,9 @@ int taco_env_import_state(TacoEnv* env, const float* in_host) {
     TACO_CUDA(cudaMemcpy(env->export_stage, in_host, bytes, cudaMemcpyHostToDevice));
     import_state_kernel<<<(env->n + 255) / 256, 256>>>(env->p, env->export_stage); TACO_LAUNCHED();
     TACO_CUDA(cudaGetLastError());
-    const int rc = log_restart(env, 0);
+    int rc = log_restart(env, 0);
+    if (rc != TACO_OK) return rc;
+    rc = rep_restart(env, 0);
     if (rc != TACO_OK) return rc;
     TACO_CUDA(cudaDeviceSynchronize());
     return TACO_OK;
@@ -991,6 +1026,87 @@ int taco_env_record_state(TacoEnv* env, const int32_t* ids_dev, int32_t k, float
     DevGuard guard(env->device);
     export_state_kernel<<<(k + 255) / 256, 256, 0, (cudaStream_t)stream>>>(env->p, ids_dev, k, out_dev); TACO_LAUNCHED();
     TACO_CUDA(cudaGetLastError());
+    return TACO_OK;
+}
+
+int taco_env_attach_rollout_episodes(TacoEnv* env, int64_t capacity, void* stream) {
+    if (!env) return fail(TACO_E_INVALID, "taco_env_attach_rollout_episodes: null argument");
+    if (capacity < 1) return fail(TACO_E_INVALID, "taco_env_attach_rollout_episodes: capacity must be >= 1");
+    if (env->rep_mem) return fail(TACO_E_INVALID, "taco_env_attach_rollout_episodes: rollout episodes are already attached");
+    DevGuard guard(env->device);
+    const size_t n = (size_t)env->n, blocks = (n + kScanBlock - 1) / kScanBlock;
+    size_t off = 256;                                                // counter at 0, blocks_done at 8
+    auto take = [&](size_t bytes) { const size_t o = off; off = align_up(off + bytes, 256); return o; };
+    const size_t oRet = take(n * sizeof(float)), oLen = take(n * sizeof(int)), oLive = take(n);
+    const size_t oPart = take(blocks * kSummaryStride * sizeof(double)), oRec = take((size_t)capacity * sizeof(TacoRolloutEpisode));
+    void* mem = nullptr;
+    const cudaError_t ce = cudaMalloc(&mem, off);
+    if (ce != cudaSuccess) { cudaGetLastError(); return fail(TACO_E_NOMEM, std::string("cudaMalloc of the rollout episodes failed: ") + cudaGetErrorString(ce)); }
+    char* base = (char*)mem;
+    env->rep_mem = mem;
+    env->rep_count = (unsigned long long*)base;
+    env->rep_blocks_done = (unsigned int*)(base + 8);
+    env->rep_ret = (float*)(base + oRet);
+    env->rep_len = (int*)(base + oLen);
+    env->rep_live = (uint8_t*)(base + oLive);
+    env->rep_partial = (double*)(base + oPart);
+    env->rep_rec = (TacoRolloutEpisode*)(base + oRec);
+    env->rep_cap = (unsigned long long)capacity;
+    cudaStream_t s = (cudaStream_t)stream;
+    TACO_CUDA(cudaMemsetAsync(base, 0, 256, s));
+    return rep_restart(env, s);
+}
+
+int taco_env_detach_rollout_episodes(TacoEnv* env) {
+    if (!env) return fail(TACO_E_INVALID, "taco_env_detach_rollout_episodes: null argument");
+    if (!env->rep_mem) return TACO_OK;
+    DevGuard guard(env->device);
+    TACO_CUDA(cudaDeviceSynchronize());
+    cudaFree(env->rep_mem);
+    env->rep_mem = nullptr; env->rep_count = nullptr; env->rep_blocks_done = nullptr;
+    env->rep_ret = nullptr; env->rep_len = nullptr; env->rep_live = nullptr; env->rep_partial = nullptr; env->rep_rec = nullptr;
+    env->rep_cap = 0; env->rep_scanned = 0;
+    return TACO_OK;
+}
+
+int taco_env_rollout_episodes_buffers(TacoEnv* env, TacoRolloutEpisode** records_dev, uint64_t** count_dev, int64_t* capacity) {
+    if (!env || !records_dev || !count_dev) return fail(TACO_E_INVALID, "taco_env_rollout_episodes_buffers: null argument");
+    if (!env->rep_mem) return fail(TACO_E_INVALID, "taco_env_rollout_episodes_buffers: no rollout episodes attached");
+    *records_dev = env->rep_rec;
+    *count_dev = (uint64_t*)env->rep_count;
+    if (capacity) *capacity = (int64_t)env->rep_cap;
+    return TACO_OK;
+}
+
+int taco_env_rollout_episodes_clear(TacoEnv* env, void* stream) {
+    if (!env) return fail(TACO_E_INVALID, "taco_env_rollout_episodes_clear: null argument");
+    if (!env->rep_mem) return fail(TACO_E_INVALID, "taco_env_rollout_episodes_clear: no rollout episodes attached");
+    DevGuard guard(env->device);
+    TACO_CUDA(cudaMemsetAsync(env->rep_count, 0, sizeof(unsigned long long), (cudaStream_t)stream));
+    return TACO_OK;
+}
+
+int taco_env_scan_rollout_episodes(TacoEnv* env, double* summary_dev, void* stream) {
+    if (!env || !summary_dev) return fail(TACO_E_INVALID, "taco_env_scan_rollout_episodes: null argument");
+    if (!env->rep_mem) return fail(TACO_E_INVALID, "taco_env_scan_rollout_episodes: no rollout episodes attached");
+    if (!env->ring_slots || !env->ring_rew)
+        return fail(TACO_E_INVALID, "taco_env_scan_rollout_episodes: no rollout ring with rew / done / time-out rows attached");
+    DevGuard guard(env->device);
+    const int k0 = env->rep_scanned, rows = env->ring_cur - k0;
+    const size_t n = (size_t)env->n;
+    RolloutScanParams q;
+    q.rew = env->ring_rew + n * k0; q.done = env->ring_done + n * k0; q.tout = env->ring_tout + n * k0;
+    q.n = env->n; q.rows = rows;
+    // step index of row k0: the ring cursor and the step index advance together
+    q.step0 = (env->graph_mode ? env->step_index - env->graph_origin : env->step_index) - (uint32_t)rows;
+    q.step_base = env->graph_mode ? env->step_counter : nullptr;
+    q.env_offset = env->p.env_offset; q.mix_n1 = env->p.mix_n1; q.mix_n2 = env->p.mix_n2; q.task_mode = env->p.task_mode;
+    q.ret = env->rep_ret; q.len = env->rep_len; q.live = env->rep_live;
+    q.rec = env->rep_rec; q.count = env->rep_count; q.capacity = env->rep_cap;
+    q.partial = env->rep_partial; q.blocks_done = env->rep_blocks_done; q.summary = summary_dev;
+    rollout_episodes_scan_kernel<<<(env->n + kScanBlock - 1) / kScanBlock, kScanBlock, 0, (cudaStream_t)stream>>>(q); TACO_LAUNCHED();
+    TACO_CUDA(cudaGetLastError());
+    env->rep_scanned = env->ring_cur;
     return TACO_OK;
 }
 

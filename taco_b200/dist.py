@@ -44,6 +44,37 @@ def summarise(stats):
             "timeout_fraction": s["n_timeout"] / eps, **s}
 
 
+EPISODE_SUMMARY_FIELDS = ("episodes", "time_outs", "sum_length", "sum_ret", "sum_ret2")
+TASK_NAMES = ("pos", "rotate", "flip")
+
+
+def allreduce_episode_summary(summary, group=None):
+    """In-place SUM over ranks of the (15,) float64 per-task episode summary of a rollout (taco_env_scan_rollout_episodes); no-op
+    without an initialised process group."""
+    if summary.dtype != torch.float64 or summary.numel() != len(TASK_NAMES) * len(EPISODE_SUMMARY_FIELDS):
+        raise ValueError("summary must be a float64 tensor of 15 elements")
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(summary, op=dist.ReduceOp.SUM, group=group)
+    return summary
+
+
+def summarise_episode_summary(summary):
+    """Per-task scalars from a (reduced) episode summary: one dict per task with episodes, keyed "pos" / "rotate" / "flip", holding
+    the raw sums plus survival (time-outs / episodes), ret_mean, ret_std (population) and length_mean."""
+    v = summary.tolist() if hasattr(summary, "tolist") else list(summary)
+    out = {}
+    for t, name in enumerate(TASK_NAMES):
+        s = dict(zip(EPISODE_SUMMARY_FIELDS, v[5 * t:5 * t + 5]))
+        n = s["episodes"]
+        if n <= 0:
+            continue
+        mean = s["sum_ret"] / n
+        s.update(survival=s["time_outs"] / n, ret_mean=mean, ret_std=max(s["sum_ret2"] / n - mean * mean, 0.0) ** 0.5,
+                 length_mean=s["sum_length"] / n)
+        out[name] = s
+    return out
+
+
 def bind_to_gpu_numa(gpu_index):
     """Pin the calling process to the CPUs NVML reports as local to GPU ``gpu_index`` (its NUMA node), so that pinned host
     buffers allocated afterwards -- the action / result buffers of ``step_host`` -- live in memory next to that GPU's PCIe root

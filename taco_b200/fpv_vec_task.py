@@ -113,11 +113,11 @@ class FpvVecTask:
         handle = C.c_void_p()
         _capi.check(self._lib.taco_env_create(C.byref(c), self.device_id, C.byref(handle)), "taco_env_create")
         self._h = handle
+        self.rollout_buffer = None          # RolloutBuffer whose ring the step kernel writes into (attach_rollout)
         self._wrap_buffers()
         self.extras = {}
         self.obs_dict = {}
         self._actions_keepalive = None
-        self.rollout_buffer = None          # RolloutBuffer whose ring the step kernel writes into (attach_rollout)
         self._ring_cur = 0
         self.step_count = 0                 # RL steps since construction / reset_all = the Philox step index of the next step
 
@@ -136,7 +136,8 @@ class FpvVecTask:
         self.reset_buf = _capi.wrap(b.reset, (N,), "<i8", dev, self)
         self.timeout_buf = _capi.wrap(b.time_outs, (N,), "|b1", dev, self)
         self._progress_i32 = _capi.wrap(b.progress, (N,), "<i4", dev, self)
-        self._cur = self._ab_ptr.index(int(b.obs))
+        if self.rollout_buffer is None:           # with a ring attached, obs points into the ring (reset_all keeps the ring)
+            self._cur = self._ab_ptr.index(int(b.obs))
 
     @property
     def obs_buf(self):

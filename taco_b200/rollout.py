@@ -17,7 +17,9 @@ and ``batch_idx_generator``.  Differences, all on purpose:
     the per-step ``store`` copies of the reference (2.7 GB per rollout at 262144 envs x 20 steps) disappear; ``store`` then
     takes ``None`` for those fields;
   * ``reset`` only rewinds the write index (the reference re-allocates every buffer each epoch, buffer_asymmetry.py:70-91;
-    every slot is overwritten by the next rollout before it is read).
+    every slot is overwritten by the next rollout before it is read);
+  * ``RolloutEpisodes``: one record per finished training episode and a per-task summary, from one scan of the ring's result
+    rows per rollout (``episodes=`` of ``collect_rollout`` / ``GraphedRollout``).
 There is no CPU fallback: the buffer lives on a CUDA device.
 """
 import ctypes as C
@@ -124,6 +126,73 @@ class RolloutBuffer:
         return torch.randperm(n).reshape(self.mini_batch_num, -1).tolist()
 
 
+class RolloutEpisodes:
+    """Training-time episode records and per-task summaries (``taco_env_attach_rollout_episodes``): ``scan()`` -- one launch, run
+    by ``collect_rollout`` / ``GraphedRollout`` after the horizon's steps when passed as ``episodes`` -- walks the ring rows the
+    step kernel wrote since the last scan and appends one ``ROLLOUT_EPISODE_DTYPE`` record per finished episode (``capacity``
+    records on the device; past it they are dropped but counted) and writes the float64 per-task summary of those episodes to
+    ``summary_vec``.  Only whole episodes are recorded; the record order is unspecified.  Needs a rollout ring with result rows
+    attached at scan time."""
+
+    def __init__(self, env, capacity):
+        self.env = env
+        self._lib = _capi.lib()
+        _capi.check(self._lib.taco_env_attach_rollout_episodes(env._h, int(capacity), self._stream()), "taco_env_attach_rollout_episodes")
+        rec, cnt, cap = C.c_void_p(), C.c_void_p(), C.c_int64()
+        _capi.check(self._lib.taco_env_rollout_episodes_buffers(env._h, C.byref(rec), C.byref(cnt), C.byref(cap)),
+                    "taco_env_rollout_episodes_buffers")
+        self.capacity = int(cap.value)
+        self._count = _capi.wrap(cnt.value, (1,), "<i8", env.device, self)
+        self._records = _capi.wrap(rec.value, (self.capacity * _capi.ROLLOUT_EPISODE_DTYPE.itemsize,), "|u1", env.device, self)
+        self.summary_vec = torch.zeros(_capi.EPISODE_SUMMARY_WORDS, dtype=torch.float64, device=env.device)
+        self._open = True
+
+    def _stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.env.device_id).cuda_stream)
+
+    def scan(self):
+        """Scan the ring rows written since the last scan or rewind into records and ``summary_vec`` (asynchronous, capturable)."""
+        _capi.check(self._lib.taco_env_scan_rollout_episodes(self.env._h, C.c_void_p(self.summary_vec.data_ptr()), self._stream()),
+                    "taco_env_scan_rollout_episodes")
+        return self.summary_vec
+
+    @property
+    def count(self):
+        """Records appended since attach / the last ``clear`` (dropped ones included).  Synchronises."""
+        return int(self._count.item())
+
+    @property
+    def dropped(self):
+        return max(0, self.count - self.capacity)
+
+    def read(self):
+        """The records as a numpy structured array (``ROLLOUT_EPISODE_DTYPE``)."""
+        n = min(self.count, self.capacity)
+        return self._records[:n * _capi.ROLLOUT_EPISODE_DTYPE.itemsize].cpu().numpy().view(_capi.ROLLOUT_EPISODE_DTYPE)
+
+    def clear(self):
+        """Rewind the counter; the episodes in progress continue."""
+        _capi.check(self._lib.taco_env_rollout_episodes_clear(self.env._h, self._stream()), "taco_env_rollout_episodes_clear")
+
+    def summary(self):
+        """Per-task dict of the last scan's summary (all-reduced when the rollout ran under torch.distributed); see
+        ``taco_b200.dist.summarise_episode_summary``.  Synchronises."""
+        from .dist import summarise_episode_summary
+        return summarise_episode_summary(self.summary_vec)
+
+    def close(self):
+        if self._open:
+            self._open = False
+            self._records = self._count = None
+            _capi.check(self._lib.taco_env_detach_rollout_episodes(self.env._h), "taco_env_detach_rollout_episodes")
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 _warned_fp32 = set()
 
 
@@ -137,7 +206,7 @@ def _warn_fp32_fallback(actor_tc, critic_tc):
                       "falling back to the FP32 CUDA-core kernel, which is 70-100x slower at large env counts", RuntimeWarning, stacklevel=3)
 
 
-def collect_rollout(env, actor, buffer, value_fn, seed=0, tensor_cores=True, group=None):
+def collect_rollout(env, actor, buffer, value_fn, seed=0, tensor_cores=True, group=None, episodes=None):
     """One rollout of ``buffer.horizon_len`` steps: the data-collection loop of ``PPO.run``
     (IsaacGymEnvs/algorithms/ppo_asymmetry.py:305-342) with no host round trip inside it.
 
@@ -147,7 +216,8 @@ def collect_rollout(env, actor, buffer, value_fn, seed=0, tensor_cores=True, gro
     rows, the critic kernel values the state history, the step kernel writes the next observation history into ring slot s+1
     and reward / done / time-out into row s.  The time-out bootstrap, GAE and the advantage normalisation (with the moments
     all-reduced under torch.distributed) run in ``buffer.compute_returns_and_advantage``; episode statistics come from the
-    env's device-side vector, all-reduced once.  Returns the (8,) float64 statistics tensor (see taco_b200.dist.STAT_NAMES)."""
+    env's device-side vector, all-reduced once.  Returns the (8,) float64 statistics tensor (see taco_b200.dist.STAT_NAMES).
+    ``episodes``: a ``RolloutEpisodes`` of ``env``, scanned after the H steps (before GAE); its ``summary_vec`` is all-reduced too."""
     from . import dist as tdist
     from .critic import CriticLSTM
     torch.cuda.nvtx.range_push("taco.rollout")                    # NVTX: rollout / gae / update ranges (SURVEY.md section 5)
@@ -173,6 +243,8 @@ def collect_rollout(env, actor, buffer, value_fn, seed=0, tensor_cores=True, gro
             value = value_fn(obs, states)
         env.step(out[1])
         buffer.store(None, None, out[0], None, out[2], None, value, out[3], sigma, time_outs=True)
+    if episodes is not None:
+        episodes.scan()
     if native_critic:
         last_value = value_fn.forward(buffer.states_ring[H], tensor_cores=critic_tc)
     else:
@@ -181,6 +253,8 @@ def collect_rollout(env, actor, buffer, value_fn, seed=0, tensor_cores=True, gro
     torch.cuda.nvtx.range_push("taco.gae")
     buffer.compute_returns_and_advantage(last_value, group=group)
     torch.cuda.nvtx.range_pop()
+    if episodes is not None:
+        tdist.allreduce_episode_summary(episodes.summary_vec, group=group)
     return tdist.allreduce_rollout_stats(env.stats(), group=group)
 
 
@@ -196,14 +270,17 @@ class GraphedRollout:
     ``critic`` must be a ``CriticLSTM``; weights may be reloaded between replays (``ActorMLP.load`` / ``CriticLSTM.load`` write the
     same device buffers, ``ActorMLP.set_log_std`` the sampler constants the captured kernels read from device memory) and
     ``env.difficulty`` may be set between replays (graph-mode launches read its device copy).  Single-process statistics / advantage normalisation are inside the
-    graph; under torch.distributed the two small all-reduces run after the replay."""
+    graph; under torch.distributed the two small all-reduces run after the replay.  ``episodes``: a ``RolloutEpisodes`` of ``env``
+    whose scan is captured after the H steps; every ``run()`` leaves that rollout's summary in ``episodes.summary_vec``
+    (all-reduced under torch.distributed, like the statistics)."""
 
-    def __init__(self, env, actor, buffer, critic, seed=0, tensor_cores=True, group=None):
+    def __init__(self, env, actor, buffer, critic, seed=0, tensor_cores=True, group=None, episodes=None):
         from . import dist as tdist
         from .critic import CriticLSTM
         if not isinstance(critic, CriticLSTM):
             raise TypeError("GraphedRollout needs the native critic (CriticLSTM)")
         self.env, self.actor, self.buffer, self.critic, self.group = env, actor, buffer, critic, group
+        self.episodes = episodes
         self.seed = int(seed)
         self.tc_actor = bool(tensor_cores and actor.tensor_cores_available)
         self.tc_critic = bool(tensor_cores and critic.tensor_cores_available)
@@ -212,7 +289,8 @@ class GraphedRollout:
         # The FIRST rollout is collected eagerly, here: it leaves the ring cursor at H (so that the captured rewind contains the
         # slot H -> slot 0 copy), runs every lazy initialisation outside the capture, and its experience is in ``buffer`` like
         # that of any later ``run()``.
-        self.first_stats = collect_rollout(env, actor, buffer, critic, seed=self.seed, tensor_cores=tensor_cores, group=group)
+        self.first_stats = collect_rollout(env, actor, buffer, critic, seed=self.seed, tensor_cores=tensor_cores, group=group,
+                                           episodes=episodes)
         H = buffer.horizon_len
         self.stats = torch.zeros(8, dtype=torch.float64, device=buffer.device)
         self.last_value = torch.empty(buffer.num_envs, 1, dtype=torch.float32, device=buffer.device)
@@ -249,6 +327,8 @@ class GraphedRollout:
             self.actor.act(buf.obs_ring[s], env.step_count - base, seed=self.seed, env_offset=env.env_offset, tensor_cores=self.tc_actor,
                            out=out, step_base=counter)
             env.step_raw(out[1])
+        if self.episodes is not None:
+            self.episodes.scan()                                  # before graph_advance: it reads the counter the steps used
         env.graph_advance(H)
         done = torch.cuda.Event()
         done.record(side)
@@ -267,6 +347,8 @@ class GraphedRollout:
         self.env.step_count += self.buffer.horizon_len
         if self.world > 1:
             self.buffer.compute_returns_and_advantage(self.last_value, group=self.group)
+        if self.episodes is not None:
+            self._tdist.allreduce_episode_summary(self.episodes.summary_vec, group=self.group)
         return self._tdist.allreduce_rollout_stats(self.stats, group=self.group)
 
     def close(self):
